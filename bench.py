@@ -49,9 +49,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-geometry", action="store_true", help="skip the config-5 geometry sweep")
     ap.add_argument("--no-extra", action="store_true", help="skip front step, _find_dot latency and the C1 / C3 configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float64; rank 0's frame-sets and cameras)")
     a = ap.parse_args()
     if a.steps is None:
         a.steps = 300 if a.impl == "b200" else 20
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     return a
 
 
@@ -280,6 +284,36 @@ def _parity_check(rig, frames, det, corr, cams_local):
             "ok": bool(cen_ok and pairs_ok and rel is not None and rel < 1e-4)}
 
 
+DUMP_BYTES = 64_000_000
+
+
+def _dump_outputs(out_dir, det, corr, cams_local):
+    """Write the results of one step as float64 .npy files, one per array the caller receives: the detection of rank 0's cameras
+    (det_xy [FS, cams, max_blobs, 2], det_count, det_flags) and the matching of its frame-sets (corr_obj, corr_n_obj, corr_img,
+    corr_n_valid, corr_err, corr_flags), frame-set s in row s.  Entries past a count are zeroed (the kernels leave them
+    unspecified), so two builds compare element for element.  Above DUMP_BYTES a fixed seeded sample of the frame-sets is written;
+    frame_sets.npy names the frame-sets the rows are."""
+    S = corr.n_obj.shape[0]
+    host = lambda t: t.cpu().numpy().astype(np.float64)
+    out = {"det_xy": host(det.xy).reshape(-1, cams_local, *det.xy.shape[1:])[:S],
+           "det_count": host(det.count).reshape(-1, cams_local)[:S], "det_flags": host(det.flags).reshape(-1, cams_local)[:S],
+           "corr_obj": host(corr.obj), "corr_n_obj": host(corr.n_obj), "corr_img": host(corr.img),
+           "corr_n_valid": host(corr.n_valid), "corr_err": host(corr.err), "corr_flags": host(corr.flags)}
+    slots = np.arange(out["det_xy"].shape[2])
+    out["det_xy"][slots[None, None, :] >= out["det_count"][..., None]] = 0
+    rows = np.arange(corr.obj.shape[1])[None, :] >= out["corr_n_valid"][:, None]
+    out["corr_img"][rows] = 0
+    out["corr_err"][rows] = 0
+    out["corr_obj"][np.arange(corr.obj.shape[1])[None, :] >= out["corr_n_obj"][:, None]] = 0
+    keep = min(S, (DUMP_BYTES - 4096) // (sum(a.nbytes for a in out.values()) // S + 8))     # (4096: the .npy headers)
+    fs = np.arange(S) if keep == S else np.sort(np.random.default_rng(0).choice(S, keep, replace=False))
+    out = {k: a[fs] for k, a in out.items()}
+    out["frame_sets"] = fs.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _time_loop(fn, reps, warm=3):
     import torch
     for _ in range(warm):
@@ -467,6 +501,8 @@ def run_b200(args):
     ev1.record()
     gpu_launches = eng.launches - launches0
     barrier()
+    if args.dump_outputs and rank == 0:     # before the steps below reuse the lanes' result buffers
+        _dump_outputs(args.dump_outputs, det, corr, pipe.cams_local)
     # nvidia-smi delivers a sample every ~50-100 ms: if the timed region was shorter than a second keep the same step loop
     # running (untimed) so that the clock record is taken under this very load
     # (the number of extra steps follows from the all-reduced time: every rank runs the same number of steps and lane turns)
