@@ -97,28 +97,17 @@ int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, in
                        void* workspace, size_t workspace_bytes, void* stream, void* stage_timer_or_null);
 
 /* ---- overlapped detection (same results as mocap_detect_batch without the parity outputs) ----------------------------
- * The batch is cut into chunks of `chunk_frames` frames.  The streaming scan -- one TMA-fed kernel (cp.async.bulk.tensor +
- * mbarrier ring in shared memory, one small CTA per SM) over the whole batch on a high-priority stream of the pipe -- runs
- * beside the instruction-bound stages (group, piece filter, borders) of the chunks it has already finished, which wait for
- * its per-chunk flag with a stream memory operation.  A pipe owns those streams and events: create one per caller thread,
- * keep it for the life of the engine; a call is asynchronous on `stream` like every other entry point (fork / join with
- * events).  Shapes the TMA unit cannot describe (rows not a multiple of 16 bytes, thresh outside 0..254) use the classic scan
- * kernels chunk by chunk; frame sizes the per-cluster units do not support return MOCAP_ERR_UNSUPPORTED (use
- * mocap_detect_batch). */
-typedef struct {
-    int chunk_frames;          /* frames per chunk (<= 0: one chunk) */
-    int sync_mode;             /* 1: one scan kernel + per-chunk flags (stream memory operations); 0: one scan launch per chunk + events */
-    int scan_variant;          /* 1: TMA ring scan where the shape allows; 0: classic register-staged scan */
-    int filter_ctas_per_sm;    /* persistent piece-filter CTAs per SM (<= 0: 6 beside the TMA scan, else 8) */
-    int cand_ctas_per_sm;      /* <= 0: 12 */
-    int record_timeline;       /* record CUDA events for mocap_detect_pipe_timeline */
-    int stream_plan;           /* 0: a chunk's stages run as a chain on worker (chunk mod workers); 1: stage streams -- worker 0 groups,
-                                  worker 1 filters, workers 2.. take the border stages of alternate chunks (needs >= 3 workers);
-                                  2: worker 0 groups and filters, workers 1.. take the borders; 3: like 2, grouping one chunk ahead */
-    int scan_stages;           /* 8 KB ring slots of the TMA scan per SM: 6 (default) or 3 (leaves room for seven filter CTAs) */
-} MocapPipeOpts;
-/* prio_mode 0: all workers at the lowest stream priority; 1 / 2 (for stream_plan 1): earlier / later stages first */
-void* mocap_detect_pipe_create(int n_worker_streams, int prio_mode);
+ * The batch is cut into chunks of `chunk_frames` frames (<= 0: one chunk); chunk k's stages (group, piece filter, borders) run as
+ * one chain on worker stream k mod n_worker_streams of the pipe.  The streaming scan -- one TMA-fed kernel (cp.async.bulk.tensor +
+ * mbarrier ring in shared memory, one small CTA per SM) over the whole batch on the pipe's high-priority scan stream -- runs
+ * beside the stages of the chunks it has already finished, which wait for its per-chunk flag with a stream memory operation.
+ * Frames the TMA unit cannot describe (rows or frame stride not a multiple of 16 bytes, thresh outside 0..254), or a driver
+ * without stream memory operations, take the classic scan kernels chunk by chunk, handed over with events; with cell boxes handed in (mocap_detect_pipe_set_cellbox) there is no
+ * scan.  A pipe owns those streams and events: create one per caller thread, keep it for the life of the engine; a call is
+ * asynchronous on `stream` like every other entry point (fork / join with events).  record_timeline != 0 keeps the call's
+ * timeline for mocap_detect_pipe_timeline.  Frame sizes the per-cluster units do not support return MOCAP_ERR_UNSUPPORTED
+ * (use mocap_detect_batch). */
+void* mocap_detect_pipe_create(int n_worker_streams);
 void mocap_detect_pipe_destroy(void* pipe);
 size_t mocap_detect_pipelined_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs, int chunk_frames);
 int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
@@ -126,7 +115,7 @@ int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_fr
                                  int max_blobs, int max_contours, int max_runs,
                                  int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
                                  double* out_contours, int32_t* out_contour_count,
-                                 void* workspace, size_t workspace_bytes, void* stream, const MocapPipeOpts* opts);
+                                 void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline);
 /* Store-to-peer epilogue (multi-GPU): with per-frame destination addresses set (device arrays [n_frames] of pointers, valid for the
  * following calls of this pipe; NULL, NULL switches it off) every frame's record is ALSO copied -- chunk by chunk, behind the chunk's
  * border stage -- to xy_dst[f] (its centroids, int32 pairs) and count_dst[f] (its count): addresses in the receive buffer of the rank that
@@ -143,12 +132,14 @@ int mocap_detect_pipe_set_cellbox(void* pipe, const uint32_t* cellbox_dev);
 /* ms since the fork of the last call with record_timeline: [scan done, join] then per chunk [scan seen, grouped, filtered,
  * borders done]; returns the number of floats written, 0 without a timeline */
 int mocap_detect_pipe_timeline(void* pipe, float* ms_out, int cap);
-/* what the last call ran: out3 = {scan kernel (1 TMA ring, 0 classic), chunks, sync mode used} */
+/* what the last call ran: out3 = {scan kernel (1 TMA ring, 0 classic or none), chunks, sync mode (1 the workers waited on the TMA
+ * scan's chunk flags, 0 on events or on nothing)} */
 int mocap_detect_pipe_info(void* pipe, int* out3);
 
 /* stage entry points of the same path (used by the parity tests and the bench's per-kernel timing) */
 /* the streaming scan alone: cellbox_out [n][ceil(H/32)][ceil(W/32)] hot bounding box of every 32x32 source cell
- * (x0 | x1 << 8 | y0 << 16 | y1 << 24, 0xffffffff: no pixel > thresh).  variant 0 classic kernels, 1 TMA ring (workspace >= 1 KB) */
+ * (x0 | x1 << 8 | y0 << 16 | y1 << 24, 0xffffffff: no pixel > thresh).  variant 0 classic kernels, 1 TMA ring (workspace >= 1 KB);
+ * any other variant returns MOCAP_ERR_INVALID */
 int mocap_scan_cells_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride, const void* table_dev,
                            int thresh, int variant, uint32_t* cellbox_out, void* workspace, size_t workspace_bytes, void* stream);
 int mocap_filter_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,

@@ -12,7 +12,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB = os.path.join(HERE, "libmocap_b200.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 MAX_CAND = 8
 MAX_CAMS = 16
 CAM_STRIDE = 40
@@ -44,11 +44,11 @@ SIGNATURES = {
     "mocap_stage_timer_destroy": (None, [_p]),
     "mocap_stage_timer_read": (_i, [_p, _p]),
     "mocap_stage_name": (C.c_char_p, [_i]),
-    "mocap_detect_pipe_create": (_p, [_i, _i]),
+    "mocap_detect_pipe_create": (_p, [_i]),
     "mocap_detect_pipe_destroy": (None, [_p]),
     "mocap_detect_pipelined_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i]),
     "mocap_detect_batch_pipelined": (_i, [_p, _p, _i, _i, _i, _i64, _p, _i, _d, _d, _i, _i, _i,
-                                          _p, _p, _p, _p, _p, _p, _sz, _p, _p]),
+                                          _p, _p, _p, _p, _p, _p, _sz, _p, _i, _i]),
     "mocap_detect_pipe_set_scatter": (_i, [_p, _p, _p]),
     "mocap_detect_pipe_set_scan_token": (_i, [_p, _p, _p]),
     "mocap_detect_pipe_set_cellbox": (_i, [_p, _p]),
@@ -72,12 +72,6 @@ SIGNATURES = {
     "mocap_correspond_batch_blocked": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _d, _i, _i, _i,
                                             _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
 }
-
-
-class PipeOpts(C.Structure):
-    """MocapPipeOpts of include/mocap_b200.h"""
-    _fields_ = [("chunk_frames", _i), ("sync_mode", _i), ("scan_variant", _i), ("filter_ctas_per_sm", _i),
-                ("cand_ctas_per_sm", _i), ("record_timeline", _i), ("stream_plan", _i), ("scan_stages", _i)]
 
 
 class MocapError(RuntimeError):

@@ -10,10 +10,10 @@ int launch_scan(const uint8_t* frames, int n, int H, int W, int64_t fstride, con
 int launch_tiles(const uint8_t* frames, int n, int H, int W, int64_t fstride, const TableView& tv, int thresh,
                  const FilterWs& ws, int max_fg, int* flags, const int* need_general, cudaStream_t s);
 // detect_cluster.cu
-size_t cluster_ws_bytes(int n, int H, int W, int max_contours, size_t* offs);
+size_t cluster_ws_bytes(int n, int H, int W, int max_contours, ClusterLayout* L);
 bool cluster_path_supported(int H, int W);
 int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstride, const TableView& tv, int thresh,
-                        const uint32_t* cellbox, char* ws_base, const size_t* offs, int* need_general,
+                        const uint32_t* cellbox, char* ws_base, const ClusterLayout& L, int* need_general,
                         int max_contours, int max_blobs, double min_area, double min_circ,
                         int32_t* out_xy, int32_t* out_count, int32_t* out_flags, double* out_contours, int32_t* out_contour_count,
                         cudaStream_t s, StageTimer* timer, const ClusterLaunch& how);
@@ -21,8 +21,9 @@ int launch_materialize_bits(const FilterWs& ws, int n, int H, int W, const Table
 // detect_scan_tma.cu
 bool scan_tma_supported(const uint8_t* frames, int n, int H, int W, int64_t fstride, int thresh);
 size_t scan_tma_ctrl_bytes(int chunks);
+const int* scan_tma_chunk_flag(const int* ctrl, int chunks, int chunk);
 int launch_scan_tma(const uint8_t* frames, int n, int H, int W, int64_t fstride, const TableView& tv, int thresh, uint32_t* cellbox,
-                    int* ctrl, int chunks, int chunk_frames, int widx, int item_begin, int item_end, int stages, cudaStream_t s);
+                    int* ctrl, int chunks, int chunk_frames, cudaStream_t s);
 int stream_wait_geq(cudaStream_t s, const int* addr_dev, int value);
 bool stream_wait_supported();
 // detect_blobs.cu
@@ -91,7 +92,7 @@ extern "C" int mocap_stage_timer_read(void* timer, float* ms_out)
 struct DetectLayout {
     size_t off_active, off_list, off_counters, off_bits, off_fg, off_nfg, off_flags, off_cellbox, off_blob, off_cluster;
     size_t blob_stride, total;
-    size_t cl_offs[16];
+    ClusterLayout cl;
     int TX, TY, TXW, max_fg;
 };
 
@@ -114,7 +115,7 @@ static int detect_layout(int n, int H, int W, int max_contours, int max_runs, bo
     L->off_cellbox = take((size_t)n * L->TX * L->TY * 4);
     L->blob_stride = with_blobs ? blob_ws_stride(H, max_runs, max_contours) : 0;
     L->off_blob = take(L->blob_stride * (size_t)n);
-    L->off_cluster = take(cluster_ws_bytes(n, H, W, max_contours, L->cl_offs));
+    L->off_cluster = take(cluster_ws_bytes(n, H, W, max_contours, &L->cl));
     L->total = off;
     return MOCAP_OK;
 }
@@ -190,12 +191,12 @@ extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H
     const bool extras = out_bits || out_labels || out_blob_sums || out_blob_count;
     const bool use_cluster = !extras && cluster_path_supported(H, W);
     char* cl_base = (char*)workspace + L.off_cluster;
-    int* need_general = (int*)(cl_base + L.cl_offs[0]);
+    int* need_general = (int*)(cl_base + L.cl.need_general);
     st = launch_scan(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws, s, timer);
     if (st != MOCAP_OK) return st;
     CUDA_TRY(cudaMemsetAsync(need_general, use_cluster ? 0 : 1, (size_t)n_frames * 4, s));
     if (use_cluster) {
-        st = launch_cluster_path(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, cl_base, L.cl_offs, need_general,
+        st = launch_cluster_path(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, cl_base, L.cl, need_general,
                                  max_contours, max_blobs, min_area, min_circ, out_xy, out_count, out_flags, out_contours,
                                  out_contour_count, s, timer, ClusterLaunch());
         if (st != MOCAP_OK) return st;
@@ -244,18 +245,22 @@ extern "C" int mocap_blobs_batch(const uint32_t* bits_dev, int n_frames, int H, 
 
 // =========================================================================================================
 // Overlapped detection: the batch is cut into chunks of frames; the HBM-bound streaming scan of chunk k+1 runs
-// beside the instruction-bound stages (group / piece filter / borders) of chunk k on the same SMs.
-//   sync_mode 1: ONE TMA-fed scan kernel over the whole batch on its own (high-priority) stream; it publishes a flag per
-//                finished chunk and the chunk's stages, on a worker stream, wait for it with a stream memory operation
-//                (cuStreamWaitValue32) -- the scan CTA of an SM stays resident from the first byte to the last.
-//   sync_mode 0: one scan launch per chunk + CUDA events (same kernels; the fallback when stream memory operations are
-//                not available, and the A/B for the design note).
+// beside the instruction-bound stages (group / piece filter / borders) of chunk k on the same SMs.  Chunk k's stages run as
+// one chain on worker stream k mod workers.  The scan follows from the input:
+//   cell boxes handed in (mocap_detect_pipe_set_cellbox): no scan.
+//   frames a tensor map can describe, and stream memory operations available: ONE TMA-fed scan kernel over the whole batch
+//     on the pipe's high-priority scan stream; it publishes a flag per finished chunk, which the chunk's worker stream waits
+//     for with cuStreamWaitValue32 -- the scan CTA of an SM stays resident from the first byte to the last.
+//   otherwise (and in the CPU emulation build, which has neither): the classic scan kernels chunk by chunk on the scan
+//     stream, handed to the worker streams with one event per chunk.
 // Whatever the cluster path hands to the general path is finished for the whole batch after the join.
 // =========================================================================================================
 #define PIPE_MAX_PROC 6
-#define PIPE_CTRL_WORK 64            // == SCAN_CTRL_WORK of detect_scan_tma.cu: work-counter slots ahead of chunk_done[] / chunk_flag[]
 #define PIPE_MAX_CHUNKS 64
 #define PIPE_TL_PER_CHUNK 4          // timeline marks per chunk: scan seen, grouped, filtered, borders done
+#define PIPE_FILTER_CTAS_TMA 6       // persistent piece-filter CTAs per SM beside the TMA scan CTA
+#define PIPE_FILTER_CTAS 8           // ... without it
+#define PIPE_CAND_CTAS 12            // candidates_kernel CTAs per SM
 
 // Store-to-peer epilogue of the multi-GPU pipeline: every frame's record (count + centroids) is copied to the address its consumer
 // reads it from -- for the frame-sets of another rank that is a slot of THAT rank's receive buffer, mapped into this process
@@ -290,37 +295,25 @@ struct DetectPipe {
     void* tok_wait = nullptr;                       // scan token (mocap_detect_pipe_set_scan_token): cudaEvent_t the scan waits for / records
     void* tok_done = nullptr;
     const uint32_t* pre_cellbox = nullptr;          // hot cell boxes of the next calls' frames, computed by the caller (mocap_detect_pipe_set_cellbox)
-#ifndef MOCAP_EMU
     cudaStream_t s_scan = nullptr, s_proc[PIPE_MAX_PROC] = {};
     cudaEvent_t ev_fork = nullptr, ev_scan_done = nullptr, ev_proc_done[PIPE_MAX_PROC] = {}, ev_join = nullptr;
-    cudaEvent_t ev_scan[PIPE_MAX_CHUNKS] = {};                       // sync_mode 0
+    cudaEvent_t ev_scan[PIPE_MAX_CHUNKS] = {};                       // classic scan: chunk c scanned
     cudaEvent_t ev_tl[PIPE_MAX_CHUNKS][PIPE_TL_PER_CHUNK] = {};      // timeline (timing enabled)
-#endif
     int n_proc = 0;
     int tl_chunks = 0;               // chunks of the last call that recorded a timeline
-    int last_scan = -1, last_chunks = 0, last_mode = -1;
+    int last_tma = -1, last_chunks = 0;  // what the last call ran (mocap_detect_pipe_info)
 };
 
-extern "C" void* mocap_detect_pipe_create(int n_proc_streams, int prio_mode)
+extern "C" void* mocap_detect_pipe_create(int n_proc_streams)
 {
     if (n_proc_streams < 1) n_proc_streams = 1;
     if (n_proc_streams > PIPE_MAX_PROC) n_proc_streams = PIPE_MAX_PROC;
     DetectPipe* p = new DetectPipe();
     p->n_proc = n_proc_streams;
-#ifndef MOCAP_EMU
     int lo = 0, hi = 0;
     bool ok = cudaDeviceGetStreamPriorityRange(&lo, &hi) == cudaSuccess;      // hi = numerically smallest = highest priority
     ok = ok && cudaStreamCreateWithPriority(&p->s_scan, cudaStreamNonBlocking, hi) == cudaSuccess;
-    for (int i = 0; ok && i < n_proc_streams; ++i) {
-        // prio_mode 0: every worker at the lowest priority.  1 / 2 (stage plan: worker 0 groups, worker 1 filters, the others take
-        // the borders): 1 = earlier stages first (group > filter > borders), 2 = later stages first (borders > filter > group).
-        int pr = lo;
-        const int stage = i < 2 ? i : 2;
-        if (prio_mode == 1) pr = hi + 1 + stage;
-        if (prio_mode == 2) pr = hi + 3 - stage;
-        if (pr > lo) pr = lo;
-        ok = cudaStreamCreateWithPriority(&p->s_proc[i], cudaStreamNonBlocking, pr) == cudaSuccess;
-    }
+    for (int i = 0; ok && i < n_proc_streams; ++i) ok = cudaStreamCreateWithPriority(&p->s_proc[i], cudaStreamNonBlocking, lo) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&p->ev_fork, cudaEventDefault) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&p->ev_scan_done, cudaEventDefault) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&p->ev_join, cudaEventDefault) == cudaSuccess;
@@ -330,7 +323,6 @@ extern "C" void* mocap_detect_pipe_create(int n_proc_streams, int prio_mode)
         for (int k = 0; ok && k < PIPE_TL_PER_CHUNK; ++k) ok = cudaEventCreateWithFlags(&p->ev_tl[c][k], cudaEventDefault) == cudaSuccess;
     }
     if (!ok) { delete p; return nullptr; }
-#endif
     return p;
 }
 
@@ -364,7 +356,6 @@ extern "C" void mocap_detect_pipe_destroy(void* pipe)
 {
     DetectPipe* p = (DetectPipe*)pipe;
     if (!p) return;
-#ifndef MOCAP_EMU
     if (p->s_scan) cudaStreamDestroy(p->s_scan);
     for (int i = 0; i < PIPE_MAX_PROC; ++i) { if (p->s_proc[i]) cudaStreamDestroy(p->s_proc[i]); if (p->ev_proc_done[i]) cudaEventDestroy(p->ev_proc_done[i]); }
     if (p->ev_fork) cudaEventDestroy(p->ev_fork);
@@ -374,14 +365,13 @@ extern "C" void mocap_detect_pipe_destroy(void* pipe)
         if (p->ev_scan[c]) cudaEventDestroy(p->ev_scan[c]);
         for (int k = 0; k < PIPE_TL_PER_CHUNK; ++k) if (p->ev_tl[c][k]) cudaEventDestroy(p->ev_tl[c][k]);
     }
-#endif
     delete p;
 }
 
 struct PipeLayout {
     DetectLayout L;                  // general-path arrays of the whole batch (its cluster part serves chunk 0 .. see below)
     size_t off_ctrl, off_need, off_chunks, chunk_bytes, total;
-    size_t cl_offs[16];              // offsets inside one chunk's cluster workspace
+    ClusterLayout cl;                // inside one chunk's cluster workspace
     int chunks, chunk_frames;
 };
 
@@ -397,7 +387,7 @@ static int pipe_layout(int n, int H, int W, int max_contours, int max_runs, int 
     auto take = [&](size_t bytes) { size_t r = off; off += align_up(bytes, 256); return r; };
     P->off_ctrl = take(scan_tma_ctrl_bytes(chunks));
     P->off_need = take((size_t)n * 4);
-    P->chunk_bytes = align_up(cluster_ws_bytes(chunk_frames, H, W, max_contours, P->cl_offs), 256);
+    P->chunk_bytes = align_up(cluster_ws_bytes(chunk_frames, H, W, max_contours, &P->cl), 256);
     P->off_chunks = take(P->chunk_bytes * (size_t)chunks);
     P->total = off > P->L.total ? off : P->L.total;
     return MOCAP_OK;
@@ -417,14 +407,14 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
                                             int max_blobs, int max_contours, int max_runs,
                                             int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
                                             double* out_contours, int32_t* out_contour_count,
-                                            void* workspace, size_t workspace_bytes, void* stream, const MocapPipeOpts* opts)
+                                            void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
 {
     DetectPipe* dp = (DetectPipe*)pipe;
-    if (!dp || !frames_dev || !table_dev || !out_xy || !out_count || !out_flags || !workspace || !opts) return MOCAP_ERR_INVALID;
+    if (!dp || !frames_dev || !table_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
     if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
     if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
     PipeLayout P;
-    int st = pipe_layout(n_frames, H, W, max_contours, max_runs, opts->chunk_frames, &P);
+    int st = pipe_layout(n_frames, H, W, max_contours, max_runs, chunk_frames, &P);
     if (st != MOCAP_OK) return st;
     if (workspace_bytes < P.total) return MOCAP_ERR_WORKSPACE;
     if (!cluster_path_supported(H, W)) return MOCAP_ERR_UNSUPPORTED;         // such shapes take mocap_detect_batch
@@ -438,109 +428,52 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
     int* ctrl = (int*)(base + P.off_ctrl);
     int* need_general = (int*)(base + P.off_need);
     const int chunks = P.chunks, cf = P.chunk_frames;
-    const int per_frame_items = tv.TY * cdiv(W, 256);
-    const bool tma = !prescanned && opts->scan_variant != 0 && scan_tma_supported(frames_dev, n_frames, H, W, frame_stride, thresh);
-    int mode = opts->sync_mode;
-    if (mode == 1 && !(tma && stream_wait_supported())) mode = 0;
-    dp->last_scan = tma ? 1 : 0; dp->last_chunks = chunks; dp->last_mode = mode;
+    const bool tma = !prescanned && scan_tma_supported(frames_dev, n_frames, H, W, frame_stride, thresh) && stream_wait_supported();
+    dp->last_tma = tma ? 1 : 0; dp->last_chunks = chunks;
     dp->tl_chunks = 0;
     ClusterLaunch how;
-    how.zero = 1;
-    how.filter_ctas_per_sm = opts->filter_ctas_per_sm > 0 ? opts->filter_ctas_per_sm : (tma ? 6 : 8);
-    how.cand_ctas_per_sm = opts->cand_ctas_per_sm > 0 ? opts->cand_ctas_per_sm : 12;
+    how.zero = 0;                    // the chunk loop clears each chunk's block on its worker stream ahead of its scan wait
+    how.filter_ctas = tma ? PIPE_FILTER_CTAS_TMA : PIPE_FILTER_CTAS;
+    how.cand_ctas = PIPE_CAND_CTAS;
     CUDA_TRY(cudaMemsetAsync(out_flags, 0, (size_t)n_frames * 4, s));
     CUDA_TRY(cudaMemsetAsync(need_general, 0, (size_t)n_frames * 4, s));
     CUDA_TRY(cudaMemsetAsync(ctrl, 0, scan_tma_ctrl_bytes(chunks), s));
-#ifdef MOCAP_EMU
-    // CPU emulation build (tests/emu): no streams; the chunks run one after the other through the same launchers
-    for (int c = 0; c < chunks; ++c) {
-        const int f0 = c * cf, nc = (n_frames - f0) < cf ? (n_frames - f0) : cf;
-        FilterWs wc = ws; wc.cellbox = ws.cellbox + (size_t)f0 * tv.TX * tv.TY;
-        st = prescanned ? MOCAP_OK : launch_scan(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, wc, s, nullptr);
-        if (st != MOCAP_OK) return st;
-        st = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, wc.cellbox,
-                                 base + P.off_chunks + (size_t)c * P.chunk_bytes, P.cl_offs, need_general + f0, max_contours, max_blobs, min_area, min_circ,
-                                 out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, out_flags + f0,
-                                 out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,
-                                 s, nullptr, how);
-        if (st != MOCAP_OK) return st;
-        if (dp->sc_xy) {
-            st = launch_scatter(out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, dp->sc_xy + f0, dp->sc_count + f0, nc, max_blobs, need_general + f0, 0, s);
-            if (st != MOCAP_OK) return st;
-        }
-    }
-#else
-    const bool tl = opts->record_timeline != 0;
     CUDA_TRY(cudaEventRecord(dp->ev_fork, s));
     CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, dp->ev_fork, 0));
     if (dp->tok_wait) CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, (cudaEvent_t)dp->tok_wait, 0));    // scans of several pipes one after the other
-    if (mode == 1) {
-        st = launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, ctrl, chunks, cf, 0, 0, -1, opts->scan_stages, dp->s_scan);
+    if (tma) {
+        st = launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, ctrl, chunks, cf, dp->s_scan);
         if (st != MOCAP_OK) return st;
     }
-    // Stream plans (which worker stream runs which stage of which chunk):
-    //   0  a chunk's stages as one chain on worker (chunk mod workers)
-    //   1  stage streams: worker 0 groups, worker 1 filters, workers 2.. take the borders of alternate chunks
-    //   2  worker 0 groups and filters chunk after chunk; workers 1.. take the borders (they fill the filter kernels' tails)
-    //   3  like 2, grouping one chunk ahead of the filter (group(k+1) is issued before filter(k): never waits for filter CTAs to leave)
-    int plan = opts->stream_plan;
-    if ((plan == 1 && dp->n_proc < 3) || ((plan == 2 || plan == 3) && dp->n_proc < 2) || plan < 0 || plan > 3) plan = 0;
     for (int i = 0; i < dp->n_proc; ++i) CUDA_TRY(cudaStreamWaitEvent(dp->s_proc[i], dp->ev_fork, 0));
-    auto group_stream = [&](int c) { return plan == 0 ? dp->s_proc[c % dp->n_proc] : dp->s_proc[0]; };
-    auto run_stages = [&](int c, int stages) -> int {
-        const int f0 = c * cf, nc = (n_frames - f0) < cf ? (n_frames - f0) : cf;
-        char* cws = base + P.off_chunks + (size_t)c * P.chunk_bytes;
-        uint32_t* cb = ws.cellbox + (size_t)f0 * tv.TX * tv.TY;
-        cudaStream_t ps = group_stream(c);
-        ClusterLaunch hc = how;
-        hc.zero = 0;
-        hc.stages = stages;
-        hc.ev_group = dp->ev_tl[c][1]; hc.ev_filter = dp->ev_tl[c][2]; hc.ev_borders = dp->ev_tl[c][3];
-        if (plan == 1) { hc.s_filter = dp->s_proc[1]; hc.s_borders = dp->s_proc[2 + c % (dp->n_proc - 2)]; }
-        if (plan == 2 || plan == 3) { hc.s_filter = dp->s_proc[0]; hc.s_borders = dp->s_proc[1 + c % (dp->n_proc - 1)]; }
-        int rc = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, cb, cws, P.cl_offs, need_general + f0,
-                                     max_contours, max_blobs, min_area, min_circ,
-                                     out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, out_flags + f0,
-                                     out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,
-                                     ps, nullptr, hc);
-        if (rc == MOCAP_OK && (stages & 4) && dp->sc_xy) {      // the chunk's records go where their consumers read them, off the critical path
-            cudaStream_t sb = hc.s_borders ? hc.s_borders : (hc.s_filter ? hc.s_filter : ps);
-            rc = launch_scatter(out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, dp->sc_xy + f0, dp->sc_count + f0, nc, max_blobs, need_general + f0, 0, sb);
-        }
-        return rc;
-    };
     for (int c = 0; c < chunks; ++c) {
         const int f0 = c * cf, nc = (n_frames - f0) < cf ? (n_frames - f0) : cf;
-        cudaStream_t ps = group_stream(c);
+        cudaStream_t ps = dp->s_proc[c % dp->n_proc];
         char* cws = base + P.off_chunks + (size_t)c * P.chunk_bytes;
-        CUDA_TRY(cudaMemsetAsync(cws + P.cl_offs[14], 0, P.cl_offs[15], ps));     // the chunk's counters / lists, off the critical path
-        if (prescanned) {
-            // nothing to wait for: the boxes were complete before the fork
-        } else if (mode == 1) {
-            st = stream_wait_geq(ps, ctrl + PIPE_CTRL_WORK + chunks + c, 1);
+        uint32_t* cb = ws.cellbox + (size_t)f0 * tv.TX * tv.TY;
+        CUDA_TRY(cudaMemsetAsync(cws + P.cl.zero_begin, 0, P.cl.zero_bytes, ps));     // the chunk's counters / lists, off the critical path
+        if (tma) {
+            st = stream_wait_geq(ps, scan_tma_chunk_flag(ctrl, chunks, c), 1);
             if (st != MOCAP_OK) return st;
-        } else {
-            if (tma) {
-                // all launches share the batch-wide tensor map and item numbering; launch c covers the boxes of chunk c
-                const int ib = f0 * per_frame_items, ie = (f0 + nc) * per_frame_items;
-                st = launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, ctrl, chunks, cf, c, ib, ie, opts->scan_stages, dp->s_scan);
-            } else {
-                FilterWs wc = ws; wc.cellbox = ws.cellbox + (size_t)f0 * tv.TX * tv.TY;
-                st = launch_scan(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, wc, dp->s_scan, nullptr);
-            }
+        } else if (!prescanned) {                                                   // (handed-in boxes were complete before the fork)
+            FilterWs wc = ws; wc.cellbox = cb;
+            st = launch_scan(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, wc, dp->s_scan, nullptr);
             if (st != MOCAP_OK) return st;
             CUDA_TRY(cudaEventRecord(dp->ev_scan[c], dp->s_scan));
             CUDA_TRY(cudaStreamWaitEvent(ps, dp->ev_scan[c], 0));
         }
-        if (tl) CUDA_TRY(cudaEventRecord(dp->ev_tl[c][0], ps));
-        if (plan == 3) {
-            st = run_stages(c, 1);
-            if (st == MOCAP_OK && c > 0) st = run_stages(c - 1, 2 | 4);
-            if (st == MOCAP_OK && c == chunks - 1) st = run_stages(c, 2 | 4);
-        } else {
-            st = run_stages(c, 1 | 2 | 4);
-        }
+        if (record_timeline) CUDA_TRY(cudaEventRecord(dp->ev_tl[c][0], ps));
+        how.ev_group = dp->ev_tl[c][1]; how.ev_filter = dp->ev_tl[c][2]; how.ev_borders = dp->ev_tl[c][3];
+        st = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, cb, cws, P.cl, need_general + f0,
+                                 max_contours, max_blobs, min_area, min_circ,
+                                 out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, out_flags + f0,
+                                 out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,
+                                 ps, nullptr, how);
         if (st != MOCAP_OK) return st;
+        if (dp->sc_xy) {                                     // the chunk's records go where their consumers read them, off the critical path
+            st = launch_scatter(out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, dp->sc_xy + f0, dp->sc_count + f0, nc, max_blobs, need_general + f0, 0, ps);
+            if (st != MOCAP_OK) return st;
+        }
     }
     CUDA_TRY(cudaEventRecord(dp->ev_scan_done, dp->s_scan));
     if (dp->tok_done) CUDA_TRY(cudaEventRecord((cudaEvent_t)dp->tok_done, dp->s_scan));
@@ -549,8 +482,7 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
         CUDA_TRY(cudaEventRecord(dp->ev_proc_done[i], dp->s_proc[i]));
         CUDA_TRY(cudaStreamWaitEvent(s, dp->ev_proc_done[i], 0));
     }
-    if (tl) { CUDA_TRY(cudaEventRecord(dp->ev_join, s)); dp->tl_chunks = chunks; }
-#endif
+    if (record_timeline) { CUDA_TRY(cudaEventRecord(dp->ev_join, s)); dp->tl_chunks = chunks; }
     // general path for the frames the cluster units could not finish (rare), whole batch
     st = launch_tiles(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws, P.L.max_fg, out_flags, need_general, s);
     if (st != MOCAP_OK) return st;
@@ -568,10 +500,6 @@ extern "C" int mocap_detect_pipe_timeline(void* pipe, float* ms_out, int cap)
 {
     DetectPipe* dp = (DetectPipe*)pipe;
     if (!dp || !ms_out) return MOCAP_ERR_INVALID;
-#ifdef MOCAP_EMU
-    (void)cap;
-    return 0;
-#else
     const int need = 2 + PIPE_TL_PER_CHUNK * dp->tl_chunks;
     if (dp->tl_chunks == 0) return 0;
     if (cap < need) return MOCAP_ERR_INVALID;
@@ -582,15 +510,15 @@ extern "C" int mocap_detect_pipe_timeline(void* pipe, float* ms_out, int cap)
         for (int k = 0; k < PIPE_TL_PER_CHUNK; ++k)
             CUDA_TRY(cudaEventElapsedTime(&ms_out[2 + c * PIPE_TL_PER_CHUNK + k], dp->ev_fork, dp->ev_tl[c][k]));
     return need;
-#endif
 }
 
-// what the last pipelined call actually ran: [0] scan kernel (1 = TMA ring, 0 = classic), [1] chunks, [2] sync mode used
+// what the last pipelined call actually ran: [0] scan kernel (1 = TMA ring, 0 = classic or none), [1] chunks, [2] sync mode
+// (1 = the workers waited on the TMA scan's chunk flags, 0 = on events or on nothing: always equal to [0])
 extern "C" int mocap_detect_pipe_info(void* pipe, int* out3)
 {
     DetectPipe* dp = (DetectPipe*)pipe;
     if (!dp || !out3) return MOCAP_ERR_INVALID;
-    out3[0] = dp->last_scan; out3[1] = dp->last_chunks; out3[2] = dp->last_mode;
+    out3[0] = dp->last_tma; out3[1] = dp->last_chunks; out3[2] = dp->last_tma;
     return MOCAP_OK;
 }
 
@@ -600,7 +528,7 @@ extern "C" int mocap_scan_cells_batch(const uint8_t* frames_dev, int n_frames, i
                                       int thresh, int variant, uint32_t* cellbox_out, void* workspace, size_t workspace_bytes, void* stream)
 {
     if (!frames_dev || !table_dev || !cellbox_out || n_frames <= 0 || H <= 0 || W <= 0) return MOCAP_ERR_INVALID;
-    if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
+    if (frame_stride < (int64_t)H * W || (variant != 0 && variant != 1)) return MOCAP_ERR_INVALID;
     cudaStream_t s = (cudaStream_t)stream;
     TableView tv; table_view(table_dev, H, W, &tv);
     if (variant == 0) {
@@ -611,5 +539,5 @@ extern "C" int mocap_scan_cells_batch(const uint8_t* frames_dev, int n_frames, i
     if (!scan_tma_supported(frames_dev, n_frames, H, W, frame_stride, thresh)) return MOCAP_ERR_UNSUPPORTED;
     if (!workspace || workspace_bytes < scan_tma_ctrl_bytes(1)) return MOCAP_ERR_WORKSPACE;
     CUDA_TRY(cudaMemsetAsync(workspace, 0, scan_tma_ctrl_bytes(1), s));
-    return launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, cellbox_out, (int*)workspace, 1, n_frames, 0, 0, -1, variant == 2 ? 3 : 6, s);
+    return launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, cellbox_out, (int*)workspace, 1, n_frames, s);
 }

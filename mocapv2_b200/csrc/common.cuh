@@ -6,6 +6,14 @@
 #define LAUNCH(kernel, grid, block, smem, stream, ...) \
     (mocap_count_launch(), emu::launch(dim3(grid), dim3(block), (size_t)(smem), [=]() { kernel(__VA_ARGS__); }))
 #define DYN_SHARED(name) unsigned char* name = emu::dyn_smem()
+// the overlapped detection's streams and events there: launches run where they are issued, so every stream is the null
+// stream and waiting for an event has nothing to wait for
+enum { cudaStreamNonBlocking = 1, cudaEventDefault = 0, cudaEventDisableTiming = 2 };
+static inline cudaError_t cudaEventCreateWithFlags(cudaEvent_t* e, unsigned) { return cudaEventCreate(e); }
+static inline cudaError_t cudaDeviceGetStreamPriorityRange(int* lo, int* hi) { *lo = 0; *hi = 0; return 0; }
+static inline cudaError_t cudaStreamCreateWithPriority(cudaStream_t* s, unsigned, int) { *s = nullptr; return 0; }
+static inline cudaError_t cudaStreamDestroy(cudaStream_t) { return 0; }
+static inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigned) { return 0; }
 #else
 #include <cuda_runtime.h>
 #define LAUNCH(kernel, grid, block, smem, stream, ...) (mocap_count_launch(), kernel<<<grid, block, smem, stream>>>(__VA_ARGS__))
@@ -14,7 +22,7 @@
 #include <stdint.h>
 #include "../../include/mocap_b200.h"
 
-#define MOCAP_ABI_VERSION 2
+#define MOCAP_ABI_VERSION 3
 
 // every kernel launch of the library is counted (mocap_kernel_launch_count: the bench's gpu_launches is read, not estimated)
 extern unsigned long long g_mocap_launches;
@@ -120,12 +128,17 @@ __device__ __forceinline__ uint32_t pack_cellbox(uint32_t xmask, uint32_t ymask)
 // how launch_cluster_path runs a batch (or one chunk of the overlapped pipeline)
 struct ClusterLaunch {
     int zero = 1;                    // clear the counters / lists of the workspace on the stream first
-    int stages = 7;                  // which stages this call issues: 1 group, 2 piece filter, 4 borders (a chunk may be issued in parts)
-    int filter_ctas_per_sm = 8;      // persistent piece-filter CTAs per SM (fewer when the TMA scan is co-resident)
-    int cand_ctas_per_sm = 16;
-    cudaEvent_t ev_group = nullptr, ev_filter = nullptr, ev_borders = nullptr;   // recorded after the stages (timeline marks; hand-over between streams)
-    cudaStream_t s_filter = nullptr, s_borders = nullptr;   // run the piece filter / the border stage on other streams than the grouping
-                                                             // (each waits for the event of the stage before it, which must then be set)
+    int filter_ctas = 8;             // persistent piece-filter CTAs per SM (fewer when the TMA scan is co-resident)
+    int cand_ctas = 16;              // candidates_kernel CTAs per SM
+    cudaEvent_t ev_group = nullptr, ev_filter = nullptr, ev_borders = nullptr;   // recorded after the stages (timeline marks)
+};
+
+// byte offsets of the cluster path's arrays in its workspace (cluster_ws_bytes)
+struct ClusterLayout {
+    size_t need_general;             // int [n] (the chunked path keeps one array for the whole batch instead)
+    size_t zero_begin, zero_bytes;   // the block a call has to zero first: counters, rec_count, cand_count, frame_clusters
+    size_t counters, rec_count, cand_count, frame_clusters;
+    size_t clusters, pieces, rec_start, rec_a, rec_per, memb, rows_out, cand_list, rec_info;
 };
 
 // workspace slices of the filter stage (carved by api.cu)

@@ -1156,27 +1156,26 @@ static int cl_cap_of(int n) { return n * 256 + 1024; }
 static int pc_cap_of(int n) { return n * 512 + 2048; }
 static size_t rows_cap_of(int n, int H, int W) { size_t w = (size_t)n * ((size_t)H * W / 128 + 4096); return w > 0xf0000000ull ? 0xf0000000ull : w; }   // a quarter of the frame area per frame
 
-size_t cluster_ws_bytes(int n, int H, int W, int max_contours, size_t* offs /*[16]*/)
+size_t cluster_ws_bytes(int n, int H, int W, int max_contours, ClusterLayout* L)
 {
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t r = off; off += align_up(bytes, 256); return r; };
-    offs[0] = take((size_t)n * 4);                         // need_general (the chunked path keeps one array for the whole batch instead)
-    // everything a call has to zero first lies in one block: offs[14] = its start, offs[15] = its size
-    offs[14] = off;
-    offs[1] = take(64);                                    // counters
-    offs[4] = take((size_t)n * 4);                         // rec_count
-    offs[11] = take((size_t)n * 4);                        // cand_count
-    offs[13] = take((size_t)n * 8);                        // frame_clusters
-    offs[15] = off - offs[14];
-    offs[2] = take((size_t)cl_cap_of(n) * 32);             // clusters
-    offs[3] = take((size_t)pc_cap_of(n) * 32);             // pieces
-    offs[5] = take((size_t)n * max_contours * 4);          // rec_start
-    offs[6] = take((size_t)n * max_contours * 24);         // rec_a
-    offs[7] = take((size_t)n * max_contours * 8);          // rec_per
-    offs[8] = take((size_t)n * HOT_MAX * 8);               // memb
-    offs[9] = take(rows_cap_of(n, H, W) * 4);              // rows_out
-    offs[10] = take((size_t)n * CAND_PER_FRAME * 8);       // cand_list
-    offs[12] = take((size_t)n * max_contours * 16);        // rec_info
+    L->need_general = take((size_t)n * 4);
+    L->zero_begin = off;
+    L->counters = take(64);
+    L->rec_count = take((size_t)n * 4);
+    L->cand_count = take((size_t)n * 4);
+    L->frame_clusters = take((size_t)n * 8);
+    L->zero_bytes = off - L->zero_begin;
+    L->clusters = take((size_t)cl_cap_of(n) * 32);
+    L->pieces = take((size_t)pc_cap_of(n) * 32);
+    L->rec_start = take((size_t)n * max_contours * 4);
+    L->rec_a = take((size_t)n * max_contours * 24);
+    L->rec_per = take((size_t)n * max_contours * 8);
+    L->memb = take((size_t)n * HOT_MAX * 8);
+    L->rows_out = take(rows_cap_of(n, H, W) * 4);
+    L->cand_list = take((size_t)n * CAND_PER_FRAME * 8);
+    L->rec_info = take((size_t)n * max_contours * 16);
     return off;
 }
 
@@ -1186,30 +1185,30 @@ bool cluster_path_supported(int H, int W)
 }
 
 int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstride, const TableView& tv, int thresh,
-                        const uint32_t* cellbox, char* ws_base, const size_t* offs, int* need_general,
+                        const uint32_t* cellbox, char* ws_base, const ClusterLayout& L, int* need_general,
                         int max_contours, int max_blobs, double min_area, double min_circ,
                         int32_t* out_xy, int32_t* out_count, int32_t* out_flags, double* out_contours, int32_t* out_contour_count,
                         cudaStream_t s, StageTimer* timer, const ClusterLaunch& how)
 {
     ClusterWs cw;
     cw.need_general = need_general;
-    cw.counters = (int*)(ws_base + offs[1]);
-    cw.clusters = (int*)(ws_base + offs[2]);
-    cw.pieces = (int*)(ws_base + offs[3]);
+    cw.counters = (int*)(ws_base + L.counters);
+    cw.clusters = (int*)(ws_base + L.clusters);
+    cw.pieces = (int*)(ws_base + L.pieces);
     cw.cl_cap = cl_cap_of(n); cw.pc_cap = pc_cap_of(n);
-    cw.rec_count = (int*)(ws_base + offs[4]);
-    cw.rec_start = (int*)(ws_base + offs[5]);
-    cw.rec_a = (long long*)(ws_base + offs[6]);
-    cw.rec_per = (double*)(ws_base + offs[7]);
-    cw.memb = (short*)(ws_base + offs[8]);
-    cw.rows_out = (uint32_t*)(ws_base + offs[9]);
+    cw.rec_count = (int*)(ws_base + L.rec_count);
+    cw.rec_start = (int*)(ws_base + L.rec_start);
+    cw.rec_a = (long long*)(ws_base + L.rec_a);
+    cw.rec_per = (double*)(ws_base + L.rec_per);
+    cw.memb = (short*)(ws_base + L.memb);
+    cw.rows_out = (uint32_t*)(ws_base + L.rows_out);
     cw.rows_cap = (unsigned)rows_cap_of(n, H, W);
-    cw.cand_list = (int*)(ws_base + offs[10]);
-    cw.cand_count = (int*)(ws_base + offs[11]);
-    cw.rec_info = (int*)(ws_base + offs[12]);
-    cw.frame_clusters = (int*)(ws_base + offs[13]);
+    cw.cand_list = (int*)(ws_base + L.cand_list);
+    cw.cand_count = (int*)(ws_base + L.cand_count);
+    cw.rec_info = (int*)(ws_base + L.rec_info);
+    cw.frame_clusters = (int*)(ws_base + L.frame_clusters);
     cw.n_frames = n;
-    if (how.zero) CUDA_TRY(cudaMemsetAsync(ws_base + offs[14], 0, offs[15], s));
+    if (how.zero) CUDA_TRY(cudaMemsetAsync(ws_base + L.zero_begin, 0, L.zero_bytes, s));
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -1219,47 +1218,33 @@ int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstr
     static bool attr_done = false;                          // (idempotent; a race only repeats the call)
     if (!attr_done) { CUDA_TRY(cudaFuncSetAttribute(form_clusters_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024)); attr_done = true; }
 #endif
-    if (how.stages & 1) {
-        stage_begin(timer, 1, s);
-        LAUNCH(form_clusters_kernel, n, CL_THREADS, sm_form, s, cellbox, tv, cw);
-        stage_end(timer, 1, s);
-        if (how.ev_group) cudaEventRecord(how.ev_group, s);
-    }
-    cudaStream_t sf = how.s_filter ? how.s_filter : s;
-    if (how.stages & 2) {
-#ifndef MOCAP_EMU
-        if (sf != s) { if (!how.ev_group) return MOCAP_ERR_INVALID; CUDA_TRY(cudaStreamWaitEvent(sf, how.ev_group, 0)); }
-#endif
-        stage_begin(timer, 2, sf);
+    stage_begin(timer, 1, s);
+    LAUNCH(form_clusters_kernel, n, CL_THREADS, sm_form, s, cellbox, tv, cw);
+    stage_end(timer, 1, s);
+    if (how.ev_group) cudaEventRecord(how.ev_group, s);
+    stage_begin(timer, 2, s);
 #ifdef MOCAP_EMU
-        LAUNCH(piece_filter_kernel, sms * how.filter_ctas_per_sm, CL_THREADS, 0, sf, frames, fstride, tv, thresh, cw);
+    LAUNCH(piece_filter_kernel, sms * how.filter_ctas, CL_THREADS, 0, s, frames, fstride, tv, thresh, cw);
 #else
-        {
-            CUtensorMap tmap, tmap_low;
-            memset(&tmap, 0, sizeof(tmap)); memset(&tmap_low, 0, sizeof(tmap_low));
-            const int T = thresh + 1;
-            const int use_tma = (T >= 0 && T <= 256 && frames_tensor_map(&tmap, frames, n, H, W, fstride, WIN_W, WIN_H, PF_WIN_L2_PROMO) &&
-                                 frames_tensor_map(&tmap_low, frames, n, H, W, fstride, WIN_W, WIN_H_LOW, PF_WIN_L2_PROMO)) ? 1 : 0;
-            LAUNCH(piece_filter_kernel, sms * how.filter_ctas_per_sm, CL_THREADS, 0, sf, frames, fstride, tv, thresh, cw, tmap, tmap_low, use_tma);
-        }
-#endif
-        stage_end(timer, 2, sf);
-        if (how.ev_filter) cudaEventRecord(how.ev_filter, sf);
+    {
+        CUtensorMap tmap, tmap_low;
+        memset(&tmap, 0, sizeof(tmap)); memset(&tmap_low, 0, sizeof(tmap_low));
+        const int T = thresh + 1;
+        const int use_tma = (T >= 0 && T <= 256 && frames_tensor_map(&tmap, frames, n, H, W, fstride, WIN_W, WIN_H, PF_WIN_L2_PROMO) &&
+                             frames_tensor_map(&tmap_low, frames, n, H, W, fstride, WIN_W, WIN_H_LOW, PF_WIN_L2_PROMO)) ? 1 : 0;
+        LAUNCH(piece_filter_kernel, sms * how.filter_ctas, CL_THREADS, 0, s, frames, fstride, tv, thresh, cw, tmap, tmap_low, use_tma);
     }
-    cudaStream_t sb = how.s_borders ? how.s_borders : sf;
-    if (how.stages & 4) {
-#ifndef MOCAP_EMU
-        if (sb != sf) { if (!how.ev_filter) return MOCAP_ERR_INVALID; CUDA_TRY(cudaStreamWaitEvent(sb, how.ev_filter, 0)); }
 #endif
-        stage_begin(timer, 3, sb);
-        LAUNCH(candidates_kernel, sms * how.cand_ctas_per_sm, 128, 0, sb, cw);
-        int frame_step = 1;
-        for (int pr : {61, 67, 71, 73}) if (n % pr != 0) { frame_step = pr; break; }          // a prime that does not divide n
-        LAUNCH(borders_finalize_kernel, n, BF_THREADS, (size_t)max_contours + 16, sb, cw, W, frame_step, max_contours, max_blobs, min_area, min_circ,
-               out_xy, out_count, out_flags, out_contours, out_contour_count);
-        stage_end(timer, 3, sb);
-        if (how.ev_borders) cudaEventRecord(how.ev_borders, sb);
-    }
+    stage_end(timer, 2, s);
+    if (how.ev_filter) cudaEventRecord(how.ev_filter, s);
+    stage_begin(timer, 3, s);
+    LAUNCH(candidates_kernel, sms * how.cand_ctas, 128, 0, s, cw);
+    int frame_step = 1;
+    for (int pr : {61, 67, 71, 73}) if (n % pr != 0) { frame_step = pr; break; }          // a prime that does not divide n
+    LAUNCH(borders_finalize_kernel, n, BF_THREADS, (size_t)max_contours + 16, s, cw, W, frame_step, max_contours, max_blobs, min_area, min_circ,
+           out_xy, out_count, out_flags, out_contours, out_contour_count);
+    stage_end(timer, 3, s);
+    if (how.ev_borders) cudaEventRecord(how.ev_borders, s);
     CUDA_TRY(cudaGetLastError());
     return MOCAP_OK;
 }

@@ -19,7 +19,11 @@
 // memory operation (cuStreamWaitValue32) -- no kernel ever spins on another kernel.
 #include "common.cuh"
 
-#define SCAN_CTRL_WORK 64          // work-counter slots at the head of the control block (one per scan launch of a call)
+// Control block of a launch: int [SCAN_CTRL_WORK + 2 chunks] = the work counter (slot 0, the rest of the head is unused), then
+// chunk_done[], chunk_flag[].
+#define SCAN_CTRL_WORK 64
+size_t scan_tma_ctrl_bytes(int chunks) { return align_up((size_t)(SCAN_CTRL_WORK + 2 * chunks) * 4, 256); }
+const int* scan_tma_chunk_flag(const int* ctrl, int chunks, int chunk) { return ctrl + SCAN_CTRL_WORK + chunks + chunk; }
 
 #include "tma.cuh"
 #ifndef MOCAP_EMU
@@ -28,7 +32,7 @@
 #define ST_BOX_H 32
 #define ST_STAGE_BYTES (ST_BOX_W * ST_BOX_H)
 #define ST_CONSUMERS 4
-#define ST_STAGES_MAX 6            // ring slots of 8 KB: 6 when the scan has the SM (almost) to itself, 3 beside seven filter CTAs
+#define ST_STAGES 6                // ring slots of 8 KB
 #define ST_GRAB 8                  // boxes a producer draws from the work counter at a time (one 2048-pixel band of cells)
 #define ST_THREADS (32 * (ST_CONSUMERS + 1))
 
@@ -56,7 +60,7 @@ __device__ __forceinline__ void scan_publish(const ScanTmaArgs& a, int ch, int c
     }
 }
 
-template <int MODE, int ST_STAGES>
+template <int MODE>
 __global__ void __launch_bounds__(ST_THREADS, 8) scan_tma_kernel(const __grid_constant__ CUtensorMap tmap, ScanTmaArgs a)
 {
     extern __shared__ unsigned char st_raw[];
@@ -216,12 +220,9 @@ bool scan_tma_supported(const uint8_t* frames, int n, int H, int W, int64_t fstr
     return have;
 }
 
-size_t scan_tma_ctrl_bytes(int chunks) { return align_up((size_t)(SCAN_CTRL_WORK + 2 * chunks) * 4, 256); }
-
-// One launch over the boxes [item_begin, item_end) of the batch (all of them: item_end < 0).  ctrl: int [SCAN_CTRL_WORK + 2 chunks],
-// zeroed by the caller on an earlier point of the stream: work counters (one per launch index `widx`), then chunk_done[], chunk_flag[].
+// One launch over every box of the batch.  ctrl: the control block, zeroed by the caller on an earlier point of the stream.
 int launch_scan_tma(const uint8_t* frames, int n, int H, int W, int64_t fstride, const TableView& tv, int thresh, uint32_t* cellbox,
-                    int* ctrl, int chunks, int chunk_frames, int widx, int item_begin, int item_end, int stages, cudaStream_t s)
+                    int* ctrl, int chunks, int chunk_frames, cudaStream_t s)
 {
     CUtensorMap map;
     if (!frames_tensor_map(&map, frames, n, H, W, fstride, ST_BOX_W, ST_BOX_H, 256)) return MOCAP_ERR_UNSUPPORTED;
@@ -231,7 +232,7 @@ int launch_scan_tma(const uint8_t* frames, int n, int H, int W, int64_t fstride,
     const HotTest ht = make_hot_test(thresh);
     ScanTmaArgs a;
     a.cellbox = cellbox;
-    a.work = ctrl + widx;
+    a.work = ctrl;
     a.chunk_done = ctrl + SCAN_CTRL_WORK;
     a.chunk_flag = ctrl + SCAN_CTRL_WORK + chunks;
     a.TX = tv.TX; a.TY = tv.TY; a.XB = cdiv(W, ST_BOX_W);
@@ -239,25 +240,18 @@ int launch_scan_tma(const uint8_t* frames, int n, int H, int W, int64_t fstride,
     if (per_frame * n >= (1LL << 31) - 64 * ST_GRAB * sms) return MOCAP_ERR_UNSUPPORTED;
     a.total_items = (int)(per_frame * n);
     a.items_per_chunk = (int)(per_frame * chunk_frames);
-    a.item_begin = item_begin; a.item_end = item_end < 0 ? a.total_items : item_end;
+    a.item_begin = 0; a.item_end = a.total_items;
     a.add = ht.add;
-    const int S = stages == 3 ? 3 : ST_STAGES_MAX;
-    const size_t smem = (size_t)S * ST_STAGE_BYTES + 4 * S * 8 + 16 + S * sizeof(StageRec) + 128;
+    const int smem = ST_STAGES * ST_STAGE_BYTES + 4 * ST_STAGES * 8 + 16 + ST_STAGES * (int)sizeof(StageRec) + 128;
     static bool attr_done = false;
     if (!attr_done) {
-        const int big = ST_STAGES_MAX * ST_STAGE_BYTES + 4 * ST_STAGES_MAX * 8 + 16 + ST_STAGES_MAX * (int)sizeof(StageRec) + 128;
-        CUDA_TRY(cudaFuncSetAttribute(scan_tma_kernel<0, ST_STAGES_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-        CUDA_TRY(cudaFuncSetAttribute(scan_tma_kernel<1, ST_STAGES_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+        CUDA_TRY(cudaFuncSetAttribute(scan_tma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        CUDA_TRY(cudaFuncSetAttribute(scan_tma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         attr_done = true;
     }
     mocap_count_launch();
-    if (S == 3) {
-        if (ht.mode == 0) scan_tma_kernel<0, 3><<<sms, ST_THREADS, smem, s>>>(map, a);
-        else scan_tma_kernel<1, 3><<<sms, ST_THREADS, smem, s>>>(map, a);
-    } else {
-        if (ht.mode == 0) scan_tma_kernel<0, ST_STAGES_MAX><<<sms, ST_THREADS, smem, s>>>(map, a);
-        else scan_tma_kernel<1, ST_STAGES_MAX><<<sms, ST_THREADS, smem, s>>>(map, a);
-    }
+    if (ht.mode == 0) scan_tma_kernel<0><<<sms, ST_THREADS, smem, s>>>(map, a);
+    else scan_tma_kernel<1><<<sms, ST_THREADS, smem, s>>>(map, a);
     CUDA_TRY(cudaGetLastError());
     return MOCAP_OK;
 }
@@ -278,8 +272,7 @@ bool stream_wait_supported()
 #else   // MOCAP_EMU: the CPU emulation build of the kernel sources (tests/emu) has no TMA unit; the classic scan kernels serve there
 
 bool scan_tma_supported(const uint8_t*, int, int, int, int64_t, int) { return false; }
-size_t scan_tma_ctrl_bytes(int chunks) { return align_up((size_t)(SCAN_CTRL_WORK + 2 * chunks) * 4, 256); }
-int launch_scan_tma(const uint8_t*, int, int, int, int64_t, const TableView&, int, uint32_t*, int*, int, int, int, int, int, int, cudaStream_t) { return MOCAP_ERR_UNSUPPORTED; }
+int launch_scan_tma(const uint8_t*, int, int, int, int64_t, const TableView&, int, uint32_t*, int*, int, int, cudaStream_t) { return MOCAP_ERR_UNSUPPORTED; }
 int stream_wait_geq(cudaStream_t, const int*, int) { return MOCAP_ERR_UNSUPPORTED; }
 bool stream_wait_supported() { return false; }
 

@@ -92,7 +92,6 @@ class CaptureEngine:
         self._lock = threading.RLock()
         self._launch_base = int(self.lib.mocap_kernel_launch_count())
         self.pipe_workers = 3                   # worker streams of the overlapped detection
-        self.pipe_prio_mode = 0
         self.last_pipe_info = None
 
     def clone(self) -> "CaptureEngine":
@@ -104,7 +103,7 @@ class CaptureEngine:
         other._init_state()
         other._tables = self._tables
         other._lock = self._lock                 # one lock for the shared table cache
-        other.pipe_workers, other.pipe_prio_mode = self.pipe_workers, self.pipe_prio_mode
+        other.pipe_workers = self.pipe_workers
         return other
 
     # ---- plumbing ------------------------------------------------------------------------------------------------
@@ -268,12 +267,12 @@ class CaptureEngine:
     # ---- overlapped detection (chunks: TMA scan of chunk k+1 beside the filter / border stages of chunk k) ----------------------
     def _pipe(self):
         """The calling thread's detection pipe (worker streams + events of the overlapped detection)."""
-        key = (int(self.pipe_workers), int(self.pipe_prio_mode))
+        key = int(self.pipe_workers)
         pipes = getattr(self._tls, "pipes", None)
         if pipes is None:
             pipes = self._tls.pipes = {}
         if key not in pipes:
-            h = self.lib.mocap_detect_pipe_create(*key)
+            h = self.lib.mocap_detect_pipe_create(key)
             if not h:
                 raise _cabi.MocapError("mocap_detect_pipe_create failed")
             pipes[key] = h
@@ -281,8 +280,7 @@ class CaptureEngine:
 
     def detect_pipelined(self, frames: torch.Tensor, K, dist, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
                          max_blobs=None, max_contours=None, max_runs=None, outputs=(), out: DetectResult | None = None,
-                         chunk_frames=128, sync_mode=1, scan_variant=1, filter_ctas_per_sm=0, cand_ctas_per_sm=0,
-                         stream_plan=0, scan_stages=6, timeline=False, cellbox: torch.Tensor | None = None) -> DetectResult:
+                         chunk_frames=128, timeline=False, cellbox: torch.Tensor | None = None) -> DetectResult:
         """Same results as detect() (centroid lists, optionally the contour table), computed chunk by chunk with the streaming
         scan overlapped with the other stages (mocap_detect_batch_pipelined).  cellbox: the frames' hot cell boxes from
         bayer_gr2gray_scan (same thresh) -- the call then has no streaming scan."""
@@ -308,8 +306,6 @@ class CaptureEngine:
         nbytes = self.lib.mocap_detect_pipelined_workspace_bytes(n, H, W, max_blobs, max_contours, max_runs, int(chunk_frames))
         if nbytes == 0:
             raise _cabi.MocapError("mocap_detect_pipelined_workspace_bytes: unsupported shape")
-        opts = _cabi.PipeOpts(int(chunk_frames), int(sync_mode), int(scan_variant), int(filter_ctas_per_sm), int(cand_ctas_per_sm),
-                              1 if timeline else 0, int(stream_plan), int(scan_stages))
         ws = self._workspace(nbytes)
         if cellbox is not None:
             if tuple(cellbox.shape) != (n, (H + 31) // 32, (W + 31) // 32):
@@ -321,16 +317,14 @@ class CaptureEngine:
                 self._pipe(), self._ptr(frames), n, H, W, stride, self._ptr(tab), int(thresh), float(min_area), float(min_circ),
                 max_blobs, max_contours, max_runs, self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags),
                 self._ptr(ex.get("contours")), self._ptr(ex.get("contour_count")), self._ptr(ws), nbytes, self._stream(),
-                ctypes.byref(opts))
+                int(chunk_frames), 1 if timeline else 0)
         finally:
             if cellbox is not None:
                 self.lib.mocap_detect_pipe_set_cellbox(self._pipe(), None)
         _cabi.check(self.lib, st, "mocap_detect_batch_pipelined")
         info = (ctypes.c_int * 3)()
         self.lib.mocap_detect_pipe_info(self._pipe(), info)
-        chunks = int(info[1])
-        scans = 1 if int(info[2]) == 1 else chunks
-        self.last_pipe_info = {"tma_scan": bool(info[0]), "chunks": chunks, "sync_mode": int(info[2])}
+        self.last_pipe_info = {"tma_scan": bool(info[0]), "chunks": int(info[1]), "sync_mode": int(info[2])}
         return out
 
     def set_detect_scatter(self, xy_dst: torch.Tensor | None, count_dst: torch.Tensor | None):

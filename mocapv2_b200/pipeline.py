@@ -64,7 +64,8 @@ class CapturePipeline:
         self.peer_exchange = True
         self._peer = None                       # {"bufs", "hdls", "tables", "views", "turn", "n", "per"}
         # overlapped detection (engine.detect_pipelined) for batches large enough to pipeline: 8 chunks on 6 worker streams
-        # (tools/pipe_probe.py on the C4 batch: 1.75 ms against 2.03 ms for the one-shot call; 4 chunks / 4 workers 1.78 ms)
+        # (chunks x workers sweep on the C4 batch, profiles/r2_pipe_probe.log: 1.75 ms against 2.03 ms for the one-shot call;
+        # 4 chunks / 4 workers 1.78 ms; tools/stage_probe.py --grid chunks,workers times other splits)
         self.scan_token = None                  # (wait, done) events of the coming overlapped detection, set by StepsInFlight
         self.pipelined_min_frames = 256
         self.engine_pipe = {"workers": 6, "chunks": 8}

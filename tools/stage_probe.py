@@ -66,8 +66,7 @@ def main():
     print(f"one-shot call   {t:.4f} ms", flush=True)
     refxy, refc = ref.xy.clone(), ref.count.clone()
     for g in a.grid.split(";"):
-        chunks, workers, *rest = (int(x) for x in g.split(","))
-        fc = rest[0] if rest else 0
+        chunks, workers = (int(x) for x in g.split(","))
         e = CaptureEngine(dev)
         e._tables = eng._tables
         e.pipe_workers = workers
@@ -79,16 +78,16 @@ def main():
         e.detect_pipelined(frames, K, D, max_blobs=mb, chunk_frames=cf, out=res, timeline=True)
         torch.cuda.synchronize()
         tl = e.pipe_timeline()
-        print(f"overlapped chunks {chunks:2d} workers {workers} filter_ctas {fc}: {t:.4f} ms  same={same}  scan done {tl['scan_done']:.3f} join {tl['join']:.3f}", flush=True)
+        print(f"overlapped chunks {chunks:2d} workers {workers}: {t:.4f} ms  same={same}  scan done {tl['scan_done']:.3f} join {tl['join']:.3f}", flush=True)
         for depth in (2, 3):
-            t2, outs = two_in_flight(eng, frames, K, D, mb, 2 * a.reps, chunks, workers, depth, fc)
+            t2, outs = two_in_flight(eng, frames, K, D, mb, 2 * a.reps, chunks, workers, depth)
             same2 = all(bool(torch.equal(o.count, refc)) for o in outs)
             print(f"   {depth} calls in flight: {t2:.4f} ms per call  same={same2}", flush=True)
         for c, r in enumerate(tl["chunks"]):
             print(f"    {c:2d}: seen {r[0]:.3f}  +group {r[1] - r[0]:.3f}  +filter {r[2] - r[1]:.3f}  +borders {r[3] - r[2]:.3f}  (end {r[3]:.3f})")
 
 
-def two_in_flight(eng, frames, K, D, mb, reps, chunks=8, workers=6, depth=2, fc=0):
+def two_in_flight(eng, frames, K, D, mb, reps, chunks=8, workers=6, depth=2):
     """`depth` overlapped detection calls in flight on their own streams (own pipe, workspace and outputs each)"""
     n = frames.shape[0]
     cf = -(-n // chunks)
@@ -100,7 +99,7 @@ def two_in_flight(eng, frames, K, D, mb, reps, chunks=8, workers=6, depth=2, fc=
         e._tables = eng._tables
         e.pipe_workers = workers
         with torch.cuda.stream(s):
-            outs.append(e.detect_pipelined(frames, K, D, max_blobs=mb, chunk_frames=cf, filter_ctas_per_sm=fc))
+            outs.append(e.detect_pipelined(frames, K, D, max_blobs=mb, chunk_frames=cf))
         engs.append(e)
     torch.cuda.synchronize()
 
@@ -108,7 +107,7 @@ def two_in_flight(eng, frames, K, D, mb, reps, chunks=8, workers=6, depth=2, fc=
         for i in range(k):
             j = i % depth
             with torch.cuda.stream(streams[j]):
-                engs[j].detect_pipelined(frames, K, D, max_blobs=mb, chunk_frames=cf, out=outs[j], filter_ctas_per_sm=fc)
+                engs[j].detect_pipelined(frames, K, D, max_blobs=mb, chunk_frames=cf, out=outs[j])
     run(4)
     torch.cuda.synchronize()
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
