@@ -1143,6 +1143,7 @@ __global__ void __launch_bounds__(CL_THREADS, BORDERS_MIN_CTAS) borders_finalize
     // cameras in the same order, so a plain b -> frame map would hand every SM frames of the same few cameras
     const int f = (int)(((long long)blockIdx.x * frame_step) % cw.n_frames);
     if (cw.need_general[f]) return;
+    step_table_build();                                     // (frame_traces synchronises before its traces)
     frame_traces(cw, f, W, max_contours);
     __syncthreads();
     if (cw.need_general[f]) return;                         // trace budget, unresolved hole parent or nested contour tree

@@ -37,6 +37,7 @@ def main():
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--lib", default="", help="a variant library (tools/build_variant.py) instead of the product library")
     ap.add_argument("--grid", default="8,6;8,4;4,4;16,6", help="semicolon list of chunks,workers")
+    ap.add_argument("--kernel-times", action="store_true", help="also the device time of every kernel of the one-shot call (torch.profiler)")
     a = ap.parse_args()
     if a.lib:
         from mocapv2_b200 import _cabi
@@ -64,6 +65,8 @@ def main():
     print("one-shot stages (ms):", {k: round(v, 4) for k, v in acc.items()}, "sum", round(sum(acc.values()), 4), flush=True)
     t = timed(lambda: eng.detect(frames, K, D, max_blobs=mb, out=ref), a.reps)
     print(f"one-shot call   {t:.4f} ms", flush=True)
+    if a.kernel_times:
+        kernel_times(lambda: eng.detect(frames, K, D, max_blobs=mb, out=ref), a.reps)
     refxy, refc = ref.xy.clone(), ref.count.clone()
     for g in a.grid.split(";"):
         chunks, workers = (int(x) for x in g.split(","))
@@ -85,6 +88,23 @@ def main():
             print(f"   {depth} calls in flight: {t2:.4f} ms per call  same={same2}", flush=True)
         for c, r in enumerate(tl["chunks"]):
             print(f"    {c:2d}: seen {r[0]:.3f}  +group {r[1] - r[0]:.3f}  +filter {r[2] - r[1]:.3f}  +borders {r[3] - r[2]:.3f}  (end {r[3]:.3f})")
+
+
+def kernel_times(fn, reps):
+    """mean device time per call of every kernel `fn` launches (a separate, profiled run)"""
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            fn()
+        torch.cuda.synchronize()
+    acc = {}
+    for ev in prof.events():
+        if ev.device_type.name == "CUDA" and ev.device_time_total > 0:
+            acc[ev.name] = acc.get(ev.name, 0.0) + ev.device_time_total / 1000.0 / reps
+    for name, ms in sorted(acc.items(), key=lambda kv: -kv[1]):
+        print(f"  kernel {ms:8.4f} ms per call  {name.split('(')[0]}", flush=True)
 
 
 def two_in_flight(eng, frames, K, D, mb, reps, chunks=8, workers=6, depth=2):
