@@ -38,6 +38,8 @@ extern "C" {
                                           2 too many hot cells, 3 too many clusters, 5 cluster storage full, 7 too many border
                                           starts, 8 border trace / hole parent outside the fast rules, 9 nested outer border,
                                           10 lens displacement varies by more than 8 px inside a 32-px cell */
+#define MOCAP_FLAG_LENS_INDEX 128      /* the frame's lens index (MocapLensSet::frame_lens_dev) lies outside [0, n_lenses): count 0,
+                                          no table was read for the frame */
 
 /* per-frame-set flags written by mocap_correspond_batch */
 #define MOCAP_CFLAG_GROUP_CAP 1        /* a root had more candidate groups than max_groups: mean over the first max_groups */
@@ -96,6 +98,27 @@ int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, in
                        double* out_contours, int32_t* out_contour_count,
                        void* workspace, size_t workspace_bytes, void* stream, void* stage_timer_or_null);
 
+/* ---- lens set: one undistortion table per camera ------------------------------------------------------------------------
+ * n_lenses tables of one frame size, each built by mocap_undistort_table_build, lens l at tables_dev + l * lens_stride (one device
+ * allocation).  frame_lens_dev [n_frames] int32: the lens of every frame of a call (device memory, complete on the call's stream);
+ * NULL = lens 0 for every frame.  A frame whose index lies outside [0, n_lenses) gets count 0 and MOCAP_FLAG_LENS_INDEX.
+ * MOCAP_ERR_INVALID: n_lenses < 1, lens_stride < mocap_undistort_table_bytes(H, W) or not a multiple of 256. */
+typedef struct MocapLensSet {
+    const void* tables_dev;
+    int n_lenses;
+    size_t lens_stride;
+    const int32_t* frame_lens_dev;
+} MocapLensSet;
+/* mocap_detect_batch with a lens set in place of table_dev (parity outputs included); mocap_detect_batch is this call with a
+ * one-lens set */
+int mocap_detect_batch_lenses(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                              const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                              int max_blobs, int max_contours, int max_runs,
+                              int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
+                              uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                              double* out_contours, int32_t* out_contour_count,
+                              void* workspace, size_t workspace_bytes, void* stream, void* stage_timer_or_null);
+
 /* ---- overlapped detection (same results as mocap_detect_batch without the parity outputs) ----------------------------
  * The batch is cut into chunks of `chunk_frames` frames (<= 0: one chunk); chunk k's stages (group, piece filter, borders) run as
  * one chain on worker stream k mod n_worker_streams of the pipe.  The streaming scan -- one TMA-fed kernel (cp.async.bulk.tensor +
@@ -129,6 +152,10 @@ int mocap_detect_pipe_set_scan_token(void* pipe, void* wait_event, void* done_ev
  * cellbox_dev [n_frames][ceil(H/32)][ceil(W/32)] (complete on the call's stream before the call; as written by mocap_scan_cells_batch
  * or mocap_bayer_gr2gray_scan_batch for the same frames and thresh) instead.  NULL switches back. */
 int mocap_detect_pipe_set_cellbox(void* pipe, const uint32_t* cellbox_dev);
+/* Lens set (see MocapLensSet, copied; its device arrays must stay valid): the following mocap_detect_batch_pipelined calls of this
+ * pipe undistort every frame with its own lens and take table_dev == NULL (anything else returns MOCAP_ERR_INVALID).  NULL
+ * switches back to table_dev.  Works with handed-in cell boxes, the scatter epilogue and the scan token (the scan reads no table). */
+int mocap_detect_pipe_set_lenses(void* pipe, const MocapLensSet* lenses);
 /* ms since the fork of the last call with record_timeline: [scan done, join] then per chunk [scan seen, grouped, filtered,
  * borders done]; returns the number of floats written, 0 without a timeline */
 int mocap_detect_pipe_timeline(void* pipe, float* ms_out, int cap);

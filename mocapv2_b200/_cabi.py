@@ -12,7 +12,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB = os.path.join(HERE, "libmocap_b200.so")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_CAND = 8
 MAX_CAMS = 16
 CAM_STRIDE = 40
@@ -21,7 +21,8 @@ N_STAGES = 5
 OK = 0
 FLAG_RUN_OVERFLOW, FLAG_BLOB_OVERFLOW, FLAG_CONTOUR_OVERFLOW, FLAG_TILE_OVERFLOW, FLAG_DEPTH_OVERFLOW, FLAG_TRACE_OVERFLOW = 1, 2, 4, 8, 16, 32
 FLAG_GENERAL_PATH = 64          # informational
-FLAG_ERRORS = 1 | 2 | 4 | 8 | 32
+FLAG_LENS_INDEX = 128           # the frame's lens index lies outside the lens set: count 0
+FLAG_ERRORS = 1 | 2 | 4 | 8 | 32 | 128
 CFLAG_GROUP_CAP, CFLAG_CAND_CAP, CFLAG_TIE = 1, 2, 4
 
 _p = C.c_void_p
@@ -29,6 +30,14 @@ _i = C.c_int
 _i64 = C.c_int64
 _sz = C.c_size_t
 _d = C.c_double
+
+
+class LensSet(C.Structure):
+    """MocapLensSet: n_lenses undistortion tables lens_stride bytes apart, frame_lens_dev [n] int32 (or NULL: lens 0)."""
+    _fields_ = [("tables_dev", C.c_void_p), ("n_lenses", C.c_int), ("lens_stride", C.c_size_t), ("frame_lens_dev", C.c_void_p)]
+
+
+_ls = C.POINTER(LensSet)
 
 # name -> (restype, argtypes); mirrors include/mocap_b200.h declaration by declaration
 SIGNATURES = {
@@ -40,6 +49,8 @@ SIGNATURES = {
     "mocap_detect_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i]),
     "mocap_detect_batch": (_i, [_p, _i, _i, _i, _i64, _p, _i, _d, _d, _i, _i, _i,
                                 _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _p]),
+    "mocap_detect_batch_lenses": (_i, [_p, _i, _i, _i, _i64, _ls, _i, _d, _d, _i, _i, _i,
+                                       _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _p]),
     "mocap_stage_timer_create": (_p, []),
     "mocap_stage_timer_destroy": (None, [_p]),
     "mocap_stage_timer_read": (_i, [_p, _p]),
@@ -52,6 +63,7 @@ SIGNATURES = {
     "mocap_detect_pipe_set_scatter": (_i, [_p, _p, _p]),
     "mocap_detect_pipe_set_scan_token": (_i, [_p, _p, _p]),
     "mocap_detect_pipe_set_cellbox": (_i, [_p, _p]),
+    "mocap_detect_pipe_set_lenses": (_i, [_p, _ls]),
     "mocap_detect_pipe_timeline": (_i, [_p, _p, _i]),
     "mocap_detect_pipe_info": (_i, [_p, _p]),
     "mocap_scan_cells_batch": (_i, [_p, _i, _i, _i, _i64, _p, _i, _i, _p, _p, _sz, _p]),

@@ -164,6 +164,26 @@ extern "C" int mocap_filter_batch(const uint8_t* frames_dev, int n_frames, int H
     return launch_materialize_bits(ws, n_frames, H, W, tv, out_bits, s);
 }
 
+// The view of a lens set (MocapLensSet) for frames of H x W
+static int lens_set_view(const MocapLensSet* ls, int H, int W, TableView* tv)
+{
+    if (!ls || !ls->tables_dev || ls->n_lenses < 1) return MOCAP_ERR_INVALID;
+    if (ls->lens_stride < mocap_undistort_table_bytes(H, W) || ls->lens_stride % 256 != 0) return MOCAP_ERR_INVALID;
+    table_view(ls->tables_dev, H, W, tv);
+    tv->lens_words = ls->lens_stride / 4;
+    tv->n_lenses = ls->n_lenses;
+    tv->frame_lens = ls->frame_lens_dev;
+    return MOCAP_OK;
+}
+
+// one table = a set of one lens
+static MocapLensSet one_lens(const void* table_dev, int H, int W)
+{
+    MocapLensSet ls;
+    ls.tables_dev = table_dev; ls.n_lenses = 1; ls.lens_stride = mocap_undistort_table_bytes(H, W); ls.frame_lens_dev = nullptr;
+    return ls;
+}
+
 extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
                                   const void* table_dev, int thresh, double min_area, double min_circ,
                                   int max_blobs, int max_contours, int max_runs,
@@ -172,8 +192,22 @@ extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H
                                   double* out_contours, int32_t* out_contour_count,
                                   void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
 {
+    const MocapLensSet ls = one_lens(table_dev, H, W);
+    return mocap_detect_batch_lenses(frames_dev, n_frames, H, W, frame_stride, &ls, thresh, min_area, min_circ, max_blobs, max_contours,
+                                     max_runs, out_xy, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count,
+                                     out_contours, out_contour_count, workspace, workspace_bytes, stream, stage_timer);
+}
+
+extern "C" int mocap_detect_batch_lenses(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                         const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                         int max_blobs, int max_contours, int max_runs,
+                                         int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
+                                         uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                                         double* out_contours, int32_t* out_contour_count,
+                                         void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
+{
     StageTimer* timer = (StageTimer*)stage_timer;
-    if (!frames_dev || !table_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
+    if (!frames_dev || !lenses || !lenses->tables_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
     if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
     if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
     DetectLayout L;
@@ -181,7 +215,9 @@ extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H
     if (st != MOCAP_OK) return st;
     if (workspace_bytes < L.total) return MOCAP_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
-    TableView tv; table_view(table_dev, H, W, &tv);
+    TableView tv;
+    st = lens_set_view(lenses, H, W, &tv);
+    if (st != MOCAP_OK) return st;
     FilterWs ws = filter_ws((char*)workspace, L);
     CUDA_TRY(cudaMemsetAsync(out_flags, 0, (size_t)n_frames * 4, s));
     if (out_labels) CUDA_TRY(cudaMemsetAsync(out_labels, 0, (size_t)n_frames * H * W * 4, s));
@@ -295,6 +331,7 @@ struct DetectPipe {
     void* tok_wait = nullptr;                       // scan token (mocap_detect_pipe_set_scan_token): cudaEvent_t the scan waits for / records
     void* tok_done = nullptr;
     const uint32_t* pre_cellbox = nullptr;          // hot cell boxes of the next calls' frames, computed by the caller (mocap_detect_pipe_set_cellbox)
+    MocapLensSet lenses = {};                       // lens set of the next calls (mocap_detect_pipe_set_lenses); tables_dev null: none
     cudaStream_t s_scan = nullptr, s_proc[PIPE_MAX_PROC] = {};
     cudaEvent_t ev_fork = nullptr, ev_scan_done = nullptr, ev_proc_done[PIPE_MAX_PROC] = {}, ev_join = nullptr;
     cudaEvent_t ev_scan[PIPE_MAX_CHUNKS] = {};                       // classic scan: chunk c scanned
@@ -349,6 +386,16 @@ extern "C" int mocap_detect_pipe_set_cellbox(void* pipe, const uint32_t* cellbox
     DetectPipe* p = (DetectPipe*)pipe;
     if (!p) return MOCAP_ERR_INVALID;
     p->pre_cellbox = cellbox_dev;
+    return MOCAP_OK;
+}
+
+extern "C" int mocap_detect_pipe_set_lenses(void* pipe, const MocapLensSet* lenses)
+{
+    DetectPipe* p = (DetectPipe*)pipe;
+    if (!p) return MOCAP_ERR_INVALID;
+    if (!lenses) { p->lenses = MocapLensSet(); return MOCAP_OK; }
+    if (!lenses->tables_dev || lenses->n_lenses < 1 || lenses->lens_stride % 256 != 0) return MOCAP_ERR_INVALID;    // (the size: per call)
+    p->lenses = *lenses;
     return MOCAP_OK;
 }
 
@@ -410,7 +457,9 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
                                             void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
 {
     DetectPipe* dp = (DetectPipe*)pipe;
-    if (!dp || !frames_dev || !table_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
+    if (!dp || !frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
+    const bool with_set = dp->lenses.tables_dev != nullptr;
+    if (with_set ? table_dev != nullptr : table_dev == nullptr) return MOCAP_ERR_INVALID;     // a lens set attached: no table_dev
     if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
     if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
     PipeLayout P;
@@ -419,7 +468,10 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
     if (workspace_bytes < P.total) return MOCAP_ERR_WORKSPACE;
     if (!cluster_path_supported(H, W)) return MOCAP_ERR_UNSUPPORTED;         // such shapes take mocap_detect_batch
     cudaStream_t s = (cudaStream_t)stream;
-    TableView tv; table_view(table_dev, H, W, &tv);
+    const MocapLensSet one = one_lens(table_dev, H, W);
+    TableView tv;
+    st = lens_set_view(with_set ? &dp->lenses : &one, H, W, &tv);
+    if (st != MOCAP_OK) return st;
     char* base = (char*)workspace;
     FilterWs ws = filter_ws(base, P.L);
     // hot cell boxes handed in (the Bayer front step computes them while it writes the grey frames): no streaming scan in this call
@@ -464,7 +516,9 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
         }
         if (record_timeline) CUDA_TRY(cudaEventRecord(dp->ev_tl[c][0], ps));
         how.ev_group = dp->ev_tl[c][1]; how.ev_filter = dp->ev_tl[c][2]; how.ev_borders = dp->ev_tl[c][3];
-        st = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, cb, cws, P.cl, need_general + f0,
+        TableView tc = tv;                                                          // the chunk's frames are numbered from 0
+        if (tc.frame_lens) tc.frame_lens += f0;
+        st = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tc, thresh, cb, cws, P.cl, need_general + f0,
                                  max_contours, max_blobs, min_area, min_circ,
                                  out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, out_flags + f0,
                                  out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,

@@ -22,7 +22,7 @@ static inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigne
 #include <stdint.h>
 #include "../../include/mocap_b200.h"
 
-#define MOCAP_ABI_VERSION 3
+#define MOCAP_ABI_VERSION 4
 
 // every kernel launch of the library is counted (mocap_kernel_launch_count: the bench's gpu_launches is read, not estimated)
 extern unsigned long long g_mocap_launches;
@@ -67,6 +67,7 @@ struct TableHeader {
 #define WIN_W 96             // row stride of the staged source window of a filter piece (detect_cluster.cu); the fast map is built for it
 #define FAST_INVALID 0x80000000u
 
+// The arrays of lens 0; lens l's table lies l * lens_words int32 words further (a lens set, MocapLensSet).
 struct TableView {
     const int32_t* map;
     const int32_t* cell;
@@ -75,7 +76,26 @@ struct TableView {
     const int32_t* fast;
     const int32_t* tflag;
     int H, W, TX, TY;
+    size_t lens_words;           // lens_stride / 4 (0 with one table)
+    int n_lenses;
+    const int32_t* frame_lens;   // [n] lens of every frame of the call, or null: lens 0
 };
+
+// Lens of frame f, -1 when its index lies outside [0, n_lenses) (the frame is flagged MOCAP_FLAG_LENS_INDEX and no table is read
+// for it).  Read once per frame, by the kernel that first reads the frame's table.
+__device__ __forceinline__ int frame_lens_of(const TableView& tv, int f)
+{
+    if (!tv.frame_lens) return 0;
+    const int l = tv.frame_lens[f];
+    return (unsigned)l < (unsigned)tv.n_lenses ? l : -1;
+}
+// tv with its arrays moved to lens l's table
+__device__ __forceinline__ TableView lens_table(TableView tv, int l)
+{
+    const size_t o = (size_t)l * tv.lens_words;
+    tv.map += o; tv.cell += o; tv.tile += o; tv.cellinv += o; tv.fast += o; tv.tflag += o;
+    return tv;
+}
 
 // per-stage CUDA events of one mocap_detect_batch call (mocap_stage_timer_*)
 struct StageTimer {

@@ -24,6 +24,9 @@
 #ifndef PF_WIN_L2_PROMO
 #define PF_WIN_L2_PROMO 64      // bytes a window fetch is widened to in L2 (rows are 96 bytes; 64: 0.99 GB of DRAM reads per 1024 frames, 128 or none: 1.30 GB)
 #endif
+#ifndef PF_MAP_EVICT
+#define PF_MAP_EVICT evict_last // L2 priority of the fast-map reads (build-time A/B: evict_normal, see tools/lens_probe.py)
+#endif
 #ifndef BF_THREADS
 #define BF_THREADS 128          // threads of a border CTA (one frame): with fewer threads a lane follows several borders one after the other
 #endif
@@ -101,11 +104,11 @@ __device__ __forceinline__ bool boxes_touch(const int* a, const int* b)
 //   [0] frame            [1] px0 | py0 << 16 (piece origin)
 //   [2] mw | mh << 8 | hl << 16 | hr << 18 | ht << 20 | hb << 22 | packed << 24 | window fits << 25 | fast map usable << 26
 //   [3] word offset of the piece's first bit-row word      [4] words per row | window rows << 16 | 16-byte vectors per row << 24
-//   [5] window origin x (s16) | y << 16
+//   [5] window origin x (s16) | y << 16      [6] lens of the frame (its table lies [6] * lens_words words beyond lens 0's)
 // hl, hr, ht, hb (0 or 2): how far the thresholded-mean box extends beyond the piece; it stops at the cluster box.
 // packed: no frame border within reach of the piece, the tight boxes apply; else the +-4 box with clamped coordinates.
 // window = the source pixels the undistortion of the piece's U box can touch (displacement bounds of the tiles it overlaps).
-__device__ __forceinline__ void make_piece_desc(const TableView& tv, int f, int cx0, int cy0, int cx1, int cy1, int bx, int by,
+__device__ __forceinline__ void make_piece_desc(const TableView& tv, int f, int lens, int cx0, int cy0, int cx1, int cy1, int bx, int by,
                                                 unsigned cluster_rows, int wpr, int* __restrict__ d)
 {
     const int W = tv.W, H = tv.H;
@@ -155,7 +158,7 @@ __device__ __forceinline__ void make_piece_desc(const TableView& tv, int f, int 
     lo.w = (int)(cluster_rows + (unsigned)(py0 - cy0) * (unsigned)wpr + (unsigned)(bx * (PIECE / 32)));
     hi.x = wpr | (wh << 16) | (nvec << 24);
     hi.y = (wx0 & 0xffff) | (wy0 << 16);
-    hi.z = 0; hi.w = 0;
+    hi.z = lens; hi.w = 0;
     *(int4*)d = lo;
     *(int4*)(d + 4) = hi;
 }
@@ -163,12 +166,17 @@ __device__ __forceinline__ void make_piece_desc(const TableView& tv, int f, int 
 // ---------------------------------------------------------------------------------------------------------
 // per frame: hot cells -> clusters (connected components of "output boxes touch") -> cluster table + filter pieces
 // ---------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(CL_THREADS) form_clusters_kernel(const uint32_t* __restrict__ cellbox, TableView tv, ClusterWs cw)
+// The frame's lens is resolved here, once: the cluster entries and piece descriptors carry it to the later stages.
+__global__ void __launch_bounds__(CL_THREADS) form_clusters_kernel(const uint32_t* __restrict__ cellbox, TableView tv_set, ClusterWs cw,
+                                                                   int32_t* __restrict__ out_flags)
 {
     DYN_SHARED(smraw);
     const int f = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
-    const int TX = tv.TX, TY = tv.TY, cells = TX * TY, W = tv.W, H = tv.H;
+    const int TX = tv_set.TX, TY = tv_set.TY, cells = TX * TY, W = tv_set.W, H = tv_set.H;
     if (cw.need_general[f]) return;
+    const int lens = frame_lens_of(tv_set, f);
+    if (lens < 0) { if (tid == 0) out_flags[f] |= MOCAP_FLAG_LENS_INDEX; return; }      // no clusters: the border stage writes count 0
+    const TableView tv = lens_table(tv_set, lens);
     // carve: idx_of[cells] u16 | hot_cell[HOT_MAX] u16 | parent[HOT_MAX] int | box[HOT_MAX][4] short | cbox[HOT_MAX][4] int | roots[ROOTS_MAX] u16
     uint16_t* idx_of = (uint16_t*)smraw;                // dead after the neighbour pass: its memory then holds fill[] and ymax[]
     uint16_t* hot_cell = idx_of + form_idx_slots(cells);
@@ -325,7 +333,7 @@ __global__ void __launch_bounds__(CL_THREADS) form_clusters_kernel(const uint32_
         ce[1] = x0 | (y0 << 16); ce[2] = x1 | (y1 << 16); ce[3] = (int)(roff0 + (unsigned)r_words[i]); ce[4] = pbx * (PIECE / 32);
         ce[5] = cbox[4 * r + 3]; ce[6] = 0; ce[7] = 0;
         for (int q = 0; q < pbx * pby; ++q)
-            make_piece_desc(tv, f, x0, y0, x1, y1, q % pbx, q / pbx, (unsigned)ce[3], ce[4], cw.pieces + 8 * (size_t)(p00 + r_pcs[i] + q));
+            make_piece_desc(tv, f, lens, x0, y0, x1, y1, q % pbx, q / pbx, (unsigned)ce[3], ce[4], cw.pieces + 8 * (size_t)(p00 + r_pcs[i] + q));
     }
     if (tid == 0) {
         cw.frame_clusters[2 * f] = cid0; cw.frame_clusters[2 * f + 1] = bad ? 0 : nr;
@@ -598,7 +606,7 @@ __device__ __forceinline__ FastIter fast_iter_init(const int* d, const TableView
     it.q = tid - it.r * it.nq;
     it.dr = (int)(((unsigned)CL_THREADS * inv) >> 16);
     it.dq = CL_THREADS - it.dr * it.nq;
-    it.mp = tv.fast + (size_t)(py0 - ht - 2 + it.r) * tv.W + (ux0 - lead) + 4 * it.q;
+    it.mp = tv.fast + (size_t)d[6] * tv.lens_words + (size_t)(py0 - ht - 2 + it.r) * tv.W + (ux0 - lead) + 4 * it.q;
     return it;
 }
 
@@ -672,7 +680,9 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
     unsigned wphase = 0;
     uint64_t wpolicy, mpolicy;                                     // L2: the windows are read once (evict first), the fast map by every piece (evict last)
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(wpolicy));
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(mpolicy));
+#define PF_STR2(x) #x
+#define PF_STR(x) PF_STR2(x)
+    asm volatile("createpolicy.fractional.L2::" PF_STR(PF_MAP_EVICT) ".b64 %0, 1.0;" : "=l"(mpolicy));
     if (threadIdx.x == 0 && PF_USE_TMA) {
         mbar_init(&wbar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -759,6 +769,7 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
                 if (fi.q >= fi.nq) { fi.q -= fi.nq; ++fi.r; fi.mp += dmx; pw += dwx; pu += dux; }
             }
         } else {
+            const int32_t* map = tv.map + (size_t)d[6] * tv.lens_words;
             const int n_u = uw * uh;
             const unsigned inv = (1u << 20) / (unsigned)uw + 1u;              // idx / uw == (idx * inv) >> 20 for idx * uw < 2^20
             for (int base = tid; base < n_u; base += 4 * CL_THREADS) {
@@ -769,7 +780,7 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
                     int r = (int)(((unsigned)idx * inv) >> 20), c = idx - r * uw;
                     int i = uy0 + r, j = ux0 + c;
                     ii[k] = i; jj[k] = j; rc[k] = r * UW + c;
-                    m[k] = (idx < n_u && (unsigned)i < (unsigned)H && (unsigned)j < (unsigned)W) ? (uint32_t)tv.map[(size_t)i * W + j] : MAP_OUTSIDE;
+                    m[k] = (idx < n_u && (unsigned)i < (unsigned)H && (unsigned)j < (unsigned)W) ? (uint32_t)map[(size_t)i * W + j] : MAP_OUTSIDE;
                 }
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
@@ -1220,7 +1231,7 @@ int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstr
     if (!attr_done) { CUDA_TRY(cudaFuncSetAttribute(form_clusters_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024)); attr_done = true; }
 #endif
     stage_begin(timer, 1, s);
-    LAUNCH(form_clusters_kernel, n, CL_THREADS, sm_form, s, cellbox, tv, cw);
+    LAUNCH(form_clusters_kernel, n, CL_THREADS, sm_form, s, cellbox, tv, cw, out_flags);
     stage_end(timer, 1, s);
     if (how.ev_group) cudaEventRecord(how.ev_group, s);
     stage_begin(timer, 2, s);

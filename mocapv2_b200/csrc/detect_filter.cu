@@ -247,6 +247,7 @@ int table_view(const void* table_dev, int H, int W, TableView* tv)
     tv->fast = (const int32_t*)(base + h.off_fast);
     tv->tflag = (const int32_t*)(base + h.off_tflag);
     tv->H = H; tv->W = W; tv->TX = h.TX; tv->TY = h.TY;
+    tv->lens_words = 0; tv->n_lenses = 1; tv->frame_lens = nullptr;
     return MOCAP_OK;
 }
 
@@ -445,16 +446,19 @@ __global__ void scan_hot_scalar_kernel(const uint8_t* __restrict__ frames, int n
 }
 
 // general path: the output tiles the hot cells of a flagged frame can reach (one CTA per frame; frames the cluster path
-// finished leave at once)
+// finished leave at once).  A frame whose lens index is out of range marks no tile: nothing downstream reads a table for it.
 __global__ void mark_active_kernel(const uint32_t* __restrict__ cellbox, TableView tv, int n_frames, uint32_t* __restrict__ active, int TXW,
-                                   const int* __restrict__ need_general)
+                                   const int* __restrict__ need_general, int* __restrict__ flags)
 {
     const int cells = tv.TX * tv.TY;
     for (int f = blockIdx.x; f < n_frames; f += gridDim.x) {
         if (need_general && !need_general[f]) continue;
+        const int lens = frame_lens_of(tv, f);
+        if (lens < 0) { if (threadIdx.x == 0) flags[f] |= MOCAP_FLAG_LENS_INDEX; continue; }
+        const TableView tl = lens_table(tv, lens);
         const uint32_t* cb = cellbox + (size_t)f * cells;
         for (int c = threadIdx.x; c < cells; c += blockDim.x)
-            if (cb[c] != CELL_EMPTY) mark_cell(tv, active, f, c / tv.TX, c % tv.TX, TXW);
+            if (cb[c] != CELL_EMPTY) mark_cell(tl, active, f, c / tv.TX, c % tv.TX, TXW);
     }
 }
 
@@ -513,7 +517,9 @@ __global__ void __launch_bounds__(FT_WARPS * 32) filter_tiles_kernel(
         int x0 = tx * TILE, y0 = ty * TILE;
         const uint8_t* fr = frames + (size_t)f * fstride;
         uint32_t* brow = bits + ((size_t)f * H + y0) * TX + tx;
-        const int32_t* tt = tv.tile + 8 * t;
+        const size_t loff = tv.frame_lens ? (size_t)tv.frame_lens[f] * tv.lens_words : 0;     // (checked by mark_active_kernel)
+        const int32_t* tt = tv.tile + loff + 8 * t;
+        const int32_t* map = tv.map + loff;
         int sx0 = tt[0], sy0 = tt[1], sx1 = tt[2], sy1 = tt[3];
         uint32_t myword = 0;
 
@@ -560,7 +566,7 @@ __global__ void __launch_bounds__(FT_WARPS * 32) filter_tiles_kernel(
                             int i = UY0 + r, j = UX0 + c;
                             int u = 0;
                             if ((unsigned)i < (unsigned)H && (unsigned)j < (unsigned)W)
-                                u = remap_px(fr, W, H, i, j, (uint32_t)tv.map[(size_t)i * W + j]);
+                                u = remap_px(fr, W, H, i, j, (uint32_t)map[(size_t)i * W + j]);
                             S.U[(i - (y0 - HALO_U)) * REG_U + (j - (x0 - HALO_U))] = (uint8_t)u;
                         }
                     }
@@ -713,7 +719,7 @@ int launch_tiles(const uint8_t* frames, int n, int /*H*/, int W, int64_t fstride
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     CUDA_TRY(cudaMemsetAsync(ws.active, 0, (size_t)n * TY * TXW * 4, s));
-    LAUNCH(mark_active_kernel, (unsigned)(n < 65535 ? n : 65535), 256, 0, s, ws.cellbox, tv, n, ws.active, TXW, need_general);
+    LAUNCH(mark_active_kernel, (unsigned)(n < 65535 ? n : 65535), 256, 0, s, ws.cellbox, tv, n, ws.active, TXW, need_general, flags);
     long long n_words = (long long)n * TY * TXW;
     LAUNCH(compact_tiles_kernel, (unsigned)((n_words + 255) / 256), 256, 0, s, ws.active, n_words, TX, TY, TXW, ws.list, ws.counters, need_general);
     LAUNCH(filter_tiles_kernel, sms * 4, FT_WARPS * 32, 0, s, frames, fstride, tv, thresh, ws.list, ws.counters, ws.counters + 1,

@@ -63,6 +63,19 @@ class DetectResult:
 
 
 @dataclass
+class LensSet:
+    """Undistortion tables of several lenses for one frame size, `stride` bytes apart in one device allocation (MocapLensSet)."""
+    tables: torch.Tensor             # [n * stride] uint8
+    n: int
+    stride: int
+    H: int
+    W: int
+
+    def cabi(self, frame_lens: torch.Tensor | None) -> _cabi.LensSet:
+        return _cabi.LensSet(self.tables.data_ptr(), self.n, self.stride, frame_lens.data_ptr() if frame_lens is not None else None)
+
+
+@dataclass
 class CorrespondResult:
     obj: torch.Tensor        # [S, max_pts, 3] float64, sorted by mean error, first n_obj valid
     n_obj: torch.Tensor      # [S]
@@ -85,6 +98,7 @@ class CaptureEngine:
 
     def _init_state(self):
         self._tables = {}
+        self._lens_sets = {}
         # _find_dot is called from one thread per camera (RealtimeTracking_FLIR.py:309): every calling thread owns its workspace
         # (and its detection pipe), keyed by the CUDA stream it launches on, so concurrent calls never share scratch memory and
         # need no lock -- the C-ABI keeps no state.  The lock only guards the shared table cache.
@@ -102,6 +116,7 @@ class CaptureEngine:
         other.lib = self.lib
         other._init_state()
         other._tables = self._tables
+        other._lens_sets = self._lens_sets
         other._lock = self._lock                 # one lock for the shared table cache
         other.pipe_workers = self.pipe_workers
         return other
@@ -192,11 +207,16 @@ class CaptureEngine:
         return torch.empty(shape, dtype=dtype, device=self.device)
 
     # ---- undistortion table ---------------------------------------------------------------------------------------------
-    def table(self, K, dist, H: int, W: int) -> torch.Tensor:
+    @staticmethod
+    def _lens_key(K, dist):
         K = np.ascontiguousarray(np.asarray(K, dtype=np.float64).reshape(9))
         d = np.zeros(5, dtype=np.float64)
         dd = np.asarray(dist, dtype=np.float64).ravel()
         d[:min(5, dd.size)] = dd[:5]
+        return K, d
+
+    def table(self, K, dist, H: int, W: int) -> torch.Tensor:
+        K, d = self._lens_key(K, dist)
         key = (K.tobytes(), d.tobytes(), H, W)
         with self._lock:                       # concurrent first calls (one thread per camera) build the table once
             tab = self._tables.get(key)
@@ -211,6 +231,52 @@ class CaptureEngine:
                 self._tables[key] = tab
         return tab
 
+    def lens_set(self, camera_params, H: int, W: int) -> LensSet:
+        """One undistortion table per entry of camera_params ({"intrinsic_matrix", "distortion_coef"} each, the layout of the
+        reference's camera-params.json) in one device allocation: lens i = camera_params[i].  Cached like table()."""
+        lenses = [self._lens_key(cp["intrinsic_matrix"], cp["distortion_coef"]) for cp in camera_params]
+        if not lenses:
+            raise ValueError("a lens set needs at least one lens")
+        key = (tuple(K.tobytes() + d.tobytes() for K, d in lenses), H, W)
+        with self._lock:
+            ls = self._lens_sets.get(key)
+            if ls is None:
+                stride = int(self.lib.mocap_undistort_table_bytes(H, W))          # a multiple of 256
+                if stride == 0:
+                    raise _cabi.MocapError("unsupported frame size")
+                tabs = torch.zeros(len(lenses) * stride, dtype=torch.uint8, device=self.device)
+                with self._device_ctx():
+                    for i, (K, d) in enumerate(lenses):
+                        st = self.lib.mocap_undistort_table_build(K.ctypes.data, d.ctypes.data, H, W,
+                                                                  ctypes.c_void_p(tabs.data_ptr() + i * stride), stride, self._stream())
+                        _cabi.check(self.lib, st, "mocap_undistort_table_build")
+                ls = self._lens_sets[key] = LensSet(tabs, len(lenses), stride, H, W)
+        return ls
+
+    def _frame_lens(self, lenses: LensSet | None, frame_lens, n: int, H: int, W: int):
+        """Checks the lens arguments of a detection call; frame_lens as an int32 device tensor [n] (or None: lens 0)."""
+        if lenses is None:
+            if frame_lens is not None:
+                raise ValueError("frame_lens needs lenses=")
+            return None
+        if (lenses.H, lenses.W) != (H, W):
+            raise ValueError(f"lens set built for {lenses.H}x{lenses.W}, frames are {H}x{W}")
+        if frame_lens is None:
+            return None
+        if not isinstance(frame_lens, torch.Tensor):
+            frame_lens = torch.as_tensor(np.asarray(frame_lens, dtype=np.int32))
+        frame_lens = frame_lens.to(device=self.device, dtype=torch.int32).contiguous()
+        if tuple(frame_lens.shape) != (n,):
+            raise ValueError(f"frame_lens must be [{n}]")
+        return frame_lens
+
+    @staticmethod
+    def _check_lens_args(K, dist, lenses):
+        if lenses is not None and (K is not None or dist is not None):
+            raise ValueError("pass either K / dist or lenses=, not both")
+        if lenses is None and (K is None or dist is None):
+            raise ValueError("K and dist are needed without lenses=")
+
     # ---- detection ----------------------------------------------------------------------------------------------------------
     def default_caps(self, H, W, max_blobs=None, max_contours=None, max_runs=None):
         max_blobs = 256 if max_blobs is None else int(max_blobs)
@@ -218,13 +284,16 @@ class CaptureEngine:
         max_runs = 4 * H + 4096 if max_runs is None else int(max_runs)
         return max_blobs, max_contours, max_runs
 
-    def detect(self, frames: torch.Tensor, K, dist, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
+    def detect(self, frames: torch.Tensor, K=None, dist=None, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
                max_blobs=None, max_contours=None, max_runs=None, outputs=(), out: DetectResult | None = None,
-               timer=None) -> DetectResult:
+               timer=None, lenses: LensSet | None = None, frame_lens=None) -> DetectResult:
         """_find_dot(img)[1] for a batch (lib/ImageOperations.py:33-78).  frames: [n, H, W] uint8 on the device.
 
         outputs: any of "bits", "labels", "blob_sums", "contours" (parity outputs, see include/mocap_b200.h).
+        lenses (from lens_set(), in place of K / dist): frame i is undistorted with lens frame_lens[i] ([n] int, None: lens 0);
+        an index outside the set gives the frame count 0 and FLAG_LENS_INDEX.
         """
+        self._check_lens_args(K, dist, lenses)
         if frames.dim() != 3:
             raise ValueError("frames must be [n, H, W]")
         if frames.device != self.device or frames.dtype != torch.uint8:
@@ -234,7 +303,8 @@ class CaptureEngine:
             frames = frames.contiguous()
         stride = frames.stride(0) if n > 1 else H * W
         max_blobs, max_contours, max_runs = self.default_caps(H, W, max_blobs, max_contours, max_runs)
-        tab = self.table(K, dist, H, W)
+        fl = self._frame_lens(lenses, frame_lens, n, H, W)
+        tab = self.table(K, dist, H, W) if lenses is None else None
         if out is None:
             out = DetectResult(self.empty((n, max_blobs, 2), torch.int32), self.empty((n,), torch.int32),
                                self.empty((n,), torch.int32))
@@ -254,13 +324,19 @@ class CaptureEngine:
         if nbytes == 0:
             raise _cabi.MocapError("mocap_detect_workspace_bytes: unsupported shape")
         ws = self._workspace(nbytes)
-        st = self.lib.mocap_detect_batch(
-            self._ptr(frames), n, H, W, stride, self._ptr(tab), int(thresh), float(min_area), float(min_circ),
-            max_blobs, max_contours, max_runs, self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags),
-            self._ptr(ex.get("bits")), self._ptr(ex.get("labels")), self._ptr(ex.get("blob_sums")),
-            self._ptr(ex.get("blob_count")), self._ptr(ex.get("contours")), self._ptr(ex.get("contour_count")),
-            self._ptr(ws), nbytes, self._stream(), ctypes.c_void_p(timer) if timer else ctypes.c_void_p(0))
-        _cabi.check(self.lib, st, "mocap_detect_batch")
+        args = (int(thresh), float(min_area), float(min_circ),
+                max_blobs, max_contours, max_runs, self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags),
+                self._ptr(ex.get("bits")), self._ptr(ex.get("labels")), self._ptr(ex.get("blob_sums")),
+                self._ptr(ex.get("blob_count")), self._ptr(ex.get("contours")), self._ptr(ex.get("contour_count")),
+                self._ptr(ws), nbytes, self._stream(), ctypes.c_void_p(timer) if timer else ctypes.c_void_p(0))
+        if lenses is None:
+            st = self.lib.mocap_detect_batch(self._ptr(frames), n, H, W, stride, self._ptr(tab), *args)
+            _cabi.check(self.lib, st, "mocap_detect_batch")
+        else:
+            st = self.lib.mocap_detect_batch_lenses(self._ptr(frames), n, H, W, stride, ctypes.byref(lenses.cabi(fl)), *args)
+            _cabi.check(self.lib, st, "mocap_detect_batch_lenses")
+            if fl is not None:
+                self._retire(fl)
         # scan, group, filter pieces, candidates, traces+finalize + the general path's mark / compact / tiles / blobs
         return out
 
@@ -278,12 +354,14 @@ class CaptureEngine:
             pipes[key] = h
         return ctypes.c_void_p(pipes[key])
 
-    def detect_pipelined(self, frames: torch.Tensor, K, dist, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
+    def detect_pipelined(self, frames: torch.Tensor, K=None, dist=None, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
                          max_blobs=None, max_contours=None, max_runs=None, outputs=(), out: DetectResult | None = None,
-                         chunk_frames=128, timeline=False, cellbox: torch.Tensor | None = None) -> DetectResult:
+                         chunk_frames=128, timeline=False, cellbox: torch.Tensor | None = None,
+                         lenses: LensSet | None = None, frame_lens=None) -> DetectResult:
         """Same results as detect() (centroid lists, optionally the contour table), computed chunk by chunk with the streaming
         scan overlapped with the other stages (mocap_detect_batch_pipelined).  cellbox: the frames' hot cell boxes from
-        bayer_gr2gray_scan (same thresh) -- the call then has no streaming scan."""
+        bayer_gr2gray_scan (same thresh) -- the call then has no streaming scan.  lenses / frame_lens as in detect()."""
+        self._check_lens_args(K, dist, lenses)
         if frames.dim() != 3:
             raise ValueError("frames must be [n, H, W]")
         if frames.device != self.device or frames.dtype != torch.uint8:
@@ -295,7 +373,8 @@ class CaptureEngine:
             frames = frames.contiguous()
         stride = frames.stride(0) if n > 1 else H * W
         max_blobs, max_contours, max_runs = self.default_caps(H, W, max_blobs, max_contours, max_runs)
-        tab = self.table(K, dist, H, W)
+        fl = self._frame_lens(lenses, frame_lens, n, H, W)
+        tab = self.table(K, dist, H, W) if lenses is None else None
         if out is None:
             out = DetectResult(self.empty((n, max_blobs, 2), torch.int32), self.empty((n,), torch.int32),
                                self.empty((n,), torch.int32))
@@ -312,6 +391,9 @@ class CaptureEngine:
                 raise ValueError("cellbox must be [n, ceil(H/32), ceil(W/32)]")
             self._check_dev(cellbox, torch.int32, "cellbox")
             _cabi.check(self.lib, self.lib.mocap_detect_pipe_set_cellbox(self._pipe(), self._ptr(cellbox)), "mocap_detect_pipe_set_cellbox")
+        if lenses is not None:
+            _cabi.check(self.lib, self.lib.mocap_detect_pipe_set_lenses(self._pipe(), ctypes.byref(lenses.cabi(fl))),
+                        "mocap_detect_pipe_set_lenses")
         try:
             st = self.lib.mocap_detect_batch_pipelined(
                 self._pipe(), self._ptr(frames), n, H, W, stride, self._ptr(tab), int(thresh), float(min_area), float(min_circ),
@@ -321,6 +403,10 @@ class CaptureEngine:
         finally:
             if cellbox is not None:
                 self.lib.mocap_detect_pipe_set_cellbox(self._pipe(), None)
+            if lenses is not None:
+                self.lib.mocap_detect_pipe_set_lenses(self._pipe(), None)
+                if fl is not None:
+                    self._retire(fl)
         _cabi.check(self.lib, st, "mocap_detect_batch_pipelined")
         info = (ctypes.c_int * 3)()
         self.lib.mocap_detect_pipe_info(self._pipe(), info)

@@ -2,6 +2,7 @@
 
 Same names and conventions as the reference module:
   _find_dot(img, print_location=False, return_filtered=False) -> (img, image_points)   lib/ImageOperations.py:33-78
+    (+ keyword camera_number: undistort with that camera's calibration instead of camera 0's)
   image_filter_gpu(image, camera_number=0)                                             lib/ImageOperations.py:23-31
   module globals `camera_params`, `intrinsics_json`, `cuda_lock` stay assignable.
 All arithmetic runs in libmocap_b200.so on the GPU (undistort + 5x5 floor-mean + threshold + 5x5 majority +
@@ -86,12 +87,13 @@ def _detect_one(eng, fr, K, dist, outputs):
     raise _cabi.MocapError(f"_find_dot: detection capacity exceeded even with caps {caps} (flags {flags})")
 
 
-def _find_dot(img, print_location=False, return_filtered=False):
+def _find_dot(img, print_location=False, return_filtered=False, *, camera_number=None):
     """output: image with dot and dot coordinates -- (img, [[x, y], ...]) or (img, [[None, None]]).
 
-    Undistortion always uses camera 0's calibration, like lib/ImageOperations.py:36-38."""
+    camera_number=None undistorts with camera 0's calibration, like lib/ImageOperations.py:36-38; an integer selects
+    camera_params[camera_number] (the lens of the camera the frame comes from; a short list raises IndexError)."""
     eng = _engine.default_engine()
-    cp = _params()[0]
+    cp = _params()[0 if camera_number is None else camera_number]
     K = np.array(cp["intrinsic_matrix"], dtype=np.float64)
     dist = np.array(cp["distortion_coef"], dtype=np.float64)
     with eng.thread_stream():

@@ -36,7 +36,7 @@ class StepResult:
 
 class CapturePipeline:
     def __init__(self, engine: CaptureEngine, rig: dict, *, max_blobs=160, obj_count=None, max_groups=64, fp64=False,
-                 group=None):
+                 group=None, lens="camera0"):
         self.eng = engine
         self.rig = rig
         self.C = len(rig["poses"])
@@ -52,9 +52,18 @@ class CapturePipeline:
             raise ValueError(f"{self.C} cameras do not shard over {self.world} ranks")
         self.cams_local = self.C // self.world
         self.cam_begin = self.rank * self.cams_local
-        # _find_dot undistorts with camera 0's calibration for every camera (lib/ImageOperations.py:36-38)
+        # lens="camera0": _find_dot undistorts with camera 0's calibration for every camera (lib/ImageOperations.py:36-38).
+        # lens="per_camera": every camera's frames with its own calibration -- a lens set of this rank's cameras, frame i of the
+        # [FS][cams_local] batch takes lens i % cams_local.
+        if lens not in ("camera0", "per_camera"):
+            raise ValueError(f"lens must be 'camera0' or 'per_camera', not {lens!r}")
+        self.lens = lens
         self.K0 = np.asarray(rig["camera_params"][0]["intrinsic_matrix"], dtype=np.float64)
         self.dist0 = np.asarray(rig["camera_params"][0]["distortion_coef"], dtype=np.float64)
+        self.lenses = None
+        self._frame_lens = None                 # cached [n] int32 device tensor of the lens indices
+        if lens == "per_camera":
+            self.lenses = engine.lens_set(rig["camera_params"][self.cam_begin:self.cam_begin + self.cams_local], self.H, self.W)
         self.cams = engine.cameras(rig["poses"], rig["camera_params"])
         self.Fs = torch.from_numpy(np.asarray(rig["Fs"], dtype=np.float64).reshape(-1, 3, 3).copy()).to(engine.device)
         self._det = None
@@ -86,6 +95,14 @@ class CapturePipeline:
             self._rx = None
         return self._det
 
+    def _lens_args(self, n: int):
+        """The lens arguments of a detection call of n frames: K, dist or the lens set with the per-frame indices."""
+        if self.lenses is None:
+            return (self.K0, self.dist0), {}
+        if self._frame_lens is None or self._frame_lens.shape[0] != n:
+            self._frame_lens = (torch.arange(n, dtype=torch.int32) % self.cams_local).to(self.eng.device)
+        return (), {"lenses": self.lenses, "frame_lens": self._frame_lens}
+
     def detect(self, frames: torch.Tensor, timer=None, pipelined=None, timeline=False, cellbox=None) -> DetectResult:
         """frames [FS, cams_local, H, W] uint8 on the device -> centroid lists of this rank's cameras.  cellbox: the frames' hot cell
         boxes from CaptureEngine.bayer_gr2gray_scan (raw sensor input): the overlapped call then runs without its streaming scan."""
@@ -98,6 +115,7 @@ class CapturePipeline:
         if cellbox is not None and not pipelined:
             raise ValueError("cellbox is taken by the overlapped detection call only")
         buf = self._buffers(n)
+        lens_pos, lens_kw = self._lens_args(n)
         buf.extras.pop("peer_turn", None)                          # (set below when this call stores its records to the peers)
         if pipelined:
             self.eng.pipe_workers = self.engine_pipe["workers"]
@@ -109,15 +127,15 @@ class CapturePipeline:
                 peer["turn"] ^= 1
                 self.eng.set_detect_scatter(*peer["tables"][peer["turn"]])
             try:
-                self._det = self.eng.detect_pipelined(flat, self.K0, self.dist0, max_blobs=self.max_blobs, out=buf,
-                                                      chunk_frames=chunk, timeline=timeline, cellbox=cellbox)
+                self._det = self.eng.detect_pipelined(flat, *lens_pos, max_blobs=self.max_blobs, out=buf,
+                                                      chunk_frames=chunk, timeline=timeline, cellbox=cellbox, **lens_kw)
             finally:
                 if peer is not None:
                     self.eng.set_detect_scatter(None, None)
             if peer is not None:
                 self._det.extras["peer_turn"] = peer["turn"]       # the result knows which receive buffers hold its records
         else:
-            self._det = self.eng.detect(flat, self.K0, self.dist0, max_blobs=self.max_blobs, out=buf, timer=timer)
+            self._det = self.eng.detect(flat, *lens_pos, max_blobs=self.max_blobs, out=buf, timer=timer, **lens_kw)
         return self._det
 
     def _peer_setup(self, FS: int):
@@ -220,7 +238,7 @@ class StepsInFlight:
         for _ in range(self.depth - 1):
             eng = pipe.eng.clone()                                 # same library, device and calibration tables
             lane = CapturePipeline(eng, pipe.rig, max_blobs=pipe.max_blobs, obj_count=pipe.obj_count, max_groups=pipe.max_groups,
-                                   fp64=pipe.fp64, group=pipe.group)
+                                   fp64=pipe.fp64, group=pipe.group, lens=pipe.lens)
             lane.pipelined_min_frames = pipe.pipelined_min_frames
             lane.peer_exchange = pipe.peer_exchange
             self.lanes.append(lane)

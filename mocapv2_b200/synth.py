@@ -4,6 +4,8 @@ The frame recipe follows SURVEY.md section 8(d): background uint8 ~ U[0,40), eve
 disc of value 255 with radius U{14..22} px, then a sigma=1.2 Gaussian blur.  Marker centres are the pinhole
 projection of the 3-D marker through K[R|t] followed by the forward distortion model of camera 0, because
 the reference's ``_find_dot`` always undistorts with camera 0's coefficients (lib/ImageOperations.py:37-38).
+A rig built with one lens per camera (``ring_rig(..., lenses=...)``, ``per_camera_lenses``) records that
+(``rig["per_camera_lens"]``); its markers are then projected with every camera's own K and distortion.
 
 ``fundamental_from_poses`` restates CalculateCameraPoses.py:26-78 (F = K2^-T [t]x R K1^-1 for the relative
 pose cam1 -> cam2); it is how jsons/fundamentals.json is produced, needed for rigs with more than 2 cameras.
@@ -93,12 +95,40 @@ def _rot_a_to_b(a, b):
     return np.eye(3) + vx + vx @ vx / (1 + c)
 
 
-def ring_rig(n_cams, W, H, radius=6.0, K=None, dist=None, height=0.8):
+def per_camera_lenses(n_cams, seed=SEED0, scale=1.0):
+    """n_cams distinct lenses around the shipped one, [(K, dist), ...]: focal lengths within +-3 %, principal point within +-2 %
+    of the frame size of the shipped calibration (2048 px), distortion coefficients within +-15 % (times `scale`).  Camera 0 keeps
+    the shipped lens."""
+    rng = np.random.default_rng(seed)
+    out = [(np.array(SHIPPED_K, dtype=np.float64), np.array(SHIPPED_DIST, dtype=np.float64))]
+    for _ in range(1, n_cams):
+        K = np.array(SHIPPED_K, dtype=np.float64)
+        K[0, 0] *= 1 + scale * rng.uniform(-0.03, 0.03)
+        K[1, 1] *= 1 + scale * rng.uniform(-0.03, 0.03)
+        K[0, 2] += scale * rng.uniform(-40.0, 40.0)
+        K[1, 2] += scale * rng.uniform(-40.0, 40.0)
+        d = np.array(SHIPPED_DIST, dtype=np.float64) * (1 + scale * rng.uniform(-0.15, 0.15, 5))
+        out.append((K, d))
+    return out
+
+
+def camera_lens(rig, c):
+    """(K, dist) the frames of camera c are distorted with: its own with per-camera lenses, camera 0's otherwise."""
+    cp = rig["camera_params"][c if rig.get("per_camera_lens") else 0]
+    return cp["intrinsic_matrix"], cp["distortion_coef"]
+
+
+def ring_rig(n_cams, W, H, radius=6.0, K=None, dist=None, height=0.8, lenses=None):
     """n_cams cameras on a ring looking at the origin so that the origin projects to the image centre.
 
     Camera 0 is re-based to R = I, t = 0 like the reference's calibration (CalculateCameraPoses.py) does, i.e.
     world coordinates are camera-0 coordinates.  Returns dict(camera_params, poses, Fs, W, H, centre).
+    lenses: [(K_i, dist_i)] one per camera (in place of K / dist): the rig's frames are distorted per camera.
     """
+    if lenses is not None:
+        if len(lenses) != n_cams:
+            raise ValueError("one lens per camera")
+        K, dist = lenses[0]
     K = np.array(SHIPPED_K if K is None else K, dtype=np.float64)
     dist = list(SHIPPED_DIST if dist is None else dist)
     ray_c = np.linalg.inv(K) @ np.array([W / 2.0, H / 2.0, 1.0])
@@ -123,9 +153,14 @@ def ring_rig(n_cams, W, H, radius=6.0, K=None, dist=None, height=0.8):
         t = tw - R @ t0w
         poses.append({"R": R, "t": t})
     centre = R0w @ np.zeros(3) + t0w                        # the ring centre in camera-0 coordinates
-    cams = [{"intrinsic_matrix": K.tolist(), "distortion_coef": dist} for _ in range(n_cams)]
-    Fs = [fundamental_from_poses(poses[0], poses[i], K, K).tolist() for i in range(1, n_cams)]
-    return {"camera_params": cams, "poses": poses, "Fs": Fs, "W": W, "H": H, "centre": centre}
+    if lenses is None:
+        cams = [{"intrinsic_matrix": K.tolist(), "distortion_coef": dist} for _ in range(n_cams)]
+        Fs = [fundamental_from_poses(poses[0], poses[i], K, K).tolist() for i in range(1, n_cams)]
+        return {"camera_params": cams, "poses": poses, "Fs": Fs, "W": W, "H": H, "centre": centre}
+    Ks = [np.asarray(k, dtype=np.float64) for k, _ in lenses]
+    cams = [{"intrinsic_matrix": k.tolist(), "distortion_coef": list(np.asarray(d, dtype=np.float64))} for k, (_, d) in zip(Ks, lenses)]
+    Fs = [fundamental_from_poses(poses[0], poses[i], Ks[0], Ks[i]).tolist() for i in range(1, n_cams)]
+    return {"camera_params": cams, "poses": poses, "Fs": Fs, "W": W, "H": H, "centre": centre, "per_camera_lens": True}
 
 
 def shipped_rig(W=640, H=480):
@@ -137,8 +172,7 @@ def shipped_rig(W=640, H=480):
 
 def sample_markers(rig, n_markers, rng, spread=0.45, min_sep_px=56.0, margin=40.0, tries=200):
     """3-D marker positions (camera-0 coordinates) visible in every view; best-effort pixel separation."""
-    K = rig["camera_params"][0]["intrinsic_matrix"]
-    dist = rig["camera_params"][0]["distortion_coef"]
+    lens = [camera_lens(rig, c) for c in range(len(rig["poses"]))]
     W, H = rig["W"], rig["H"]
     out = []
     proj = []
@@ -146,7 +180,7 @@ def sample_markers(rig, n_markers, rng, spread=0.45, min_sep_px=56.0, margin=40.
         best = None
         for k in range(tries):
             X = rig["centre"] + rng.uniform(-spread, spread, 3)
-            uv = np.stack([project_distorted(X, p, K, dist)[0] for p in rig["poses"]])
+            uv = np.stack([project_distorted(X, p, *lens[c])[0] for c, p in enumerate(rig["poses"])])
             if (uv[:, 0] < margin).any() or (uv[:, 0] > W - margin).any() or \
                (uv[:, 1] < margin).any() or (uv[:, 1] > H - margin).any():
                 continue
@@ -167,9 +201,7 @@ def sample_markers(rig, n_markers, rng, spread=0.45, min_sep_px=56.0, margin=40.
 
 def marker_pixels(rig, X):
     """(C, M, 2) float64 ideal (distorted) pixel centres of markers X (M,3)."""
-    K = rig["camera_params"][0]["intrinsic_matrix"]
-    dist = rig["camera_params"][0]["distortion_coef"]
-    return np.stack([project_distorted(X, p, K, dist) for p in rig["poses"]])
+    return np.stack([project_distorted(X, p, *camera_lens(rig, c)) for c, p in enumerate(rig["poses"])])
 
 
 def gaussian_kernel1d(sigma=1.2):
