@@ -7,8 +7,9 @@
  *
  * Conventions: every *_dev pointer is device memory owned by the caller (torch tensors in the Python host
  * layer); `stream` is a cudaStream_t passed as void*; all calls are asynchronous on that stream, allocate
- * nothing, keep no global state and are re-entrant.  Return value: MOCAP_OK or a negative status; per-frame /
- * per-frame-set problems (capacity overflows) are reported in the flags arrays, not in the return value.
+ * nothing, keep no global state and are re-entrant.  Everything a call reads is in its arguments: a handle (stage timer, detection
+ * pipe) owns CUDA streams and events and remembers what its last call ran, nothing more.  Return value: MOCAP_OK or a negative
+ * status; per-frame / per-frame-set problems (capacity overflows) are reported in the flags arrays, not in the return value.
  */
 #ifndef MOCAP_B200_H
 #define MOCAP_B200_H
@@ -79,6 +80,20 @@ int mocap_undistort_table_build(const double* K9_host, const double* dist5_host,
  */
 size_t mocap_detect_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs);
 
+/* ---- lens set: one undistortion table per camera ------------------------------------------------------------------------
+ * n_lenses tables of one frame size, each built by mocap_undistort_table_build, lens l at tables_dev + l * lens_stride (one device
+ * allocation).  frame_lens_dev [n_frames] int32: the lens of every frame of a call (device memory, complete on the call's stream);
+ * NULL = lens 0 for every frame.  A frame whose index lies outside [0, n_lenses) gets count 0 and MOCAP_FLAG_LENS_INDEX.
+ * One table is the set {table_dev, 1, mocap_undistort_table_bytes(H, W), NULL}.  A call reads the structure before it returns; the
+ * device arrays must stay valid until its kernels have run.  MOCAP_ERR_INVALID: a NULL set or tables_dev, n_lenses < 1,
+ * lens_stride < mocap_undistort_table_bytes(H, W) or not a multiple of 256. */
+typedef struct MocapLensSet {
+    const void* tables_dev;
+    int n_lenses;
+    size_t lens_stride;
+    const int32_t* frame_lens_dev;
+} MocapLensSet;
+
 /* Optional per-stage device timing of mocap_detect_batch (bench.py's roofline line): a timer owns CUDA events that
  * the call records around its kernels on `stream`; read it after the stream has been synchronised.  Stages:
  * 0 scan (streams every source byte), 1 group (hot cells -> clusters -> 64x64 filter pieces), 2 filter (remap + floor-mean
@@ -91,33 +106,12 @@ void mocap_stage_timer_destroy(void* timer);
 int mocap_stage_timer_read(void* timer, float* ms_out);
 const char* mocap_stage_name(int stage);
 int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                       const void* table_dev, int thresh, double min_area, double min_circ,
+                       const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
                        int max_blobs, int max_contours, int max_runs,
                        int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
                        uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
                        double* out_contours, int32_t* out_contour_count,
                        void* workspace, size_t workspace_bytes, void* stream, void* stage_timer_or_null);
-
-/* ---- lens set: one undistortion table per camera ------------------------------------------------------------------------
- * n_lenses tables of one frame size, each built by mocap_undistort_table_build, lens l at tables_dev + l * lens_stride (one device
- * allocation).  frame_lens_dev [n_frames] int32: the lens of every frame of a call (device memory, complete on the call's stream);
- * NULL = lens 0 for every frame.  A frame whose index lies outside [0, n_lenses) gets count 0 and MOCAP_FLAG_LENS_INDEX.
- * MOCAP_ERR_INVALID: n_lenses < 1, lens_stride < mocap_undistort_table_bytes(H, W) or not a multiple of 256. */
-typedef struct MocapLensSet {
-    const void* tables_dev;
-    int n_lenses;
-    size_t lens_stride;
-    const int32_t* frame_lens_dev;
-} MocapLensSet;
-/* mocap_detect_batch with a lens set in place of table_dev (parity outputs included); mocap_detect_batch is this call with a
- * one-lens set */
-int mocap_detect_batch_lenses(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                              const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
-                              int max_blobs, int max_contours, int max_runs,
-                              int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
-                              uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
-                              double* out_contours, int32_t* out_contour_count,
-                              void* workspace, size_t workspace_bytes, void* stream, void* stage_timer_or_null);
 
 /* ---- overlapped detection (same results as mocap_detect_batch without the parity outputs) ----------------------------
  * The batch is cut into chunks of `chunk_frames` frames (<= 0: one chunk); chunk k's stages (group, piece filter, borders) run as
@@ -125,43 +119,38 @@ int mocap_detect_batch_lenses(const uint8_t* frames_dev, int n_frames, int H, in
  * mbarrier ring in shared memory, one small CTA per SM) over the whole batch on the pipe's high-priority scan stream -- runs
  * beside the stages of the chunks it has already finished, which wait for its per-chunk flag with a stream memory operation.
  * Frames the TMA unit cannot describe (rows or frame stride not a multiple of 16 bytes, thresh outside 0..254), or a driver
- * without stream memory operations, take the classic scan kernels chunk by chunk, handed over with events; with cell boxes handed in (mocap_detect_pipe_set_cellbox) there is no
- * scan.  A pipe owns those streams and events: create one per caller thread, keep it for the life of the engine; a call is
- * asynchronous on `stream` like every other entry point (fork / join with events).  record_timeline != 0 keeps the call's
- * timeline for mocap_detect_pipe_timeline.  Frame sizes the per-cluster units do not support return MOCAP_ERR_UNSUPPORTED
- * (use mocap_detect_batch). */
+ * without stream memory operations, take the classic scan kernels chunk by chunk, handed over with events; with cell boxes handed in
+ * there is no scan.  A pipe owns those streams and events and remembers what its last call ran: create one per caller thread, keep it
+ * for the life of the engine; a call is asynchronous on `stream` like every other entry point (fork / join with events).
+ * record_timeline != 0 keeps the call's timeline for mocap_detect_pipe_timeline.  Frame sizes the per-cluster units do not support
+ * return MOCAP_ERR_UNSUPPORTED (use mocap_detect_batch).
+ * Optional inputs of a call (NULL: not used):
+ *   cellbox_dev [n_frames][ceil(H/32)][ceil(W/32)]: the frames' hot cell boxes, complete on `stream` before the call, as written by
+ *     mocap_scan_cells_batch or mocap_bayer_gr2gray_scan_batch for the same frames and thresh.  The call then runs no streaming scan.
+ *   xy_dst_dev, count_dst_dev [n_frames] device addresses (both or neither; one without the other is MOCAP_ERR_INVALID): the
+ *     store-to-peer epilogue (multi-GPU).  Every frame's record is ALSO copied -- chunk by chunk, behind the chunk's border stage --
+ *     to xy_dst[f] (its centroids, int32 pairs) and count_dst[f] (its count): addresses in the receive buffer of the rank that
+ *     matches the frame's frame-set, mapped into this process (symmetric memory over NVLink).  The exchange step is then a barrier.
+ *   scan_wait_event, scan_done_event (cudaEvent_t owned by the caller): the scan token of several pipes in flight on one GPU
+ *     (pipeline.StepsInFlight).  The call's streaming scan waits for scan_wait_event and records scan_done_event behind it.
+ *     Chained from call to call across the pipes, the HBM-bound scans run one after the other instead of side by side: one ring
+ *     of TMA boxes per SM instead of two. */
 void* mocap_detect_pipe_create(int n_worker_streams);
 void mocap_detect_pipe_destroy(void* pipe);
 size_t mocap_detect_pipelined_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs, int chunk_frames);
 int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                 const void* table_dev, int thresh, double min_area, double min_circ,
+                                 const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
                                  int max_blobs, int max_contours, int max_runs,
                                  int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
                                  double* out_contours, int32_t* out_contour_count,
+                                 const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
+                                 void* scan_wait_event, void* scan_done_event,
                                  void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline);
-/* Store-to-peer epilogue (multi-GPU): with per-frame destination addresses set (device arrays [n_frames] of pointers, valid for the
- * following calls of this pipe; NULL, NULL switches it off) every frame's record is ALSO copied -- chunk by chunk, behind the chunk's
- * border stage -- to xy_dst[f] (its centroids, int32 pairs) and count_dst[f] (its count): addresses in the receive buffer of the rank that
- * matches the frame's frame-set, mapped into this process (symmetric memory over NVLink).  The exchange step is then a barrier. */
-int mocap_detect_pipe_set_scatter(void* pipe, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev);
-/* Scan token (several pipes in flight on one GPU, pipeline.StepsInFlight): the following calls of this pipe let their streaming scan wait
- * for `wait_event` and record `done_event` behind it (cudaEvent_t handles owned by the caller, NULL = none).  Chained from call to call
- * across the pipes, the HBM-bound scans run one after the other instead of side by side: one ring of TMA boxes per SM instead of two. */
-int mocap_detect_pipe_set_scan_token(void* pipe, void* wait_event, void* done_event);
-/* Hot cell boxes from the caller: the following mocap_detect_batch_pipelined calls of this pipe skip their streaming scan and take
- * cellbox_dev [n_frames][ceil(H/32)][ceil(W/32)] (complete on the call's stream before the call; as written by mocap_scan_cells_batch
- * or mocap_bayer_gr2gray_scan_batch for the same frames and thresh) instead.  NULL switches back. */
-int mocap_detect_pipe_set_cellbox(void* pipe, const uint32_t* cellbox_dev);
-/* Lens set (see MocapLensSet, copied; its device arrays must stay valid): the following mocap_detect_batch_pipelined calls of this
- * pipe undistort every frame with its own lens and take table_dev == NULL (anything else returns MOCAP_ERR_INVALID).  NULL
- * switches back to table_dev.  Works with handed-in cell boxes, the scatter epilogue and the scan token (the scan reads no table). */
-int mocap_detect_pipe_set_lenses(void* pipe, const MocapLensSet* lenses);
 /* ms since the fork of the last call with record_timeline: [scan done, join] then per chunk [scan seen, grouped, filtered,
  * borders done]; returns the number of floats written, 0 without a timeline */
 int mocap_detect_pipe_timeline(void* pipe, float* ms_out, int cap);
-/* what the last call ran: out3 = {scan kernel (1 TMA ring, 0 classic or none), chunks, sync mode (1 the workers waited on the TMA
- * scan's chunk flags, 0 on events or on nothing)} */
-int mocap_detect_pipe_info(void* pipe, int* out3);
+/* what the last call ran: out2 = {scan kernel (1 TMA ring: the workers waited on its chunk flags; 0 classic scan or none), chunks} */
+int mocap_detect_pipe_info(void* pipe, int* out2);
 
 /* stage entry points of the same path (used by the parity tests and the bench's per-kernel timing) */
 /* the streaming scan alone: cellbox_out [n][ceil(H/32)][ceil(W/32)] hot bounding box of every 32x32 source cell
@@ -197,9 +186,9 @@ int mocap_median5_threshold_batch(const uint8_t* frames_dev, int n_frames, int H
  * (RealtimeTracking_FLIR.py:103-104), fused: raw u8 [n][H][W] -> grey u8 [n][H][W].  H, W >= 3. */
 int mocap_bayer_gr2gray_batch(const uint8_t* raw_dev, int n_frames, int H, int W, uint8_t* out_dev, void* stream);
 /* The same front step, which also delivers what the streaming scan of the detection would compute from the grey frames it writes:
- * cellbox_out [n][ceil(H/32)][ceil(W/32)] as mocap_scan_cells_batch (the grey bytes are tested while they are in registers).  Handed to
- * mocap_detect_pipe_set_cellbox, the detection of raw sensor frames (RealtimeTracking_FLIR.py:103-105) reads every frame byte once
- * less.  workspace >= n * ceil(H/32) * ceil(W/32) * 8 bytes. */
+ * cellbox_out [n][ceil(H/32)][ceil(W/32)] as mocap_scan_cells_batch (the grey bytes are tested while they are in registers).  Passed as
+ * cellbox_dev of mocap_detect_batch_pipelined, the detection of raw sensor frames (RealtimeTracking_FLIR.py:103-105) reads every frame
+ * byte once less.  workspace >= n * ceil(H/32) * ceil(W/32) * 8 bytes. */
 int mocap_bayer_gr2gray_scan_batch(const uint8_t* raw_dev, int n_frames, int H, int W, uint8_t* out_dev, int thresh,
                                    uint32_t* cellbox_out, void* workspace, size_t workspace_bytes, void* stream);
 /* cv.undistort alone (lib/ImageOperations.py:38), for stage parity */

@@ -164,7 +164,7 @@ extern "C" int mocap_filter_batch(const uint8_t* frames_dev, int n_frames, int H
     return launch_materialize_bits(ws, n_frames, H, W, tv, out_bits, s);
 }
 
-// The view of a lens set (MocapLensSet) for frames of H x W
+// The view of a lens set (MocapLensSet) for frames of H x W: the whole set is checked here, by every call that takes one
 static int lens_set_view(const MocapLensSet* ls, int H, int W, TableView* tv)
 {
     if (!ls || !ls->tables_dev || ls->n_lenses < 1) return MOCAP_ERR_INVALID;
@@ -176,48 +176,26 @@ static int lens_set_view(const MocapLensSet* ls, int H, int W, TableView* tv)
     return MOCAP_OK;
 }
 
-// one table = a set of one lens
-static MocapLensSet one_lens(const void* table_dev, int H, int W)
-{
-    MocapLensSet ls;
-    ls.tables_dev = table_dev; ls.n_lenses = 1; ls.lens_stride = mocap_undistort_table_bytes(H, W); ls.frame_lens_dev = nullptr;
-    return ls;
-}
-
 extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                  const void* table_dev, int thresh, double min_area, double min_circ,
+                                  const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
                                   int max_blobs, int max_contours, int max_runs,
                                   int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
                                   uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
                                   double* out_contours, int32_t* out_contour_count,
                                   void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
 {
-    const MocapLensSet ls = one_lens(table_dev, H, W);
-    return mocap_detect_batch_lenses(frames_dev, n_frames, H, W, frame_stride, &ls, thresh, min_area, min_circ, max_blobs, max_contours,
-                                     max_runs, out_xy, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count,
-                                     out_contours, out_contour_count, workspace, workspace_bytes, stream, stage_timer);
-}
-
-extern "C" int mocap_detect_batch_lenses(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                         const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
-                                         int max_blobs, int max_contours, int max_runs,
-                                         int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
-                                         uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
-                                         double* out_contours, int32_t* out_contour_count,
-                                         void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
-{
     StageTimer* timer = (StageTimer*)stage_timer;
-    if (!frames_dev || !lenses || !lenses->tables_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
+    if (!frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
     if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
     if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
     DetectLayout L;
     int st = detect_layout(n_frames, H, W, max_contours, max_runs, true, &L);
     if (st != MOCAP_OK) return st;
-    if (workspace_bytes < L.total) return MOCAP_ERR_WORKSPACE;
-    cudaStream_t s = (cudaStream_t)stream;
     TableView tv;
     st = lens_set_view(lenses, H, W, &tv);
     if (st != MOCAP_OK) return st;
+    if (workspace_bytes < L.total) return MOCAP_ERR_WORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream;
     FilterWs ws = filter_ws((char*)workspace, L);
     CUDA_TRY(cudaMemsetAsync(out_flags, 0, (size_t)n_frames * 4, s));
     if (out_labels) CUDA_TRY(cudaMemsetAsync(out_labels, 0, (size_t)n_frames * H * W * 4, s));
@@ -283,7 +261,7 @@ extern "C" int mocap_blobs_batch(const uint32_t* bits_dev, int n_frames, int H, 
 // Overlapped detection: the batch is cut into chunks of frames; the HBM-bound streaming scan of chunk k+1 runs
 // beside the instruction-bound stages (group / piece filter / borders) of chunk k on the same SMs.  Chunk k's stages run as
 // one chain on worker stream k mod workers.  The scan follows from the input:
-//   cell boxes handed in (mocap_detect_pipe_set_cellbox): no scan.
+//   cell boxes handed in (cellbox_dev): no scan.
 //   frames a tensor map can describe, and stream memory operations available: ONE TMA-fed scan kernel over the whole batch
 //     on the pipe's high-priority scan stream; it publishes a flag per finished chunk, which the chunk's worker stream waits
 //     for with cuStreamWaitValue32 -- the scan CTA of an SM stays resident from the first byte to the last.
@@ -325,13 +303,8 @@ static int launch_scatter(const int32_t* xy, const int32_t* count, const unsigne
     return MOCAP_OK;
 }
 
+// A pipe owns streams and events and remembers what its last call ran; everything a call reads is in its arguments.
 struct DetectPipe {
-    const unsigned long long* sc_xy = nullptr;      // per-frame destinations of the store-to-peer epilogue (device arrays [n]), or null
-    const unsigned long long* sc_count = nullptr;
-    void* tok_wait = nullptr;                       // scan token (mocap_detect_pipe_set_scan_token): cudaEvent_t the scan waits for / records
-    void* tok_done = nullptr;
-    const uint32_t* pre_cellbox = nullptr;          // hot cell boxes of the next calls' frames, computed by the caller (mocap_detect_pipe_set_cellbox)
-    MocapLensSet lenses = {};                       // lens set of the next calls (mocap_detect_pipe_set_lenses); tables_dev null: none
     cudaStream_t s_scan = nullptr, s_proc[PIPE_MAX_PROC] = {};
     cudaEvent_t ev_fork = nullptr, ev_scan_done = nullptr, ev_proc_done[PIPE_MAX_PROC] = {}, ev_join = nullptr;
     cudaEvent_t ev_scan[PIPE_MAX_CHUNKS] = {};                       // classic scan: chunk c scanned
@@ -361,42 +334,6 @@ extern "C" void* mocap_detect_pipe_create(int n_proc_streams)
     }
     if (!ok) { delete p; return nullptr; }
     return p;
-}
-
-extern "C" int mocap_detect_pipe_set_scatter(void* pipe, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev)
-{
-    DetectPipe* p = (DetectPipe*)pipe;
-    if (!p || ((xy_dst_dev == nullptr) != (count_dst_dev == nullptr))) return MOCAP_ERR_INVALID;
-    p->sc_xy = (const unsigned long long*)xy_dst_dev;
-    p->sc_count = (const unsigned long long*)count_dst_dev;
-    return MOCAP_OK;
-}
-
-extern "C" int mocap_detect_pipe_set_scan_token(void* pipe, void* wait_event, void* done_event)
-{
-    DetectPipe* p = (DetectPipe*)pipe;
-    if (!p) return MOCAP_ERR_INVALID;
-    p->tok_wait = wait_event;
-    p->tok_done = done_event;
-    return MOCAP_OK;
-}
-
-extern "C" int mocap_detect_pipe_set_cellbox(void* pipe, const uint32_t* cellbox_dev)
-{
-    DetectPipe* p = (DetectPipe*)pipe;
-    if (!p) return MOCAP_ERR_INVALID;
-    p->pre_cellbox = cellbox_dev;
-    return MOCAP_OK;
-}
-
-extern "C" int mocap_detect_pipe_set_lenses(void* pipe, const MocapLensSet* lenses)
-{
-    DetectPipe* p = (DetectPipe*)pipe;
-    if (!p) return MOCAP_ERR_INVALID;
-    if (!lenses) { p->lenses = MocapLensSet(); return MOCAP_OK; }
-    if (!lenses->tables_dev || lenses->n_lenses < 1 || lenses->lens_stride % 256 != 0) return MOCAP_ERR_INVALID;    // (the size: per call)
-    p->lenses = *lenses;
-    return MOCAP_OK;
 }
 
 extern "C" void mocap_detect_pipe_destroy(void* pipe)
@@ -450,33 +387,35 @@ extern "C" size_t mocap_detect_pipelined_workspace_bytes(int n_frames, int H, in
 }
 
 extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                            const void* table_dev, int thresh, double min_area, double min_circ,
+                                            const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
                                             int max_blobs, int max_contours, int max_runs,
                                             int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
                                             double* out_contours, int32_t* out_contour_count,
+                                            const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
+                                            void* scan_wait_event, void* scan_done_event,
                                             void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
 {
     DetectPipe* dp = (DetectPipe*)pipe;
     if (!dp || !frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
-    const bool with_set = dp->lenses.tables_dev != nullptr;
-    if (with_set ? table_dev != nullptr : table_dev == nullptr) return MOCAP_ERR_INVALID;     // a lens set attached: no table_dev
+    if ((xy_dst_dev == nullptr) != (count_dst_dev == nullptr)) return MOCAP_ERR_INVALID;
     if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
     if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
     PipeLayout P;
     int st = pipe_layout(n_frames, H, W, max_contours, max_runs, chunk_frames, &P);
     if (st != MOCAP_OK) return st;
+    TableView tv;
+    st = lens_set_view(lenses, H, W, &tv);
+    if (st != MOCAP_OK) return st;
     if (workspace_bytes < P.total) return MOCAP_ERR_WORKSPACE;
     if (!cluster_path_supported(H, W)) return MOCAP_ERR_UNSUPPORTED;         // such shapes take mocap_detect_batch
     cudaStream_t s = (cudaStream_t)stream;
-    const MocapLensSet one = one_lens(table_dev, H, W);
-    TableView tv;
-    st = lens_set_view(with_set ? &dp->lenses : &one, H, W, &tv);
-    if (st != MOCAP_OK) return st;
+    const unsigned long long* sc_xy = (const unsigned long long*)xy_dst_dev;
+    const unsigned long long* sc_count = (const unsigned long long*)count_dst_dev;
     char* base = (char*)workspace;
     FilterWs ws = filter_ws(base, P.L);
     // hot cell boxes handed in (the Bayer front step computes them while it writes the grey frames): no streaming scan in this call
-    const bool prescanned = dp->pre_cellbox != nullptr;
-    if (prescanned) ws.cellbox = (uint32_t*)dp->pre_cellbox;
+    const bool prescanned = cellbox_dev != nullptr;
+    if (prescanned) ws.cellbox = (uint32_t*)cellbox_dev;
     int* ctrl = (int*)(base + P.off_ctrl);
     int* need_general = (int*)(base + P.off_need);
     const int chunks = P.chunks, cf = P.chunk_frames;
@@ -492,7 +431,7 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
     CUDA_TRY(cudaMemsetAsync(ctrl, 0, scan_tma_ctrl_bytes(chunks), s));
     CUDA_TRY(cudaEventRecord(dp->ev_fork, s));
     CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, dp->ev_fork, 0));
-    if (dp->tok_wait) CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, (cudaEvent_t)dp->tok_wait, 0));    // scans of several pipes one after the other
+    if (scan_wait_event) CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, (cudaEvent_t)scan_wait_event, 0));    // scans of several pipes one after the other
     if (tma) {
         st = launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, ctrl, chunks, cf, dp->s_scan);
         if (st != MOCAP_OK) return st;
@@ -524,13 +463,13 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
                                  out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,
                                  ps, nullptr, how);
         if (st != MOCAP_OK) return st;
-        if (dp->sc_xy) {                                     // the chunk's records go where their consumers read them, off the critical path
-            st = launch_scatter(out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, dp->sc_xy + f0, dp->sc_count + f0, nc, max_blobs, need_general + f0, 0, ps);
+        if (sc_xy) {                                         // the chunk's records go where their consumers read them, off the critical path
+            st = launch_scatter(out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, sc_xy + f0, sc_count + f0, nc, max_blobs, need_general + f0, 0, ps);
             if (st != MOCAP_OK) return st;
         }
     }
     CUDA_TRY(cudaEventRecord(dp->ev_scan_done, dp->s_scan));
-    if (dp->tok_done) CUDA_TRY(cudaEventRecord((cudaEvent_t)dp->tok_done, dp->s_scan));
+    if (scan_done_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)scan_done_event, dp->s_scan));
     CUDA_TRY(cudaStreamWaitEvent(s, dp->ev_scan_done, 0));
     for (int i = 0; i < dp->n_proc; ++i) {
         CUDA_TRY(cudaEventRecord(dp->ev_proc_done[i], dp->s_proc[i]));
@@ -543,7 +482,7 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
     st = launch_blobs(ws.bits, ws.fg_tiles, ws.n_fg, n_frames, H, W, P.L.TX, P.L.max_fg, max_runs, max_blobs, max_contours,
                       min_area, min_circ, base + P.L.off_blob, P.L.blob_stride,
                       out_xy, out_count, out_flags, nullptr, nullptr, out_contours, out_contour_count, nullptr, need_general, s);
-    if (st == MOCAP_OK && dp->sc_xy) st = launch_scatter(out_xy, out_count, dp->sc_xy, dp->sc_count, n_frames, max_blobs, need_general, 1, s);
+    if (st == MOCAP_OK && sc_xy) st = launch_scatter(out_xy, out_count, sc_xy, sc_count, n_frames, max_blobs, need_general, 1, s);
     return st;
 }
 
@@ -566,13 +505,13 @@ extern "C" int mocap_detect_pipe_timeline(void* pipe, float* ms_out, int cap)
     return need;
 }
 
-// what the last pipelined call actually ran: [0] scan kernel (1 = TMA ring, 0 = classic or none), [1] chunks, [2] sync mode
-// (1 = the workers waited on the TMA scan's chunk flags, 0 = on events or on nothing: always equal to [0])
-extern "C" int mocap_detect_pipe_info(void* pipe, int* out3)
+// what the last pipelined call actually ran: [0] scan kernel (1 = TMA ring, the workers waited on its chunk flags; 0 = classic or
+// none), [1] chunks
+extern "C" int mocap_detect_pipe_info(void* pipe, int* out2)
 {
     DetectPipe* dp = (DetectPipe*)pipe;
-    if (!dp || !out3) return MOCAP_ERR_INVALID;
-    out3[0] = dp->last_tma; out3[1] = dp->last_chunks; out3[2] = dp->last_tma;
+    if (!dp || !out2) return MOCAP_ERR_INVALID;
+    out2[0] = dp->last_tma; out2[1] = dp->last_chunks;
     return MOCAP_OK;
 }
 

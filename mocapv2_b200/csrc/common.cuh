@@ -22,7 +22,7 @@ static inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigne
 #include <stdint.h>
 #include "../../include/mocap_b200.h"
 
-#define MOCAP_ABI_VERSION 4
+#define MOCAP_ABI_VERSION 5
 
 // every kernel launch of the library is counted (mocap_kernel_launch_count: the bench's gpu_launches is read, not estimated)
 extern unsigned long long g_mocap_launches;

@@ -64,7 +64,8 @@ class DetectResult:
 
 @dataclass
 class LensSet:
-    """Undistortion tables of several lenses for one frame size, `stride` bytes apart in one device allocation (MocapLensSet)."""
+    """Undistortion tables of one or more lenses for one frame size, `stride` bytes apart in one device allocation (MocapLensSet).
+    With one lens, `tables` is that lens's table."""
     tables: torch.Tensor             # [n * stride] uint8
     n: int
     stride: int
@@ -97,8 +98,7 @@ class CaptureEngine:
         self._init_state()
 
     def _init_state(self):
-        self._tables = {}
-        self._lens_sets = {}
+        self._tables = {}                       # (lenses, H, W) -> LensSet; table() is the one-lens entry
         # _find_dot is called from one thread per camera (RealtimeTracking_FLIR.py:309): every calling thread owns its workspace
         # (and its detection pipe), keyed by the CUDA stream it launches on, so concurrent calls never share scratch memory and
         # need no lock -- the C-ABI keeps no state.  The lock only guards the shared table cache.
@@ -116,7 +116,6 @@ class CaptureEngine:
         other.lib = self.lib
         other._init_state()
         other._tables = self._tables
-        other._lens_sets = self._lens_sets
         other._lock = self._lock                 # one lock for the shared table cache
         other.pipe_workers = self.pipe_workers
         return other
@@ -215,31 +214,12 @@ class CaptureEngine:
         d[:min(5, dd.size)] = dd[:5]
         return K, d
 
-    def table(self, K, dist, H: int, W: int) -> torch.Tensor:
-        K, d = self._lens_key(K, dist)
-        key = (K.tobytes(), d.tobytes(), H, W)
-        with self._lock:                       # concurrent first calls (one thread per camera) build the table once
-            tab = self._tables.get(key)
-            if tab is None:
-                nbytes = self.lib.mocap_undistort_table_bytes(H, W)
-                if nbytes == 0:
-                    raise _cabi.MocapError("unsupported frame size")
-                tab = torch.zeros(int(nbytes), dtype=torch.uint8, device=self.device)
-                with self._device_ctx():
-                    st = self.lib.mocap_undistort_table_build(K.ctypes.data, d.ctypes.data, H, W, self._ptr(tab), nbytes, self._stream())
-                _cabi.check(self.lib, st, "mocap_undistort_table_build")
-                self._tables[key] = tab
-        return tab
-
-    def lens_set(self, camera_params, H: int, W: int) -> LensSet:
-        """One undistortion table per entry of camera_params ({"intrinsic_matrix", "distortion_coef"} each, the layout of the
-        reference's camera-params.json) in one device allocation: lens i = camera_params[i].  Cached like table()."""
-        lenses = [self._lens_key(cp["intrinsic_matrix"], cp["distortion_coef"]) for cp in camera_params]
-        if not lenses:
-            raise ValueError("a lens set needs at least one lens")
+    def _lens_set(self, lenses, H: int, W: int) -> LensSet:
+        """The tables of lenses [(K, d), ...] (as _lens_key returns them) in one device allocation, lens i at i * stride; built once
+        per list of lenses and frame size."""
         key = (tuple(K.tobytes() + d.tobytes() for K, d in lenses), H, W)
-        with self._lock:
-            ls = self._lens_sets.get(key)
+        with self._lock:                       # concurrent first calls (one thread per camera) build the tables once
+            ls = self._tables.get(key)
             if ls is None:
                 stride = int(self.lib.mocap_undistort_table_bytes(H, W))          # a multiple of 256
                 if stride == 0:
@@ -250,32 +230,19 @@ class CaptureEngine:
                         st = self.lib.mocap_undistort_table_build(K.ctypes.data, d.ctypes.data, H, W,
                                                                   ctypes.c_void_p(tabs.data_ptr() + i * stride), stride, self._stream())
                         _cabi.check(self.lib, st, "mocap_undistort_table_build")
-                ls = self._lens_sets[key] = LensSet(tabs, len(lenses), stride, H, W)
+                ls = self._tables[key] = LensSet(tabs, len(lenses), stride, H, W)
         return ls
 
-    def _frame_lens(self, lenses: LensSet | None, frame_lens, n: int, H: int, W: int):
-        """Checks the lens arguments of a detection call; frame_lens as an int32 device tensor [n] (or None: lens 0)."""
-        if lenses is None:
-            if frame_lens is not None:
-                raise ValueError("frame_lens needs lenses=")
-            return None
-        if (lenses.H, lenses.W) != (H, W):
-            raise ValueError(f"lens set built for {lenses.H}x{lenses.W}, frames are {H}x{W}")
-        if frame_lens is None:
-            return None
-        if not isinstance(frame_lens, torch.Tensor):
-            frame_lens = torch.as_tensor(np.asarray(frame_lens, dtype=np.int32))
-        frame_lens = frame_lens.to(device=self.device, dtype=torch.int32).contiguous()
-        if tuple(frame_lens.shape) != (n,):
-            raise ValueError(f"frame_lens must be [{n}]")
-        return frame_lens
+    def table(self, K, dist, H: int, W: int) -> torch.Tensor:
+        return self._lens_set([self._lens_key(K, dist)], H, W).tables
 
-    @staticmethod
-    def _check_lens_args(K, dist, lenses):
-        if lenses is not None and (K is not None or dist is not None):
-            raise ValueError("pass either K / dist or lenses=, not both")
-        if lenses is None and (K is None or dist is None):
-            raise ValueError("K and dist are needed without lenses=")
+    def lens_set(self, camera_params, H: int, W: int) -> LensSet:
+        """One undistortion table per entry of camera_params ({"intrinsic_matrix", "distortion_coef"} each, the layout of the
+        reference's camera-params.json) in one device allocation: lens i = camera_params[i].  Cached like table()."""
+        lenses = [self._lens_key(cp["intrinsic_matrix"], cp["distortion_coef"]) for cp in camera_params]
+        if not lenses:
+            raise ValueError("a lens set needs at least one lens")
+        return self._lens_set(lenses, H, W)
 
     # ---- detection ----------------------------------------------------------------------------------------------------------
     def default_caps(self, H, W, max_blobs=None, max_contours=None, max_runs=None):
@@ -283,6 +250,50 @@ class CaptureEngine:
         max_contours = max(2 * max_blobs, 512) if max_contours is None else int(max_contours)
         max_runs = 4 * H + 4096 if max_runs is None else int(max_runs)
         return max_blobs, max_contours, max_runs
+
+    def _detect_prologue(self, frames, K, dist, lenses, frame_lens, caps, outputs, out):
+        """What both detection calls check and prepare: contiguous frames and their stride, the caps, the lens set (K / dist: the
+        one-lens set of its table) with the per-frame indices as an int32 device tensor [n] (or None: lens 0), and the outputs."""
+        if lenses is not None and (K is not None or dist is not None):
+            raise ValueError("pass either K / dist or lenses=, not both")
+        if lenses is None and (K is None or dist is None):
+            raise ValueError("K and dist are needed without lenses=")
+        if frames.dim() != 3:
+            raise ValueError("frames must be [n, H, W]")
+        if frames.device != self.device or frames.dtype != torch.uint8:
+            raise ValueError(f"frames must be uint8 on {self.device}")
+        n, H, W = frames.shape
+        if frames.stride(2) != 1 or frames.stride(1) != W:
+            frames = frames.contiguous()
+        stride = frames.stride(0) if n > 1 else H * W
+        max_blobs, max_contours, max_runs = caps = self.default_caps(H, W, *caps)
+        if lenses is None:
+            if frame_lens is not None:
+                raise ValueError("frame_lens needs lenses=")
+            lenses = self._lens_set([self._lens_key(K, dist)], H, W)
+        elif (lenses.H, lenses.W) != (H, W):
+            raise ValueError(f"lens set built for {lenses.H}x{lenses.W}, frames are {H}x{W}")
+        if frame_lens is not None:
+            if not isinstance(frame_lens, torch.Tensor):
+                frame_lens = torch.as_tensor(np.asarray(frame_lens, dtype=np.int32))
+            frame_lens = frame_lens.to(device=self.device, dtype=torch.int32).contiguous()
+            if tuple(frame_lens.shape) != (n,):
+                raise ValueError(f"frame_lens must be [{n}]")
+        if out is None:
+            out = DetectResult(self.empty((n, max_blobs, 2), torch.int32), self.empty((n,), torch.int32),
+                               self.empty((n,), torch.int32))
+        ex = out.extras
+        if "bits" in outputs and "bits" not in ex:
+            ex["bits"] = self.empty((n, H, (W + 31) // 32), torch.int32)
+        if "labels" in outputs and "labels" not in ex:
+            ex["labels"] = self.empty((n, H, W), torch.int32)
+        if "blob_sums" in outputs and "blob_sums" not in ex:
+            ex["blob_sums"] = torch.zeros((n, max_blobs, 3), dtype=torch.int64, device=self.device)
+            ex["blob_count"] = self.empty((n,), torch.int32)
+        if "contours" in outputs and "contours" not in ex:
+            ex["contours"] = torch.zeros((n, max_contours, 8), dtype=torch.float64, device=self.device)
+            ex["contour_count"] = self.empty((n,), torch.int32)
+        return frames, stride, caps, lenses, frame_lens, out
 
     def detect(self, frames: torch.Tensor, K=None, dist=None, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
                max_blobs=None, max_contours=None, max_runs=None, outputs=(), out: DetectResult | None = None,
@@ -293,50 +304,23 @@ class CaptureEngine:
         lenses (from lens_set(), in place of K / dist): frame i is undistorted with lens frame_lens[i] ([n] int, None: lens 0);
         an index outside the set gives the frame count 0 and FLAG_LENS_INDEX.
         """
-        self._check_lens_args(K, dist, lenses)
-        if frames.dim() != 3:
-            raise ValueError("frames must be [n, H, W]")
-        if frames.device != self.device or frames.dtype != torch.uint8:
-            raise ValueError(f"frames must be uint8 on {self.device}")
+        frames, stride, caps, lenses, fl, out = self._detect_prologue(frames, K, dist, lenses, frame_lens,
+                                                                      (max_blobs, max_contours, max_runs), outputs, out)
         n, H, W = frames.shape
-        if frames.stride(2) != 1 or frames.stride(1) != W:
-            frames = frames.contiguous()
-        stride = frames.stride(0) if n > 1 else H * W
-        max_blobs, max_contours, max_runs = self.default_caps(H, W, max_blobs, max_contours, max_runs)
-        fl = self._frame_lens(lenses, frame_lens, n, H, W)
-        tab = self.table(K, dist, H, W) if lenses is None else None
-        if out is None:
-            out = DetectResult(self.empty((n, max_blobs, 2), torch.int32), self.empty((n,), torch.int32),
-                               self.empty((n,), torch.int32))
         ex = out.extras
-        TX = (W + 31) // 32
-        if "bits" in outputs and "bits" not in ex:
-            ex["bits"] = self.empty((n, H, TX), torch.int32)
-        if "labels" in outputs and "labels" not in ex:
-            ex["labels"] = self.empty((n, H, W), torch.int32)
-        if "blob_sums" in outputs and "blob_sums" not in ex:
-            ex["blob_sums"] = torch.zeros((n, max_blobs, 3), dtype=torch.int64, device=self.device)
-            ex["blob_count"] = self.empty((n,), torch.int32)
-        if "contours" in outputs and "contours" not in ex:
-            ex["contours"] = torch.zeros((n, max_contours, 8), dtype=torch.float64, device=self.device)
-            ex["contour_count"] = self.empty((n,), torch.int32)
-        nbytes = self.lib.mocap_detect_workspace_bytes(n, H, W, max_blobs, max_contours, max_runs)
+        nbytes = self.lib.mocap_detect_workspace_bytes(n, H, W, *caps)
         if nbytes == 0:
             raise _cabi.MocapError("mocap_detect_workspace_bytes: unsupported shape")
         ws = self._workspace(nbytes)
-        args = (int(thresh), float(min_area), float(min_circ),
-                max_blobs, max_contours, max_runs, self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags),
-                self._ptr(ex.get("bits")), self._ptr(ex.get("labels")), self._ptr(ex.get("blob_sums")),
-                self._ptr(ex.get("blob_count")), self._ptr(ex.get("contours")), self._ptr(ex.get("contour_count")),
-                self._ptr(ws), nbytes, self._stream(), ctypes.c_void_p(timer) if timer else ctypes.c_void_p(0))
-        if lenses is None:
-            st = self.lib.mocap_detect_batch(self._ptr(frames), n, H, W, stride, self._ptr(tab), *args)
-            _cabi.check(self.lib, st, "mocap_detect_batch")
-        else:
-            st = self.lib.mocap_detect_batch_lenses(self._ptr(frames), n, H, W, stride, ctypes.byref(lenses.cabi(fl)), *args)
-            _cabi.check(self.lib, st, "mocap_detect_batch_lenses")
-            if fl is not None:
-                self._retire(fl)
+        st = self.lib.mocap_detect_batch(
+            self._ptr(frames), n, H, W, stride, ctypes.byref(lenses.cabi(fl)), int(thresh), float(min_area), float(min_circ), *caps,
+            self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags),
+            self._ptr(ex.get("bits")), self._ptr(ex.get("labels")), self._ptr(ex.get("blob_sums")),
+            self._ptr(ex.get("blob_count")), self._ptr(ex.get("contours")), self._ptr(ex.get("contour_count")),
+            self._ptr(ws), nbytes, self._stream(), ctypes.c_void_p(timer) if timer else ctypes.c_void_p(0))
+        _cabi.check(self.lib, st, "mocap_detect_batch")
+        if fl is not None:
+            self._retire(fl)
         # scan, group, filter pieces, candidates, traces+finalize + the general path's mark / compact / tiles / blobs
         return out
 
@@ -357,32 +341,20 @@ class CaptureEngine:
     def detect_pipelined(self, frames: torch.Tensor, K=None, dist=None, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
                          max_blobs=None, max_contours=None, max_runs=None, outputs=(), out: DetectResult | None = None,
                          chunk_frames=128, timeline=False, cellbox: torch.Tensor | None = None,
-                         lenses: LensSet | None = None, frame_lens=None) -> DetectResult:
+                         lenses: LensSet | None = None, frame_lens=None, scatter=None, scan_token=None) -> DetectResult:
         """Same results as detect() (centroid lists, optionally the contour table), computed chunk by chunk with the streaming
         scan overlapped with the other stages (mocap_detect_batch_pipelined).  cellbox: the frames' hot cell boxes from
-        bayer_gr2gray_scan (same thresh) -- the call then has no streaming scan.  lenses / frame_lens as in detect()."""
-        self._check_lens_args(K, dist, lenses)
-        if frames.dim() != 3:
-            raise ValueError("frames must be [n, H, W]")
-        if frames.device != self.device or frames.dtype != torch.uint8:
-            raise ValueError(f"frames must be uint8 on {self.device}")
+        bayer_gr2gray_scan (same thresh) -- the call then has no streaming scan.  lenses / frame_lens as in detect().
+        scatter=(xy_dst, count_dst): per-frame destination addresses (int64 device tensors [n]) of the store-to-peer epilogue.
+        scan_token=(wait, done): torch.cuda.Event objects (recorded at least once, or None) the call's streaming scan waits for and
+        records behind it; StepsInFlight chains the scans of its lanes this way."""
         if any(o != "contours" for o in outputs):
             raise ValueError("detect_pipelined offers the contour table only; use detect() for bits / labels / blob_sums")
+        frames, stride, caps, lenses, fl, out = self._detect_prologue(frames, K, dist, lenses, frame_lens,
+                                                                      (max_blobs, max_contours, max_runs), outputs, out)
         n, H, W = frames.shape
-        if frames.stride(2) != 1 or frames.stride(1) != W:
-            frames = frames.contiguous()
-        stride = frames.stride(0) if n > 1 else H * W
-        max_blobs, max_contours, max_runs = self.default_caps(H, W, max_blobs, max_contours, max_runs)
-        fl = self._frame_lens(lenses, frame_lens, n, H, W)
-        tab = self.table(K, dist, H, W) if lenses is None else None
-        if out is None:
-            out = DetectResult(self.empty((n, max_blobs, 2), torch.int32), self.empty((n,), torch.int32),
-                               self.empty((n,), torch.int32))
         ex = out.extras
-        if "contours" in outputs and "contours" not in ex:
-            ex["contours"] = torch.zeros((n, max_contours, 8), dtype=torch.float64, device=self.device)
-            ex["contour_count"] = self.empty((n,), torch.int32)
-        nbytes = self.lib.mocap_detect_pipelined_workspace_bytes(n, H, W, max_blobs, max_contours, max_runs, int(chunk_frames))
+        nbytes = self.lib.mocap_detect_pipelined_workspace_bytes(n, H, W, *caps, int(chunk_frames))
         if nbytes == 0:
             raise _cabi.MocapError("mocap_detect_pipelined_workspace_bytes: unsupported shape")
         ws = self._workspace(nbytes)
@@ -390,47 +362,25 @@ class CaptureEngine:
             if tuple(cellbox.shape) != (n, (H + 31) // 32, (W + 31) // 32):
                 raise ValueError("cellbox must be [n, ceil(H/32), ceil(W/32)]")
             self._check_dev(cellbox, torch.int32, "cellbox")
-            _cabi.check(self.lib, self.lib.mocap_detect_pipe_set_cellbox(self._pipe(), self._ptr(cellbox)), "mocap_detect_pipe_set_cellbox")
-        if lenses is not None:
-            _cabi.check(self.lib, self.lib.mocap_detect_pipe_set_lenses(self._pipe(), ctypes.byref(lenses.cabi(fl))),
-                        "mocap_detect_pipe_set_lenses")
-        try:
-            st = self.lib.mocap_detect_batch_pipelined(
-                self._pipe(), self._ptr(frames), n, H, W, stride, self._ptr(tab), int(thresh), float(min_area), float(min_circ),
-                max_blobs, max_contours, max_runs, self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags),
-                self._ptr(ex.get("contours")), self._ptr(ex.get("contour_count")), self._ptr(ws), nbytes, self._stream(),
-                int(chunk_frames), 1 if timeline else 0)
-        finally:
-            if cellbox is not None:
-                self.lib.mocap_detect_pipe_set_cellbox(self._pipe(), None)
-            if lenses is not None:
-                self.lib.mocap_detect_pipe_set_lenses(self._pipe(), None)
-                if fl is not None:
-                    self._retire(fl)
+        xy_dst, count_dst = scatter if scatter is not None else (None, None)
+        for t in (xy_dst, count_dst):
+            if t is not None:
+                self._check_dev(t, torch.int64, "scatter")
+        wait, done = scan_token if scan_token is not None else (None, None)
+        ev = lambda e: ctypes.c_void_p(int(e.cuda_event)) if e is not None else ctypes.c_void_p(0)
+        st = self.lib.mocap_detect_batch_pipelined(
+            self._pipe(), self._ptr(frames), n, H, W, stride, ctypes.byref(lenses.cabi(fl)), int(thresh), float(min_area), float(min_circ),
+            *caps, self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags), self._ptr(ex.get("contours")),
+            self._ptr(ex.get("contour_count")), self._ptr(cellbox), self._ptr(xy_dst), self._ptr(count_dst), ev(wait), ev(done),
+            self._ptr(ws), nbytes, self._stream(), int(chunk_frames), 1 if timeline else 0)
         _cabi.check(self.lib, st, "mocap_detect_batch_pipelined")
-        info = (ctypes.c_int * 3)()
+        for t in (fl, xy_dst, count_dst):
+            if t is not None:
+                self._retire(t)
+        info = (ctypes.c_int * 2)()
         self.lib.mocap_detect_pipe_info(self._pipe(), info)
-        self.last_pipe_info = {"tma_scan": bool(info[0]), "chunks": int(info[1]), "sync_mode": int(info[2])}
+        self.last_pipe_info = {"tma_scan": bool(info[0]), "chunks": int(info[1]), "sync_mode": int(info[0])}
         return out
-
-    def set_detect_scatter(self, xy_dst: torch.Tensor | None, count_dst: torch.Tensor | None):
-        """Per-frame destination addresses (int64 device tensors [n]) of the store-to-peer epilogue of detect_pipelined, for the
-        calling thread's pipe; None, None switches it off (include/mocap_b200.h, mocap_detect_pipe_set_scatter)."""
-        if xy_dst is not None:
-            xy_dst = self._check_dev(xy_dst, torch.int64, "xy_dst")
-            count_dst = self._check_dev(count_dst, torch.int64, "count_dst")
-        self._tls.scatter = (xy_dst, count_dst)                  # keeps the tables alive
-        _cabi.check(self.lib, self.lib.mocap_detect_pipe_set_scatter(self._pipe(), self._ptr(xy_dst), self._ptr(count_dst)),
-                    "mocap_detect_pipe_set_scatter")
-
-    def set_scan_token(self, wait_event=None, done_event=None):
-        """The following detect_pipelined calls of the calling thread let their streaming scan wait for `wait_event` and record
-        `done_event` behind it (torch.cuda.Event objects that have been recorded at least once, or None): StepsInFlight chains the
-        scans of its lanes this way (include/mocap_b200.h, mocap_detect_pipe_set_scan_token)."""
-        self._tls.scan_token = (wait_event, done_event)          # keeps the events alive
-        h = lambda e: ctypes.c_void_p(int(e.cuda_event)) if e is not None else ctypes.c_void_p(0)
-        _cabi.check(self.lib, self.lib.mocap_detect_pipe_set_scan_token(self._pipe(), h(wait_event), h(done_event)),
-                    "mocap_detect_pipe_set_scan_token")
 
     def pipe_timeline(self):
         """ms since the fork of the last detect_pipelined(timeline=True): {"scan_done", "join", "chunks": [[seen, grouped, filtered, borders], ...]}"""

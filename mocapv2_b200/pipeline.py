@@ -12,7 +12,7 @@ kernels on the step path.  No floating-point reduction crosses ranks, so N-rank 
 On a GPU box with peer access (NVLink / NVSwitch) the exchange needs no collective at all: the receive buffers live in
 torch symmetric memory, every rank maps its peers' buffers, and the overlapped detection call stores each frame's record
 straight into the slot of the rank that matches its frame-set, chunk by chunk behind the chunk's border stage
-(`mocap_detect_pipe_set_scatter`: store-to-peer epilogue).  The exchange step is then one symmetric-memory barrier; two
+(`detect_pipelined(scatter=...)`: store-to-peer epilogue).  The exchange step is then one symmetric-memory barrier; two
 receive buffers alternate so that a rank may already store step t + 1 while a peer still matches step t.
 """
 from __future__ import annotations
@@ -96,12 +96,12 @@ class CapturePipeline:
         return self._det
 
     def _lens_args(self, n: int):
-        """The lens arguments of a detection call of n frames: K, dist or the lens set with the per-frame indices."""
+        """The lens keyword arguments of a detection call of n frames: K, dist or the lens set with the per-frame indices."""
         if self.lenses is None:
-            return (self.K0, self.dist0), {}
+            return {"K": self.K0, "dist": self.dist0}
         if self._frame_lens is None or self._frame_lens.shape[0] != n:
             self._frame_lens = (torch.arange(n, dtype=torch.int32) % self.cams_local).to(self.eng.device)
-        return (), {"lenses": self.lenses, "frame_lens": self._frame_lens}
+        return {"lenses": self.lenses, "frame_lens": self._frame_lens}
 
     def detect(self, frames: torch.Tensor, timer=None, pipelined=None, timeline=False, cellbox=None) -> DetectResult:
         """frames [FS, cams_local, H, W] uint8 on the device -> centroid lists of this rank's cameras.  cellbox: the frames' hot cell
@@ -115,27 +115,21 @@ class CapturePipeline:
         if cellbox is not None and not pipelined:
             raise ValueError("cellbox is taken by the overlapped detection call only")
         buf = self._buffers(n)
-        lens_pos, lens_kw = self._lens_args(n)
+        lens_kw = self._lens_args(n)
         buf.extras.pop("peer_turn", None)                          # (set below when this call stores its records to the peers)
         if pipelined:
             self.eng.pipe_workers = self.engine_pipe["workers"]
-            if self.scan_token is not None:
-                self.eng.set_scan_token(*self.scan_token)
             chunk = -(-n // self.engine_pipe["chunks"])
             peer = self._peer_setup(FS) if (self.world > 1 and self.peer_exchange) else None
             if peer is not None:
                 peer["turn"] ^= 1
-                self.eng.set_detect_scatter(*peer["tables"][peer["turn"]])
-            try:
-                self._det = self.eng.detect_pipelined(flat, *lens_pos, max_blobs=self.max_blobs, out=buf,
-                                                      chunk_frames=chunk, timeline=timeline, cellbox=cellbox, **lens_kw)
-            finally:
-                if peer is not None:
-                    self.eng.set_detect_scatter(None, None)
+            self._det = self.eng.detect_pipelined(flat, max_blobs=self.max_blobs, out=buf, chunk_frames=chunk, timeline=timeline,
+                                                  cellbox=cellbox, scatter=peer["tables"][peer["turn"]] if peer is not None else None,
+                                                  scan_token=self.scan_token, **lens_kw)
             if peer is not None:
                 self._det.extras["peer_turn"] = peer["turn"]       # the result knows which receive buffers hold its records
         else:
-            self._det = self.eng.detect(flat, *lens_pos, max_blobs=self.max_blobs, out=buf, timer=timer, **lens_kw)
+            self._det = self.eng.detect(flat, max_blobs=self.max_blobs, out=buf, timer=timer, **lens_kw)
         return self._det
 
     def _peer_setup(self, FS: int):

@@ -1,4 +1,5 @@
-"""Detection with a lens set: one undistortion table per camera in one call (mocap_detect_batch_lenses, mocap_detect_pipe_set_lenses).
+"""Detection with a lens set: one undistortion table per camera in one call (MocapLensSet in mocap_detect_batch and
+mocap_detect_batch_pipelined).
 
 Every frame of a batch that mixes lenses must give exactly what the single-table call gives with that frame's K / dist, and what
 the oracle gives; a set of copies of one table must give the single-table call bit for bit; a lens index outside the set flags
@@ -117,7 +118,7 @@ def test_pipelined_lens_set_equals_one_shot(engine):
                                       cellbox=cb)
         for i in range(n):
             same_frame(got, i, want, i)
-    # the pipe is back on table_dev after the lens-set calls
+    # a K / dist call on the same pipe after the lens-set calls undistorts with its own table
     K, D = LENSES[0]
     plain = engine.detect_pipelined(fr, K, D, min_area=MIN_AREA, chunk_frames=3)
     one = engine.detect(fr, K, D, min_area=MIN_AREA)
@@ -180,7 +181,9 @@ def test_lens_index_outside_the_set_flags_the_frame(engine, outputs):
     assert any(want.points(i) != [[None, None]] for i in (1, 3))    # the flagged frames do hold blobs
 
 
-def test_lens_set_argument_errors(engine):
+def test_both_calls_check_the_lens_set_argument(engine):
+    """Both detection calls check the whole lens set they are given: zero lenses, a stride below the table size or not a multiple
+    of 256, NULL tables and a NULL set are invalid arguments."""
     lib = engine.lib
     n = 2
     frames = dev(engine, scene(35, n))
@@ -190,40 +193,27 @@ def test_lens_set_argument_errors(engine):
     mb, mc, mr = engine.default_caps(H, W)
     out = [engine.empty((n, mb, 2), torch.int32), engine.empty((n,), torch.int32), engine.empty((n,), torch.int32)]
     nbytes = lib.mocap_detect_workspace_bytes(n, H, W, mb, mc, mr)
-    ws = engine._workspace(nbytes)
+    pn = lib.mocap_detect_pipelined_workspace_bytes(n, H, W, mb, mc, mr, 1)
+    ws = engine._workspace(max(pn, nbytes))
     P = engine._ptr
     null = ctypes.c_void_p(0)
+    ref = lambda lset: ctypes.byref(lset) if lset is not None else None
 
     def one_shot(lset):
-        return lib.mocap_detect_batch_lenses(P(frames), n, H, W, H * W, ctypes.byref(lset) if lset is not None else None, 216, 30.0, 0.5,
-                                             mb, mc, mr, P(out[0]), P(out[1]), P(out[2]), null, null, null, null, null, null,
-                                             P(ws), nbytes, engine._stream(), null)
+        return lib.mocap_detect_batch(P(frames), n, H, W, H * W, ref(lset), 216, 30.0, 0.5, mb, mc, mr, P(out[0]), P(out[1]), P(out[2]),
+                                      null, null, null, null, null, null, P(ws), nbytes, engine._stream(), null)
+
+    def piped(lset):
+        return lib.mocap_detect_batch_pipelined(engine._pipe(), P(frames), n, H, W, H * W, ref(lset), 216, 30.0, 0.5, mb, mc, mr,
+                                                P(out[0]), P(out[1]), P(out[2]), null, null, null, null, null, null, null,
+                                                P(ws), pn, engine._stream(), 1, 0)
 
     base = ls.tables.data_ptr()
-    assert one_shot(_cabi.LensSet(base, 2, tb, None)) == _cabi.OK
-    for bad in (_cabi.LensSet(base, 0, tb, None), _cabi.LensSet(base, 2, tb - 256, None), _cabi.LensSet(base, 2, tb + 16, None),
-                _cabi.LensSet(None, 2, tb, None)):
-        assert one_shot(bad) == -1
-        assert lib.mocap_detect_pipe_set_lenses(engine._pipe(), ctypes.byref(bad)) == (_cabi.OK if bad.lens_stride == tb - 256 else -1)
-    assert one_shot(None) == -1
-    # pipelined: a set whose stride is below the table size is refused by the call, table_dev with a set attached too
-    pn = lib.mocap_detect_pipelined_workspace_bytes(n, H, W, mb, mc, mr, 1)
-    pws = engine._workspace(max(pn, nbytes))
-    tab = engine.table(*LENSES[0], H, W)
-
-    def piped(table):
-        return lib.mocap_detect_batch_pipelined(engine._pipe(), P(frames), n, H, W, H * W, table, 216, 30.0, 0.5, mb, mc, mr,
-                                                P(out[0]), P(out[1]), P(out[2]), null, null, P(pws), pn, engine._stream(), 1, 0)
-
-    pipe = engine._pipe()
-    assert lib.mocap_detect_pipe_set_lenses(pipe, ctypes.byref(_cabi.LensSet(base, 2, tb - 256, None))) == _cabi.OK
-    assert piped(null) == -1
-    assert lib.mocap_detect_pipe_set_lenses(pipe, ctypes.byref(_cabi.LensSet(base, 2, tb, None))) == _cabi.OK
-    assert piped(P(tab)) == -1
-    assert piped(null) == _cabi.OK
-    assert lib.mocap_detect_pipe_set_lenses(pipe, None) == _cabi.OK            # detached: table_dev again
-    assert piped(null) == -1
-    assert piped(P(tab)) == _cabi.OK
+    for call in (one_shot, piped):
+        assert call(_cabi.LensSet(base, 2, tb, None)) == _cabi.OK
+        for bad in (_cabi.LensSet(base, 0, tb, None), _cabi.LensSet(base, 2, tb - 256, None), _cabi.LensSet(base, 2, tb + 16, None),
+                    _cabi.LensSet(None, 2, tb, None), None):
+            assert call(bad) == -1, (call.__name__, bad)
     if is_gpu(engine):
         torch.cuda.synchronize()
     with pytest.raises(ValueError):

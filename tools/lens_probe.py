@@ -131,7 +131,7 @@ def main():
     set_c = e0.lens_set(rig_c["camera_params"], H, W)
     for es in E.values():
         for e in es:
-            e._tables, e._lens_sets = e0._tables, e0._lens_sets
+            e._tables = e0._tables
     arms = {"a": (frames_a, {"K": K0, "dist": D0}), "b": (frames_a, {"lenses": set_b, "frame_lens": frame_lens}),
             "c": (frames_c, {"lenses": set_c, "frame_lens": frame_lens})}
     print(f"C4 {n} frames of {H}x{W}; lens-set bytes: (b) {set_b.tables.numel() / 1e6:.1f} MB, (c) {set_c.tables.numel() / 1e6:.1f} MB; "
