@@ -506,9 +506,8 @@ __device__ __forceinline__ void packed_stage_c2(PieceSmem& S, const PackedDims& 
     }
 }
 
-// stages 2 and 3 of a piece: floor-mean of the in-frame taps > thresh (sum >= T * count), 5x5 majority with replicated
-// frame border (clamped coordinates), bit rows via ballot.  INTERIOR: the frame border is out of reach -> count = 25, no clamps.
-template <bool INTERIOR>
+// stages 2 and 3 of a piece with the frame border within reach: floor-mean of the in-frame taps > thresh (sum >= T * count),
+// 5x5 majority with replicated frame border (clamped coordinates), bit rows via ballot
 __device__ __forceinline__ void piece_threshold_majority(PieceSmem& S, int px0, int py0, int mw, int mh, int W, int H, int T,
                                                          uint32_t* __restrict__ out, int wpr)
 {
@@ -518,40 +517,30 @@ __device__ __forceinline__ void piece_threshold_majority(PieceSmem& S, int px0, 
     const int bw = mw + 4, bh = mh + 4;
     for (int r = wy; r < bh; r += NWARP) {
         int i = py0 - 2 + r;
-        int cnty = INTERIOR ? 5 : min(i + 2, H - 1) - max(i - 2, 0) + 1;
-        bool rowin = INTERIOR || (unsigned)i < (unsigned)H;
+        int cnty = min(i + 2, H - 1) - max(i - 2, 0) + 1;
+        bool rowin = (unsigned)i < (unsigned)H;
         for (int c = lane; c < bw; c += 32) {
             int j = px0 - 2 + c, b = 0;
-            if (rowin && (INTERIOR || (unsigned)j < (unsigned)W)) {
+            if (rowin && (unsigned)j < (unsigned)W) {
                 const uint16_t* h = &S.HS[r * HSW + c];
                 int s = h[0] + h[HSW] + h[2 * HSW] + h[3 * HSW] + h[4 * HSW];
-                int cnt = INTERIOR ? 25 : cnty * (min(j + 2, W - 1) - max(j - 2, 0) + 1);
+                int cnt = cnty * (min(j + 2, W - 1) - max(j - 2, 0) + 1);
                 b = s >= T * cnt;
             }
             S.B[r * BW + c] = (uint8_t)b;
         }
         __syncwarp();
-        if (INTERIOR) {
-            for (int c = lane; c < mw; c += 32) {
-                const uint8_t* b = &S.B[r * BW + c];
-                MH[r * PIECE + c] = (uint8_t)(b[0] + b[1] + b[2] + b[3] + b[4]);
-            }
-        } else {
-            const uint8_t* b = &S.B[r * BW] - (px0 - 2);               // indexed by frame column
-            for (int c = lane; c < mw; c += 32) {
-                int j = px0 + c;
-                MH[r * PIECE + c] = (uint8_t)(b[max(j - 2, 0)] + b[max(j - 1, 0)] + b[j] + b[min(j + 1, W - 1)] + b[min(j + 2, W - 1)]);
-            }
+        const uint8_t* b = &S.B[r * BW] - (px0 - 2);                   // indexed by frame column
+        for (int c = lane; c < mw; c += 32) {
+            int j = px0 + c;
+            MH[r * PIECE + c] = (uint8_t)(b[max(j - 2, 0)] + b[max(j - 1, 0)] + b[j] + b[min(j + 1, W - 1)] + b[min(j + 2, W - 1)]);
         }
     }
     __syncthreads();
     for (int r = wy; r < mh; r += NWARP) {
         int i = py0 + r;
-        int r0 = r, r1 = r + 1, r2 = r + 2, r3 = r + 3, r4 = r + 4;
-        if (!INTERIOR) {
-            r0 = max(i - 2, 0) - (py0 - 2); r1 = max(i - 1, 0) - (py0 - 2);
-            r3 = min(i + 1, H - 1) - (py0 - 2); r4 = min(i + 2, H - 1) - (py0 - 2);
-        }
+        const int r0 = max(i - 2, 0) - (py0 - 2), r1 = max(i - 1, 0) - (py0 - 2), r2 = r + 2;
+        const int r3 = min(i + 1, H - 1) - (py0 - 2), r4 = min(i + 2, H - 1) - (py0 - 2);
 #pragma unroll
         for (int c0 = 0; c0 < PIECE; c0 += 32) {
             int c = c0 + lane, s = 0;
@@ -563,8 +552,12 @@ __device__ __forceinline__ void piece_threshold_majority(PieceSmem& S, int px0, 
 }
 
 // four fast-map words, kept in L2 (evict last: every piece of every frame reads the map, the frames stream past it)
+// The L2 policies of the piece filter: the windows are read once (evict first), the fast map by every piece (PF_MAP_EVICT).  The
+// kernel creates them where it uses them, once per piece: a 64-bit policy held across the piece loop costs it spills at 64 registers.
 #ifdef MOCAP_EMU
-#define ld_map4(p, policy) (*(const int4*)(p))
+static inline int4 ld_map4(const int32_t* p, uint64_t) { return *(const int4*)p; }
+static inline uint64_t window_l2_policy() { return 0; }
+static inline uint64_t map_l2_policy() { return 0; }
 #else
 __device__ __forceinline__ int4 ld_map4(const int32_t* p, uint64_t policy)
 {
@@ -572,17 +565,27 @@ __device__ __forceinline__ int4 ld_map4(const int32_t* p, uint64_t policy)
     asm volatile("ld.global.nc.L2::cache_hint.v4.s32 {%0,%1,%2,%3}, [%4], %5;" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p), "l"(policy));
     return r;
 }
+#define PF_STR2(x) #x
+#define PF_STR(x) PF_STR2(x)
+__device__ __forceinline__ uint64_t window_l2_policy()
+{
+    uint64_t p;
+    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
+__device__ __forceinline__ uint64_t map_l2_policy()
+{
+    uint64_t p;
+    asm volatile("createpolicy.fractional.L2::" PF_STR(PF_MAP_EVICT) ".b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
 #endif
 
 // one undistorted pixel from the staged window: m = fast-map word (fx | fy << 8 | tap offset << 16), p = the pixel's own place in the window
 __device__ __forceinline__ uint32_t fast_tap(const uint8_t* p, uint32_t m)
 {
     const uint8_t* q = p + ((int)m >> 16);
-#ifdef MOCAP_EMU
-    const int fx = (int)(m & 0xffu), fy = (int)((m >> 8) & 0xffu);
-#else
     const int fx = (int)(m & 0xffu), fy = (int)__byte_perm(m, 0, 0x4441);      // byte 1, one PRMT
-#endif
     const int r0 = (32 - fx) * q[0] + fx * q[1];
     const int r1 = (32 - fx) * q[WIN_W] + fx * q[WIN_W + 1];
     return (uint32_t)(((32 - fy) * r0 + fy * r1 + 512) >> 10);
@@ -610,92 +613,42 @@ __device__ __forceinline__ FastIter fast_iter_init(const int* d, const TableView
     return it;
 }
 
-// 16 bytes global -> shared without a register round trip (lands asynchronously; piece_copy_wait before the data is used)
-__device__ __forceinline__ void piece_copy16(void* dst_smem, const void* src)
+// The source window of a piece comes in as ONE TMA box (cp.async.bulk.tensor.3d of the frame batch viewed as [n][H][W], WIN_W x
+// WIN_H_LOW or WIN_W x WIN_H bytes at (wx0, wy0, frame); what lies outside the frame is zero-filled by the TMA unit), issued by thread
+// 0 and completing on `wbar`.  Pieces whose window does not fit take their taps from global memory and post nothing.  Readers of
+// the window wait on `wbar` and then pass a __syncthreads() that the issuing thread reaches after posting (the emulation build's
+// synchronous box copy and no-op barrier rely on that).
+__device__ __forceinline__ void post_piece_window(uint8_t* win, const int* d, const CUtensorMap& tmap, const CUtensorMap& tmap_low, uint64_t* wbar)
 {
-#ifdef MOCAP_EMU
-    *(uint4*)dst_smem = *(const uint4*)src;
-#else
-    unsigned d = (unsigned)__cvta_generic_to_shared(dst_smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" :: "r"(d), "l"(src) : "memory");
-#endif
-}
-__device__ __forceinline__ void piece_copy_wait()
-{
-#ifndef MOCAP_EMU
-    asm volatile("cp.async.wait_all;\n" ::: "memory");
-#endif
-}
-
-// source window of a piece -> shared memory, 16 bytes per copy, zero outside the frame
-__device__ __forceinline__ void piece_issue_window(uint8_t* win, const int* d, const uint8_t* __restrict__ frames, int64_t fstride, int W, int H)
-{
-    const int wh = (d[4] >> 16) & 0xff, nvec = (d[4] >> 24) & 0xff;
-    const int wx0 = (int)(int16_t)(d[5] & 0xffff), wy0 = d[5] >> 16;
-    const uint8_t* fr = frames + (size_t)d[0] * fstride;
-    const unsigned inv_v = nvec ? (1u << 16) / (unsigned)nvec + 1u : 0u;            // idx / nvec for idx * nvec < 2^16
-    for (int idx = threadIdx.x; idx < wh * nvec; idx += CL_THREADS) {
-        int row = (int)(((unsigned)idx * inv_v) >> 16), v = idx - row * nvec;
-        int gy = wy0 + row, gx = wx0 + 16 * v;
-        uint8_t* dst = &win[row * WIN_W + 16 * v];
-        if ((unsigned)gy < (unsigned)H && gx >= 0 && gx + 16 <= W) piece_copy16(dst, fr + (size_t)gy * W + gx);
-        else *(uint4*)dst = make_uint4(0, 0, 0, 0);
-    }
+    if (threadIdx.x != 0 || !((d[2] >> 25) & 1)) return;
+    const bool low = ((d[4] >> 16) & 0xff) <= WIN_H_LOW;                           // window rows needed
+    mbar_expect_tx(wbar, WIN_W * (low ? WIN_H_LOW : WIN_H));
+    tma_load_box(win, low ? &tmap_low : &tmap, (int)(int16_t)(d[5] & 0xffff), d[5] >> 16, d[0], wbar, window_l2_policy());
 }
 
 // Persistent CTAs over the piece list.  The loop is software-pipelined over pieces: as soon as the remap of piece i has
-// consumed `win`, every thread posts the source window of piece i + 1 into it (cp.async, lands while the stages of piece i
-// run), warp 0 fetches the descriptor of piece i + 2 and thread 0 draws the index of piece i + 3 -- no descriptor, window or
-// work-counter latency is waited for inside the loop.
-#ifdef MOCAP_EMU
-#define PF_ISSUE_WINDOW(desc) piece_issue_window(win, desc, frames, fstride, W, H)
-#else
-#define PF_ISSUE_WINDOW(desc)                                                                                                   \
-    do {                                                                                                                        \
-        if (!PF_USE_TMA) piece_issue_window(win, desc, frames, fstride, W, H);                                                  \
-        else if (tid == 0 && (((desc)[2] >> 25) & 1)) {                                                                         \
-            const bool low_ = (((desc)[4] >> 16) & 0xff) <= WIN_H_LOW;        /* window rows needed */                          \
-            mbar_expect_tx(&wbar, WIN_W * (low_ ? WIN_H_LOW : WIN_H));                                                          \
-            tma_load_box(win, low_ ? &tmap_low : &tmap, (int)(int16_t)((desc)[5] & 0xffff), (desc)[5] >> 16, (desc)[0], &wbar, wpolicy); \
-        }                                                                                                                       \
-    } while (0)
-#endif
-#ifdef MOCAP_EMU
-#define PF_TMA_PARAM
-#define PF_USE_TMA false
-#else
-#define PF_TMA_PARAM , const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_low, int use_tma
-#define PF_USE_TMA (use_tma != 0)
-#endif
-// The source window of a piece comes in as ONE TMA box (cp.async.bulk.tensor.3d of the frame batch viewed as [n][H][W], WIN_W x WIN_H
-// bytes at (wx0, wy0, frame); what lies outside the frame is zero-filled by the TMA unit) issued by thread 0 and completing on an
-// mbarrier; batches the tensor map cannot describe use 16-byte cp.async copies per thread instead.
+// consumed `win`, thread 0 posts the source window of piece i + 1 into it (it lands while the stages of piece i run), warp 0
+// fetches the descriptor of piece i + 2 and thread 0 draws the index of piece i + 3 -- no descriptor, window or work-counter
+// latency is waited for inside the loop.  use_window: the host encoded both window tensor maps (the batch is one a tensor map
+// can describe) and T lies in 0..256; else every piece takes its taps from global memory.
 __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8_t* __restrict__ frames, int64_t fstride, TableView tv, int thresh,
-                                                                  ClusterWs cw PF_TMA_PARAM)
+                                                                  ClusterWs cw, const __grid_constant__ CUtensorMap tmap,
+                                                                  const __grid_constant__ CUtensorMap tmap_low, int use_window)
 {
     __shared__ PieceSmem S;
     __align__(128) __shared__ uint8_t win[WIN_W * WIN_H];          // staged source window
-#ifndef MOCAP_EMU
-    __shared__ uint64_t wbar;                                      // "window landed" barrier of the TMA path
+    __shared__ uint64_t wbar;                                      // "window landed" barrier
     unsigned wphase = 0;
-    uint64_t wpolicy, mpolicy;                                     // L2: the windows are read once (evict first), the fast map by every piece (evict last)
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(wpolicy));
-#define PF_STR2(x) #x
-#define PF_STR(x) PF_STR2(x)
-    asm volatile("createpolicy.fractional.L2::" PF_STR(PF_MAP_EVICT) ".b64 %0, 1.0;" : "=l"(mpolicy));
-    if (threadIdx.x == 0 && PF_USE_TMA) {
+    if (threadIdx.x == 0 && use_window) {
         mbar_init(&wbar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-#endif
     __align__(16) __shared__ int s_desc[2][8];
     __shared__ int s_next;
     constexpr int UW = PieceSmem::UW, HSW = PieceSmem::HSW;
-    const bool vec_ok = (tv.W % 16 == 0) && (fstride % 16 == 0) && (((uintptr_t)frames) % 16 == 0);
     const int tid = threadIdx.x, lane = tid & 31, wy = tid >> 5, NWARP = CL_THREADS / 32;
     const int H = tv.H, W = tv.W, T = thresh + 1;
     const bool t_ok = T >= 0 && T <= 256;                          // thresholds the packed stages can represent
-    const bool use_win = vec_ok && t_ok;                           // else: descriptors' windows are ignored, taps come from global memory
     const int total = min(cw.counters[CN_PIECES], cw.pc_cap);
     if (tid == 0) s_next = atomicAdd(&cw.counters[CN_PIECE_CUR], 1);
     __syncthreads();
@@ -711,7 +664,7 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
         if (lane == 0) next = atomicAdd(&cw.counters[CN_PIECE_CUR], 1);
     }
     __syncthreads();
-    if (use_win) PF_ISSUE_WINDOW(s_desc[0]);
+    if (use_window) post_piece_window(win, s_desc[0], tmap, tmap_low, &wbar);
     int slot = 0;
     for (;;) {
         const int* d = s_desc[slot];
@@ -723,8 +676,8 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
         pd.lead = 0;
         const int mw = pd.mw, mh = pd.mh;
         const bool packed = ((dims >> 24) & 1) && t_ok;
-        const bool staged = ((dims >> 25) & 1) && use_win;
-        const bool fastp = ((dims >> 26) & 1) && use_win;
+        const bool staged = ((dims >> 25) & 1) && use_window;
+        const bool fastp = ((dims >> 26) & 1) && use_window;
         const int wpr = d[4] & 0xffff;
         const int wx0 = (int)(int16_t)(d[5] & 0xffff), wy0 = d[5] >> 16;
         uint32_t* out = cw.rows_out + (unsigned)d[3];
@@ -733,11 +686,7 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
         const int ux1 = packed ? px1 + pd.hr + 2 : px1 + 4, uy1 = packed ? py1 + pd.hb + 2 : py1 + 4;
         const int uw = ux1 - ux0 + 1, uh = uy1 - uy0 + 1, bw = mw + 4;
         const uint8_t* fr = frames + (size_t)f * fstride;
-#ifndef MOCAP_EMU
-        if (PF_USE_TMA) { if (((dims >> 25) & 1) && use_win) { mbar_wait(&wbar, wphase); wphase ^= 1; } }
-        else
-#endif
-        piece_copy_wait();
+        if (staged) { mbar_wait(&wbar, wphase); wphase ^= 1; }
         __syncthreads();                                            // the window of this piece has landed; the other descriptor slot is free
         if (wy == 0 && lane < 8) s_desc[slot ^ 1][lane] = dn;
         if (tid == 0) s_next = nx;
@@ -756,6 +705,7 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
             // (the byte taps of a warp then fall into consecutive bytes: no 2-way bank conflicts, but four 32-bit map loads and four byte
             // stores): 0.680 against 0.687 ms, and no gain with two calls in flight.
             FastIter fi = fast_iter_init(d, tv, tid);
+            const uint64_t mpolicy = map_l2_policy();
             pd.lead = ux0 & 3;
             const uint8_t* pw = win + (uy0 - wy0 + fi.r) * WIN_W + (ux0 - pd.lead - wx0) + 4 * fi.q;
             uint8_t* pu = S.U + fi.r * UW + 4 * fi.q;
@@ -805,7 +755,7 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
         }
         __syncthreads();                                            // U complete; the window is free again
         // post the next piece's window (it lands while the stages below run), fetch the descriptor of the piece after it
-        if (s_next < total && use_win) PF_ISSUE_WINDOW(s_desc[slot ^ 1]);
+        if (s_next < total && use_window) post_piece_window(win, s_desc[slot ^ 1], tmap, tmap_low, &wbar);
         if (wy == 0) {
             nx = __shfl_sync(0xffffffffu, next, 0);
             dn = (lane < 8 && nx < total) ? cw.pieces[8 * (size_t)nx + lane] : 0;
@@ -827,7 +777,7 @@ __global__ void __launch_bounds__(CL_THREADS, 8) piece_filter_kernel(const uint8
                     S.HS[r * HSW + c] = (uint16_t)(up[0] + up[1] + up[2] + up[3] + up[4]);
                 }
             __syncthreads();
-            piece_threshold_majority<false>(S, px0, py0, mw, mh, W, H, T, out, wpr);
+            piece_threshold_majority(S, px0, py0, mw, mh, W, H, T, out, wpr);
         }
         if (s_next >= total) break;
         slot ^= 1;
@@ -1235,18 +1185,14 @@ int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstr
     stage_end(timer, 1, s);
     if (how.ev_group) cudaEventRecord(how.ev_group, s);
     stage_begin(timer, 2, s);
-#ifdef MOCAP_EMU
-    LAUNCH(piece_filter_kernel, sms * how.filter_ctas, CL_THREADS, 0, s, frames, fstride, tv, thresh, cw);
-#else
     {
         CUtensorMap tmap, tmap_low;
         memset(&tmap, 0, sizeof(tmap)); memset(&tmap_low, 0, sizeof(tmap_low));
         const int T = thresh + 1;
-        const int use_tma = (T >= 0 && T <= 256 && frames_tensor_map(&tmap, frames, n, H, W, fstride, WIN_W, WIN_H, PF_WIN_L2_PROMO) &&
-                             frames_tensor_map(&tmap_low, frames, n, H, W, fstride, WIN_W, WIN_H_LOW, PF_WIN_L2_PROMO)) ? 1 : 0;
-        LAUNCH(piece_filter_kernel, sms * how.filter_ctas, CL_THREADS, 0, s, frames, fstride, tv, thresh, cw, tmap, tmap_low, use_tma);
+        const int use_window = (T >= 0 && T <= 256 && frames_tensor_map(&tmap, frames, n, H, W, fstride, WIN_W, WIN_H, PF_WIN_L2_PROMO) &&
+                                frames_tensor_map(&tmap_low, frames, n, H, W, fstride, WIN_W, WIN_H_LOW, PF_WIN_L2_PROMO)) ? 1 : 0;
+        LAUNCH(piece_filter_kernel, sms * how.filter_ctas, CL_THREADS, 0, s, frames, fstride, tv, thresh, cw, tmap, tmap_low, use_window);
     }
-#endif
     stage_end(timer, 2, s);
     if (how.ev_filter) cudaEventRecord(how.ev_filter, s);
     stage_begin(timer, 3, s);

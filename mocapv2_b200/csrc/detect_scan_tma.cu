@@ -79,7 +79,7 @@ __global__ void __launch_bounds__(ST_THREADS, 8) scan_tma_kernel(const __grid_co
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) {
         for (int s = 0; s < ST_STAGES; ++s) { for (int b = 0; b < NB; ++b) mbar_init(&full[NB * s + b], 1); mbar_init(&empty[s], 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
 
@@ -269,8 +269,16 @@ bool stream_wait_supported()
     return have;
 }
 
-#else   // MOCAP_EMU: the CPU emulation build of the kernel sources (tests/emu) has no TMA unit; the classic scan kernels serve there
+#else   // MOCAP_EMU: the CPU emulation build of the kernel sources (tests/emu) runs no TMA scan; the classic scan kernels serve there
 
+// the stand-in tensor map of the emulation build (tma.cuh), for the same batches the driver describes above
+bool frames_tensor_map(CUtensorMap* out, const uint8_t* frames, int n, int H, int W, int64_t fstride, int box_w, int box_h, int)
+{
+    if (n <= 0 || H <= 0 || W <= 0) return false;
+    if (W % 16 || fstride % 16 || ((uintptr_t)frames) % 16) return false;    // tensor-map strides are multiples of 16 bytes
+    *out = CUtensorMap{frames, n, H, W, fstride, box_w, box_h};
+    return true;
+}
 bool scan_tma_supported(const uint8_t*, int, int, int, int64_t, int) { return false; }
 int launch_scan_tma(const uint8_t*, int, int, int, int64_t, const TableView&, int, uint32_t*, int*, int, int, cudaStream_t) { return MOCAP_ERR_UNSUPPORTED; }
 int stream_wait_geq(cudaStream_t, const int*, int) { return MOCAP_ERR_UNSUPPORTED; }
