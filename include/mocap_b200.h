@@ -70,6 +70,10 @@ int mocap_undistort_table_build(const double* K9_host, const double* dist5_host,
  * frames_dev: n_frames x H x W uint8 (row stride W, frame stride `frame_stride` bytes).
  * out_xy[n][max_blobs][2] int32 centroids in the reference's output order, out_count[n] how many
  * (0 = the reference's [[None, None]]), out_flags[n] MOCAP_FLAG_*.
+ * Centroid of a kept contour: q = (m10 / m00, m01 / m00), the FP64 quotients of cv.moments of the contour polygon (lib/ImageOperations.py:
+ * 59-62).  The entry points without a suffix store int(q) (truncated toward zero, the reference's whole pixels); the *_subpixel entry
+ * points store (float)q, the float32 nearest to q (spacing <= 2^-10 px below 16384), in the same 8-byte slot: out_xy[n][max_blobs][2]
+ * float32.  Contours, filter, order, counts and flags do not depend on the format.
  * Optional (may be NULL) parity outputs:
  *   out_bits[n][H][ceil(W/32)]   the filtered binary image (image_filter_gpu, :23-31), LSB = leftmost pixel
  *   out_labels[n][H][W] int32    8-connected blob labels, 0 = background, k = k-th blob in raster order
@@ -112,6 +116,14 @@ int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, in
                        uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
                        double* out_contours, int32_t* out_contour_count,
                        void* workspace, size_t workspace_bytes, void* stream, void* stage_timer_or_null);
+/* The same with sub-pixel centroids: out_xy [n][max_blobs][2] float32 (see the centroid definition above). */
+int mocap_detect_batch_subpixel(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                int max_blobs, int max_contours, int max_runs,
+                                float* out_xy, int32_t* out_count, int32_t* out_flags,
+                                uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                                double* out_contours, int32_t* out_contour_count,
+                                void* workspace, size_t workspace_bytes, void* stream, void* stage_timer_or_null);
 
 /* ---- overlapped detection (same results as mocap_detect_batch without the parity outputs) ----------------------------
  * The batch is cut into chunks of `chunk_frames` frames (<= 0: one chunk); chunk k's stages (group, piece filter, borders) run as
@@ -129,7 +141,7 @@ int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, in
  *     mocap_scan_cells_batch or mocap_bayer_gr2gray_scan_batch for the same frames and thresh.  The call then runs no streaming scan.
  *   xy_dst_dev, count_dst_dev [n_frames] device addresses (both or neither; one without the other is MOCAP_ERR_INVALID): the
  *     store-to-peer epilogue (multi-GPU).  Every frame's record is ALSO copied -- chunk by chunk, behind the chunk's border stage --
- *     to xy_dst[f] (its centroids, int32 pairs) and count_dst[f] (its count): addresses in the receive buffer of the rank that
+ *     to xy_dst[f] (its centroids, int32 pairs; float32 pairs in the _subpixel call) and count_dst[f] (its count): addresses in the receive buffer of the rank that
  *     matches the frame's frame-set, mapped into this process (symmetric memory over NVLink).  The exchange step is then a barrier.
  *   scan_wait_event, scan_done_event (cudaEvent_t owned by the caller): the scan token of several pipes in flight on one GPU
  *     (pipeline.StepsInFlight).  The call's streaming scan waits for scan_wait_event and records scan_done_event behind it.
@@ -146,6 +158,15 @@ int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_fr
                                  const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
                                  void* scan_wait_event, void* scan_done_event,
                                  void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline);
+/* The same with sub-pixel centroids: out_xy [n][max_blobs][2] float32, and xy_dst[f] receives float32 pairs. */
+int mocap_detect_batch_pipelined_subpixel(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                          const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                          int max_blobs, int max_contours, int max_runs,
+                                          float* out_xy, int32_t* out_count, int32_t* out_flags,
+                                          double* out_contours, int32_t* out_contour_count,
+                                          const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
+                                          void* scan_wait_event, void* scan_done_event,
+                                          void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline);
 /* ms since the fork of the last call with record_timeline: [scan done, join] then per chunk [scan seen, grouped, filtered,
  * borders done]; returns the number of floats written, 0 without a timeline */
 int mocap_detect_pipe_timeline(void* pipe, float* ms_out, int cap);
@@ -240,6 +261,16 @@ int mocap_correspond_batch_blocked(const int32_t* xy_dev, const int32_t* count_d
                                    double* obj_out, int32_t* n_obj_out, int32_t* img_out, int32_t* n_valid_out,
                                    double* err_out, int32_t* cand_out, int32_t* flags_out,
                                    void* workspace, size_t workspace_bytes, void* stream);
+
+/* mocap_correspond_batch_blocked on sub-pixel centroid lists (mocap_detect_batch_subpixel): xy_dev float32 and img_out
+ * [S][max_pts][C][2] float32, everything else as there.  The roots' epilines are computed from the float32 points as the reference
+ * does (Helpers.py:205-208), the distances and the DLT read them exactly. */
+int mocap_correspond_batch_subpixel(const float* xy_dev, const int32_t* count_dev, int S, int C, int max_pts, int cams_per_block,
+                                    const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
+                                    int max_groups, int fp64_mode,
+                                    double* obj_out, int32_t* n_obj_out, float* img_out, int32_t* n_valid_out,
+                                    double* err_out, int32_t* cand_out, int32_t* flags_out,
+                                    void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

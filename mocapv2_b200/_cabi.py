@@ -12,7 +12,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB = os.path.join(HERE, "libmocap_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_CAND = 8
 MAX_CAMS = 16
 CAM_STRIDE = 40
@@ -49,6 +49,8 @@ SIGNATURES = {
     "mocap_detect_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i]),
     "mocap_detect_batch": (_i, [_p, _i, _i, _i, _i64, _ls, _i, _d, _d, _i, _i, _i,
                                 _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _p]),
+    "mocap_detect_batch_subpixel": (_i, [_p, _i, _i, _i, _i64, _ls, _i, _d, _d, _i, _i, _i,
+                                         _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _p]),
     "mocap_stage_timer_create": (_p, []),
     "mocap_stage_timer_destroy": (None, [_p]),
     "mocap_stage_timer_read": (_i, [_p, _p]),
@@ -58,6 +60,8 @@ SIGNATURES = {
     "mocap_detect_pipelined_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i]),
     "mocap_detect_batch_pipelined": (_i, [_p, _p, _i, _i, _i, _i64, _ls, _i, _d, _d, _i, _i, _i,
                                           _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i, _i]),
+    "mocap_detect_batch_pipelined_subpixel": (_i, [_p, _p, _i, _i, _i, _i64, _ls, _i, _d, _d, _i, _i, _i,
+                                                   _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i, _i]),
     "mocap_detect_pipe_timeline": (_i, [_p, _p, _i]),
     "mocap_detect_pipe_info": (_i, [_p, _p]),
     "mocap_scan_cells_batch": (_i, [_p, _i, _i, _i, _i64, _p, _i, _i, _p, _p, _sz, _p]),
@@ -77,6 +81,8 @@ SIGNATURES = {
                                     _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "mocap_correspond_batch_blocked": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _d, _i, _i, _i,
                                             _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "mocap_correspond_batch_subpixel": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _d, _i, _i, _i,
+                                             _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
 }
 
 

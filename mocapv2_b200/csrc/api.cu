@@ -15,7 +15,7 @@ bool cluster_path_supported(int H, int W);
 int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstride, const TableView& tv, int thresh,
                         const uint32_t* cellbox, char* ws_base, const ClusterLayout& L, int* need_general,
                         int max_contours, int max_blobs, double min_area, double min_circ,
-                        int32_t* out_xy, int32_t* out_count, int32_t* out_flags, double* out_contours, int32_t* out_contour_count,
+                        int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags, double* out_contours, int32_t* out_contour_count,
                         cudaStream_t s, StageTimer* timer, const ClusterLaunch& how);
 int launch_materialize_bits(const FilterWs& ws, int n, int H, int W, const TableView& tv, uint32_t* out, cudaStream_t s);
 // detect_scan_tma.cu
@@ -32,7 +32,7 @@ size_t blob_ws_stride(int H, int max_runs, int max_contours);
 int launch_blobs(const uint32_t* bits, const uint32_t* fg_tiles, const int* n_fg, int n, int H, int W, int TX,
                  int max_fg, int max_runs, int max_blobs, int max_contours, double min_area, double min_circ,
                  char* ws, size_t ws_stride,
-                 int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
+                 int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags,
                  int64_t* out_blob_sums, int32_t* out_blob_count, double* out_contours, int32_t* out_contour_count,
                  int32_t* out_labels, const int* need_general, cudaStream_t s);
 
@@ -176,13 +176,14 @@ static int lens_set_view(const MocapLensSet* ls, int H, int W, TableView* tv)
     return MOCAP_OK;
 }
 
-extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                  const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
-                                  int max_blobs, int max_contours, int max_runs,
-                                  int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
-                                  uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
-                                  double* out_contours, int32_t* out_contour_count,
-                                  void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
+// mocap_detect_batch and mocap_detect_batch_subpixel: out_xy holds int32 (xy_float 0) or float32 (1) centroid pairs
+static int detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                        const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                        int max_blobs, int max_contours, int max_runs,
+                        int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags,
+                        uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                        double* out_contours, int32_t* out_contour_count,
+                        void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
 {
     StageTimer* timer = (StageTimer*)stage_timer;
     if (!frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
@@ -211,7 +212,7 @@ extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H
     CUDA_TRY(cudaMemsetAsync(need_general, use_cluster ? 0 : 1, (size_t)n_frames * 4, s));
     if (use_cluster) {
         st = launch_cluster_path(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, cl_base, L.cl, need_general,
-                                 max_contours, max_blobs, min_area, min_circ, out_xy, out_count, out_flags, out_contours,
+                                 max_contours, max_blobs, min_area, min_circ, out_xy, xy_float, out_count, out_flags, out_contours,
                                  out_contour_count, s, timer, ClusterLaunch());
         if (st != MOCAP_OK) return st;
     }
@@ -224,10 +225,36 @@ extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H
     }
     st = launch_blobs(ws.bits, ws.fg_tiles, ws.n_fg, n_frames, H, W, L.TX, L.max_fg, max_runs, max_blobs, max_contours,
                       min_area, min_circ, (char*)workspace + L.off_blob, L.blob_stride,
-                      out_xy, out_count, out_flags, out_blob_sums, out_blob_count, out_contours, out_contour_count,
+                      out_xy, xy_float, out_count, out_flags, out_blob_sums, out_blob_count, out_contours, out_contour_count,
                       out_labels, need_general, s);
     stage_end(timer, 4, s);
     return st;
+}
+
+extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                  const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                  int max_blobs, int max_contours, int max_runs,
+                                  int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
+                                  uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                                  double* out_contours, int32_t* out_contour_count,
+                                  void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
+{
+    return detect_batch(frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours, max_runs,
+                        out_xy, 0, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count, out_contours, out_contour_count,
+                        workspace, workspace_bytes, stream, stage_timer);
+}
+
+extern "C" int mocap_detect_batch_subpixel(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                           const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                           int max_blobs, int max_contours, int max_runs,
+                                           float* out_xy, int32_t* out_count, int32_t* out_flags,
+                                           uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                                           double* out_contours, int32_t* out_contour_count,
+                                           void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
+{
+    return detect_batch(frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours, max_runs,
+                        (int32_t*)out_xy, 1, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count, out_contours,
+                        out_contour_count, workspace, workspace_bytes, stream, stage_timer);
 }
 
 // findContours -> filter -> moments on a given packed binary image (lib/ImageOperations.py:41-65), stage parity entry
@@ -252,7 +279,7 @@ extern "C" int mocap_blobs_batch(const uint32_t* bits_dev, int n_frames, int H, 
     if (st != MOCAP_OK) return st;
     return launch_blobs(bits_dev, ws.fg_tiles, ws.n_fg, n_frames, H, W, L.TX, L.max_fg, max_runs, max_blobs, max_contours,
                         min_area, min_circ, (char*)workspace + L.off_blob, L.blob_stride,
-                        out_xy, out_count, out_flags, out_blob_sums, out_blob_count, out_contours, out_contour_count,
+                        out_xy, 0, out_count, out_flags, out_blob_sums, out_blob_count, out_contours, out_contour_count,
                         out_labels, nullptr, s);
 }
 
@@ -386,14 +413,16 @@ extern "C" size_t mocap_detect_pipelined_workspace_bytes(int n_frames, int H, in
     return P.total;
 }
 
-extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                            const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
-                                            int max_blobs, int max_contours, int max_runs,
-                                            int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
-                                            double* out_contours, int32_t* out_contour_count,
-                                            const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
-                                            void* scan_wait_event, void* scan_done_event,
-                                            void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
+// mocap_detect_batch_pipelined and mocap_detect_batch_pipelined_subpixel: int32 (xy_float 0) or float32 (1) centroid pairs.  The
+// store-to-peer epilogue copies 8-byte records and does not care which.
+static int detect_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                            const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                            int max_blobs, int max_contours, int max_runs,
+                            int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags,
+                            double* out_contours, int32_t* out_contour_count,
+                            const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
+                            void* scan_wait_event, void* scan_done_event,
+                            void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
 {
     DetectPipe* dp = (DetectPipe*)pipe;
     if (!dp || !frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
@@ -459,7 +488,7 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
         if (tc.frame_lens) tc.frame_lens += f0;
         st = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tc, thresh, cb, cws, P.cl, need_general + f0,
                                  max_contours, max_blobs, min_area, min_circ,
-                                 out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, out_flags + f0,
+                                 out_xy + (size_t)f0 * max_blobs * 2, xy_float, out_count + f0, out_flags + f0,
                                  out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,
                                  ps, nullptr, how);
         if (st != MOCAP_OK) return st;
@@ -481,9 +510,37 @@ extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_de
     if (st != MOCAP_OK) return st;
     st = launch_blobs(ws.bits, ws.fg_tiles, ws.n_fg, n_frames, H, W, P.L.TX, P.L.max_fg, max_runs, max_blobs, max_contours,
                       min_area, min_circ, base + P.L.off_blob, P.L.blob_stride,
-                      out_xy, out_count, out_flags, nullptr, nullptr, out_contours, out_contour_count, nullptr, need_general, s);
+                      out_xy, xy_float, out_count, out_flags, nullptr, nullptr, out_contours, out_contour_count, nullptr, need_general, s);
     if (st == MOCAP_OK && sc_xy) st = launch_scatter(out_xy, out_count, sc_xy, sc_count, n_frames, max_blobs, need_general, 1, s);
     return st;
+}
+
+extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                            const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                            int max_blobs, int max_contours, int max_runs,
+                                            int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
+                                            double* out_contours, int32_t* out_contour_count,
+                                            const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
+                                            void* scan_wait_event, void* scan_done_event,
+                                            void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
+{
+    return detect_pipelined(pipe, frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours,
+                            max_runs, out_xy, 0, out_count, out_flags, out_contours, out_contour_count, cellbox_dev, xy_dst_dev,
+                            count_dst_dev, scan_wait_event, scan_done_event, workspace, workspace_bytes, stream, chunk_frames, record_timeline);
+}
+
+extern "C" int mocap_detect_batch_pipelined_subpixel(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                                     const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                                     int max_blobs, int max_contours, int max_runs,
+                                                     float* out_xy, int32_t* out_count, int32_t* out_flags,
+                                                     double* out_contours, int32_t* out_contour_count,
+                                                     const uint32_t* cellbox_dev, const uint64_t* xy_dst_dev, const uint64_t* count_dst_dev,
+                                                     void* scan_wait_event, void* scan_done_event,
+                                                     void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
+{
+    return detect_pipelined(pipe, frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours,
+                            max_runs, (int32_t*)out_xy, 1, out_count, out_flags, out_contours, out_contour_count, cellbox_dev, xy_dst_dev,
+                            count_dst_dev, scan_wait_event, scan_done_event, workspace, workspace_bytes, stream, chunk_frames, record_timeline);
 }
 
 // Timeline of the last mocap_detect_batch_pipelined call that had record_timeline set (read it after the stream has been

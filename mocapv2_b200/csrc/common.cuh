@@ -22,7 +22,7 @@ static inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigne
 #include <stdint.h>
 #include "../../include/mocap_b200.h"
 
-#define MOCAP_ABI_VERSION 5
+#define MOCAP_ABI_VERSION 6
 
 // every kernel launch of the library is counted (mocap_kernel_launch_count: the bench's gpu_launches is read, not estimated)
 extern unsigned long long g_mocap_launches;
@@ -143,6 +143,14 @@ __device__ __forceinline__ uint32_t pack_cellbox(uint32_t xmask, uint32_t ymask)
     if (!xmask) return CELL_EMPTY;
     uint32_t x0 = __ffs(xmask) - 1, x1 = 31 - __clz(xmask), y0 = __ffs(ymask) - 1, y1 = 31 - __clz(ymask);
     return x0 | (x1 << 8) | (y0 << 16) | (y1 << 24);
+}
+
+// The centroid record of a kept contour: (m10 / m00, m01 / m00) as the FP64 quotients of cv.moments, stored in the 8-byte slot
+// xy[0..1] as int32 truncated toward zero (int(), lib/ImageOperations.py:59-62) or, sub-pixel, as the float32 nearest to them.
+__device__ __forceinline__ void store_centroid(int32_t* xy, double qx, double qy, int xy_float)
+{
+    if (xy_float) { float* p = (float*)xy; p[0] = (float)qx; p[1] = (float)qy; }
+    else { xy[0] = (int32_t)qx; xy[1] = (int32_t)qy; }
 }
 
 // how launch_cluster_path runs a batch (or one chunk of the overlapped pipeline)

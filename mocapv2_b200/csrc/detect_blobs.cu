@@ -90,6 +90,7 @@ struct BlobParams {
     int H, W, TX;
     int max_fg, max_runs, max_blobs, max_contours;
     double min_area, min_circ;
+    int xy_float;                    // centroid records as float32 pairs (sub-pixel), else int32 (store_centroid)
 };
 
 __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
@@ -510,8 +511,7 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
             double m00 = __dmul_rn((double)a00, sgn * 0.5);
             double m10 = __dmul_rn((double)a10, sgn * 0.16666666666666666);
             double m01 = __dmul_rn((double)a01, sgn * 0.16666666666666666);
-            out_xy[((size_t)f * P.max_blobs + pos) * 2 + 0] = (int32_t)__ddiv_rn(m10, m00);   // int(): toward zero
-            out_xy[((size_t)f * P.max_blobs + pos) * 2 + 1] = (int32_t)__ddiv_rn(m01, m00);
+            store_centroid(out_xy + ((size_t)f * P.max_blobs + pos) * 2, __ddiv_rn(m10, m00), __ddiv_rn(m01, m00), P.xy_float);
         }
     }
     __syncthreads();
@@ -566,13 +566,13 @@ size_t blob_ws_stride(int H, int max_runs, int max_contours)
 int launch_blobs(const uint32_t* bits, const uint32_t* fg_tiles, const int* n_fg, int n, int H, int W, int TX,
                  int max_fg, int max_runs, int max_blobs, int max_contours, double min_area, double min_circ,
                  char* ws, size_t ws_stride,
-                 int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
+                 int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags,
                  int64_t* out_blob_sums, int32_t* out_blob_count, double* out_contours, int32_t* out_contour_count,
                  int32_t* out_labels, const int* need_general, cudaStream_t s)
 {
     BlobParams P;
     P.H = H; P.W = W; P.TX = TX; P.max_fg = max_fg; P.max_runs = max_runs; P.max_blobs = max_blobs;
-    P.max_contours = max_contours; P.min_area = min_area; P.min_circ = min_circ;
+    P.max_contours = max_contours; P.min_area = min_area; P.min_circ = min_circ; P.xy_float = xy_float;
     LAUNCH(blobs_kernel, n, BLOB_THREADS, 0, s, bits, fg_tiles, n_fg, P, ws, ws_stride, out_xy, out_count, out_flags,
                                             out_blob_sums, out_blob_count, out_contours, out_contour_count, out_labels, need_general);
     CUDA_TRY(cudaGetLastError());

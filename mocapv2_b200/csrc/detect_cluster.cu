@@ -1015,7 +1015,7 @@ __device__ void frame_traces(const ClusterWs& cw, int f, int W, int max_contours
 // ---------------------------------------------------------------------------------------------------------
 __device__ void frame_finalize(const ClusterWs& cw, int f, uint8_t* keepv /*[max_contours], shared*/, int max_contours, int max_blobs,
                                double min_area, double min_circ,
-                               int32_t* __restrict__ out_xy, int32_t* __restrict__ out_count, int32_t* __restrict__ out_flags,
+                               int32_t* __restrict__ out_xy, int xy_float, int32_t* __restrict__ out_count, int32_t* __restrict__ out_flags,
                                double* __restrict__ out_contours, int32_t* __restrict__ out_contour_count)
 {
     const int tid = threadIdx.x;
@@ -1080,8 +1080,7 @@ __device__ void frame_finalize(const ClusterWs& cw, int f, uint8_t* keepv /*[max
             double m00 = __dmul_rn((double)a00, sgn * 0.5);
             double m10 = __dmul_rn((double)a10, sgn * 0.16666666666666666);
             double m01 = __dmul_rn((double)a01, sgn * 0.16666666666666666);
-            out_xy[((size_t)f * max_blobs + pos) * 2 + 0] = (int32_t)__ddiv_rn(m10, m00);
-            out_xy[((size_t)f * max_blobs + pos) * 2 + 1] = (int32_t)__ddiv_rn(m01, m00);
+            store_centroid(out_xy + ((size_t)f * max_blobs + pos) * 2, __ddiv_rn(m10, m00), __ddiv_rn(m01, m00), xy_float);
         }
     }
     __syncthreads();
@@ -1096,7 +1095,7 @@ __device__ void frame_finalize(const ClusterWs& cw, int f, uint8_t* keepv /*[max
 // One CTA per frame: the traces of the frame's border-start candidates, the nesting check and -- unless the frame was
 // handed to the general path on the way -- the reference's filter / centroid / output order.
 __global__ void __launch_bounds__(CL_THREADS, BORDERS_MIN_CTAS) borders_finalize_kernel(ClusterWs cw, int W, int frame_step, int max_contours, int max_blobs, double min_area, double min_circ,
-                                                                      int32_t* __restrict__ out_xy, int32_t* __restrict__ out_count, int32_t* __restrict__ out_flags,
+                                                                      int32_t* __restrict__ out_xy, int xy_float, int32_t* __restrict__ out_count, int32_t* __restrict__ out_flags,
                                                                       double* __restrict__ out_contours, int32_t* __restrict__ out_contour_count)
 {
     DYN_SHARED(smraw);
@@ -1108,7 +1107,7 @@ __global__ void __launch_bounds__(CL_THREADS, BORDERS_MIN_CTAS) borders_finalize
     frame_traces(cw, f, W, max_contours);
     __syncthreads();
     if (cw.need_general[f]) return;                         // trace budget, unresolved hole parent or nested contour tree
-    frame_finalize(cw, f, (uint8_t*)smraw, max_contours, max_blobs, min_area, min_circ, out_xy, out_count, out_flags, out_contours, out_contour_count);
+    frame_finalize(cw, f, (uint8_t*)smraw, max_contours, max_blobs, min_area, min_circ, out_xy, xy_float, out_count, out_flags, out_contours, out_contour_count);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1149,7 +1148,7 @@ bool cluster_path_supported(int H, int W)
 int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstride, const TableView& tv, int thresh,
                         const uint32_t* cellbox, char* ws_base, const ClusterLayout& L, int* need_general,
                         int max_contours, int max_blobs, double min_area, double min_circ,
-                        int32_t* out_xy, int32_t* out_count, int32_t* out_flags, double* out_contours, int32_t* out_contour_count,
+                        int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags, double* out_contours, int32_t* out_contour_count,
                         cudaStream_t s, StageTimer* timer, const ClusterLaunch& how)
 {
     ClusterWs cw;
@@ -1200,7 +1199,7 @@ int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstr
     int frame_step = 1;
     for (int pr : {61, 67, 71, 73}) if (n % pr != 0) { frame_step = pr; break; }          // a prime that does not divide n
     LAUNCH(borders_finalize_kernel, n, BF_THREADS, (size_t)max_contours + 16, s, cw, W, frame_step, max_contours, max_blobs, min_area, min_circ,
-           out_xy, out_count, out_flags, out_contours, out_contour_count);
+           out_xy, xy_float, out_count, out_flags, out_contours, out_contour_count);
     stage_end(timer, 3, s);
     if (how.ev_borders) cudaEventRecord(how.ev_borders, s);
     CUDA_TRY(cudaGetLastError());

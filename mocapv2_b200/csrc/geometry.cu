@@ -475,11 +475,13 @@ struct CorrWs { int32_t* cand; int32_t* ncand; };
 
 // Centroid lists of S frame-sets, camera blocks outermost: xy [C / cpb][S][cpb][max_pts][2], count [C / cpb][S][cpb].  cpb = C is the
 // plain [S][C] layout; cpb = cameras per rank is what the shard exchange of the multi-GPU pipeline delivers (one block per source
-// rank), so the kernels read the received buffer as it is.
+// rank), so the kernels read the received buffer as it is.  Pt: int32_t (whole-pixel centroids) or float (sub-pixel); both convert to
+// float and double exactly, so the epilines, distances, cutoff and ties are the same expressions for either.
+template <typename Pt>
 struct CorrIn {
-    const int32_t* xy; const int32_t* count;
+    const Pt* xy; const int32_t* count;
     int S, cpb, max_pts;
-    __device__ __forceinline__ const int32_t* pts(int s, int cam) const {
+    __device__ __forceinline__ const Pt* pts(int s, int cam) const {
         const int blk = cam / cpb, ci = cam - blk * cpb;
         return xy + (((size_t)blk * S + s) * cpb + ci) * (size_t)max_pts * 2;
     }
@@ -495,16 +497,16 @@ struct CorrIn {
 
 // Part 1, grid (S, ceil(max_pts / CORR_RPC)): candidates per (root, camera), candidate groups, triangulation and mean
 // reprojection error of the CTA's roots -> workspace.  Roots are independent until the ranking (Helpers.py:203-273).
-template <typename T>
+template <typename T, typename Pt>
 __global__ void __launch_bounds__(CORR_THREADS) correspond_kernel(
-    CorrIn in, int C, int max_pts,
+    CorrIn<Pt> in, int C, int max_pts,
     const double* __restrict__ Fs, const double* __restrict__ cams, double cutoff, int max_groups,
     int32_t* __restrict__ cand_out, int32_t* __restrict__ flags_out, char* __restrict__ ws_base, size_t ws_stride)
 {
     DYN_SHARED(smraw);
     T* sm = (T*)smraw;
     const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, nw = blockDim.x >> 5;
-    const int32_t* root_xy = in.pts(s, 0);
+    const Pt* root_xy = in.pts(s, 0);
     const int R = min(in.n(s, 0), max_pts);
     const int j0 = blockIdx.y * CORR_RPC, j1 = min(j0 + CORR_RPC, R);
     if (j0 >= R) return;
@@ -533,7 +535,7 @@ __global__ void __launch_bounds__(CORR_THREADS) correspond_kernel(
         nu = nu != 0.0 ? __ddiv_rn(1.0, sqrt(nu)) : 1.0;
         a = (double)(float)__dmul_rn(a, nu); b = (double)(float)__dmul_rn(b, nu); c = (double)(float)__dmul_rn(c, nu);
         double den = sqrt(__dadd_rn(__dmul_rn(a, a), __dmul_rn(b, b)));
-        const int32_t* pp = in.pts(s, i);
+        const Pt* pp = in.pts(s, i);
         int np = min(in.n(s, i), max_pts), n = 0, fl = 0;
         double dist[MOCAP_MAX_CAND];
         // points farther than cutoff + 2e-5 can neither pass the cutoff nor register as a tie: they are rejected on the
@@ -579,7 +581,7 @@ __global__ void __launch_bounds__(CORR_THREADS) correspond_kernel(
                 int k;
                 if (i == 0) k = j;
                 else { int n = ncand[j * C + i]; int q = rem / n; k = cand[((size_t)j * C + i) * MOCAP_MAX_CAND + (rem - q * n)]; rem = q; }
-                const int32_t* pt = in.pts(s, i) + 2 * k;
+                const Pt* pt = in.pts(s, i) + 2 * k;
                 px[i] = (T)pt[0]; py[i] = (T)pt[1];
                 acc.add_view(sm + i * CAM_T_STRIDE + CAM_P, px[i], py[i]);
             }
@@ -608,9 +610,10 @@ __global__ void __launch_bounds__(CORR_THREADS) correspond_kernel(
 }
 
 // Part 2, one CTA per frame-set: compact the complete roots in root order, rank them by mean error (Helpers.py:274-279)
+template <typename Pt>
 __global__ void __launch_bounds__(CORR_THREADS) correspond_rank_kernel(
-    CorrIn in, int C, int max_pts, int obj_count,
-    double* __restrict__ obj_out, int32_t* __restrict__ n_obj_out, int32_t* __restrict__ img_out, int32_t* __restrict__ n_valid_out,
+    CorrIn<Pt> in, int C, int max_pts, int obj_count,
+    double* __restrict__ obj_out, int32_t* __restrict__ n_obj_out, Pt* __restrict__ img_out, int32_t* __restrict__ n_valid_out,
     double* __restrict__ err_out, char* __restrict__ ws_base, size_t ws_stride)
 {
     const int s = blockIdx.x, tid = threadIdx.x;
@@ -645,10 +648,10 @@ __global__ void __launch_bounds__(CORR_THREADS) correspond_rank_kernel(
             o[0] = rX[3 * j]; o[1] = rX[3 * j + 1]; o[2] = rX[3 * j + 2];
         }
         err_out[(size_t)s * max_pts + v] = e;
-        int32_t* io = img_out + ((size_t)s * max_pts + v) * C * 2;
+        Pt* io = img_out + ((size_t)s * max_pts + v) * C * 2;
         for (int i = 0; i < C; ++i) {
             int k = i == 0 ? j : cand[((size_t)j * C + i) * MOCAP_MAX_CAND];
-            const int32_t* pt = in.pts(s, i) + 2 * k;
+            const Pt* pt = in.pts(s, i) + 2 * k;
             io[2 * i] = pt[0];
             io[2 * i + 1] = pt[1];
         }
@@ -672,30 +675,14 @@ extern "C" size_t mocap_correspond_workspace_bytes(int S, int C, int max_pts, in
     return corr_ws_stride(C, max_pts) * (size_t)S;
 }
 
-extern "C" int mocap_correspond_batch_blocked(const int32_t* xy_dev, const int32_t* count_dev, int S, int C, int max_pts, int cams_per_block,
-                                              const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
-                                              int max_groups, int fp64_mode,
-                                              double* obj_out, int32_t* n_obj_out, int32_t* img_out, int32_t* n_valid_out,
-                                              double* err_out, int32_t* cand_out, int32_t* flags_out,
-                                              void* workspace, size_t workspace_bytes, void* stream);
-
-extern "C" int mocap_correspond_batch(const int32_t* xy_dev, const int32_t* count_dev, int S, int C, int max_pts,
-                                      const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
-                                      int max_groups, int fp64_mode,
-                                      double* obj_out, int32_t* n_obj_out, int32_t* img_out, int32_t* n_valid_out,
-                                      double* err_out, int32_t* cand_out, int32_t* flags_out,
-                                      void* workspace, size_t workspace_bytes, void* stream)
-{
-    return mocap_correspond_batch_blocked(xy_dev, count_dev, S, C, max_pts, C, F_dev, cams_dev, cutoff, obj_count, max_groups, fp64_mode,
-                                          obj_out, n_obj_out, img_out, n_valid_out, err_out, cand_out, flags_out, workspace, workspace_bytes, stream);
-}
-
-extern "C" int mocap_correspond_batch_blocked(const int32_t* xy_dev, const int32_t* count_dev, int S, int C, int max_pts, int cams_per_block,
-                                              const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
-                                              int max_groups, int fp64_mode,
-                                              double* obj_out, int32_t* n_obj_out, int32_t* img_out, int32_t* n_valid_out,
-                                              double* err_out, int32_t* cand_out, int32_t* flags_out,
-                                              void* workspace, size_t workspace_bytes, void* stream)
+// every correspondence entry point: int32 (Pt = int32_t) or float32 (Pt = float) centroid lists, camera-blocked
+template <typename Pt>
+static int correspond_blocked(const Pt* xy_dev, const int32_t* count_dev, int S, int C, int max_pts, int cams_per_block,
+                              const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
+                              int max_groups, int fp64_mode,
+                              double* obj_out, int32_t* n_obj_out, Pt* img_out, int32_t* n_valid_out,
+                              double* err_out, int32_t* cand_out, int32_t* flags_out,
+                              void* workspace, size_t workspace_bytes, void* stream)
 {
     if (cams_per_block < 1 || (C > 0 && C % cams_per_block != 0)) return MOCAP_ERR_INVALID;
     if (!xy_dev || !count_dev || !cams_dev || !obj_out || !n_obj_out || !img_out || !n_valid_out || !err_out || !flags_out || !workspace)
@@ -708,16 +695,52 @@ extern "C" int mocap_correspond_batch_blocked(const int32_t* xy_dev, const int32
     cudaStream_t s = (cudaStream_t)stream;
     CUDA_TRY(cudaMemsetAsync(flags_out, 0, (size_t)S * 4, s));
     dim3 grid(S, cdiv(max_pts, CORR_RPC));
-    CorrIn in;
+    CorrIn<Pt> in;
     in.xy = xy_dev; in.count = count_dev; in.S = S; in.cpb = cams_per_block; in.max_pts = max_pts;
+    auto corr_f64 = correspond_kernel<double, Pt>;
+    auto corr_f32 = correspond_kernel<float, Pt>;
+    auto rank = correspond_rank_kernel<Pt>;
     if (fp64_mode)
-        LAUNCH(correspond_kernel<double>, grid, CORR_THREADS, (size_t)C * CAM_T_STRIDE * sizeof(double), s,
+        LAUNCH(corr_f64, grid, CORR_THREADS, (size_t)C * CAM_T_STRIDE * sizeof(double), s,
             in, C, max_pts, F_dev, cams_dev, cutoff, max_groups, cand_out, flags_out, (char*)workspace, stride);
     else
-        LAUNCH(correspond_kernel<float>, grid, CORR_THREADS, (size_t)C * CAM_T_STRIDE * sizeof(float), s,
+        LAUNCH(corr_f32, grid, CORR_THREADS, (size_t)C * CAM_T_STRIDE * sizeof(float), s,
             in, C, max_pts, F_dev, cams_dev, cutoff, max_groups, cand_out, flags_out, (char*)workspace, stride);
-    LAUNCH(correspond_rank_kernel, S, CORR_THREADS, 0, s, in, C, max_pts, obj_count, obj_out, n_obj_out, img_out,
+    LAUNCH(rank, S, CORR_THREADS, 0, s, in, C, max_pts, obj_count, obj_out, n_obj_out, img_out,
            n_valid_out, err_out, (char*)workspace, stride);
     CUDA_TRY(cudaGetLastError());
     return MOCAP_OK;
+}
+
+extern "C" int mocap_correspond_batch_blocked(const int32_t* xy_dev, const int32_t* count_dev, int S, int C, int max_pts, int cams_per_block,
+                                              const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
+                                              int max_groups, int fp64_mode,
+                                              double* obj_out, int32_t* n_obj_out, int32_t* img_out, int32_t* n_valid_out,
+                                              double* err_out, int32_t* cand_out, int32_t* flags_out,
+                                              void* workspace, size_t workspace_bytes, void* stream)
+{
+    return correspond_blocked(xy_dev, count_dev, S, C, max_pts, cams_per_block, F_dev, cams_dev, cutoff, obj_count, max_groups, fp64_mode,
+                              obj_out, n_obj_out, img_out, n_valid_out, err_out, cand_out, flags_out, workspace, workspace_bytes, stream);
+}
+
+extern "C" int mocap_correspond_batch_subpixel(const float* xy_dev, const int32_t* count_dev, int S, int C, int max_pts, int cams_per_block,
+                                               const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
+                                               int max_groups, int fp64_mode,
+                                               double* obj_out, int32_t* n_obj_out, float* img_out, int32_t* n_valid_out,
+                                               double* err_out, int32_t* cand_out, int32_t* flags_out,
+                                               void* workspace, size_t workspace_bytes, void* stream)
+{
+    return correspond_blocked(xy_dev, count_dev, S, C, max_pts, cams_per_block, F_dev, cams_dev, cutoff, obj_count, max_groups, fp64_mode,
+                              obj_out, n_obj_out, img_out, n_valid_out, err_out, cand_out, flags_out, workspace, workspace_bytes, stream);
+}
+
+extern "C" int mocap_correspond_batch(const int32_t* xy_dev, const int32_t* count_dev, int S, int C, int max_pts,
+                                      const double* F_dev, const double* cams_dev, double cutoff, int obj_count,
+                                      int max_groups, int fp64_mode,
+                                      double* obj_out, int32_t* n_obj_out, int32_t* img_out, int32_t* n_valid_out,
+                                      double* err_out, int32_t* cand_out, int32_t* flags_out,
+                                      void* workspace, size_t workspace_bytes, void* stream)
+{
+    return correspond_blocked(xy_dev, count_dev, S, C, max_pts, C, F_dev, cams_dev, cutoff, obj_count, max_groups, fp64_mode,
+                              obj_out, n_obj_out, img_out, n_valid_out, err_out, cand_out, flags_out, workspace, workspace_bytes, stream);
 }

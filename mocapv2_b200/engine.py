@@ -49,17 +49,18 @@ def pack_cameras(camera_poses, camera_params) -> np.ndarray:
 
 @dataclass
 class DetectResult:
-    xy: torch.Tensor                 # [n, max_blobs, 2] int32, reference output order
+    xy: torch.Tensor                 # [n, max_blobs, 2] int32 (float32 sub-pixel centroids), reference output order
     count: torch.Tensor              # [n] int32 (0 == the reference's [[None, None]])
     flags: torch.Tensor              # [n] int32 MOCAP_FLAG_*
     extras: dict = field(default_factory=dict)
 
     def points(self, i: int):
-        """Frame i as the reference returns it: [[x, y], ...] Python ints, or [[None, None]]."""
+        """Frame i as the reference returns it: [[x, y], ...] Python ints (floats for sub-pixel centroids), or [[None, None]]."""
         n = int(self.count[i])
         if n == 0:
             return [[None, None]]
-        return [[int(a), int(b)] for a, b in self.xy[i, :n].tolist()]
+        conv = float if self.xy.dtype == torch.float32 else int
+        return [[conv(a), conv(b)] for a, b in self.xy[i, :n].tolist()]
 
 
 @dataclass
@@ -80,7 +81,7 @@ class LensSet:
 class CorrespondResult:
     obj: torch.Tensor        # [S, max_pts, 3] float64, sorted by mean error, first n_obj valid
     n_obj: torch.Tensor      # [S]
-    img: torch.Tensor        # [S, max_pts, C, 2] int32, first n_valid valid (root order)
+    img: torch.Tensor        # [S, max_pts, C, 2] in the dtype of the centroid lists (int32 / float32), first n_valid valid (root order)
     n_valid: torch.Tensor    # [S]
     err: torch.Tensor        # [S, max_pts] float64 mean error per complete root (root order)
     flags: torch.Tensor      # [S]
@@ -251,9 +252,10 @@ class CaptureEngine:
         max_runs = 4 * H + 4096 if max_runs is None else int(max_runs)
         return max_blobs, max_contours, max_runs
 
-    def _detect_prologue(self, frames, K, dist, lenses, frame_lens, caps, outputs, out):
+    def _detect_prologue(self, frames, K, dist, lenses, frame_lens, caps, outputs, out, subpixel):
         """What both detection calls check and prepare: contiguous frames and their stride, the caps, the lens set (K / dist: the
-        one-lens set of its table) with the per-frame indices as an int32 device tensor [n] (or None: lens 0), and the outputs."""
+        one-lens set of its table) with the per-frame indices as an int32 device tensor [n] (or None: lens 0), and the outputs
+        (centroids int32, float32 with subpixel)."""
         if lenses is not None and (K is not None or dist is not None):
             raise ValueError("pass either K / dist or lenses=, not both")
         if lenses is None and (K is None or dist is None):
@@ -279,9 +281,12 @@ class CaptureEngine:
             frame_lens = frame_lens.to(device=self.device, dtype=torch.int32).contiguous()
             if tuple(frame_lens.shape) != (n,):
                 raise ValueError(f"frame_lens must be [{n}]")
+        xy_dtype = torch.float32 if subpixel else torch.int32
         if out is None:
-            out = DetectResult(self.empty((n, max_blobs, 2), torch.int32), self.empty((n,), torch.int32),
+            out = DetectResult(self.empty((n, max_blobs, 2), xy_dtype), self.empty((n,), torch.int32),
                                self.empty((n,), torch.int32))
+        else:
+            self._check_dev(out.xy, xy_dtype, "out.xy")                # the centroid format of the call
         ex = out.extras
         if "bits" in outputs and "bits" not in ex:
             ex["bits"] = self.empty((n, H, (W + 31) // 32), torch.int32)
@@ -297,28 +302,32 @@ class CaptureEngine:
 
     def detect(self, frames: torch.Tensor, K=None, dist=None, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
                max_blobs=None, max_contours=None, max_runs=None, outputs=(), out: DetectResult | None = None,
-               timer=None, lenses: LensSet | None = None, frame_lens=None) -> DetectResult:
+               timer=None, lenses: LensSet | None = None, frame_lens=None, subpixel=False) -> DetectResult:
         """_find_dot(img)[1] for a batch (lib/ImageOperations.py:33-78).  frames: [n, H, W] uint8 on the device.
+
+        subpixel=False: int32 centroids, int(m10/m00) like the reference.  subpixel=True: float32 centroids, the float32 nearest to
+        m10/m00 (include/mocap_b200.h); everything else is the same.
 
         outputs: any of "bits", "labels", "blob_sums", "contours" (parity outputs, see include/mocap_b200.h).
         lenses (from lens_set(), in place of K / dist): frame i is undistorted with lens frame_lens[i] ([n] int, None: lens 0);
         an index outside the set gives the frame count 0 and FLAG_LENS_INDEX.
         """
         frames, stride, caps, lenses, fl, out = self._detect_prologue(frames, K, dist, lenses, frame_lens,
-                                                                      (max_blobs, max_contours, max_runs), outputs, out)
+                                                                      (max_blobs, max_contours, max_runs), outputs, out, subpixel)
         n, H, W = frames.shape
         ex = out.extras
         nbytes = self.lib.mocap_detect_workspace_bytes(n, H, W, *caps)
         if nbytes == 0:
             raise _cabi.MocapError("mocap_detect_workspace_bytes: unsupported shape")
         ws = self._workspace(nbytes)
-        st = self.lib.mocap_detect_batch(
+        name = "mocap_detect_batch_subpixel" if subpixel else "mocap_detect_batch"
+        st = getattr(self.lib, name)(
             self._ptr(frames), n, H, W, stride, ctypes.byref(lenses.cabi(fl)), int(thresh), float(min_area), float(min_circ), *caps,
             self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags),
             self._ptr(ex.get("bits")), self._ptr(ex.get("labels")), self._ptr(ex.get("blob_sums")),
             self._ptr(ex.get("blob_count")), self._ptr(ex.get("contours")), self._ptr(ex.get("contour_count")),
             self._ptr(ws), nbytes, self._stream(), ctypes.c_void_p(timer) if timer else ctypes.c_void_p(0))
-        _cabi.check(self.lib, st, "mocap_detect_batch")
+        _cabi.check(self.lib, st, name)
         if fl is not None:
             self._retire(fl)
         # scan, group, filter pieces, candidates, traces+finalize + the general path's mark / compact / tiles / blobs
@@ -341,17 +350,18 @@ class CaptureEngine:
     def detect_pipelined(self, frames: torch.Tensor, K=None, dist=None, *, thresh=THRESH_U8, min_area=MIN_AREA, min_circ=MIN_CIRC,
                          max_blobs=None, max_contours=None, max_runs=None, outputs=(), out: DetectResult | None = None,
                          chunk_frames=128, timeline=False, cellbox: torch.Tensor | None = None,
-                         lenses: LensSet | None = None, frame_lens=None, scatter=None, scan_token=None) -> DetectResult:
+                         lenses: LensSet | None = None, frame_lens=None, scatter=None, scan_token=None, subpixel=False) -> DetectResult:
         """Same results as detect() (centroid lists, optionally the contour table), computed chunk by chunk with the streaming
         scan overlapped with the other stages (mocap_detect_batch_pipelined).  cellbox: the frames' hot cell boxes from
         bayer_gr2gray_scan (same thresh) -- the call then has no streaming scan.  lenses / frame_lens as in detect().
         scatter=(xy_dst, count_dst): per-frame destination addresses (int64 device tensors [n]) of the store-to-peer epilogue.
         scan_token=(wait, done): torch.cuda.Event objects (recorded at least once, or None) the call's streaming scan waits for and
-        records behind it; StepsInFlight chains the scans of its lanes this way."""
+        records behind it; StepsInFlight chains the scans of its lanes this way.  subpixel as in detect(); the scatter destinations
+        then receive float32 pairs."""
         if any(o != "contours" for o in outputs):
             raise ValueError("detect_pipelined offers the contour table only; use detect() for bits / labels / blob_sums")
         frames, stride, caps, lenses, fl, out = self._detect_prologue(frames, K, dist, lenses, frame_lens,
-                                                                      (max_blobs, max_contours, max_runs), outputs, out)
+                                                                      (max_blobs, max_contours, max_runs), outputs, out, subpixel)
         n, H, W = frames.shape
         ex = out.extras
         nbytes = self.lib.mocap_detect_pipelined_workspace_bytes(n, H, W, *caps, int(chunk_frames))
@@ -368,12 +378,13 @@ class CaptureEngine:
                 self._check_dev(t, torch.int64, "scatter")
         wait, done = scan_token if scan_token is not None else (None, None)
         ev = lambda e: ctypes.c_void_p(int(e.cuda_event)) if e is not None else ctypes.c_void_p(0)
-        st = self.lib.mocap_detect_batch_pipelined(
+        name = "mocap_detect_batch_pipelined_subpixel" if subpixel else "mocap_detect_batch_pipelined"
+        st = getattr(self.lib, name)(
             self._pipe(), self._ptr(frames), n, H, W, stride, ctypes.byref(lenses.cabi(fl)), int(thresh), float(min_area), float(min_circ),
             *caps, self._ptr(out.xy), self._ptr(out.count), self._ptr(out.flags), self._ptr(ex.get("contours")),
             self._ptr(ex.get("contour_count")), self._ptr(cellbox), self._ptr(xy_dst), self._ptr(count_dst), ev(wait), ev(done),
             self._ptr(ws), nbytes, self._stream(), int(chunk_frames), 1 if timeline else 0)
-        _cabi.check(self.lib, st, "mocap_detect_batch_pipelined")
+        _cabi.check(self.lib, st, name)
         for t in (fl, xy_dst, count_dst):
             if t is not None:
                 self._retire(t)
@@ -602,11 +613,14 @@ class CaptureEngine:
                    cutoff=EPI_CUTOFF, max_groups=4096, fp64=False, want_cand=False, out: CorrespondResult | None = None) -> CorrespondResult:
         """find_point_correspondance_and_object_points (lib/Helpers.py:178-280) for S frame-sets.
 
-        xy [S, C, max_pts, 2] int32 centroid lists, count [S, C] int32, Fs [C-1, 3, 3] float64 (Fs[i-1]: camera 0 -> camera i).
+        xy [S, C, max_pts, 2] centroid lists, count [S, C] int32, Fs [C-1, 3, 3] float64 (Fs[i-1]: camera 0 -> camera i).
+        xy is int32 (whole-pixel centroids) or float32 (sub-pixel, detect(subpixel=True)); res.img has the dtype of xy.
         Camera-blocked input (what the shard exchange of the multi-GPU pipeline delivers) is read in place:
         xy [B, S, C/B, max_pts, 2], count [B, S, C/B] with block b holding cameras b*C/B .. (b+1)*C/B - 1.
         """
-        xy = self._check_dev(xy, torch.int32, "xy")
+        if xy.dtype not in (torch.int32, torch.float32):
+            raise ValueError(f"xy: centroid lists must be int32 or float32, not {xy.dtype}")
+        xy = self._check_dev(xy, xy.dtype, "xy")
         count = self._check_dev(count, torch.int32, "count")
         cams = self._check_dev(cams, torch.float64, "cams")
         if xy.dim() == 5:
@@ -623,19 +637,22 @@ class CaptureEngine:
                 raise IndexError("Fs shorter than camera count - 1")        # the reference raises IndexError (Helpers.py:206)
         res = out if out is not None else CorrespondResult(
             obj=torch.zeros((S, max_pts, 3), dtype=torch.float64, device=self.device), n_obj=self.empty((S,), torch.int32),
-            img=torch.zeros((S, max_pts, C, 2), dtype=torch.int32, device=self.device), n_valid=self.empty((S,), torch.int32),
+            img=torch.zeros((S, max_pts, C, 2), dtype=xy.dtype, device=self.device), n_valid=self.empty((S,), torch.int32),
             err=torch.zeros((S, max_pts), dtype=torch.float64, device=self.device), flags=self.empty((S,), torch.int32),
             cand=self.empty((S, max_pts, C, _cabi.MAX_CAND), torch.int32) if want_cand else None)
+        if out is not None:
+            self._check_dev(res.img, xy.dtype, "out.img")              # written in the centroid format of xy
         if S == 0:
             return res
         nbytes = self.lib.mocap_correspond_workspace_bytes(S, C, max_pts, max_groups)
         ws = self._workspace(nbytes)
-        st = self.lib.mocap_correspond_batch_blocked(
+        name = "mocap_correspond_batch_subpixel" if xy.dtype == torch.float32 else "mocap_correspond_batch_blocked"
+        st = getattr(self.lib, name)(
             self._ptr(xy), self._ptr(count), S, C, max_pts, cpb, self._ptr(Fs) if C > 1 else ctypes.c_void_p(0), self._ptr(cams),
             float(cutoff), int(obj_count), int(max_groups), 1 if fp64 else 0,
             self._ptr(res.obj), self._ptr(res.n_obj), self._ptr(res.img), self._ptr(res.n_valid), self._ptr(res.err),
             self._ptr(res.cand), self._ptr(res.flags), self._ptr(ws), nbytes, self._stream())
-        _cabi.check(self.lib, st, "mocap_correspond_batch_blocked")
+        _cabi.check(self.lib, st, name)
         return res
 
 

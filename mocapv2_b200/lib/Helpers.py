@@ -205,7 +205,9 @@ def bundle_adjustment(image_points, camera_poses):
 def find_point_correspondance_and_object_points(image_points, camera_poses, obj_count=0, debug=False):
     """image_points shape = [camera_count, obj points, 2] -> (object_points sorted by error, image_points_all).
 
-    Mutates the per-camera lists like the reference (one [None, None] removed from each, Helpers.py:184-188)."""
+    Mutates the per-camera lists like the reference (one [None, None] removed from each, Helpers.py:184-188).
+    The points are whole pixels (the output of _find_dot; image_points_all int64) or sub-pixel centroids whose every coordinate is a
+    float32 value (the output of _find_dot(..., subpixel=True); image_points_all float64, as the reference returns float lists)."""
     read_camera_params()
     for image_points_i in image_points:
         try:
@@ -222,12 +224,17 @@ def find_point_correspondance_and_object_points(image_points, camera_poses, obj_
     lists = []
     for cam in list(image_points)[:C]:
         pts = [p for p in np.asarray(cam, dtype=object).reshape(-1, 2).tolist() if not _is_none(p)] if len(cam) else []
-        arr = np.asarray(pts, dtype=np.float64).reshape(-1, 2)
-        if arr.size and not np.array_equal(arr, np.rint(arr)):
-            raise ValueError("image points must be integer pixel coordinates (the output of _find_dot)")
-        lists.append(arr.astype(np.int32))
+        lists.append(np.asarray(pts, dtype=np.float64).reshape(-1, 2))
+    if all(np.array_equal(a, np.rint(a)) for a in lists):
+        dtype = np.int32
+    elif all(np.array_equal(a, a.astype(np.float32)) for a in lists):
+        dtype = np.float32                                       # sub-pixel centroids: every coordinate exactly a float32 value
+    else:
+        raise ValueError("image points must be integer pixel coordinates (the output of _find_dot) or float32 values "
+                         "(the output of _find_dot(..., subpixel=True))")
+    lists = [a.astype(dtype) for a in lists]
     max_pts = max(1, max(len(a) for a in lists))
-    xy = np.zeros((1, C, max_pts, 2), dtype=np.int32)
+    xy = np.zeros((1, C, max_pts, 2), dtype=dtype)
     cnt = np.zeros((1, C), dtype=np.int32)
     for c, a in enumerate(lists):
         cnt[0, c] = len(a)
@@ -244,4 +251,4 @@ def find_point_correspondance_and_object_points(image_points, camera_poses, obj_
     nv, no = int(res.n_valid[0]), int(res.n_obj[0])
     if nv == 0:
         return np.array([]), np.array([])
-    return res.obj[0, :no].cpu().numpy(), res.img[0, :nv].cpu().numpy().astype(np.int64)
+    return res.obj[0, :no].cpu().numpy(), res.img[0, :nv].cpu().numpy().astype(np.int64 if dtype == np.int32 else np.float64)

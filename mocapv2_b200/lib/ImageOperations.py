@@ -2,7 +2,8 @@
 
 Same names and conventions as the reference module:
   _find_dot(img, print_location=False, return_filtered=False) -> (img, image_points)   lib/ImageOperations.py:33-78
-    (+ keyword camera_number: undistort with that camera's calibration instead of camera 0's)
+    (+ keyword camera_number: undistort with that camera's calibration instead of camera 0's;
+     keyword subpixel: float centroids m10/m00 rounded to float32 instead of int(m10/m00))
   image_filter_gpu(image, camera_number=0)                                             lib/ImageOperations.py:23-31
   module globals `camera_params`, `intrinsics_json`, `cuda_lock` stay assignable.
 All arithmetic runs in libmocap_b200.so on the GPU (undistort + 5x5 floor-mean + threshold + 5x5 majority +
@@ -71,13 +72,13 @@ def image_filter_gpu(image, camera_number=0):
     return (np.unpackbits(b, axis=1, bitorder="little")[:, :W] * 255).astype(np.uint8)
 
 
-def _detect_one(eng, fr, K, dist, outputs):
+def _detect_one(eng, fr, K, dist, outputs, subpixel):
     """eng.detect on one frame; capacity overflows (MOCAP_FLAG_*_OVERFLOW: more blobs / contours / runs than the default
     caps hold) are never returned as a silently short list -- the call is repeated with larger caps, like the reference,
     which has none (lib/ImageOperations.py:41-65)."""
     caps = {}
     for attempt in range(6):
-        res = eng.detect(fr, K, dist, outputs=outputs, **caps)
+        res = eng.detect(fr, K, dist, outputs=outputs, subpixel=subpixel, **caps)
         flags = int(res.flags[0])                              # device -> host read of the result
         if not flags & _cabi.FLAG_ERRORS:
             return res
@@ -87,11 +88,14 @@ def _detect_one(eng, fr, K, dist, outputs):
     raise _cabi.MocapError(f"_find_dot: detection capacity exceeded even with caps {caps} (flags {flags})")
 
 
-def _find_dot(img, print_location=False, return_filtered=False, *, camera_number=None):
+def _find_dot(img, print_location=False, return_filtered=False, *, camera_number=None, subpixel=False):
     """output: image with dot and dot coordinates -- (img, [[x, y], ...]) or (img, [[None, None]]).
 
     camera_number=None undistorts with camera 0's calibration, like lib/ImageOperations.py:36-38; an integer selects
-    camera_params[camera_number] (the lens of the camera the frame comes from; a short list raises IndexError)."""
+    camera_params[camera_number] (the lens of the camera the frame comes from; a short list raises IndexError).
+    subpixel=False returns int(m10/m00), int(m01/m00) like the reference (:59-62); subpixel=True returns Python floats, the
+    float32 nearest to m10/m00 and m01/m00 -- the same blobs in the same order, without the reference's truncation bias of about
+    half a pixel.  find_point_correspondance_and_object_points takes either."""
     eng = _engine.default_engine()
     cp = _params()[0 if camera_number is None else camera_number]
     K = np.array(cp["intrinsic_matrix"], dtype=np.float64)
@@ -102,10 +106,10 @@ def _find_dot(img, print_location=False, return_filtered=False, *, camera_number
         if not ANNOTATE and not return_filtered:
             # everything of the call is queued before the first host read: H2D, the undistorted image and its way back, detection
             fetch = eng.download_image_async(eng.undistort(fr, K, dist)[0])
-            res = _detect_one(eng, fr, K, dist, ())
+            res = _detect_one(eng, fr, K, dist, (), subpixel)
         else:
             # with the reference's overlays: the contour outline needs the binary image and the contour table of the same call
-            res = _detect_one(eng, fr, K, dist, ("bits", "contours"))
+            res = _detect_one(eng, fr, K, dist, ("bits", "contours"), subpixel)
             if return_filtered:                               # the reference then draws on (and returns) the filtered image (:53)
                 b = res.extras["bits"][0].cpu().numpy().view(np.uint8)
                 canvas = eng.upload_image((np.unpackbits(b, axis=1, bitorder="little")[:, :W] * 255).astype(np.uint8))
@@ -121,6 +125,7 @@ def _find_dot(img, print_location=False, return_filtered=False, *, camera_number
         try:                                                  # display-only overlays (lib/ImageOperations.py:67-73)
             import cv2 as cv
             for i, (x, y) in enumerate(image_points):
+                x, y = int(x), int(y)                         # (sub-pixel centroids: drawn at the truncated pixel)
                 label = f"({x}, {y})" if print_location else str(i)
                 org = (x - 240, y - 15) if print_location else (x - 20, y - 15)
                 cv.putText(out, label, org, cv.FONT_HERSHEY_SIMPLEX, 2, (0, 0, 255), 4)

@@ -36,7 +36,7 @@ class StepResult:
 
 class CapturePipeline:
     def __init__(self, engine: CaptureEngine, rig: dict, *, max_blobs=160, obj_count=None, max_groups=64, fp64=False,
-                 group=None, lens="camera0"):
+                 group=None, lens="camera0", centroids="int"):
         self.eng = engine
         self.rig = rig
         self.C = len(rig["poses"])
@@ -58,6 +58,13 @@ class CapturePipeline:
         if lens not in ("camera0", "per_camera"):
             raise ValueError(f"lens must be 'camera0' or 'per_camera', not {lens!r}")
         self.lens = lens
+        # centroids="int": int(m10/m00) like _find_dot (lib/ImageOperations.py:59-62).  centroids="subpixel": the float32 nearest to
+        # m10/m00 -- the same 8-byte records, so the exchange moves the same bytes; the matching then reads float32 lists.
+        if centroids not in ("int", "subpixel"):
+            raise ValueError(f"centroids must be 'int' or 'subpixel', not {centroids!r}")
+        self.centroids = centroids
+        self.subpixel = centroids == "subpixel"
+        self.xy_dtype = torch.float32 if self.subpixel else torch.int32
         self.K0 = np.asarray(rig["camera_params"][0]["intrinsic_matrix"], dtype=np.float64)
         self.dist0 = np.asarray(rig["camera_params"][0]["distortion_coef"], dtype=np.float64)
         self.lenses = None
@@ -89,7 +96,7 @@ class CapturePipeline:
         """Detection outputs of n frames [FS * cams_local, ...] (frame-set major: the slice of a destination rank is contiguous)."""
         if self._det is None or self._det.xy.shape[0] != n:
             mb = self.max_blobs
-            self._det = DetectResult(torch.zeros((n, mb, 2), dtype=torch.int32, device=self.eng.device),
+            self._det = DetectResult(torch.zeros((n, mb, 2), dtype=self.xy_dtype, device=self.eng.device),
                                      torch.zeros(n, dtype=torch.int32, device=self.eng.device),
                                      torch.zeros(n, dtype=torch.int32, device=self.eng.device))
             self._rx = None
@@ -125,11 +132,11 @@ class CapturePipeline:
                 peer["turn"] ^= 1
             self._det = self.eng.detect_pipelined(flat, max_blobs=self.max_blobs, out=buf, chunk_frames=chunk, timeline=timeline,
                                                   cellbox=cellbox, scatter=peer["tables"][peer["turn"]] if peer is not None else None,
-                                                  scan_token=self.scan_token, **lens_kw)
+                                                  scan_token=self.scan_token, subpixel=self.subpixel, **lens_kw)
             if peer is not None:
                 self._det.extras["peer_turn"] = peer["turn"]       # the result knows which receive buffers hold its records
         else:
-            self._det = self.eng.detect(flat, max_blobs=self.max_blobs, out=buf, timer=timer, **lens_kw)
+            self._det = self.eng.detect(flat, max_blobs=self.max_blobs, out=buf, timer=timer, subpixel=self.subpixel, **lens_kw)
         return self._det
 
     def _peer_setup(self, FS: int):
@@ -160,7 +167,7 @@ class CapturePipeline:
                 xy_dst = (base[dst] + slot * (mb * 2 * 4)).to(self.eng.device)
                 cnt_dst = (base[dst] + (xy_elems + slot) * 4).to(self.eng.device)
                 bufs.append(buf); hdls.append(hdl); tables.append((xy_dst, cnt_dst))
-                views.append((buf[:xy_elems].view(self.world, per, cl, mb, 2), buf[xy_elems:].view(self.world, per, cl)))
+                views.append((buf[:xy_elems].view(self.xy_dtype).view(self.world, per, cl, mb, 2), buf[xy_elems:].view(self.world, per, cl)))
             self._peer = {"bufs": bufs, "hdls": hdls, "tables": tables, "views": views, "turn": 1, "per": per}
         except Exception as ex:                                            # no peer mapping on this box: NCCL send/recv it is
             import warnings
@@ -185,7 +192,7 @@ class CapturePipeline:
             self.collectives += 1
             return peer["views"][turn]
         if self._rx is None or self._rx[0].shape[1] != per:
-            self._rx = (torch.empty((self.world, per, cl, mb, 2), dtype=torch.int32, device=self.eng.device),
+            self._rx = (torch.empty((self.world, per, cl, mb, 2), dtype=self.xy_dtype, device=self.eng.device),
                         torch.empty((self.world, per, cl), dtype=torch.int32, device=self.eng.device))
         rxy, rcnt = self._rx
         sxy = det.xy.view(self.world, per, cl, mb, 2)                  # [destination rank][its frame-sets][my cameras]
@@ -232,7 +239,7 @@ class StepsInFlight:
         for _ in range(self.depth - 1):
             eng = pipe.eng.clone()                                 # same library, device and calibration tables
             lane = CapturePipeline(eng, pipe.rig, max_blobs=pipe.max_blobs, obj_count=pipe.obj_count, max_groups=pipe.max_groups,
-                                   fp64=pipe.fp64, group=pipe.group, lens=pipe.lens)
+                                   fp64=pipe.fp64, group=pipe.group, lens=pipe.lens, centroids=pipe.centroids)
             lane.pipelined_min_frames = pipe.pipelined_min_frames
             lane.peer_exchange = pipe.peer_exchange
             self.lanes.append(lane)
