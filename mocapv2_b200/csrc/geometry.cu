@@ -10,6 +10,7 @@
 // point (or candidate group) per thread, FP32 main mode and FP64 check mode (template parameter).  No tensor
 // cores: these are tiny independent solves, not dense contractions.
 #include "common.cuh"
+#include <type_traits>
 
 #define CAM_P 0
 #define CAM_R 12
@@ -27,26 +28,6 @@ static inline float sfu_rcp(float x) { return 1.0f / x; }
 __device__ __forceinline__ float sfu_rsqrt(float x) { float y; asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float sfu_rcp(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 #endif
-
-template <typename T> struct Num;
-template <> struct Num<float> {
-    static __device__ __forceinline__ float sqrt_(float x) { return sqrtf(x); }
-    static __device__ __forceinline__ float abs_(float x) { return fabsf(x); }
-    static __device__ __forceinline__ float tiny() { return 1e-30f; }
-    // Jacobi rotations are self-correcting: an angle that is off by a few ulp only leaves a slightly larger off-diagonal
-    // for the next sweep, so the FP32 main mode uses the SFU reciprocal / rsqrt (the FP64 check mode stays IEEE)
-    static __device__ __forceinline__ float rcp_(float x) { return __frcp_rn(x); }
-    static __device__ __forceinline__ float rsqrt_(float x) { return rsqrtf(x); }
-    static constexpr int sweeps = 8;
-};
-template <> struct Num<double> {
-    static __device__ __forceinline__ double sqrt_(double x) { return sqrt(x); }
-    static __device__ __forceinline__ double abs_(double x) { return fabs(x); }
-    static __device__ __forceinline__ double tiny() { return 1e-280; }
-    static __device__ __forceinline__ double rcp_(double x) { return 1.0 / x; }
-    static __device__ __forceinline__ double rsqrt_(double x) { return 1.0 / sqrt(x); }
-    static constexpr int sweeps = 12;
-};
 
 // Smallest-eigenvalue eigenvector of a symmetric PSD 4x4 (upper triangle a[10]: 00 01 02 03 11 12 13 22 23 33).
 // FP32 main mode: FIVE cyclic sweeps, no data-dependent branch (the lanes of a warp never diverge, nothing is tested between
@@ -99,77 +80,71 @@ __device__ __forceinline__ void jacobi_min_eigvec_f32(float b00, float b01, floa
     }
 }
 
-template <typename T>
-__device__ __forceinline__ void jacobi_min_eigvec(T b00, T b01, T b02, T b03, T b11, T b12, T b13, T b22, T b23, T b33, T v[4])
+// FP64 check mode: IEEE theta / tau rotations, up to twelve cyclic sweeps; the solve ends at a sweep that starts diagonal, and from
+// the fourth sweep on an off-diagonal that no longer registers against either diagonal entry is dropped without a rotation (the
+// classic Jacobi shortcut), so the last sweeps cost almost nothing.
+__device__ __forceinline__ void jacobi_min_eigvec_f64(double b00, double b01, double b02, double b03, double b11, double b12,
+                                                      double b13, double b22, double b23, double b33, double v[4])
 {
-    T A[4][4] = {{b00, b01, b02, b03}, {b01, b11, b12, b13}, {b02, b12, b22, b23}, {b03, b13, b23, b33}};
-    T V[4][4] = {{1, 0, 0, 0}, {0, 1, 0, 0}, {0, 0, 1, 0}, {0, 0, 0, 1}};
+    double A[4][4] = {{b00, b01, b02, b03}, {b01, b11, b12, b13}, {b02, b12, b22, b23}, {b03, b13, b23, b33}};
+    double V[4][4] = {{1, 0, 0, 0}, {0, 1, 0, 0}, {0, 0, 1, 0}, {0, 0, 0, 1}};
 #pragma unroll 1
-    for (int sweep = 0; sweep < Num<T>::sweeps; ++sweep) {
-        T off = Num<T>::abs_(A[0][1]) + Num<T>::abs_(A[0][2]) + Num<T>::abs_(A[0][3]) +
-                Num<T>::abs_(A[1][2]) + Num<T>::abs_(A[1][3]) + Num<T>::abs_(A[2][3]);
-        if (off == (T)0) break;
+    for (int sweep = 0; sweep < 12; ++sweep) {
+        const double off = fabs(A[0][1]) + fabs(A[0][2]) + fabs(A[0][3]) + fabs(A[1][2]) + fabs(A[1][3]) + fabs(A[2][3]);
+        if (off == 0.0) break;
 #pragma unroll
         for (int p = 0; p < 3; ++p) {
 #pragma unroll
             for (int q = p + 1; q < 4; ++q) {
-                T apq = A[p][q];
-                // after the first sweeps an off-diagonal that no longer registers against either diagonal entry is dropped
-                // without a rotation (the classic Jacobi shortcut), so the last sweeps cost almost nothing
-                if (sweep >= 3 && apq != (T)0) {
-                    T g = (T)100 * Num<T>::abs_(apq), dp = Num<T>::abs_(A[p][p]), dq = Num<T>::abs_(A[q][q]);
-                    if (g + dp == dp && g + dq == dq) { A[p][q] = (T)0; A[q][p] = (T)0; apq = (T)0; }
+                double apq = A[p][q];
+                if (sweep >= 3 && apq != 0.0) {
+                    const double g = 100.0 * fabs(apq), dp = fabs(A[p][p]), dq = fabs(A[q][q]);
+                    if (g + dp == dp && g + dq == dq) { A[p][q] = 0.0; A[q][p] = 0.0; apq = 0.0; }
                 }
-                if (sizeof(T) == 4 && apq != (T)0) {
-                    // FP32 main mode: the rotation from delta = aqq - app directly, t = 2 apq / (delta + sign(delta) sqrt(delta^2 +
-                    // 4 apq^2)), applied as (c, s) -- three SFU operations (sqrt, rcp, rsqrt) instead of the five of the theta /
-                    // tau form below, which the FP64 check mode keeps
-                    T dl = A[q][q] - A[p][p], two = (T)2 * apq;
-                    T r = Num<T>::sqrt_(dl * dl + two * two);
-                    T t = two * Num<T>::rcp_(dl + (dl < (T)0 ? -r : r));
-                    T c = Num<T>::rsqrt_(t * t + (T)1), s = t * c;
-                    A[p][p] -= t * apq; A[q][q] += t * apq; A[p][q] = (T)0; A[q][p] = (T)0;
+                if (apq == 0.0) continue;
+                const double theta = (A[q][q] - A[p][p]) * (1.0 / (2.0 * apq));
+                const double at = fabs(theta);
+                double t;
+                if (at > 1e15) t = 0.5 * (1.0 / theta);                      // avoid theta^2 overflow
+                else { t = 1.0 / (at + sqrt(theta * theta + 1.0)); if (theta < 0.0) t = -t; }
+                const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+                const double tau = s * (1.0 / (1.0 + c));
+                A[p][p] -= t * apq; A[q][q] += t * apq; A[p][q] = 0.0; A[q][p] = 0.0;
 #pragma unroll
-                    for (int r2 = 0; r2 < 4; ++r2) {
-                        if (r2 != p && r2 != q) {
-                            T arp = A[r2][p], arq = A[r2][q];
-                            A[r2][p] = c * arp - s * arq; A[p][r2] = A[r2][p];
-                            A[r2][q] = s * arp + c * arq; A[q][r2] = A[r2][q];
-                        }
-                        T vrp = V[r2][p], vrq = V[r2][q];
-                        V[r2][p] = c * vrp - s * vrq;
-                        V[r2][q] = s * vrp + c * vrq;
+                for (int r = 0; r < 4; ++r) {
+                    if (r != p && r != q) {
+                        const double arp = A[r][p], arq = A[r][q];
+                        A[r][p] = arp - s * (arq + tau * arp); A[p][r] = A[r][p];
+                        A[r][q] = arq + s * (arp - tau * arq); A[q][r] = A[r][q];
                     }
-                } else if (apq != (T)0) {
-                    T theta = (A[q][q] - A[p][p]) * Num<T>::rcp_((T)2 * apq);
-                    T at = Num<T>::abs_(theta);
-                    T t;
-                    if (at > (T)1e15) t = (T)0.5 * Num<T>::rcp_(theta);         // avoid theta^2 overflow
-                    else { t = Num<T>::rcp_(at + Num<T>::sqrt_(theta * theta + (T)1)); if (theta < (T)0) t = -t; }
-                    T c = Num<T>::rsqrt_(t * t + (T)1), s = t * c;
-                    T tau = s * Num<T>::rcp_((T)1 + c);
-                    A[p][p] -= t * apq; A[q][q] += t * apq; A[p][q] = (T)0; A[q][p] = (T)0;
-#pragma unroll
-                    for (int r = 0; r < 4; ++r) {
-                        if (r != p && r != q) {
-                            T arp = A[r][p], arq = A[r][q];
-                            A[r][p] = arp - s * (arq + tau * arp); A[p][r] = A[r][p];
-                            A[r][q] = arq + s * (arp - tau * arq); A[q][r] = A[r][q];
-                        }
-                        T vrp = V[r][p], vrq = V[r][q];
-                        V[r][p] = vrp - s * (vrq + tau * vrp);
-                        V[r][q] = vrq + s * (vrp - tau * vrq);
-                    }
+                    const double vrp = V[r][p], vrq = V[r][q];
+                    V[r][p] = vrp - s * (vrq + tau * vrp);
+                    V[r][q] = vrq + s * (vrp - tau * vrq);
                 }
             }
         }
     }
     int k = 0;
-    T best = Num<T>::abs_(A[0][0]);
+    double best = fabs(A[0][0]);
 #pragma unroll
-    for (int i = 1; i < 4; ++i) { T e = Num<T>::abs_(A[i][i]); if (e < best) { best = e; k = i; } }
+    for (int i = 1; i < 4; ++i) { const double e = fabs(A[i][i]); if (e < best) { best = e; k = i; } }
 #pragma unroll
     for (int r = 0; r < 4; ++r) v[r] = (k == 0) ? V[r][0] : (k == 1) ? V[r][1] : (k == 2) ? V[r][2] : V[r][3];
+}
+
+// X = v[:3] / v[3] for the smallest eigenvector v of B (upper triangle b[10])
+__device__ __forceinline__ void dlt_solve(const float b[10], float X[3])
+{
+    float w[4];
+    jacobi_min_eigvec_f32(b[0], b[1], b[2], b[3], b[4], b[5], b[6], b[7], b[8], b[9], w);
+    const float iw = 1.0f / w[3];                          // one IEEE reciprocal instead of three divisions
+    X[0] = w[0] * iw; X[1] = w[1] * iw; X[2] = w[2] * iw;
+}
+__device__ __forceinline__ void dlt_solve(const double b[10], double X[3])
+{
+    double v[4];
+    jacobi_min_eigvec_f64(b[0], b[1], b[2], b[3], b[4], b[5], b[6], b[7], b[8], b[9], v);
+    X[0] = v[0] / v[3]; X[1] = v[1] / v[3]; X[2] = v[2] / v[3];
 }
 
 // twelve consecutive values (a 3x4 P, or R | t of a camera record): three 128-bit loads for floats that are 16-byte aligned
@@ -212,19 +187,7 @@ struct Accum {                          // B = A^T A accumulated view by view
         for (int c = 0; c < 4; ++c) { r1[c] = y * Pv[8 + c] - Pv[4 + c]; r2[c] = Pv[c] - x * Pv[8 + c]; }
         add_row(r1); add_row(r2);
     }
-    __device__ __forceinline__ void solve(T X[3]) {
-        T v[4];
-        if (sizeof(T) == 4) {
-            float w[4];
-            jacobi_min_eigvec_f32((float)b[0], (float)b[1], (float)b[2], (float)b[3], (float)b[4], (float)b[5], (float)b[6], (float)b[7],
-                                  (float)b[8], (float)b[9], w);
-            const float iw = 1.0f / w[3];                      // one IEEE reciprocal instead of three divisions
-            X[0] = (T)(w[0] * iw); X[1] = (T)(w[1] * iw); X[2] = (T)(w[2] * iw);
-            return;
-        }
-        jacobi_min_eigvec<T>(b[0], b[1], b[2], b[3], b[4], b[5], b[6], b[7], b[8], b[9], v);
-        X[0] = v[0] / v[3]; X[1] = v[1] / v[3]; X[2] = v[2] / v[3];
-    }
+    __device__ __forceinline__ void solve(T X[3]) { dlt_solve(b, X); }
 };
 
 // cv.projectPoints restated (SURVEY App. A9).  FP64: reproduces the float32 roundings of X and of (u, v).
@@ -311,6 +274,46 @@ template <> __device__ __forceinline__ void load_xy<float>(const float* p, float
 }
 #endif
 
+// for (c = 0; c < C; ++c) f(c): unrolled for a compile-time view count CT > 0 (C == CT), else a loop that is not unrolled at all (the
+// compiler's partial unrolling of the run-time view loops only adds instructions to the correspondence kernel)
+template <int CT, class F>
+__device__ __forceinline__ void for_views(int C, F f)
+{
+    if constexpr (CT > 0) {
+#pragma unroll
+        for (int c = 0; c < CT; ++c) f(c);
+    } else {
+#pragma unroll 1
+        for (int c = 0; c < C; ++c) f(c);
+    }
+}
+
+// DLT of one point seen by every view 0 .. C-1: X.  xy(c, x, y) supplies view c's image point.  With sq_residual_all_views (the sum of
+// the squared x and y residuals of X over the same views) this is the view loop of every caller whose views are all valid -- the generic
+// and the dense triangulation and each candidate group of the correspondence -- so they agree by construction.  The mean (division by
+// 2C) stays with the caller: correspondence averages it again over a root's groups.
+template <typename T, int CT, class XY>
+__device__ __forceinline__ void dlt_all_views(const T* cams, int C, XY xy, T X[3])
+{
+    Accum<T> acc; acc.clear();
+    for_views<CT>(C, [&](int c) { T x, y; xy(c, x, y); acc.add_view(cams + c * CAM_T_STRIDE + CAM_P, x, y); });
+    acc.solve(X);
+}
+
+template <typename T, int CT, class XY>
+__device__ __forceinline__ T sq_residual_all_views(const T* cams, int C, XY xy, const T X[3])
+{
+    T s = (T)0;
+    for_views<CT>(C, [&](int c) {
+        T u, v, x, y;
+        project<T>(cams + c * CAM_T_STRIDE + CAM_R, cams + c * CAM_T_STRIDE + CAM_K, X, u, v);
+        xy(c, x, y);
+        const T dx = x - u, dy = y - v;
+        s += dx * dx; s += dy * dy;
+    });
+    return s;
+}
+
 template <typename T, bool TRIANGULATE>
 __global__ void __launch_bounds__(128) triangulate_kernel(const T* __restrict__ pts, const uint8_t* __restrict__ valid,
                                                           const T* __restrict__ xyz_in, const double* __restrict__ cams,
@@ -328,15 +331,23 @@ __global__ void __launch_bounds__(128) triangulate_kernel(const T* __restrict__ 
         const T* p = pts + (size_t)i * C * 2;
         const uint8_t* vm = valid ? valid + (size_t)i * C : nullptr;
         T X[3];
+        if (TRIANGULATE && !vm && C > 1) {
+            auto xy = [&](int c, T& x, T& y) { load_xy(p + 2 * c, x, y); };
+            dlt_all_views<T, 0>(sm, C, xy, X);
+            if (xyz_out) { xyz_out[(size_t)i * 3] = X[0]; xyz_out[(size_t)i * 3 + 1] = X[1]; xyz_out[(size_t)i * 3 + 2] = X[2]; }
+            if (err_out) err_out[i] = sq_residual_all_views<T, 0>(sm, C, xy, X) / (T)(2 * C);
+            continue;
+        }
+        // with a mask, P and the residual take K of the view's rank among the valid views (make_P); given points are reprojected here too
         int nv = 0;
         if (TRIANGULATE) {
             Accum<T> acc; acc.clear();
             for (int c = 0; c < C; ++c) {
                 if (vm && !vm[c]) continue;
-                T x, y;
+                T x, y, P[12];
                 load_xy(p + 2 * c, x, y);
-                if (vm) { T P[12]; make_P<T>(sm + nv * CAM_T_STRIDE, sm + c * CAM_T_STRIDE, P); acc.add_view(P, x, y); }
-                else acc.add_view(sm + c * CAM_T_STRIDE + CAM_P, x, y);
+                make_P<T>(sm + nv * CAM_T_STRIDE, sm + c * CAM_T_STRIDE, P);
+                acc.add_view(P, x, y);
                 ++nv;
             }
             if (nv <= 1) { X[0] = X[1] = X[2] = nan; }
@@ -368,9 +379,8 @@ __global__ void __launch_bounds__(128) triangulate_kernel(const T* __restrict__ 
     }
 }
 
-// The bulk case of BASELINE config 5 (every point seen by all CT cameras, FP32, triangulation + reprojection error): the same
-// arithmetic as triangulate_kernel<float, true> with the view loops unrolled -- the camera records sit at constant shared-memory
-// offsets, no validity tests, no per-view address arithmetic (in the generic kernel ~45 of the ~150 instructions per view).
+// The bulk case of BASELINE config 5 (every point seen by all CT cameras, FP32): the image points of all CT views loaded into registers
+// up front, then the shared view loop unrolled, so the camera records sit at constant shared-memory offsets.
 template <int CT>
 __global__ void __launch_bounds__(128) triangulate_dense_f32_kernel(const float* __restrict__ pts, const double* __restrict__ cams,
                                                                     long long n, float* __restrict__ xyz_out, float* __restrict__ err_out)
@@ -383,23 +393,11 @@ __global__ void __launch_bounds__(128) triangulate_dense_f32_kernel(const float*
         float px[CT], py[CT];
 #pragma unroll
         for (int c = 0; c < CT; ++c) load_xy(p + 2 * c, px[c], py[c]);
-        Accum<float> acc; acc.clear();
-#pragma unroll
-        for (int c = 0; c < CT; ++c) acc.add_view(sm + c * CAM_T_STRIDE + CAM_P, px[c], py[c]);
         float X[3];
-        acc.solve(X);
+        auto xy = [&](int c, float& x, float& y) { x = px[c]; y = py[c]; };
+        dlt_all_views<float, CT>(sm, CT, xy, X);
         if (xyz_out) { xyz_out[(size_t)i * 3] = X[0]; xyz_out[(size_t)i * 3 + 1] = X[1]; xyz_out[(size_t)i * 3 + 2] = X[2]; }
-        if (err_out) {
-            float s = 0.f;
-#pragma unroll
-            for (int c = 0; c < CT; ++c) {
-                float u, v;
-                project<float>(sm + c * CAM_T_STRIDE + CAM_R, sm + c * CAM_T_STRIDE + CAM_K, X, u, v);
-                const float dx = px[c] - u, dy = py[c] - v;
-                s += dx * dx; s += dy * dy;
-            }
-            err_out[i] = s / (float)(2 * CT);
-        }
+        if (err_out) err_out[i] = sq_residual_all_views<float, CT>(sm, CT, xy, X) / (float)(2 * CT);
     }
 }
 
@@ -425,12 +423,14 @@ static int launch_tri(const void* pts, const uint8_t* valid, const void* xyz_in,
     auto k_rep = triangulate_kernel<T, false>;
     const T* no_in = nullptr;
     T* no_out = nullptr;
-    if (tri && sizeof(T) == 4 && !valid && n_sets == 1 && (C == 2 || C == 4 || C == 6 || C == 8 || C == 16)) {
-        if (C == 2) launch_dense<2>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s);
-        else if (C == 4) launch_dense<4>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s);
-        else if (C == 6) launch_dense<6>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s);
-        else if (C == 8) launch_dense<8>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s);
-        else launch_dense<16>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s);
+    if (tri && std::is_same<T, float>::value && !valid && n_sets == 1 && (C == 2 || C == 4 || C == 6 || C == 8 || C == 16)) {
+        switch (C) {
+        case 2: launch_dense<2>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s); break;
+        case 4: launch_dense<4>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s); break;
+        case 6: launch_dense<6>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s); break;
+        case 8: launch_dense<8>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s); break;
+        default: launch_dense<16>(pts, cams, n, xyz_out, err_out, (unsigned)blocks, s); break;
+        }
     } else if (tri) LAUNCH(k_tri, dim3((unsigned)blocks, (unsigned)n_sets), 128, smem, s, (const T*)pts, valid, no_in, cams, C, n, (T*)xyz_out, (T*)err_out);
     else LAUNCH(k_rep, (unsigned)blocks, 128, smem, s, (const T*)pts, valid, (const T*)xyz_in, cams, C, n, no_out, (T*)err_out);
     CUDA_TRY(cudaGetLastError());
@@ -470,8 +470,6 @@ extern "C" int mocap_reproject_batch(const void* pts_dev, const uint8_t* valid_d
 // correspondence: one CTA per frame-set
 // ---------------------------------------------------------------------------------------------------------
 #define CORR_THREADS 128
-
-struct CorrWs { int32_t* cand; int32_t* ncand; };
 
 // Centroid lists of S frame-sets, camera blocks outermost: xy [C / cpb][S][cpb][max_pts][2], count [C / cpb][S][cpb].  cpb = C is the
 // plain [S][C] layout; cpb = cameras per rank is what the shard exchange of the multi-GPU pipeline delivers (one block per source
@@ -574,27 +572,20 @@ __global__ void __launch_bounds__(CORR_THREADS) correspond_kernel(
         T X0[3] = {0, 0, 0};
         for (int g = lane; g < ne; g += 32) {
             // mixed radix: camera 1 varies fastest (Helpers.py:239-245 appends the newest camera as the outer loop)
-            Accum<T> acc; acc.clear();
             T px[MOCAP_MAX_CAMS], py[MOCAP_MAX_CAMS];
             int rem = g;
+#pragma unroll 1                                            // unrolled, this loop spills in the FP32 kernel
             for (int i = 0; i < C; ++i) {
                 int k;
                 if (i == 0) k = j;
                 else { int n = ncand[j * C + i]; int q = rem / n; k = cand[((size_t)j * C + i) * MOCAP_MAX_CAND + (rem - q * n)]; rem = q; }
                 const Pt* pt = in.pts(s, i) + 2 * k;
                 px[i] = (T)pt[0]; py[i] = (T)pt[1];
-                acc.add_view(sm + i * CAM_T_STRIDE + CAM_P, px[i], py[i]);
             }
             T X[3];
-            acc.solve(X);
-            T sq = (T)0;
-            for (int i = 0; i < C; ++i) {
-                T u, v;
-                project<T>(sm + i * CAM_T_STRIDE + CAM_R, sm + i * CAM_T_STRIDE + CAM_K, X, u, v);
-                T dx = px[i] - u, dy = py[i] - v;
-                sq += dx * dx; sq += dy * dy;
-            }
-            esum += sq / (T)(2 * C);
+            auto xy = [&](int i, T& x, T& y) { x = px[i]; y = py[i]; };
+            dlt_all_views<T, 0>(sm, C, xy, X);
+            esum += sq_residual_all_views<T, 0>(sm, C, xy, X) / (T)(2 * C);
             if (g == 0) { X0[0] = X[0]; X0[1] = X[1]; X0[2] = X[2]; }
         }
         // fixed-order warp reduction (bit-identical on any GPU count)
