@@ -467,7 +467,7 @@ extern "C" int mocap_reproject_batch(const void* pts_dev, const uint8_t* valid_d
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// correspondence: one CTA per frame-set
+// correspondence: CTAs of CORR_RPC roots of one frame-set, then one CTA per frame-set ranks
 // ---------------------------------------------------------------------------------------------------------
 #define CORR_THREADS 128
 
@@ -492,6 +492,20 @@ struct CorrIn {
 #ifndef CORR_RPC
 #define CORR_RPC 8        // roots per CTA of the candidate / group kernel
 #endif
+#define CORR_WARPS (CORR_THREADS / 32)
+
+// Workspace of one frame-set: per root the mean error, the first group's point, the first candidate of every camera (the image points
+// of the output) and the root's state; per CTA of the group kernel its flags.  Nothing in it grows with max_groups.
+struct CorrWs {
+    double* rerr; double* rX; int32_t* first; int32_t* vidx; int32_t* flags;
+    __device__ __forceinline__ CorrWs(char* wp, int C, int max_pts) {
+        rerr = (double*)wp;                                                 // [max_pts] mean error per root
+        rX = rerr + max_pts;                                                // [max_pts][3] first group's point
+        first = (int32_t*)(rX + 3 * (size_t)max_pts);                       // [max_pts][C] first candidate per camera
+        vidx = first + (size_t)max_pts * C;                                 // [max_pts] 0 = complete root, -1 = incomplete
+        flags = vidx + max_pts;                                             // [ceil(max_pts / CORR_RPC)] flags per CTA
+    }
+};
 
 // Part 1, grid (S, ceil(max_pts / CORR_RPC)): candidates per (root, camera), candidate groups, triangulation and mean
 // reprojection error of the CTA's roots -> workspace.  Roots are independent until the ranking (Helpers.py:203-273).
@@ -499,163 +513,249 @@ template <typename T, typename Pt>
 __global__ void __launch_bounds__(CORR_THREADS) correspond_kernel(
     CorrIn<Pt> in, int C, int max_pts,
     const double* __restrict__ Fs, const double* __restrict__ cams, double cutoff, int max_groups,
-    int32_t* __restrict__ cand_out, int32_t* __restrict__ flags_out, char* __restrict__ ws_base, size_t ws_stride)
+    int32_t* __restrict__ cand_out, char* __restrict__ ws_base, size_t ws_stride)
 {
     DYN_SHARED(smraw);
-    T* sm = (T*)smraw;
-    const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, nw = blockDim.x >> 5;
+    T* sm = (T*)smraw;                                                      // camera records [C][CAM_T_STRIDE]
+    T* s_cp = sm + C * CAM_T_STRIDE;                                        // candidate points [CORR_RPC][C][MAX_CAND][2] as T
+    __shared__ double s_line[CORR_RPC][MOCAP_MAX_CAMS][5];                  // epiline a, b, c, |(a, b)|, far bound per (root, camera)
+    __shared__ double s_cd[CORR_RPC][MOCAP_MAX_CAMS][MOCAP_MAX_CAND];       // candidates: distance, point index, count
+    __shared__ int s_ck[CORR_RPC][MOCAP_MAX_CAMS][MOCAP_MAX_CAND];
+    __shared__ int s_cn[CORR_RPC][MOCAP_MAX_CAMS];
+    __shared__ int s_off[CORR_RPC + 1], s_root[CORR_RPC], s_ncomp, s_flags;  // complete roots: group offsets, local root index
+    __shared__ T s_part[CORR_RPC][32];                                      // per (complete root, lane of the reference's warp) error sums
+    __shared__ T s_e[2][CORR_THREADS];                                      // one round's group errors (double-buffered)
+    const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const Pt* root_xy = in.pts(s, 0);
     const int R = min(in.n(s, 0), max_pts);
-    const int j0 = blockIdx.y * CORR_RPC, j1 = min(j0 + CORR_RPC, R);
-    if (j0 >= R) return;
-    load_cams<T>(cams, C, sm);
-    __shared__ int s_flags;
+    const int j0 = blockIdx.y * CORR_RPC, nr = min(CORR_RPC, R - j0);
+    if (nr <= 0) return;
     if (tid == 0) s_flags = 0;
-    char* wp = ws_base + (size_t)s * ws_stride;
-    double* rerr = (double*)wp;                                             // [max_pts] mean error per root
-    double* rX = rerr + max_pts;                                            // [max_pts][3] first group's point
-    int32_t* cand = (int32_t*)(rX + 3 * (size_t)max_pts);                   // [max_pts][C][MAX_CAND]
-    int32_t* ncand = cand + (size_t)max_pts * C * MOCAP_MAX_CAND;           // [max_pts][C]
-    int32_t* vidx = ncand + (size_t)max_pts * C;                            // [max_pts] 0 = complete root, -1 = incomplete
-    __syncthreads();
+    load_cams<T>(cams, C, sm);                                              // ends in __syncthreads
+    CorrWs ws(ws_base + (size_t)s * ws_stride, C, max_pts);
 
-    // ---- candidates per (root, camera): epiline (FP64 -> f32) and point-line distances (FP64) --------------------------
-    for (int it = tid; it < (j1 - j0) * C; it += blockDim.x) {
-        int j = j0 + it / C, i = it % C;
-        int32_t* cl = cand + ((size_t)j * C + i) * MOCAP_MAX_CAND;
-        if (i == 0) { ncand[j * C] = 1; cl[0] = j; continue; }
-        const double* F = Fs + (size_t)(i - 1) * 9;
-        double x = (double)(float)root_xy[2 * j], y = (double)(float)root_xy[2 * j + 1];      // root is camera-0 point j
-        double a = __dadd_rn(__dadd_rn(__dmul_rn(F[0], x), __dmul_rn(F[1], y)), F[2]);
-        double b = __dadd_rn(__dadd_rn(__dmul_rn(F[3], x), __dmul_rn(F[4], y)), F[5]);
-        double c = __dadd_rn(__dadd_rn(__dmul_rn(F[6], x), __dmul_rn(F[7], y)), F[8]);
-        double nu = __dadd_rn(__dmul_rn(a, a), __dmul_rn(b, b));
-        nu = nu != 0.0 ? __ddiv_rn(1.0, sqrt(nu)) : 1.0;
-        a = (double)(float)__dmul_rn(a, nu); b = (double)(float)__dmul_rn(b, nu); c = (double)(float)__dmul_rn(c, nu);
-        double den = sqrt(__dadd_rn(__dmul_rn(a, a), __dmul_rn(b, b)));
+    // ---- candidates: one warp per camera, lanes over its points, all roots of the CTA -------------------------------------------
+    // Each (root, camera) keeps the MOCAP_MAX_CAND smallest (distance, point index) among the points under the cutoff, merged chunk
+    // by chunk of 32 points: a passing point's rank is the number of kept entries at or below its distance (they have smaller
+    // indices) plus the passing points of its chunk before it in (distance, index) order.
+    int fl = 0;
+    for (int i = 1 + wid; i < C; i += CORR_WARPS) {
+        if (lane < nr) {                                                    // epiline (FP64 -> f32) of root j0 + lane in camera i
+            const int j = j0 + lane;
+            const double* F = Fs + (size_t)(i - 1) * 9;
+            double x = (double)(float)root_xy[2 * j], y = (double)(float)root_xy[2 * j + 1];
+            double a = __dadd_rn(__dadd_rn(__dmul_rn(F[0], x), __dmul_rn(F[1], y)), F[2]);
+            double b = __dadd_rn(__dadd_rn(__dmul_rn(F[3], x), __dmul_rn(F[4], y)), F[5]);
+            double c = __dadd_rn(__dadd_rn(__dmul_rn(F[6], x), __dmul_rn(F[7], y)), F[8]);
+            double nu = __dadd_rn(__dmul_rn(a, a), __dmul_rn(b, b));
+            nu = nu != 0.0 ? __ddiv_rn(1.0, sqrt(nu)) : 1.0;
+            a = (double)(float)__dmul_rn(a, nu); b = (double)(float)__dmul_rn(b, nu); c = (double)(float)__dmul_rn(c, nu);
+            const double den = sqrt(__dadd_rn(__dmul_rn(a, a), __dmul_rn(b, b)));
+            double* L = s_line[lane][i];
+            L[0] = a; L[1] = b; L[2] = c; L[3] = den;
+            // points farther than cutoff + 2e-5 can neither pass the cutoff nor register as a tie: they are rejected on the
+            // numerator alone (the margin dwarfs the rounding of the division), so the FP64 divide runs for near points only
+            L[4] = __dmul_rn(__dmul_rn(den, cutoff + 2e-5), 1.0 + 1e-12);
+            s_cn[lane][i] = 0;
+        }
+        __syncwarp();
         const Pt* pp = in.pts(s, i);
-        int np = min(in.n(s, i), max_pts), n = 0, fl = 0;
-        double dist[MOCAP_MAX_CAND];
-        // points farther than cutoff + 2e-5 can neither pass the cutoff nor register as a tie: they are rejected on the
-        // numerator alone (the margin dwarfs the rounding of the division), so the FP64 divide runs for near points only
-        const double far = __dmul_rn(__dmul_rn(den, cutoff + 2e-5), 1.0 + 1e-12);
-        for (int k = 0; k < np; ++k) {
-            double num = fabs(__dadd_rn(__dadd_rn(__dmul_rn(a, (double)pp[2 * k]), __dmul_rn(b, (double)pp[2 * k + 1])), c));
-            if (num > far) continue;
-            double d = __ddiv_rn(num, den);
-            if (fabs(d - cutoff) < 1e-5) fl |= MOCAP_CFLAG_TIE;
-            if (!(d < cutoff)) continue;
-            int pos;                                           // keep the MOCAP_MAX_CAND smallest, stable on ties
-            if (n < MOCAP_MAX_CAND) { pos = n; ++n; }
-            else { fl |= MOCAP_CFLAG_CAND_CAP; if (!(d < dist[MOCAP_MAX_CAND - 1])) continue; pos = MOCAP_MAX_CAND - 1; }
-            while (pos > 0 && d < dist[pos - 1]) { dist[pos] = dist[pos - 1]; cl[pos] = cl[pos - 1]; --pos; }
-            dist[pos] = d; cl[pos] = k;
+        const int np = min(in.n(s, i), max_pts);
+        for (int k0 = 0; k0 < np; k0 += 32) {
+            const int k = k0 + lane;
+            double px = 0.0, py = 0.0;
+            if (k < np) { px = (double)pp[2 * k]; py = (double)pp[2 * k + 1]; }
+#pragma unroll 1
+            for (int r = 0; r < nr; ++r) {
+                const double* L = s_line[r][i];
+                double d = 0.0;
+                bool ok = false;
+                if (k < np) {
+                    const double num = fabs(__dadd_rn(__dadd_rn(__dmul_rn(L[0], px), __dmul_rn(L[1], py)), L[2]));
+                    if (!(num > L[4])) {
+                        d = __ddiv_rn(num, L[3]);
+                        if (fabs(d - cutoff) < 1e-5) fl |= MOCAP_CFLAG_TIE;
+                        ok = d < cutoff;
+                    }
+                }
+                const unsigned pass = __ballot_sync(0xffffffffu, ok);
+                if (!pass) continue;
+                double* cd = s_cd[r][i];
+                int* ck = s_ck[r][i];
+                const int n = s_cn[r][i];
+                const double de = lane < n ? cd[lane] : 0.0;
+                const int ke = lane < n ? ck[lane] : 0;
+                int below = 0, moved = 0;                                   // passing points before mine / before kept entry `lane`
+                for (unsigned m = pass; m; m &= m - 1) {
+                    const int q = __ffs(m) - 1;
+                    const double dq = __shfl_sync(0xffffffffu, d, q);
+                    below += dq < d || (dq == d && q < lane);
+                    moved += dq < de;
+                }
+                for (int e = 0; e < n; ++e) below += cd[e] <= d;
+                __syncwarp();
+                if (lane < n && lane + moved < MOCAP_MAX_CAND) { cd[lane + moved] = de; ck[lane + moved] = ke; }
+                if (ok && below < MOCAP_MAX_CAND) { cd[below] = d; ck[below] = k; }
+                const int total = n + __popc(pass);
+                if (total > MOCAP_MAX_CAND) fl |= MOCAP_CFLAG_CAND_CAP;
+                __syncwarp();
+                if (lane == 0) s_cn[r][i] = min(total, MOCAP_MAX_CAND);
+                __syncwarp();
+            }
         }
-        ncand[j * C + i] = n;
-        if (fl) atomicOr(&s_flags, fl);
-        if (cand_out) {
-            int32_t* co = cand_out + (((size_t)s * max_pts + j) * C + i) * MOCAP_MAX_CAND;
-            for (int k = 0; k < MOCAP_MAX_CAND; ++k) co[k] = k < n ? cl[k] : -1;
+    }
+    if (fl) atomicOr(&s_flags, fl);
+    __syncthreads();
+
+    // ---- stage every candidate point as T, first candidates and cand_out to global ------------------------------------------------
+    for (int it = tid; it < nr * C * MOCAP_MAX_CAND; it += CORR_THREADS) {
+        const int m = it % MOCAP_MAX_CAND, ri = it / MOCAP_MAX_CAND, r = ri / C, i = ri - r * C, j = j0 + r;
+        T* cp = s_cp + (size_t)it * 2;
+        if (i == 0) {
+            if (m == 0) { cp[0] = (T)root_xy[2 * j]; cp[1] = (T)root_xy[2 * j + 1]; }
+            continue;
         }
+        const int n = s_cn[r][i], k = m < n ? s_ck[r][i][m] : -1;
+        if (k >= 0) { const Pt* pt = in.pts(s, i) + 2 * k; cp[0] = (T)pt[0]; cp[1] = (T)pt[1]; }
+        if (m == 0) ws.first[(size_t)j * C + i] = k;
+        if (cand_out) cand_out[(((size_t)s * max_pts + j) * C + i) * MOCAP_MAX_CAND + m] = k;
+    }
+    // complete roots of the CTA and their group counts (the first max_groups groups of each)
+    if (wid == 0) {
+        long long ng = 1;
+        bool complete = C >= 2 && lane < nr;
+        if (complete)
+            for (int i = 1; i < C; ++i) { int n = s_cn[lane][i]; if (n == 0) complete = false; ng *= n; if (ng > (1LL << 40)) ng = 1LL << 40; }
+        if (lane < nr) ws.vidx[j0 + lane] = complete ? 0 : -1;
+        if (complete && ng > max_groups) atomicOr(&s_flags, MOCAP_CFLAG_GROUP_CAP);
+        const unsigned cm = __ballot_sync(0xffffffffu, complete);
+        const int ne = complete ? (int)min(ng, (long long)max_groups) : 0;
+        int incl = ne;                                                      // inclusive scan of the group counts over the lanes
+        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
+        if (complete) {
+            const int q = __popc(cm & ((1u << lane) - 1));
+            s_root[q] = lane; s_off[q + 1] = incl;
+        }
+        if (lane == 0) { s_ncomp = __popc(cm); s_off[0] = 0; }
+        if (lane < CORR_RPC) for (int g = 0; g < 32; ++g) s_part[lane][g] = (T)0;
     }
     __syncthreads();
 
-    // ---- per root (one warp each): enumerate candidate groups, triangulate, mean reprojection error ----------------------
-    for (int j = j0 + wid; j < j1; j += nw) {
-        long long ng = 1;
-        bool complete = C >= 2;
-        for (int i = 1; i < C; ++i) { int n = ncand[j * C + i]; if (n == 0) complete = false; ng *= n; if (ng > (1LL << 40)) ng = 1LL << 40; }
-        if (!complete) { if (lane == 0) vidx[j] = -1; continue; }
-        int ne = (int)min(ng, (long long)max_groups);
-        if (ng > max_groups && lane == 0) atomicOr(&s_flags, MOCAP_CFLAG_GROUP_CAP);
-        T esum = (T)0;
-        T X0[3] = {0, 0, 0};
-        for (int g = lane; g < ne; g += 32) {
-            // mixed radix: camera 1 varies fastest (Helpers.py:239-245 appends the newest camera as the outer loop)
-            T px[MOCAP_MAX_CAMS], py[MOCAP_MAX_CAMS];
-            int rem = g;
-#pragma unroll 1                                            // unrolled, this loop spills in the FP32 kernel
-            for (int i = 0; i < C; ++i) {
-                int k;
-                if (i == 0) k = j;
-                else { int n = ncand[j * C + i]; int q = rem / n; k = cand[((size_t)j * C + i) * MOCAP_MAX_CAND + (rem - q * n)]; rem = q; }
-                const Pt* pt = in.pts(s, i) + 2 * k;
-                px[i] = (T)pt[0]; py[i] = (T)pt[1];
+    // ---- candidate groups of all complete roots, CORR_THREADS at a time ---------------------------------------------------------
+    // Flat group index f over the complete roots; group g of root q sits at s_off[q] + g.  The mean error keeps the reference
+    // kernel's summation order: per root, "lane" g % 32 sums its groups g, g + 32, ... in ascending order from (T)0, then a
+    // shuffle tree over offsets 16 .. 1.  Warp 0 adds a round's errors into those 32 partial sums in four steps of 32 consecutive
+    // groups (within a step no two groups share a partial sum), so every partial sum takes its groups in ascending order.
+    const int ncomp = s_ncomp, total = s_off[ncomp];
+    auto root_of = [&](int f) { int q = 0; while (q + 1 < ncomp && f >= s_off[q + 1]) ++q; return q; };
+    for (int base = 0, buf = 0; base < total; base += CORR_THREADS, buf ^= 1) {
+        const int f = base + tid;
+        if (f < total) {
+            const int q = root_of(f), r = s_root[q], g = f - s_off[q];
+            // mixed radix: camera 1 varies fastest (Helpers.py:239-245 appends the newest camera as the outer loop); 3 bits per view
+            unsigned long long dig = 0;
+            unsigned rem = (unsigned)g;
+            for (int i = 1; i < C; ++i) {
+                const unsigned n = (unsigned)s_cn[r][i], qt = rem / n;
+                dig |= (unsigned long long)(rem - qt * n) << (3 * i);
+                rem = qt;
             }
+            const T* cp = s_cp + (size_t)r * C * MOCAP_MAX_CAND * 2;
+            auto xy = [&](int i, T& x, T& y) { const T* p = cp + (i * MOCAP_MAX_CAND + (int)((dig >> (3 * i)) & 7)) * 2; x = p[0]; y = p[1]; };
             T X[3];
-            auto xy = [&](int i, T& x, T& y) { x = px[i]; y = py[i]; };
             dlt_all_views<T, 0>(sm, C, xy, X);
-            esum += sq_residual_all_views<T, 0>(sm, C, xy, X) / (T)(2 * C);
-            if (g == 0) { X0[0] = X[0]; X0[1] = X[1]; X0[2] = X[2]; }
+            s_e[buf][tid] = sq_residual_all_views<T, 0>(sm, C, xy, X) / (T)(2 * C);
+            if (g == 0) { double* o = ws.rX + 3 * (size_t)(j0 + r); o[0] = (double)X[0]; o[1] = (double)X[1]; o[2] = (double)X[2]; }
         }
-        // fixed-order warp reduction (bit-identical on any GPU count)
-        for (int o = 16; o > 0; o >>= 1) esum += __shfl_down_sync(0xffffffffu, esum, o);
-        if (lane == 0) {
-            rerr[j] = (double)esum / (double)ne;
-            rX[3 * j] = (double)X0[0]; rX[3 * j + 1] = (double)X0[1]; rX[3 * j + 2] = (double)X0[2];
-            vidx[j] = 0;
+        __syncthreads();
+        if (wid == 0) {
+            for (int w = 0; w < CORR_WARPS; ++w) {
+                const int ff = base + w * 32 + lane;
+                if (ff < total) { const int q = root_of(ff); s_part[q][(ff - s_off[q]) & 31] += s_e[buf][w * 32 + lane]; }
+                __syncwarp();
+            }
         }
     }
     __syncthreads();
-    if (tid == 0 && s_flags) atomicOr(&flags_out[s], s_flags);
+    for (int q = wid; q < ncomp; q += CORR_WARPS) {
+        T esum = s_part[q][lane];
+        for (int o = 16; o > 0; o >>= 1) esum += __shfl_down_sync(0xffffffffu, esum, o);     // fixed order: bit-identical on any GPU count
+        if (lane == 0) ws.rerr[j0 + s_root[q]] = (double)esum / (double)(s_off[q + 1] - s_off[q]);
+    }
+    if (tid == 0) ws.flags[blockIdx.y] = s_flags;
 }
 
-// Part 2, one CTA per frame-set: compact the complete roots in root order, rank them by mean error (Helpers.py:274-279)
+// Part 2, one CTA per frame-set: the flags of its group CTAs, the complete roots compacted in root order by ballot and prefix sum,
+// each ranked by mean error against all others (Helpers.py:274-279), the errors staged in shared memory a tile at a time.
 template <typename Pt>
 __global__ void __launch_bounds__(CORR_THREADS) correspond_rank_kernel(
     CorrIn<Pt> in, int C, int max_pts, int obj_count,
     double* __restrict__ obj_out, int32_t* __restrict__ n_obj_out, Pt* __restrict__ img_out, int32_t* __restrict__ n_valid_out,
-    double* __restrict__ err_out, char* __restrict__ ws_base, size_t ws_stride)
+    double* __restrict__ err_out, int32_t* __restrict__ flags_out, char* __restrict__ ws_base, size_t ws_stride)
 {
-    const int s = blockIdx.x, tid = threadIdx.x;
-    char* wp = ws_base + (size_t)s * ws_stride;
-    double* rerr = (double*)wp;
-    double* rX = rerr + max_pts;
-    int32_t* cand = (int32_t*)(rX + 3 * (size_t)max_pts);
-    int32_t* ncand = cand + (size_t)max_pts * C * MOCAP_MAX_CAND;
-    int32_t* vidx = ncand + (size_t)max_pts * C;
+    const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    CorrWs ws(ws_base + (size_t)s * ws_stride, C, max_pts);
     const int R = min(in.n(s, 0), max_pts);
-    __shared__ int s_nvalid;
-    if (tid == 0) {
-        int n = 0;
-        for (int j = 0; j < R; ++j) if (vidx[j] >= 0) vidx[j] = n++;
-        s_nvalid = n;
-    }
+    __shared__ int s_cnt[CORR_WARPS], s_fl[CORR_WARPS];
+    __shared__ double s_err[CORR_THREADS];
+    __shared__ int s_ok[CORR_THREADS];
+    int cnt = 0, fl = 0;
+    for (int j = tid; j < R; j += CORR_THREADS) cnt += ws.vidx[j] >= 0;
+    for (int b = tid; b < (max(R, 0) + CORR_RPC - 1) / CORR_RPC; b += CORR_THREADS) fl |= ws.flags[b];
+    for (int o = 16; o > 0; o >>= 1) { cnt += __shfl_down_sync(0xffffffffu, cnt, o); fl |= __shfl_down_sync(0xffffffffu, fl, o); }
+    if (lane == 0) { s_cnt[wid] = cnt; s_fl[wid] = fl; }
     __syncthreads();
-    const int nvalid = s_nvalid;
-    for (int j = tid; j < R; j += blockDim.x) {
-        int v = vidx[j];
-        if (v < 0) continue;
-        double e = rerr[j];
+    int nvalid = 0;
+    fl = 0;
+    for (int w = 0; w < CORR_WARPS; ++w) { nvalid += s_cnt[w]; fl |= s_fl[w]; }
+    const int n_obj = obj_count > nvalid ? nvalid : min(obj_count + 1, nvalid);
+    if (tid == 0) { n_valid_out[s] = nvalid; n_obj_out[s] = n_obj; flags_out[s] = fl; }
+    int vbase = 0;                                                          // complete roots before this block of roots
+    for (int j0 = 0; j0 < R; j0 += CORR_THREADS) {
+        const int j = j0 + tid;
+        const bool ok = j < R && ws.vidx[j] >= 0;
+        const double e = ok ? ws.rerr[j] : 0.0;
+        const unsigned m = __ballot_sync(0xffffffffu, ok);
+        __syncthreads();                                                    // s_cnt / s_err of the previous block are consumed
+        if (lane == 0) s_cnt[wid] = __popc(m);
+        __syncthreads();
+        int v = vbase + __popc(m & ((1u << lane) - 1)), nblk = 0;
+        for (int w = 0; w < CORR_WARPS; ++w) { const int c = s_cnt[w]; if (w < wid) v += c; nblk += c; }
+        vbase += nblk;
         int rank = 0;
-        for (int k = 0; k < R; ++k) {
-            if (vidx[k] < 0 || k == j) continue;
-            double ek = rerr[k];
-            rank += (ek < e) || (ek == e && k < j);
+        for (int k0 = 0; k0 < R; k0 += CORR_THREADS) {
+            __syncthreads();
+            const int k = k0 + tid;
+            s_ok[tid] = k < R && ws.vidx[k] >= 0;
+            s_err[tid] = s_ok[tid] ? ws.rerr[k] : 0.0;
+            __syncthreads();
+            if (ok)
+                for (int t = 0; t < CORR_THREADS; ++t) {
+                    const int kk = k0 + t;
+                    if (!s_ok[t] || kk == j) continue;
+                    const double ek = s_err[t];
+                    rank += (ek < e) || (ek == e && kk < j);
+                }
         }
-        int n_obj = obj_count > nvalid ? nvalid : min(obj_count + 1, nvalid);
+        if (!ok) continue;
         if (rank < n_obj) {
             double* o = obj_out + ((size_t)s * max_pts + rank) * 3;
-            o[0] = rX[3 * j]; o[1] = rX[3 * j + 1]; o[2] = rX[3 * j + 2];
+            o[0] = ws.rX[3 * j]; o[1] = ws.rX[3 * j + 1]; o[2] = ws.rX[3 * j + 2];
         }
         err_out[(size_t)s * max_pts + v] = e;
         Pt* io = img_out + ((size_t)s * max_pts + v) * C * 2;
         for (int i = 0; i < C; ++i) {
-            int k = i == 0 ? j : cand[((size_t)j * C + i) * MOCAP_MAX_CAND];
+            const int k = i == 0 ? j : ws.first[(size_t)j * C + i];
             const Pt* pt = in.pts(s, i) + 2 * k;
             io[2 * i] = pt[0];
             io[2 * i + 1] = pt[1];
         }
     }
-    if (tid == 0) {
-        n_valid_out[s] = nvalid;
-        n_obj_out[s] = obj_count > nvalid ? nvalid : min(obj_count + 1, nvalid);
-    }
 }
 
 static size_t corr_ws_stride(int C, int max_pts)
 {
-    size_t b = ((size_t)max_pts * C * MOCAP_MAX_CAND + (size_t)max_pts * C + (size_t)max_pts) * 4 + (size_t)max_pts * 4 * 8;
+    size_t b = (size_t)max_pts * 4 * 8 + ((size_t)max_pts * C + (size_t)max_pts + (size_t)cdiv(max_pts, CORR_RPC)) * 4;
     return (b + 255) & ~(size_t)255;
 }
 
@@ -684,21 +784,21 @@ static int correspond_blocked(const Pt* xy_dev, const int32_t* count_dev, int S,
     size_t stride = corr_ws_stride(C, max_pts);
     if (workspace_bytes < stride * (size_t)S) return MOCAP_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
-    CUDA_TRY(cudaMemsetAsync(flags_out, 0, (size_t)S * 4, s));
     dim3 grid(S, cdiv(max_pts, CORR_RPC));
     CorrIn<Pt> in;
     in.xy = xy_dev; in.count = count_dev; in.S = S; in.cpb = cams_per_block; in.max_pts = max_pts;
     auto corr_f64 = correspond_kernel<double, Pt>;
     auto corr_f32 = correspond_kernel<float, Pt>;
     auto rank = correspond_rank_kernel<Pt>;
+    const size_t smem_per_T = (size_t)C * (CAM_T_STRIDE + CORR_RPC * MOCAP_MAX_CAND * 2);
     if (fp64_mode)
-        LAUNCH(corr_f64, grid, CORR_THREADS, (size_t)C * CAM_T_STRIDE * sizeof(double), s,
-            in, C, max_pts, F_dev, cams_dev, cutoff, max_groups, cand_out, flags_out, (char*)workspace, stride);
+        LAUNCH(corr_f64, grid, CORR_THREADS, smem_per_T * sizeof(double), s,
+            in, C, max_pts, F_dev, cams_dev, cutoff, max_groups, cand_out, (char*)workspace, stride);
     else
-        LAUNCH(corr_f32, grid, CORR_THREADS, (size_t)C * CAM_T_STRIDE * sizeof(float), s,
-            in, C, max_pts, F_dev, cams_dev, cutoff, max_groups, cand_out, flags_out, (char*)workspace, stride);
+        LAUNCH(corr_f32, grid, CORR_THREADS, smem_per_T * sizeof(float), s,
+            in, C, max_pts, F_dev, cams_dev, cutoff, max_groups, cand_out, (char*)workspace, stride);
     LAUNCH(rank, S, CORR_THREADS, 0, s, in, C, max_pts, obj_count, obj_out, n_obj_out, img_out,
-           n_valid_out, err_out, (char*)workspace, stride);
+           n_valid_out, err_out, flags_out, (char*)workspace, stride);
     CUDA_TRY(cudaGetLastError());
     return MOCAP_OK;
 }
