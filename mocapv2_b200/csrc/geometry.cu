@@ -29,18 +29,23 @@ __device__ __forceinline__ float sfu_rsqrt(float x) { float y; asm("rsqrt.approx
 __device__ __forceinline__ float sfu_rcp(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 #endif
 
-// Smallest-eigenvalue eigenvector of a symmetric PSD 4x4 (upper triangle a[10]: 00 01 02 03 11 12 13 22 23 33).
-// FP32 main mode: FIVE cyclic sweeps, no data-dependent branch (the lanes of a warp never diverge, nothing is tested between
-// rotations).  Five is the budget of the flop count in SURVEY 8d; on the rigs of BASELINE configs 1-5 the smallest eigenvector has
-// converged to FP32 round-off after three to four (max relative error of X against the FP64 SVD 7e-7 at every count >= 4).
+// Eigen-decomposition of a symmetric PSD 4x4 (upper triangle b[10]: 00 01 02 03 11 12 13 22 23 33): eigenvalues lam, eigenvectors
+// the columns of V.  FP32 main mode: FIVE cyclic sweeps, no data-dependent branch (the lanes of a warp never diverge, nothing is tested
+// between rotations).  Five is the budget of the flop count in SURVEY 8d; on the rigs of BASELINE configs 1-5 the smallest eigenvector
+// has converged after three to four.
 // Rotation from delta = aqq - app: t = 2 apq / (delta + sign(delta) sqrt(delta^2 + 4 apq^2)), c = rsqrt(t^2 + 1), s = t c -- three
 // SFU operations (rsqrt, rcp, rsqrt), approximate on purpose: Jacobi rotations are self-correcting, an angle that is off by a few ulp
 // leaves a slightly larger off-diagonal for the next sweep.  apq == 0 gives t = 0 (the tiny terms keep 0 / 0 away): identity.
-__device__ __forceinline__ void jacobi_min_eigvec_f32(float b00, float b01, float b02, float b03, float b11, float b12, float b13,
-                                                      float b22, float b23, float b33, float v[4])
+// The vector that comes out carries B's FP32 rounding (about kappa * u, kappa = lam_max / (lam_2 - lam_1)) and what the rotations left:
+// over the volume each rig of configs 1-5 sees, X within 7e-7 relative and the reprojection error within 1.3-1.6e-3 px of the FP64
+// reference, over the 1e-3 px contract.  dlt_solve takes that back out with one correction step from the rows of A.
+__device__ __forceinline__ void jacobi_eig_f32(const float b[10], float lam[4], float V[4][4])
 {
-    float A[4][4] = {{b00, b01, b02, b03}, {b01, b11, b12, b13}, {b02, b12, b22, b23}, {b03, b13, b23, b33}};
-    float V[4][4] = {{1, 0, 0, 0}, {0, 1, 0, 0}, {0, 0, 1, 0}, {0, 0, 0, 1}};
+    float A[4][4] = {{b[0], b[1], b[2], b[3]}, {b[1], b[4], b[5], b[6]}, {b[2], b[5], b[7], b[8]}, {b[3], b[6], b[8], b[9]}};
+#pragma unroll
+    for (int r = 0; r < 4; ++r)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) V[r][c] = r == c ? 1.0f : 0.0f;
 #pragma unroll 1
     for (int sweep = 0; sweep < 5; ++sweep) {
 #pragma unroll
@@ -68,16 +73,8 @@ __device__ __forceinline__ void jacobi_min_eigvec_f32(float b00, float b01, floa
             }
         }
     }
-    // column of the smallest |eigenvalue| by selects
-    const float e0 = fabsf(A[0][0]), e1 = fabsf(A[1][1]), e2 = fabsf(A[2][2]), e3 = fabsf(A[3][3]);
-    const bool k01 = e1 < e0, k23 = e3 < e2;
-    const float m01 = k01 ? e1 : e0, m23 = k23 ? e3 : e2;
-    const bool hi = m23 < m01;
 #pragma unroll
-    for (int r = 0; r < 4; ++r) {
-        const float a = k01 ? V[r][1] : V[r][0], b = k23 ? V[r][3] : V[r][2];
-        v[r] = hi ? b : a;
-    }
+    for (int k = 0; k < 4; ++k) lam[k] = A[k][k];
 }
 
 // FP64 check mode: IEEE theta / tau rotations, up to twelve cyclic sweeps; the solve ends at a sweep that starts diagonal, and from
@@ -132,21 +129,6 @@ __device__ __forceinline__ void jacobi_min_eigvec_f64(double b00, double b01, do
     for (int r = 0; r < 4; ++r) v[r] = (k == 0) ? V[r][0] : (k == 1) ? V[r][1] : (k == 2) ? V[r][2] : V[r][3];
 }
 
-// X = v[:3] / v[3] for the smallest eigenvector v of B (upper triangle b[10])
-__device__ __forceinline__ void dlt_solve(const float b[10], float X[3])
-{
-    float w[4];
-    jacobi_min_eigvec_f32(b[0], b[1], b[2], b[3], b[4], b[5], b[6], b[7], b[8], b[9], w);
-    const float iw = 1.0f / w[3];                          // one IEEE reciprocal instead of three divisions
-    X[0] = w[0] * iw; X[1] = w[1] * iw; X[2] = w[2] * iw;
-}
-__device__ __forceinline__ void dlt_solve(const double b[10], double X[3])
-{
-    double v[4];
-    jacobi_min_eigvec_f64(b[0], b[1], b[2], b[3], b[4], b[5], b[6], b[7], b[8], b[9], v);
-    X[0] = v[0] / v[3]; X[1] = v[1] / v[3]; X[2] = v[2] / v[3];
-}
-
 // twelve consecutive values (a 3x4 P, or R | t of a camera record): three 128-bit loads for floats that are 16-byte aligned
 template <typename T> __device__ __forceinline__ void load12(const T* p, T out[12])
 {
@@ -167,6 +149,81 @@ template <> __device__ __forceinline__ void load12<float>(const float* p, float 
 }
 #endif
 
+// The two DLT rows of one view: y*P2 - P1 and P0 - x*P2 (P row-major 3x4)
+template <typename T>
+__device__ __forceinline__ void dlt_rows(const T Pv[12], T x, T y, T r1[4], T r2[4])
+{
+#pragma unroll
+    for (int c = 0; c < 4; ++c) { r1[c] = y * Pv[8 + c] - Pv[4 + c]; r2[c] = Pv[c] - x * Pv[8 + c]; }
+}
+
+// X = v[:3] / v[3] for the smallest eigenvector v of B = A^T A (upper triangle b[10]); views(f) calls f(P, x, y) for each view that
+// went into B.  FP32: the Jacobi vector v carries the rounding of B (about kappa * u), so one correction step follows: the residual
+// r = sum_i a_i (a_i . v) from the rows of A (not from the rounded B), projected on the other eigenvectors u_k, and
+// v -= sum_{k != min} (u_k . r) / (lam_k - lam_min) u_k.  That leaves the rounding of the rows (FP32 P and x, y): every point with
+// kappa < 1e3 of tests/test_triangulation_volume.py within 3.2e-7 relative and 4.9e-4 px of the reference on a B200 (CPU emulation build
+// 5.3e-7 / 6.2e-4 px).  Plain FP32 dot products a_i . v are enough: Dot2-compensated ones (exact products by fmaf, TwoSum) moved the
+// largest error of the emulation build by 2-20 % either way for about 30 more flops per row.
+template <class Views>
+__device__ __forceinline__ void dlt_solve(const float b[10], Views views, float X[3])
+{
+    float lam[4], V[4][4];
+    jacobi_eig_f32(b, lam, V);
+    // column of the smallest |eigenvalue| by selects
+    const float e0 = fabsf(lam[0]), e1 = fabsf(lam[1]), e2 = fabsf(lam[2]), e3 = fabsf(lam[3]);
+    const bool k01 = e1 < e0, k23 = e3 < e2;
+    const float m01 = k01 ? e1 : e0, m23 = k23 ? e3 : e2;
+    const bool hi = m23 < m01;
+    const float lmin = hi ? (k23 ? lam[3] : lam[2]) : (k01 ? lam[1] : lam[0]);
+    float v[4];
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+        const float a = k01 ? V[r][1] : V[r][0], c = k23 ? V[r][3] : V[r][2];
+        v[r] = hi ? c : a;
+    }
+    // M = sum_{k != min} u_k u_k^T / (lam_k - lam_min) (upper triangle): 10 values live across the view loop instead of V and lam
+    float M[10];
+#pragma unroll
+    for (int i = 0; i < 10; ++i) M[i] = 0.0f;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const float gap = lam[k] - lmin;
+        const float g = gap > 0.0f ? sfu_rcp(gap) : 0.0f;     // 0 for the smallest one itself
+        int i = 0;
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+#pragma unroll
+            for (int c = r; c < 4; ++c) M[i++] += g * V[r][k] * V[c][k];
+    }
+    // The rows are formed again rather than kept: an offset the compiler cannot see through stops it from holding every view's P
+    // (loaded for B) in registers across the solve, which would double the dense kernels' registers.
+    int opaque0 = 0;
+    asm volatile("" : "+r"(opaque0));
+    float res[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+    views([&](const float* P, float x, float y) {
+        float Pv[12], r1[4], r2[4];
+        load12(P + opaque0, Pv);
+        dlt_rows(Pv, x, y, r1, r2);
+        const float d1 = r1[0] * v[0] + r1[1] * v[1] + r1[2] * v[2] + r1[3] * v[3];
+        const float d2 = r2[0] * v[0] + r2[1] * v[1] + r2[2] * v[2] + r2[3] * v[3];
+#pragma unroll
+        for (int c = 0; c < 4; ++c) res[c] += r1[c] * d1 + r2[c] * d2;
+    });
+    const float w[4] = {v[0] - (M[0] * res[0] + M[1] * res[1] + M[2] * res[2] + M[3] * res[3]),
+                        v[1] - (M[1] * res[0] + M[4] * res[1] + M[5] * res[2] + M[6] * res[3]),
+                        v[2] - (M[2] * res[0] + M[5] * res[1] + M[7] * res[2] + M[8] * res[3]),
+                        v[3] - (M[3] * res[0] + M[6] * res[1] + M[8] * res[2] + M[9] * res[3])};
+    const float iw = 1.0f / w[3];                          // one IEEE reciprocal instead of three divisions
+    X[0] = w[0] * iw; X[1] = w[1] * iw; X[2] = w[2] * iw;
+}
+template <class Views>
+__device__ __forceinline__ void dlt_solve(const double b[10], Views, double X[3])
+{
+    double v[4];
+    jacobi_min_eigvec_f64(b[0], b[1], b[2], b[3], b[4], b[5], b[6], b[7], b[8], b[9], v);
+    X[0] = v[0] / v[3]; X[1] = v[1] / v[3]; X[2] = v[2] / v[3];
+}
+
 template <typename T>
 struct Accum {                          // B = A^T A accumulated view by view
     T b[10];
@@ -183,11 +240,11 @@ struct Accum {                          // B = A^T A accumulated view by view
         T Pv[12];
         load12(P, Pv);
         T r1[4], r2[4];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) { r1[c] = y * Pv[8 + c] - Pv[4 + c]; r2[c] = Pv[c] - x * Pv[8 + c]; }
+        dlt_rows(Pv, x, y, r1, r2);
         add_row(r1); add_row(r2);
     }
-    __device__ __forceinline__ void solve(T X[3]) { dlt_solve(b, X); }
+    // views(f): f(P, x, y) for each view added, in any order (the FP32 solve goes over them once more)
+    template <class Views> __device__ __forceinline__ void solve(Views views, T X[3]) { dlt_solve(b, views, X); }
 };
 
 // cv.projectPoints restated (SURVEY App. A9).  FP64: reproduces the float32 roundings of X and of (u, v).
@@ -295,9 +352,10 @@ __device__ __forceinline__ void for_views(int C, F f)
 template <typename T, int CT, class XY>
 __device__ __forceinline__ void dlt_all_views(const T* cams, int C, XY xy, T X[3])
 {
+    auto views = [&](auto f) { for_views<CT>(C, [&](int c) { T x, y; xy(c, x, y); f(cams + c * CAM_T_STRIDE + CAM_P, x, y); }); };
     Accum<T> acc; acc.clear();
-    for_views<CT>(C, [&](int c) { T x, y; xy(c, x, y); acc.add_view(cams + c * CAM_T_STRIDE + CAM_P, x, y); });
-    acc.solve(X);
+    views([&](const T* P, T x, T y) { acc.add_view(P, x, y); });
+    acc.solve(views, X);
 }
 
 template <typename T, int CT, class XY>
@@ -341,17 +399,22 @@ __global__ void __launch_bounds__(128) triangulate_kernel(const T* __restrict__ 
         // with a mask, P and the residual take K of the view's rank among the valid views (make_P); given points are reprojected here too
         int nv = 0;
         if (TRIANGULATE) {
+            auto views = [&](auto f) {
+                int rank = 0;
+                for (int c = 0; c < C; ++c) {
+                    if (vm && !vm[c]) continue;
+                    T x, y, P[12];
+                    load_xy(p + 2 * c, x, y);
+                    make_P<T>(sm + rank * CAM_T_STRIDE, sm + c * CAM_T_STRIDE, P);
+                    f(P, x, y);
+                    ++rank;
+                }
+                return rank;
+            };
             Accum<T> acc; acc.clear();
-            for (int c = 0; c < C; ++c) {
-                if (vm && !vm[c]) continue;
-                T x, y, P[12];
-                load_xy(p + 2 * c, x, y);
-                make_P<T>(sm + nv * CAM_T_STRIDE, sm + c * CAM_T_STRIDE, P);
-                acc.add_view(P, x, y);
-                ++nv;
-            }
+            nv = views([&](const T* P, T x, T y) { acc.add_view(P, x, y); });
             if (nv <= 1) { X[0] = X[1] = X[2] = nan; }
-            else acc.solve(X);
+            else acc.solve(views, X);
             if (xyz_out) { xyz_out[(size_t)i * 3] = X[0]; xyz_out[(size_t)i * 3 + 1] = X[1]; xyz_out[(size_t)i * 3 + 2] = X[2]; }
         } else {
             X[0] = xyz_in[(size_t)i * 3]; X[1] = xyz_in[(size_t)i * 3 + 1]; X[2] = xyz_in[(size_t)i * 3 + 2];

@@ -61,35 +61,6 @@ def test_eight_view_groups(engine, dtype):
     assert np.abs(np.sqrt(e2.double().cpu().numpy()) - np.sqrt(z["errors_ref"])).max() < (1e-9 if dtype == torch.float64 else TOL_PX)
 
 
-def test_missing_views(engine):
-    """[None, None] views are dropped and intrinsics are indexed by position among the remaining views
-    (Helpers.py:50-62); fewer than two views -> the reference's [None, None, None] (NaN here)."""
-    z = np.load(os.path.join(GOLDEN, "c5_groups.npz"))
-    rig = S.config_rig("c5")
-    cams = engine.cameras(rig["poses"], rig["camera_params"])
-    P = 16
-    groups = z["groups"][:P]
-    rng = np.random.default_rng(2)
-    valid = (rng.random((P, 8)) > 0.35).astype(np.uint8)
-    valid[0] = 0
-    valid[1] = 0
-    valid[1, 3] = 1
-    valid[2] = 1
-    xyz, err = engine.triangulate(dev(engine, groups), cams, dev(engine, valid))
-    X = xyz.cpu().numpy()
-    E = err.cpu().numpy()
-    Ps = R.projection_matrices(rig["poses"], rig["camera_params"])
-    for i in range(P):
-        idx = np.nonzero(valid[i])[0]
-        if len(idx) <= 1:
-            assert np.isnan(X[i]).all() and np.isnan(E[i])
-            continue
-        ref = R.triangulate_point(groups[i, idx], [Ps[k] for k in idx])
-        assert np.abs(X[i] - ref).max() / np.linalg.norm(ref) < 1e-9
-        e = R.reprojection_error(groups[i, idx], ref, [rig["poses"][k] for k in idx], rig["camera_params"])
-        assert abs(np.sqrt(E[i]) - np.sqrt(e)) < 1e-6
-
-
 def test_empty_batch(engine):
     rig = S.config_rig("c1")
     cams = engine.cameras(rig["poses"], rig["camera_params"])
