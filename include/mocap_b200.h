@@ -81,6 +81,8 @@ int mocap_undistort_table_build(const double* K9_host, const double* dist5_host,
  *   out_contours[n][max_contours][8] double: a00, a10, a01 (exact integers), perimeter, is_hole,
  *                                   parent (index in output order or -1), kept, start pixel index
  *   out_contour_count[n]
+ * Workspace: mocap_detect_workspace_bytes(), sized for the parity outputs.  The overlapped call below uses the same layout with one
+ * cluster-path block per chunk instead of one for the batch.
  */
 size_t mocap_detect_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs);
 
@@ -149,6 +151,7 @@ int mocap_detect_batch_subpixel(const uint8_t* frames_dev, int n_frames, int H, 
  *     of TMA boxes per SM instead of two. */
 void* mocap_detect_pipe_create(int n_worker_streams);
 void mocap_detect_pipe_destroy(void* pipe);
+/* the workspace layout of mocap_detect_workspace_bytes with the call's chunk count (chunk_frames as in the call) */
 size_t mocap_detect_pipelined_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs, int chunk_frames);
 int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
                                  const MocapLensSet* lenses, int thresh, double min_area, double min_circ,

@@ -1,5 +1,7 @@
-// C-ABI glue of the detection path: workspace carving and the mocap_detect_batch / mocap_filter_batch entry points
-// (include/mocap_b200.h).  _find_dot of the reference (lib/ImageOperations.py:33-78) = launch_filter + launch_blobs.
+// C-ABI glue of the detection path (include/mocap_b200.h): one workspace layout (detect_layout) and one stage schedule (detect)
+// behind the one-shot mocap_detect_batch and the overlapped mocap_detect_batch_pipelined, which differ only in a DetectSchedule;
+// the stage entry points mocap_filter_batch / mocap_blobs_batch / mocap_scan_cells_batch.
+// _find_dot of the reference (lib/ImageOperations.py:33-78) = launch_filter + launch_blobs.
 #include "common.cuh"
 #include <string.h>
 
@@ -89,20 +91,30 @@ extern "C" int mocap_stage_timer_read(void* timer, float* ms_out)
     return MOCAP_OK;
 }
 
+#define PIPE_MAX_CHUNKS 64           // chunks of one call at most (a pipe holds events per chunk)
+
+// The workspace of every detection call: the general-path arrays of the batch (all that mocap_filter_batch and mocap_blobs_batch
+// use), the control block of the TMA scan, need_general [n] and one cluster-path block per chunk.  The one-shot call is one chunk.
 struct DetectLayout {
-    size_t off_active, off_list, off_counters, off_bits, off_fg, off_nfg, off_flags, off_cellbox, off_blob, off_cluster;
-    size_t blob_stride, total;
-    ClusterLayout cl;
-    int TX, TY, TXW, max_fg;
+    size_t off_active, off_list, off_counters, off_bits, off_fg, off_nfg, off_flags, off_cellbox, off_blob, general_bytes;
+    size_t off_need, off_ctrl, off_chunks, chunk_bytes, total;
+    size_t blob_stride;
+    ClusterLayout cl;                // inside one chunk's block
+    int TX, TY, TXW, max_fg, chunks, chunk_frames;
 };
 
-static int detect_layout(int n, int H, int W, int max_contours, int max_runs, bool with_blobs, DetectLayout* L)
+// chunk_frames <= 0 or > n: one chunk
+static int detect_layout(int n, int H, int W, int max_contours, int max_runs, int chunk_frames, DetectLayout* L)
 {
     if (n <= 0 || H <= 0 || W <= 0) return MOCAP_ERR_INVALID;
     if (H > 16384 || W > 16384) return MOCAP_ERR_UNSUPPORTED;
     L->TX = cdiv(W, TILE); L->TY = cdiv(H, TILE); L->TXW = cdiv(L->TX, 32);
     L->max_fg = L->TX * L->TY;
     if ((long long)n * L->TX * L->TY >= (1LL << 31)) return MOCAP_ERR_UNSUPPORTED;   // tile codes are 32-bit
+    if (chunk_frames <= 0 || chunk_frames > n) chunk_frames = n;
+    int chunks = cdiv(n, chunk_frames);
+    if (chunks > PIPE_MAX_CHUNKS) { chunk_frames = cdiv(n, PIPE_MAX_CHUNKS); chunks = cdiv(n, chunk_frames); }
+    L->chunks = chunks; L->chunk_frames = chunk_frames;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t r = off; off += align_up(bytes, 256); return r; };
     L->off_active = take((size_t)n * L->TY * L->TXW * 4);
@@ -113,9 +125,13 @@ static int detect_layout(int n, int H, int W, int max_contours, int max_runs, bo
     L->off_nfg = take((size_t)n * 4);
     L->off_flags = take((size_t)n * 4);
     L->off_cellbox = take((size_t)n * L->TX * L->TY * 4);
-    L->blob_stride = with_blobs ? blob_ws_stride(H, max_runs, max_contours) : 0;
+    L->blob_stride = blob_ws_stride(H, max_runs, max_contours);
     L->off_blob = take(L->blob_stride * (size_t)n);
-    L->off_cluster = take(cluster_ws_bytes(n, H, W, max_contours, &L->cl));
+    L->general_bytes = off;
+    L->off_ctrl = take(scan_tma_ctrl_bytes(chunks));
+    L->off_need = take((size_t)n * 4);
+    L->chunk_bytes = align_up(cluster_ws_bytes(chunk_frames, H, W, max_contours, &L->cl), 256);
+    L->off_chunks = take(L->chunk_bytes * (size_t)chunks);
     L->total = off;
     return MOCAP_OK;
 }
@@ -133,13 +149,18 @@ static FilterWs filter_ws(char* base, const DetectLayout& L)
     return ws;
 }
 
-extern "C" size_t mocap_detect_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs)
+extern "C" size_t mocap_detect_pipelined_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs, int chunk_frames)
 {
     (void)max_blobs;
     DetectLayout L;
     if (max_contours <= 0 || max_runs <= 0) return 0;
-    if (detect_layout(n_frames, H, W, max_contours, max_runs, true, &L) != MOCAP_OK) return 0;
+    if (detect_layout(n_frames, H, W, max_contours, max_runs, chunk_frames, &L) != MOCAP_OK) return 0;
     return L.total;
+}
+
+extern "C" size_t mocap_detect_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs)
+{
+    return mocap_detect_pipelined_workspace_bytes(n_frames, H, W, max_blobs, max_contours, max_runs, 0);
 }
 
 extern "C" int mocap_filter_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
@@ -149,9 +170,9 @@ extern "C" int mocap_filter_batch(const uint8_t* frames_dev, int n_frames, int H
     if (!frames_dev || !table_dev || !out_bits || !workspace) return MOCAP_ERR_INVALID;
     if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
     DetectLayout L;
-    int st = detect_layout(n_frames, H, W, 1, 1, false, &L);
+    int st = detect_layout(n_frames, H, W, 1, 1, 0, &L);
     if (st != MOCAP_OK) return st;
-    if (workspace_bytes < L.total) return MOCAP_ERR_WORKSPACE;
+    if (workspace_bytes < L.general_bytes) return MOCAP_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
     TableView tv; table_view(table_dev, H, W, &tv);
     FilterWs ws = filter_ws((char*)workspace, L);
@@ -176,87 +197,6 @@ static int lens_set_view(const MocapLensSet* ls, int H, int W, TableView* tv)
     return MOCAP_OK;
 }
 
-// mocap_detect_batch and mocap_detect_batch_subpixel: out_xy holds int32 (xy_float 0) or float32 (1) centroid pairs
-static int detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                        const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
-                        int max_blobs, int max_contours, int max_runs,
-                        int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags,
-                        uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
-                        double* out_contours, int32_t* out_contour_count,
-                        void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
-{
-    StageTimer* timer = (StageTimer*)stage_timer;
-    if (!frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
-    if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
-    if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
-    DetectLayout L;
-    int st = detect_layout(n_frames, H, W, max_contours, max_runs, true, &L);
-    if (st != MOCAP_OK) return st;
-    TableView tv;
-    st = lens_set_view(lenses, H, W, &tv);
-    if (st != MOCAP_OK) return st;
-    if (workspace_bytes < L.total) return MOCAP_ERR_WORKSPACE;
-    cudaStream_t s = (cudaStream_t)stream;
-    FilterWs ws = filter_ws((char*)workspace, L);
-    CUDA_TRY(cudaMemsetAsync(out_flags, 0, (size_t)n_frames * 4, s));
-    if (out_labels) CUDA_TRY(cudaMemsetAsync(out_labels, 0, (size_t)n_frames * H * W * 4, s));
-    // Product path (no label / bit-image outputs wanted): scan -> groups of hot cells -> per-cluster units in shared memory
-    // -> per-frame ordering.  Frames it cannot finish locally, and every frame when the parity outputs are requested,
-    // take the general per-frame path (tiles -> packed image -> runs, labels, contour tree).
-    const bool extras = out_bits || out_labels || out_blob_sums || out_blob_count;
-    const bool use_cluster = !extras && cluster_path_supported(H, W);
-    char* cl_base = (char*)workspace + L.off_cluster;
-    int* need_general = (int*)(cl_base + L.cl.need_general);
-    st = launch_scan(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws, s, timer);
-    if (st != MOCAP_OK) return st;
-    CUDA_TRY(cudaMemsetAsync(need_general, use_cluster ? 0 : 1, (size_t)n_frames * 4, s));
-    if (use_cluster) {
-        st = launch_cluster_path(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, cl_base, L.cl, need_general,
-                                 max_contours, max_blobs, min_area, min_circ, out_xy, xy_float, out_count, out_flags, out_contours,
-                                 out_contour_count, s, timer, ClusterLaunch());
-        if (st != MOCAP_OK) return st;
-    }
-    stage_begin(timer, 4, s);
-    st = launch_tiles(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws, L.max_fg, out_flags, need_general, s);
-    if (st != MOCAP_OK) return st;
-    if (out_bits) {
-        st = launch_materialize_bits(ws, n_frames, H, W, tv, out_bits, s);
-        if (st != MOCAP_OK) return st;
-    }
-    st = launch_blobs(ws.bits, ws.fg_tiles, ws.n_fg, n_frames, H, W, L.TX, L.max_fg, max_runs, max_blobs, max_contours,
-                      min_area, min_circ, (char*)workspace + L.off_blob, L.blob_stride,
-                      out_xy, xy_float, out_count, out_flags, out_blob_sums, out_blob_count, out_contours, out_contour_count,
-                      out_labels, need_general, s);
-    stage_end(timer, 4, s);
-    return st;
-}
-
-extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                  const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
-                                  int max_blobs, int max_contours, int max_runs,
-                                  int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
-                                  uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
-                                  double* out_contours, int32_t* out_contour_count,
-                                  void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
-{
-    return detect_batch(frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours, max_runs,
-                        out_xy, 0, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count, out_contours, out_contour_count,
-                        workspace, workspace_bytes, stream, stage_timer);
-}
-
-extern "C" int mocap_detect_batch_subpixel(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
-                                           const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
-                                           int max_blobs, int max_contours, int max_runs,
-                                           float* out_xy, int32_t* out_count, int32_t* out_flags,
-                                           uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
-                                           double* out_contours, int32_t* out_contour_count,
-                                           void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
-{
-    return detect_batch(frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours, max_runs,
-                        (int32_t*)out_xy, 1, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count, out_contours,
-                        out_contour_count, workspace, workspace_bytes, stream, stage_timer);
-}
-
 // findContours -> filter -> moments on a given packed binary image (lib/ImageOperations.py:41-65), stage parity entry
 extern "C" int mocap_blobs_batch(const uint32_t* bits_dev, int n_frames, int H, int W,
                                  double min_area, double min_circ, int max_blobs, int max_contours, int max_runs,
@@ -268,9 +208,9 @@ extern "C" int mocap_blobs_batch(const uint32_t* bits_dev, int n_frames, int H, 
     if (!bits_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
     if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
     DetectLayout L;
-    int st = detect_layout(n_frames, H, W, max_contours, max_runs, true, &L);
+    int st = detect_layout(n_frames, H, W, max_contours, max_runs, 0, &L);
     if (st != MOCAP_OK) return st;
-    if (workspace_bytes < L.total) return MOCAP_ERR_WORKSPACE;
+    if (workspace_bytes < L.general_bytes) return MOCAP_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
     FilterWs ws = filter_ws((char*)workspace, L);
     CUDA_TRY(cudaMemsetAsync(out_flags, 0, (size_t)n_frames * 4, s));
@@ -285,19 +225,21 @@ extern "C" int mocap_blobs_batch(const uint32_t* bits_dev, int n_frames, int H, 
 
 
 // =========================================================================================================
-// Overlapped detection: the batch is cut into chunks of frames; the HBM-bound streaming scan of chunk k+1 runs
-// beside the instruction-bound stages (group / piece filter / borders) of chunk k on the same SMs.  Chunk k's stages run as
-// one chain on worker stream k mod workers.  The scan follows from the input:
-//   cell boxes handed in (cellbox_dev): no scan.
-//   frames a tensor map can describe, and stream memory operations available: ONE TMA-fed scan kernel over the whole batch
-//     on the pipe's high-priority scan stream; it publishes a flag per finished chunk, which the chunk's worker stream waits
-//     for with cuStreamWaitValue32 -- the scan CTA of an SM stays resident from the first byte to the last.
-//   otherwise (and in the CPU emulation build, which has neither): the classic scan kernels chunk by chunk on the scan
-//     stream, handed to the worker streams with one event per chunk.
-// Whatever the cluster path hands to the general path is finished for the whole batch after the join.
+// The detection schedule, one for the one-shot and the overlapped call; they differ only in a DetectSchedule.
+//   Product path (no label / bit-image outputs wanted): scan -> groups of hot cells -> per-cluster units in shared memory ->
+//   per-frame ordering.  Frames it cannot finish locally, and every frame when the parity outputs are requested, take the general
+//   per-frame path (tiles -> packed image -> runs, labels, contour tree), once for the whole batch at the end.
+//   The batch is cut into chunks of frames; chunk k's stages (group / piece filter / borders) run as one chain on worker stream
+//   k mod workers.  The one-shot call is one chunk on the caller's stream.  The overlapped call runs the HBM-bound scan of chunk k+1
+//   beside the instruction-bound stages of chunk k on the same SMs; its scan follows from the input:
+//     cell boxes handed in (cellbox_dev): no scan.
+//     frames a tensor map can describe, and stream memory operations available: ONE TMA-fed scan kernel over the whole batch
+//       on the pipe's high-priority scan stream; it publishes a flag per finished chunk, which the chunk's worker stream waits
+//       for with cuStreamWaitValue32 -- the scan CTA of an SM stays resident from the first byte to the last.
+//     otherwise (and in the CPU emulation build, which has neither): the classic scan kernels chunk by chunk on the scan
+//       stream, handed to the worker streams with one event per chunk.
 // =========================================================================================================
 #define PIPE_MAX_PROC 6
-#define PIPE_MAX_CHUNKS 64
 #define PIPE_TL_PER_CHUNK 4          // timeline marks per chunk: scan seen, grouped, filtered, borders done
 #define PIPE_FILTER_CTAS_TMA 6       // persistent piece-filter CTAs per SM beside the TMA scan CTA
 #define PIPE_FILTER_CTAS 8           // ... without it
@@ -379,42 +321,166 @@ extern "C" void mocap_detect_pipe_destroy(void* pipe)
     delete p;
 }
 
-struct PipeLayout {
-    DetectLayout L;                  // general-path arrays of the whole batch (its cluster part serves chunk 0 .. see below)
-    size_t off_ctrl, off_need, off_chunks, chunk_bytes, total;
-    ClusterLayout cl;                // inside one chunk's cluster workspace
-    int chunks, chunk_frames;
+// where the cell boxes come from: the classic scan kernels chunk by chunk, one TMA-fed kernel over the batch, or the caller (no scan)
+enum ScanKind { SCAN_CLASSIC, SCAN_TMA, SCAN_HANDED_IN };
+
+// Everything in which the two detection calls differ.  The defaults are the one-shot call.
+struct DetectSchedule {
+    DetectPipe* pipe = nullptr;          // scan / worker streams with fork and join events; none: every stage on the caller's stream
+    int chunk_frames = 0;                // frames per chunk (<= 0: one chunk)
+    ScanKind scan = SCAN_CLASSIC;
+    const uint32_t* cellbox = nullptr;   // SCAN_HANDED_IN: the frames' hot cell boxes
+    int filter_ctas = 8, cand_ctas = 16; // persistent piece-filter CTAs, candidates_kernel CTAs per SM
+    StageTimer* timer = nullptr;         // per-stage events (one chunk)
+    int record_timeline = 0;             // keep the call's timeline in the pipe
+    const unsigned long long *xy_dst = nullptr, *count_dst = nullptr;   // store-to-peer tables
+    cudaEvent_t scan_wait = nullptr, scan_done = nullptr;              // scan token: the scan waits for scan_wait, scan_done follows it
 };
 
-static int pipe_layout(int n, int H, int W, int max_contours, int max_runs, int chunk_frames, PipeLayout* P)
+// out_xy holds int32 (xy_float 0) or float32 (1) centroid pairs; the store-to-peer epilogue copies 8-byte records and does not care which
+static int detect(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                  const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                  int max_blobs, int max_contours, int max_runs,
+                  int32_t* out_xy, int xy_float, int32_t* out_count, int32_t* out_flags,
+                  uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                  double* out_contours, int32_t* out_contour_count,
+                  void* workspace, size_t workspace_bytes, void* stream, const DetectSchedule& sch)
 {
-    if (chunk_frames <= 0 || chunk_frames > n) chunk_frames = n;
-    int chunks = cdiv(n, chunk_frames);
-    if (chunks > PIPE_MAX_CHUNKS) { chunk_frames = cdiv(n, PIPE_MAX_CHUNKS); chunks = cdiv(n, chunk_frames); }
-    P->chunks = chunks; P->chunk_frames = chunk_frames;
-    int st = detect_layout(n, H, W, max_contours, max_runs, true, &P->L);
+    if (!frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
+    if ((sch.xy_dst == nullptr) != (sch.count_dst == nullptr)) return MOCAP_ERR_INVALID;
+    if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
+    if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
+    DetectLayout L;
+    int st = detect_layout(n_frames, H, W, max_contours, max_runs, sch.chunk_frames, &L);
     if (st != MOCAP_OK) return st;
-    size_t off = P->L.off_cluster;                                  // the whole-batch cluster workspace is replaced by the per-chunk ones
-    auto take = [&](size_t bytes) { size_t r = off; off += align_up(bytes, 256); return r; };
-    P->off_ctrl = take(scan_tma_ctrl_bytes(chunks));
-    P->off_need = take((size_t)n * 4);
-    P->chunk_bytes = align_up(cluster_ws_bytes(chunk_frames, H, W, max_contours, &P->cl), 256);
-    P->off_chunks = take(P->chunk_bytes * (size_t)chunks);
-    P->total = off > P->L.total ? off : P->L.total;
-    return MOCAP_OK;
+    TableView tv;
+    st = lens_set_view(lenses, H, W, &tv);
+    if (st != MOCAP_OK) return st;
+    if (workspace_bytes < L.total) return MOCAP_ERR_WORKSPACE;
+    const bool extras = out_bits || out_labels || out_blob_sums || out_blob_count;
+    const bool cluster = !extras && cluster_path_supported(H, W);
+    DetectPipe* dp = sch.pipe;
+    if (dp && !cluster) return MOCAP_ERR_UNSUPPORTED;                       // such shapes take the one-shot call
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaStream_t s_scan = dp ? dp->s_scan : s;
+    char* base = (char*)workspace;
+    FilterWs ws = filter_ws(base, L);
+    if (sch.scan == SCAN_HANDED_IN) ws.cellbox = (uint32_t*)sch.cellbox;
+    int* need_general = (int*)(base + L.off_need);
+    int* ctrl = (int*)(base + L.off_ctrl);
+    const int chunks = L.chunks, cf = L.chunk_frames;
+    if (dp) { dp->last_tma = sch.scan == SCAN_TMA ? 1 : 0; dp->last_chunks = chunks; dp->tl_chunks = 0; }
+    CUDA_TRY(cudaMemsetAsync(out_flags, 0, (size_t)n_frames * 4, s));
+    if (out_labels) CUDA_TRY(cudaMemsetAsync(out_labels, 0, (size_t)n_frames * H * W * 4, s));
+    CUDA_TRY(cudaMemsetAsync(need_general, cluster ? 0 : 1, (size_t)n_frames * 4, s));
+    if (sch.scan == SCAN_TMA) CUDA_TRY(cudaMemsetAsync(ctrl, 0, scan_tma_ctrl_bytes(chunks), s));
+    if (dp) {
+        CUDA_TRY(cudaEventRecord(dp->ev_fork, s));
+        CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, dp->ev_fork, 0));
+    }
+    if (sch.scan_wait) CUDA_TRY(cudaStreamWaitEvent(s_scan, sch.scan_wait, 0));     // scans of several pipes one after the other
+    if (sch.scan == SCAN_TMA) {
+        st = launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, ctrl, chunks, cf, s_scan);
+        if (st != MOCAP_OK) return st;
+    }
+    for (int i = 0; dp && i < dp->n_proc; ++i) CUDA_TRY(cudaStreamWaitEvent(dp->s_proc[i], dp->ev_fork, 0));
+    ClusterLaunch how{sch.filter_ctas, sch.cand_ctas};
+    for (int c = 0; c < chunks; ++c) {
+        const int f0 = c * cf, nc = (n_frames - f0) < cf ? (n_frames - f0) : cf;
+        cudaStream_t ps = dp ? dp->s_proc[c % dp->n_proc] : s;
+        char* cws = base + L.off_chunks + (size_t)c * L.chunk_bytes;
+        uint32_t* cb = ws.cellbox + (size_t)f0 * tv.TX * tv.TY;
+        if (cluster) CUDA_TRY(cudaMemsetAsync(cws, 0, L.cl.zero_bytes, ps));      // the chunk's counters / lists, off the critical path
+        if (sch.scan == SCAN_TMA) {
+            st = stream_wait_geq(ps, scan_tma_chunk_flag(ctrl, chunks, c), 1);
+            if (st != MOCAP_OK) return st;
+        } else if (sch.scan == SCAN_CLASSIC) {                                       // (handed-in boxes were complete before the fork)
+            FilterWs wc = ws; wc.cellbox = cb;
+            st = launch_scan(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, wc, s_scan, sch.timer);
+            if (st != MOCAP_OK) return st;
+            if (dp) {
+                CUDA_TRY(cudaEventRecord(dp->ev_scan[c], s_scan));
+                CUDA_TRY(cudaStreamWaitEvent(ps, dp->ev_scan[c], 0));
+            }
+        }
+        if (!cluster) continue;
+        if (sch.record_timeline) CUDA_TRY(cudaEventRecord(dp->ev_tl[c][0], ps));
+        if (dp) { how.ev_group = dp->ev_tl[c][1]; how.ev_filter = dp->ev_tl[c][2]; how.ev_borders = dp->ev_tl[c][3]; }
+        TableView tc = tv;                                                          // the chunk's frames are numbered from 0
+        if (tc.frame_lens) tc.frame_lens += f0;
+        st = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tc, thresh, cb, cws, L.cl, need_general + f0,
+                                 max_contours, max_blobs, min_area, min_circ,
+                                 out_xy + (size_t)f0 * max_blobs * 2, xy_float, out_count + f0, out_flags + f0,
+                                 out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,
+                                 ps, sch.timer, how);
+        if (st != MOCAP_OK) return st;
+        if (sch.xy_dst) {                                    // the chunk's records go where their consumers read them, off the critical path
+            st = launch_scatter(out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, sch.xy_dst + f0, sch.count_dst + f0, nc, max_blobs,
+                                need_general + f0, 0, ps);
+            if (st != MOCAP_OK) return st;
+        }
+    }
+    if (sch.scan_done) CUDA_TRY(cudaEventRecord(sch.scan_done, s_scan));
+    if (dp) {
+        CUDA_TRY(cudaEventRecord(dp->ev_scan_done, dp->s_scan));
+        CUDA_TRY(cudaStreamWaitEvent(s, dp->ev_scan_done, 0));
+        for (int i = 0; i < dp->n_proc; ++i) {
+            CUDA_TRY(cudaEventRecord(dp->ev_proc_done[i], dp->s_proc[i]));
+            CUDA_TRY(cudaStreamWaitEvent(s, dp->ev_proc_done[i], 0));
+        }
+        if (sch.record_timeline) { CUDA_TRY(cudaEventRecord(dp->ev_join, s)); dp->tl_chunks = chunks; }
+    }
+    // the general path for the frames the cluster path handed over (rare; every frame without the cluster path), whole batch
+    stage_begin(sch.timer, 4, s);
+    st = launch_tiles(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws, L.max_fg, out_flags, need_general, s);
+    if (st != MOCAP_OK) return st;
+    if (out_bits) {
+        st = launch_materialize_bits(ws, n_frames, H, W, tv, out_bits, s);
+        if (st != MOCAP_OK) return st;
+    }
+    st = launch_blobs(ws.bits, ws.fg_tiles, ws.n_fg, n_frames, H, W, L.TX, L.max_fg, max_runs, max_blobs, max_contours,
+                      min_area, min_circ, base + L.off_blob, L.blob_stride,
+                      out_xy, xy_float, out_count, out_flags, out_blob_sums, out_blob_count, out_contours, out_contour_count,
+                      out_labels, need_general, s);
+    stage_end(sch.timer, 4, s);
+    if (st == MOCAP_OK && sch.xy_dst) st = launch_scatter(out_xy, out_count, sch.xy_dst, sch.count_dst, n_frames, max_blobs, need_general, 1, s);
+    return st;
 }
 
-extern "C" size_t mocap_detect_pipelined_workspace_bytes(int n_frames, int H, int W, int max_blobs, int max_contours, int max_runs, int chunk_frames)
+static DetectSchedule one_shot(void* stage_timer)
 {
-    (void)max_blobs;
-    if (max_contours <= 0 || max_runs <= 0) return 0;
-    PipeLayout P;
-    if (pipe_layout(n_frames, H, W, max_contours, max_runs, chunk_frames, &P) != MOCAP_OK) return 0;
-    return P.total;
+    DetectSchedule sch;
+    sch.timer = (StageTimer*)stage_timer;
+    return sch;
 }
 
-// mocap_detect_batch_pipelined and mocap_detect_batch_pipelined_subpixel: int32 (xy_float 0) or float32 (1) centroid pairs.  The
-// store-to-peer epilogue copies 8-byte records and does not care which.
+extern "C" int mocap_detect_batch(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                  const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                  int max_blobs, int max_contours, int max_runs,
+                                  int32_t* out_xy, int32_t* out_count, int32_t* out_flags,
+                                  uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                                  double* out_contours, int32_t* out_contour_count,
+                                  void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
+{
+    return detect(frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours, max_runs,
+                  out_xy, 0, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count, out_contours, out_contour_count,
+                  workspace, workspace_bytes, stream, one_shot(stage_timer));
+}
+
+extern "C" int mocap_detect_batch_subpixel(const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
+                                           const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
+                                           int max_blobs, int max_contours, int max_runs,
+                                           float* out_xy, int32_t* out_count, int32_t* out_flags,
+                                           uint32_t* out_bits, int32_t* out_labels, int64_t* out_blob_sums, int32_t* out_blob_count,
+                                           double* out_contours, int32_t* out_contour_count,
+                                           void* workspace, size_t workspace_bytes, void* stream, void* stage_timer)
+{
+    return detect(frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours, max_runs,
+                  (int32_t*)out_xy, 1, out_count, out_flags, out_bits, out_labels, out_blob_sums, out_blob_count, out_contours,
+                  out_contour_count, workspace, workspace_bytes, stream, one_shot(stage_timer));
+}
+
+// mocap_detect_batch_pipelined and mocap_detect_batch_pipelined_subpixel
 static int detect_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,
                             const MocapLensSet* lenses, int thresh, double min_area, double min_circ,
                             int max_blobs, int max_contours, int max_runs,
@@ -424,95 +490,24 @@ static int detect_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames,
                             void* scan_wait_event, void* scan_done_event,
                             void* workspace, size_t workspace_bytes, void* stream, int chunk_frames, int record_timeline)
 {
-    DetectPipe* dp = (DetectPipe*)pipe;
-    if (!dp || !frames_dev || !out_xy || !out_count || !out_flags || !workspace) return MOCAP_ERR_INVALID;
-    if ((xy_dst_dev == nullptr) != (count_dst_dev == nullptr)) return MOCAP_ERR_INVALID;
-    if (max_blobs <= 0 || max_contours <= 0 || max_runs <= 0) return MOCAP_ERR_INVALID;
-    if (frame_stride < (int64_t)H * W) return MOCAP_ERR_INVALID;
-    PipeLayout P;
-    int st = pipe_layout(n_frames, H, W, max_contours, max_runs, chunk_frames, &P);
-    if (st != MOCAP_OK) return st;
-    TableView tv;
-    st = lens_set_view(lenses, H, W, &tv);
-    if (st != MOCAP_OK) return st;
-    if (workspace_bytes < P.total) return MOCAP_ERR_WORKSPACE;
-    if (!cluster_path_supported(H, W)) return MOCAP_ERR_UNSUPPORTED;         // such shapes take mocap_detect_batch
-    cudaStream_t s = (cudaStream_t)stream;
-    const unsigned long long* sc_xy = (const unsigned long long*)xy_dst_dev;
-    const unsigned long long* sc_count = (const unsigned long long*)count_dst_dev;
-    char* base = (char*)workspace;
-    FilterWs ws = filter_ws(base, P.L);
+    if (!pipe) return MOCAP_ERR_INVALID;
+    DetectSchedule sch;
+    sch.pipe = (DetectPipe*)pipe;
+    sch.chunk_frames = chunk_frames;
     // hot cell boxes handed in (the Bayer front step computes them while it writes the grey frames): no streaming scan in this call
-    const bool prescanned = cellbox_dev != nullptr;
-    if (prescanned) ws.cellbox = (uint32_t*)cellbox_dev;
-    int* ctrl = (int*)(base + P.off_ctrl);
-    int* need_general = (int*)(base + P.off_need);
-    const int chunks = P.chunks, cf = P.chunk_frames;
-    const bool tma = !prescanned && scan_tma_supported(frames_dev, n_frames, H, W, frame_stride, thresh) && stream_wait_supported();
-    dp->last_tma = tma ? 1 : 0; dp->last_chunks = chunks;
-    dp->tl_chunks = 0;
-    ClusterLaunch how;
-    how.zero = 0;                    // the chunk loop clears each chunk's block on its worker stream ahead of its scan wait
-    how.filter_ctas = tma ? PIPE_FILTER_CTAS_TMA : PIPE_FILTER_CTAS;
-    how.cand_ctas = PIPE_CAND_CTAS;
-    CUDA_TRY(cudaMemsetAsync(out_flags, 0, (size_t)n_frames * 4, s));
-    CUDA_TRY(cudaMemsetAsync(need_general, 0, (size_t)n_frames * 4, s));
-    CUDA_TRY(cudaMemsetAsync(ctrl, 0, scan_tma_ctrl_bytes(chunks), s));
-    CUDA_TRY(cudaEventRecord(dp->ev_fork, s));
-    CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, dp->ev_fork, 0));
-    if (scan_wait_event) CUDA_TRY(cudaStreamWaitEvent(dp->s_scan, (cudaEvent_t)scan_wait_event, 0));    // scans of several pipes one after the other
-    if (tma) {
-        st = launch_scan_tma(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws.cellbox, ctrl, chunks, cf, dp->s_scan);
-        if (st != MOCAP_OK) return st;
-    }
-    for (int i = 0; i < dp->n_proc; ++i) CUDA_TRY(cudaStreamWaitEvent(dp->s_proc[i], dp->ev_fork, 0));
-    for (int c = 0; c < chunks; ++c) {
-        const int f0 = c * cf, nc = (n_frames - f0) < cf ? (n_frames - f0) : cf;
-        cudaStream_t ps = dp->s_proc[c % dp->n_proc];
-        char* cws = base + P.off_chunks + (size_t)c * P.chunk_bytes;
-        uint32_t* cb = ws.cellbox + (size_t)f0 * tv.TX * tv.TY;
-        CUDA_TRY(cudaMemsetAsync(cws + P.cl.zero_begin, 0, P.cl.zero_bytes, ps));     // the chunk's counters / lists, off the critical path
-        if (tma) {
-            st = stream_wait_geq(ps, scan_tma_chunk_flag(ctrl, chunks, c), 1);
-            if (st != MOCAP_OK) return st;
-        } else if (!prescanned) {                                                   // (handed-in boxes were complete before the fork)
-            FilterWs wc = ws; wc.cellbox = cb;
-            st = launch_scan(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tv, thresh, wc, dp->s_scan, nullptr);
-            if (st != MOCAP_OK) return st;
-            CUDA_TRY(cudaEventRecord(dp->ev_scan[c], dp->s_scan));
-            CUDA_TRY(cudaStreamWaitEvent(ps, dp->ev_scan[c], 0));
-        }
-        if (record_timeline) CUDA_TRY(cudaEventRecord(dp->ev_tl[c][0], ps));
-        how.ev_group = dp->ev_tl[c][1]; how.ev_filter = dp->ev_tl[c][2]; how.ev_borders = dp->ev_tl[c][3];
-        TableView tc = tv;                                                          // the chunk's frames are numbered from 0
-        if (tc.frame_lens) tc.frame_lens += f0;
-        st = launch_cluster_path(frames_dev + (size_t)f0 * frame_stride, nc, H, W, frame_stride, tc, thresh, cb, cws, P.cl, need_general + f0,
-                                 max_contours, max_blobs, min_area, min_circ,
-                                 out_xy + (size_t)f0 * max_blobs * 2, xy_float, out_count + f0, out_flags + f0,
-                                 out_contours ? out_contours + (size_t)f0 * max_contours * 8 : nullptr, out_contour_count ? out_contour_count + f0 : nullptr,
-                                 ps, nullptr, how);
-        if (st != MOCAP_OK) return st;
-        if (sc_xy) {                                         // the chunk's records go where their consumers read them, off the critical path
-            st = launch_scatter(out_xy + (size_t)f0 * max_blobs * 2, out_count + f0, sc_xy + f0, sc_count + f0, nc, max_blobs, need_general + f0, 0, ps);
-            if (st != MOCAP_OK) return st;
-        }
-    }
-    CUDA_TRY(cudaEventRecord(dp->ev_scan_done, dp->s_scan));
-    if (scan_done_event) CUDA_TRY(cudaEventRecord((cudaEvent_t)scan_done_event, dp->s_scan));
-    CUDA_TRY(cudaStreamWaitEvent(s, dp->ev_scan_done, 0));
-    for (int i = 0; i < dp->n_proc; ++i) {
-        CUDA_TRY(cudaEventRecord(dp->ev_proc_done[i], dp->s_proc[i]));
-        CUDA_TRY(cudaStreamWaitEvent(s, dp->ev_proc_done[i], 0));
-    }
-    if (record_timeline) { CUDA_TRY(cudaEventRecord(dp->ev_join, s)); dp->tl_chunks = chunks; }
-    // general path for the frames the cluster units could not finish (rare), whole batch
-    st = launch_tiles(frames_dev, n_frames, H, W, frame_stride, tv, thresh, ws, P.L.max_fg, out_flags, need_general, s);
-    if (st != MOCAP_OK) return st;
-    st = launch_blobs(ws.bits, ws.fg_tiles, ws.n_fg, n_frames, H, W, P.L.TX, P.L.max_fg, max_runs, max_blobs, max_contours,
-                      min_area, min_circ, base + P.L.off_blob, P.L.blob_stride,
-                      out_xy, xy_float, out_count, out_flags, nullptr, nullptr, out_contours, out_contour_count, nullptr, need_general, s);
-    if (st == MOCAP_OK && sc_xy) st = launch_scatter(out_xy, out_count, sc_xy, sc_count, n_frames, max_blobs, need_general, 1, s);
-    return st;
+    sch.scan = cellbox_dev ? SCAN_HANDED_IN :
+               scan_tma_supported(frames_dev, n_frames, H, W, frame_stride, thresh) && stream_wait_supported() ? SCAN_TMA : SCAN_CLASSIC;
+    sch.cellbox = cellbox_dev;
+    sch.filter_ctas = sch.scan == SCAN_TMA ? PIPE_FILTER_CTAS_TMA : PIPE_FILTER_CTAS;
+    sch.cand_ctas = PIPE_CAND_CTAS;
+    sch.record_timeline = record_timeline;
+    sch.xy_dst = (const unsigned long long*)xy_dst_dev;
+    sch.count_dst = (const unsigned long long*)count_dst_dev;
+    sch.scan_wait = (cudaEvent_t)scan_wait_event;
+    sch.scan_done = (cudaEvent_t)scan_done_event;
+    return detect(frames_dev, n_frames, H, W, frame_stride, lenses, thresh, min_area, min_circ, max_blobs, max_contours, max_runs,
+                  out_xy, xy_float, out_count, out_flags, nullptr, nullptr, nullptr, nullptr, out_contours, out_contour_count,
+                  workspace, workspace_bytes, stream, sch);
 }
 
 extern "C" int mocap_detect_batch_pipelined(void* pipe, const uint8_t* frames_dev, int n_frames, int H, int W, int64_t frame_stride,

@@ -153,18 +153,16 @@ __device__ __forceinline__ void store_centroid(int32_t* xy, double qx, double qy
     else { xy[0] = (int32_t)qx; xy[1] = (int32_t)qy; }
 }
 
-// how launch_cluster_path runs a batch (or one chunk of the overlapped pipeline)
+// how launch_cluster_path runs one chunk of frames
 struct ClusterLaunch {
-    int zero = 1;                    // clear the counters / lists of the workspace on the stream first
-    int filter_ctas = 8;             // persistent piece-filter CTAs per SM (fewer when the TMA scan is co-resident)
-    int cand_ctas = 16;              // candidates_kernel CTAs per SM
+    int filter_ctas;                 // persistent piece-filter CTAs per SM (fewer when the TMA scan is co-resident)
+    int cand_ctas;                   // candidates_kernel CTAs per SM
     cudaEvent_t ev_group = nullptr, ev_filter = nullptr, ev_borders = nullptr;   // recorded after the stages (timeline marks)
 };
 
 // byte offsets of the cluster path's arrays in its workspace (cluster_ws_bytes)
 struct ClusterLayout {
-    size_t need_general;             // int [n] (the chunked path keeps one array for the whole batch instead)
-    size_t zero_begin, zero_bytes;   // the block a call has to zero first: counters, rec_count, cand_count, frame_clusters
+    size_t zero_bytes;               // the first bytes, which the caller zeroes before the launch: counters, rec_count, cand_count, frame_clusters
     size_t counters, rec_count, cand_count, frame_clusters;
     size_t clusters, pieces, rec_start, rec_a, rec_per, memb, rows_out, cand_list, rec_info;
 };

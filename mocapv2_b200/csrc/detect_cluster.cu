@@ -1121,13 +1121,11 @@ size_t cluster_ws_bytes(int n, int H, int W, int max_contours, ClusterLayout* L)
 {
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t r = off; off += align_up(bytes, 256); return r; };
-    L->need_general = take((size_t)n * 4);
-    L->zero_begin = off;
     L->counters = take(64);
     L->rec_count = take((size_t)n * 4);
     L->cand_count = take((size_t)n * 4);
     L->frame_clusters = take((size_t)n * 8);
-    L->zero_bytes = off - L->zero_begin;
+    L->zero_bytes = off;
     L->clusters = take((size_t)cl_cap_of(n) * 32);
     L->pieces = take((size_t)pc_cap_of(n) * 32);
     L->rec_start = take((size_t)n * max_contours * 4);
@@ -1169,7 +1167,6 @@ int launch_cluster_path(const uint8_t* frames, int n, int H, int W, int64_t fstr
     cw.rec_info = (int*)(ws_base + L.rec_info);
     cw.frame_clusters = (int*)(ws_base + L.frame_clusters);
     cw.n_frames = n;
-    if (how.zero) CUDA_TRY(cudaMemsetAsync(ws_base + L.zero_begin, 0, L.zero_bytes, s));
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
