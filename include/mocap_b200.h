@@ -198,7 +198,8 @@ int mocap_blobs_batch(const uint32_t* bits_dev, int n_frames, int H, int W,
 
 /* cv.drawContours(img, contours_filtered, -1, (0,0,255), 2) of _find_dot (lib/ImageOperations.py:52-55; display only): paints `value`
  * (the reference's colour on a one-channel image: 0) over the thickness-2 outline of every KEPT contour of the table returned by
- * mocap_detect_batch (out_contours / out_contour_count, with the packed binary image out_bits of the same call) into img_dev [n][H][W]. */
+ * mocap_detect_batch (out_contours / out_contour_count, with the packed binary image out_bits of the same call) into img_dev [n][H][W].
+ * H, W <= 16384 as for mocap_detect_batch. */
 int mocap_draw_contours_batch(const uint32_t* bits_dev, const double* contours_dev, const int32_t* contour_count_dev,
                               int n_frames, int H, int W, int max_contours, uint8_t* img_dev, int value, void* stream);
 

@@ -153,6 +153,30 @@ __device__ __forceinline__ void store_centroid(int32_t* xy, double qx, double qy
     else { xy[0] = (int32_t)qx; xy[1] = (int32_t)qy; }
 }
 
+// The reference's filter of a border (lib/ImageOperations.py:43-51) from its Green sum a00 (twice the signed area) and its
+// perimeter: circularity 4 pi area / perimeter^2 > min_circ and area > min_area, and m00 != 0 (a centroid exists).
+__device__ __forceinline__ int contour_keep(long long a00, double per, double min_area, double min_circ)
+{
+    const double area = (double)(a00 < 0 ? -a00 : a00) * 0.5;
+    int keep = 0;
+    if (per != 0.0) {
+        const double circ = __ddiv_rn(__dmul_rn(12.566370614359172, area), __dmul_rn(per, per));
+        keep = (circ > min_circ && area > min_area) ? 1 : 0;
+    }
+    return a00 == 0 ? 0 : keep;
+}
+
+// The centroid record of a kept border from its Green sums: cv.moments' m00, m10, m01 (a00 / 2, a10 / 6, a01 / 6 with the sign
+// of a00), then store_centroid.
+__device__ __forceinline__ void store_blob_centroid(int32_t* xy, long long a00, long long a10, long long a01, int xy_float)
+{
+    const double sgn = a00 > 0 ? 1.0 : -1.0;
+    const double m00 = __dmul_rn((double)a00, sgn * 0.5);
+    const double m10 = __dmul_rn((double)a10, sgn * 0.16666666666666666);
+    const double m01 = __dmul_rn((double)a01, sgn * 0.16666666666666666);
+    store_centroid(xy, __ddiv_rn(m10, m00), __ddiv_rn(m01, m00), xy_float);
+}
+
 // how launch_cluster_path runs one chunk of frames
 struct ClusterLaunch {
     int filter_ctas;                 // persistent piece-filter CTAs per SM (fewer when the TMA scan is co-resident)
@@ -176,36 +200,6 @@ struct FilterWs {
     uint32_t* fg_tiles;  // [n][max_fg] tiles that hold at least one foreground pixel
     int* n_fg;           // [n]
     uint32_t* cellbox;   // [n][TY][TX] hot bounding box of every 32x32 source cell (written by the scan pass)
-};
-
-// ---------------------------------------------------------------------------------------------------------
-// Packed binary image access: word (y, x>>5), bit x&31 (LSB = leftmost pixel)
-// ---------------------------------------------------------------------------------------------------------
-struct BitImg {
-    const uint32_t* p;
-    int W, H, WPR;
-    __device__ __forceinline__ int get(int x, int y) const {
-        if ((unsigned)x >= (unsigned)W || (unsigned)y >= (unsigned)H) return 0;
-        return (p[(size_t)y * WPR + (x >> 5)] >> (x & 31)) & 1;
-    }
-    // bits x-1, x, x+1 of row y (bit 0 = x-1); pixels outside the image read 0.  x must be inside the image.
-    __device__ __forceinline__ uint32_t row3(int x, int y) const {
-        if ((unsigned)y >= (unsigned)H) return 0u;
-        const uint32_t* r = p + (size_t)y * WPR;
-        int wi = x >> 5, b = x & 31;
-        uint32_t w = r[wi], out;
-        if (b == 0) out = ((w & 3u) << 1) | (wi > 0 ? r[wi - 1] >> 31 : 0u);
-        else if (b == 31) out = (w >> 30) | (wi + 1 < WPR ? (r[wi + 1] & 1u) << 2 : 0u);
-        else out = (w >> (b - 1)) & 7u;
-        if (x + 1 >= W) out &= 3u;
-        return out;
-    }
-    // 8-neighbour occupancy of (x, y), bit d = neighbour in direction d (0=E 1=NE 2=N 3=NW 4=W 5=SW 6=S 7=SE)
-    __device__ __forceinline__ uint32_t nbr8(int x, int y) const {
-        uint32_t up = row3(x, y - 1), mid = row3(x, y), dn = row3(x, y + 1);
-        return ((mid >> 2) & 1u) | (((up >> 2) & 1u) << 1) | (((up >> 1) & 1u) << 2) | ((up & 1u) << 3) |
-               ((mid & 1u) << 4) | ((dn & 1u) << 5) | (((dn >> 1) & 1u) << 6) | (((dn >> 2) & 1u) << 7);
-    }
 };
 
 // 8-neighbour codes: 0=E 1=NE 2=N 3=NW 4=W 5=SW 6=S 7=SE (y grows downwards)

@@ -7,10 +7,10 @@
 //   labelling   union-find over runs (8-connectivity, smaller raster index wins) -> blob = root run, whose
 //               first pixel is the blob's raster-first pixel = start of its outer border (SURVEY App. A5);
 //               per-blob pixel sums m00/m10/m01 accumulated with atomics (closed form per run)
-//   holes       every run's right edge starts a short Suzuki-Abe walk; the walk that returns to its own
-//               start without meeting a smaller west/east edge of the same border is a hole border start
-//   contours    one thread per border: border following with CHAIN_APPROX_SIMPLE vertices, Green sums
-//               a00/a10/a01 in int64, perimeter = sum of float32 sqrt per segment (exact in double)
+//   holes       every run's right edge starts a trace that is abandoned at the first smaller west/east edge of
+//               its border; a trace that completes is a hole border start
+//   contours    one thread per border: trace_border (walk.cuh) on the frame image, Green sums a00/a10/a01
+//               and perimeter of the CHAIN_APPROX_SIMPLE polygon
 //   tree/order  parents from the nearest foreground pixel to the left (Suzuki Table 1), output order =
 //               pre-order with siblings in reverse raster order, then the reference's filter and centroid.
 #include "common.cuh"
@@ -131,7 +131,6 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
 
     const uint32_t* bits = bits_all + (size_t)f * H * TX;
     const uint32_t* fg_tiles = fg_tiles_all + (size_t)f * P.max_fg;
-    BitImg im; im.p = bits; im.W = W; im.H = H; im.WPR = TX;
     int n_t = min(n_fg_all[f], P.max_fg);
 
     if (tid == 0) { s_flag = 0; s_nholes = 0; }
@@ -159,6 +158,7 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
         }
         return;
     }
+    step_table_build();                              // for the traces below (the next barrier publishes it)
     for (int y = tid; y < H + 1; y += nt) w.rowfill[y] = w.rowptr[y];
     __syncthreads();
     for (int it = tid; it < n_t * TILE; it += nt) {
@@ -247,7 +247,8 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
         if (n_cand <= P.max_contours) {
             for (int c = tid; c < n_cand; c += nt) {
                 int st = w.c_start[c], ty = w.c_type[c], ovf = 0;
-                int ok = trace_contour(im, st % W, st / W, ty ? 0 : 4, 2LL * st + ty, &w.c_a[3 * c], &w.c_per[c], &w.c_n[c], &ovf, 0, 0, W);
+                int ok = trace_border<true>(bits, H, TX, W, st % W, st / W, ty ? 0 : 4, 2LL * st + ty, &w.c_a[3 * c], &w.c_per[c], &w.c_n[c], &ovf,
+                                            0, 0, W, nullptr);
                 if (ovf) atomicOr(&s_flag, MOCAP_FLAG_TRACE_OVERFLOW);
                 w.c_keep[c] = ok;                      // parked: candidate is a real border start
                 if (ok && ty) atomicAdd(&s_nholes, 1);
@@ -360,8 +361,8 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
         if (xx == RUN_DEAD) continue;
         int y = w.run_y[r];
         int x1 = xx >> 16;
-        int ovf = 0;
-        if (walk_min_edge(im, x1, y, 0, 0, nullptr, &ovf)) {
+        long long a[3]; double per; int nch, ovf = 0;
+        if (trace_border<true>(bits, H, TX, W, x1, y, 0, 2LL * (y * W + x1) + 1, a, &per, &nch, &ovf, 0, 0, W, nullptr)) {
             int k = n_blobs + atomicAdd(&s_nholes, 1);
             if (k < P.max_contours) {
                 int comp = w.run_rank[w.run_parent[r]];
@@ -389,7 +390,7 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
     for (int c = tid; c < n_cont; c += nt) {
         int st = w.c_start[c];
         int ovf = 0;
-        trace_contour(im, st % W, st / W, w.c_type[c] ? 0 : 4, -1, &w.c_a[3 * c], &w.c_per[c], &w.c_n[c], &ovf, 0, 0, W);
+        trace_border<true>(bits, H, TX, W, st % W, st / W, w.c_type[c] ? 0 : 4, -1, &w.c_a[3 * c], &w.c_per[c], &w.c_n[c], &ovf, 0, 0, W, nullptr);
         if (ovf) atomicOr(&s_flag, MOCAP_FLAG_TRACE_OVERFLOW);
     }
     // ---- parents ------------------------------------------------------------------------------------------------
@@ -404,8 +405,8 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
         int q = r - 1;                                    // run ending left of us
         int other = w.run_rank[w.run_parent[q]];          // blob owning it
         if (w.holes_of[other] == 0) { w.c_parent[c] = -2 - other; continue; }
-        long long mk; int ovf = 0;
-        walk_min_edge(im, (int)(w.run_xx[q] >> 16), y, 0, 1, &mk, &ovf);
+        long long a[3], mk; double per; int nch, ovf = 0;         // smallest edge of the border through q's east edge
+        trace_border<true, true>(bits, H, TX, W, (int)(w.run_xx[q] >> 16), y, 0, -1, a, &per, &nch, &ovf, 0, 0, W, nullptr, &mk);
         if (ovf) atomicOr(&s_flag, MOCAP_FLAG_TRACE_OVERFLOW);
         if ((mk & 1) == 0) { w.c_parent[c] = -2 - other; continue; }     // smallest edge is a west edge: outer border of `other`
         int hole_start = (int)(mk >> 1), par = -1;
@@ -475,19 +476,8 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
     }   // general path
 
     // ---- the reference's filter and centroid (ImageOperations.py:43-65) -------------------------------------------------
-    for (int c = tid; c < n_arr; c += nt) {
-        if (w.c_rank[c] < 0) { w.c_keep[c] = 0; continue; }     // rejected fast-path candidate
-        long long a00 = w.c_a[3 * c];
-        double area = (double)(a00 < 0 ? -a00 : a00) * 0.5;
-        double per = w.c_per[c];
-        int keep = 0;
-        if (per != 0.0) {
-            double circ = __ddiv_rn(__dmul_rn(12.566370614359172, area), __dmul_rn(per, per));
-            keep = (circ > P.min_circ && area > P.min_area) ? 1 : 0;
-        }
-        if (a00 == 0) keep = 0;                          // moments["m00"] == 0 -> no centroid
-        w.c_keep[c] = keep;
-    }
+    for (int c = tid; c < n_arr; c += nt)                       // a rejected fast-path candidate has rank -1
+        w.c_keep[c] = w.c_rank[c] < 0 ? 0 : contour_keep(w.c_a[3 * c], w.c_per[c], P.min_area, P.min_circ);
     __syncthreads();
     if (tid == 0) s_ncont = 0;
     __syncthreads();
@@ -506,13 +496,7 @@ __global__ void __launch_bounds__(BLOB_THREADS) blobs_kernel(
         int pos = 0;
         for (int u = 0; u < n_arr; ++u) pos += (w.c_keep[u] && w.c_rank[u] < rank);
         atomicAdd(&s_ncont, 1);
-        if (pos < P.max_blobs) {
-            double sgn = a00 > 0 ? 1.0 : -1.0;
-            double m00 = __dmul_rn((double)a00, sgn * 0.5);
-            double m10 = __dmul_rn((double)a10, sgn * 0.16666666666666666);
-            double m01 = __dmul_rn((double)a01, sgn * 0.16666666666666666);
-            store_centroid(out_xy + ((size_t)f * P.max_blobs + pos) * 2, __ddiv_rn(m10, m00), __ddiv_rn(m01, m00), P.xy_float);
-        }
+        if (pos < P.max_blobs) store_blob_centroid(out_xy + ((size_t)f * P.max_blobs + pos) * 2, a00, a10, a01, P.xy_float);
     }
     __syncthreads();
     if (tid == 0) {
@@ -586,35 +570,31 @@ int launch_blobs(const uint32_t* bits, const uint32_t* fg_tiles, const int* n_fg
 // border (OpenCV widens every segment by one pixel to each side and rounds its ends with a radius-1 disc) covers exactly: the plus-
 // shaped neighbourhood of every border pixel and, for every diagonal step (x, y) -> (x + dx, y + dy), the pixels (x + dx, y),
 // (x, y + dy), (x + dx, y - dy), (x - dx, y + dy), (x + 2 dx, y), (x, y + 2 dy) (checked against cv2 on random images with holes and
-// nesting, tests/test_dropin.py).  One thread per kept contour of the table re-walks its border on the packed binary image.
+// nesting, tests/test_dropin.py).  One thread per kept contour of the table re-traces its border on the packed binary image and
+// paints at every step.
 // ---------------------------------------------------------------------------------------------------------
 __global__ void draw_contours_kernel(const uint32_t* __restrict__ bits, const double* __restrict__ contours, const int32_t* __restrict__ contour_count,
                                      int max_contours, int H, int W, int TX, uint8_t* __restrict__ img, int value)
 {
-    const int f = blockIdx.y, c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= min(contour_count[f], max_contours)) return;
+    const int f = blockIdx.y, c = blockIdx.x * blockDim.x + threadIdx.x, n_c = min(contour_count[f], max_contours);
+    if ((int)(blockIdx.x * blockDim.x) >= n_c) return;         // no contour of the frame in this CTA: no step table either
+    step_table_build();
+    __syncthreads();
+    if (c >= n_c) return;
     const double* o = contours + ((size_t)f * max_contours + c) * 8;
     if (o[6] == 0.0) return;                                   // not kept by the area / circularity filter
     const int st = (int)o[7], hole = o[4] != 0.0;
-    BitImg im; im.p = bits + (size_t)f * H * TX; im.W = W; im.H = H; im.WPR = TX;
     uint8_t* out = img + (size_t)f * H * W;
     auto put = [&](int x, int y) { if ((unsigned)x < (unsigned)W && (unsigned)y < (unsigned)H) out[(size_t)y * W + x] = (uint8_t)value; };
     auto plus = [&](int x, int y) { put(x, y); put(x - 1, y); put(x + 1, y); put(x, y - 1); put(x, y + 1); };
     const int y0 = st / W, x0 = st - y0 * W;
-    Walk w; walk_init(im, w, x0, y0, hole ? 0 : 4);           // outer borders start on a west edge, hole borders on an east edge
     plus(x0, y0);
-    if (w.single) return;
-    for (int step = 0; step < WALK_BUDGET; ++step) {
-        const int cx = w.x, cy = w.y;
-        unsigned zeros; bool done;
-        const int d = walk_step(im, w, zeros, done);
-        plus(cx, cy);
-        if (d & 1) {
-            const int dx = dir_dx(d), dy = dir_dy(d);
-            put(cx + dx, cy); put(cx, cy + dy); put(cx + dx, cy - dy); put(cx - dx, cy + dy); put(cx + 2 * dx, cy); put(cx, cy + 2 * dy);
-        }
-        if (done) break;
-    }
+    long long a[3]; double per; int nch, ovf = 0;                   // outer borders start on a west edge, hole borders on an east edge
+    trace_border<true>(bits + (size_t)f * H * TX, H, TX, W, x0, y0, hole ? 0 : 4, -1, a, &per, &nch, &ovf, 0, 0, W, nullptr, nullptr,
+                       [&](int x, int y, int dx, int dy) {
+                           plus(x, y);
+                           if (dx && dy) { put(x + dx, y); put(x, y + dy); put(x + dx, y - dy); put(x - dx, y + dy); put(x + 2 * dx, y); put(x, y + 2 * dy); }
+                       });
 }
 
 extern "C" int mocap_draw_contours_batch(const uint32_t* bits_dev, const double* contours_dev, const int32_t* contour_count_dev,
@@ -622,6 +602,7 @@ extern "C" int mocap_draw_contours_batch(const uint32_t* bits_dev, const double*
 {
     if (!bits_dev || !contours_dev || !contour_count_dev || !img_dev || n_frames <= 0 || n_frames > 65535 || H <= 0 || W <= 0 || max_contours <= 0)
         return MOCAP_ERR_INVALID;
+    if (H > 16384 || W > 16384) return MOCAP_ERR_UNSUPPORTED;          // the frame sizes of mocap_detect_batch (32-bit edge keys)
     LAUNCH(draw_contours_kernel, dim3(cdiv(max_contours, 64), n_frames), 64, 0, (cudaStream_t)stream, bits_dev, contours_dev, contour_count_dev,
            max_contours, H, W, cdiv(W, TILE), img_dev, value);
     CUDA_TRY(cudaGetLastError());

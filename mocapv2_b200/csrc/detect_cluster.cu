@@ -847,9 +847,9 @@ __global__ void __launch_bounds__(128) candidates_kernel(ClusterWs cw)
         if (mw <= 0 || cw.need_general[f]) continue;
         const int m_off = cb.y & 0xffff, m_cnt = cb.y >> 16;
         const short* memb = cw.memb + ((size_t)f * HOT_MAX + m_off) * 4;
-        BitImg im; im.p = cw.rows_out + (unsigned)ca.w; im.W = mw; im.H = mh; im.WPR = wpr;
+        const uint32_t* rows = cw.rows_out + (unsigned)ca.w;
         for (int r = lane; r < mh; r += 32) {
-            const uint32_t* row = im.p + (size_t)r * wpr;
+            const uint32_t* row = rows + (size_t)r * wpr;
             if (wpr == 2) {
                 // box at most 64 wide: the row and the row above are one 64-bit word each, runs and gaps come from bit scans
                 // (bit-row storage is handed out in even word counts, so these rows are 8-byte aligned)
@@ -894,19 +894,19 @@ __global__ void __launch_bounds__(128) candidates_kernel(ClusterWs cw)
 // Start pixel (frame index) of the outer border of the blob that owns the hole border starting at local pixel (lx, ly):
 // the west edge of the leftmost pixel of that pixel's run lies on another border of the same blob; if that border's
 // smallest edge is a west edge it is the blob's outer border, otherwise it is another hole of the blob further left and the
-// search continues from there.  -1 if it does not settle.
-__device__ long long hole_parent_start(const BitImg& im, int lx, int ly, int ox, int oy, int Wabs, int* overflow)
+// search continues from there.  -1 if it does not settle.  The box: mw x mh pixels at (ox, oy) of a frame Wabs wide.
+__device__ long long hole_parent_start(const uint32_t* rows, int mw, int mh, int wpr, int lx, int ly, int ox, int oy, int Wabs, int* overflow)
 {
     for (int hop = 0; hop < 32; ++hop) {
+        const uint32_t* row = rows + (size_t)ly * wpr;
         int x = lx;
-        while (x > 0 && im.get(x - 1, ly)) --x;                    // leftmost pixel of the run
-        long long mk;
-        walk_min_edge(im, x, ly, 4, 1, &mk, overflow);             // smallest edge of the border through that west edge (local keys)
+        while (x > 0 && ((row[(x - 1) >> 5] >> ((x - 1) & 31)) & 1u)) --x;     // leftmost pixel of the run
+        long long a[3], mk; double per; int nch;
+        trace_border<true, true>(rows, mh, wpr, mw, x, ly, 4, -1, a, &per, &nch, overflow, ox, oy, Wabs, nullptr, &mk);
         if (*overflow) return -1;
-        long long pix = mk >> 1;
-        int sx = (int)(pix % im.W), sy = (int)(pix / im.W);
-        if ((mk & 1) == 0) return (long long)(sy + oy) * Wabs + (sx + ox);
-        lx = sx; ly = sy;                                          // start pixel of another hole border of the same blob
+        const long long pix = mk >> 1;                             // smallest edge of the border through that west edge
+        if ((mk & 1) == 0) return pix;
+        ly = (int)(pix / Wabs) - oy; lx = (int)(pix % Wabs) - ox;  // start pixel of another hole border of the same blob
     }
     return -1;
 }
@@ -923,8 +923,8 @@ __device__ void frame_traces(const ClusterWs& cw, int f, int W, int max_contours
     const int n_cand = min(cw.cand_count[f], CAND_PER_FRAME);
     // Work order: a warp traces 32 borders in lockstep, so its time is its longest border.  The candidates are therefore
     // counting-sorted by the size of their cluster box (a proxy for the border length), longest first: the boxes wider than
-    // 64 pixels (several blobs next to each other; traced on a sliding 64-pixel window, generic loop only for boxes higher
-    // than 1024), then, from a warp boundary, the boxes up to 64 wide (rows cached in registers).  A second pass
+    // 64 pixels (several blobs next to each other) or higher than 1024, traced on a sliding 64-pixel window, then, from a
+    // warp boundary, the other boxes up to 64 wide (one 64-bit load per row).  A second pass
     // over the list runs in reverse thread order, so that the shortest borders follow the shortest first-pass borders.
     __shared__ uint16_t s_order[CAND_PER_FRAME + 32];          // + the padding between the two lists
     __shared__ int s_bucket[34];
@@ -965,20 +965,18 @@ __device__ void frame_traces(const ClusterWs& cw, int f, int W, int max_contours
         const int code = cw.cand_list[2 * c + 1];
         const int mx0 = ce[1] & 0xffff, my0 = ce[1] >> 16, mx1 = ce[2] & 0xffff, my1 = ce[2] >> 16;
         const int lx = code & 0xffff, ly = (code >> 16) & 0x7fff, ty = (code >> 31) & 1;
-        BitImg im; im.p = cw.rows_out + (unsigned)ce[3]; im.W = mx1 - mx0 + 1; im.H = my1 - my0 + 1; im.WPR = ce[4];
+        const uint32_t* rows = cw.rows_out + (unsigned)ce[3];
+        const int mw = mx1 - mx0 + 1, mh = my1 - my0 + 1, wpr = ce[4];
         long long st = (long long)(ly + my0) * W + (lx + mx0);
         long long a[3]; double per; int nch, ovf = 0, bbox[4];
         int ok;
-        if (it >= n_pad) ok = trace_contour64<false>(im.p, im.H, 2, 0, im.W, lx, ly, ty ? 0 : 4, 2 * st + ty, a, &per, &nch, &ovf, mx0, my0, W, bbox);
-        else if (im.W > 64 && im.H <= 1024) {
-            const int wx0 = min(max(lx - 32, 0), im.W - 64);
-            ok = trace_contour64<true>(im.p, im.H, im.WPR, wx0, im.W, lx - wx0, ly, ty ? 0 : 4, 2 * st + ty, a, &per, &nch, &ovf, mx0 + wx0, my0, W, bbox);
-        } else ok = trace_contour(im, lx, ly, ty ? 0 : 4, 2 * st + ty, a, &per, &nch, &ovf, mx0, my0, W, bbox);
+        if (it >= n_pad) ok = trace_border<false>(rows, mh, 2, mw, lx, ly, ty ? 0 : 4, 2 * st + ty, a, &per, &nch, &ovf, mx0, my0, W, bbox);
+        else ok = trace_border<true>(rows, mh, wpr, mw, lx, ly, ty ? 0 : 4, 2 * st + ty, a, &per, &nch, &ovf, mx0, my0, W, bbox);
         if (ovf) { cw.need_general[f] = 8; continue; }
         if (!ok) continue;
         long long parent = -1;
         if (ty) {
-            parent = hole_parent_start(im, lx, ly, mx0, my0, W, &ovf);
+            parent = hole_parent_start(rows, mw, mh, wpr, lx, ly, mx0, my0, W, &ovf);
             if (parent < 0) { cw.need_general[f] = 8; continue; }
             atomicAdd(&s_holes, 1);
         }
@@ -1031,17 +1029,7 @@ __device__ void frame_finalize(const ClusterWs& cw, int f, uint8_t* keepv /*[max
     const long long* ra = cw.rec_a + (size_t)f * max_contours * 3;
     const double* rper = cw.rec_per + (size_t)f * max_contours;
     const int* info = cw.rec_info + (size_t)f * max_contours * 4;
-    for (int c = tid; c < n; c += (int)blockDim.x) {
-        long long a00 = ra[3 * c];
-        double area = (double)(a00 < 0 ? -a00 : a00) * 0.5, per = rper[c];
-        int keep = 0;
-        if (per != 0.0) {
-            double circ = __ddiv_rn(__dmul_rn(12.566370614359172, area), __dmul_rn(per, per));
-            keep = (circ > min_circ && area > min_area) ? 1 : 0;
-        }
-        if (a00 == 0) keep = 0;                              // moments["m00"] == 0 -> no centroid
-        keepv[c] = (uint8_t)keep;
-    }
+    for (int c = tid; c < n; c += (int)blockDim.x) keepv[c] = (uint8_t)contour_keep(ra[3 * c], rper[c], min_area, min_circ);
     __syncthreads();
     for (int c = tid; c < n; c += (int)blockDim.x) {
         long long a00 = ra[3 * c], a10 = ra[3 * c + 1], a01 = ra[3 * c + 2];
@@ -1075,13 +1063,7 @@ __device__ void frame_finalize(const ClusterWs& cw, int f, uint8_t* keepv /*[max
         }
         if (!keep) continue;
         atomicAdd(&s_kept, 1);
-        if (pos < max_blobs) {
-            double sgn = a00 > 0 ? 1.0 : -1.0;
-            double m00 = __dmul_rn((double)a00, sgn * 0.5);
-            double m10 = __dmul_rn((double)a10, sgn * 0.16666666666666666);
-            double m01 = __dmul_rn((double)a01, sgn * 0.16666666666666666);
-            store_centroid(out_xy + ((size_t)f * max_blobs + pos) * 2, __ddiv_rn(m10, m00), __ddiv_rn(m01, m00), xy_float);
-        }
+        if (pos < max_blobs) store_blob_centroid(out_xy + ((size_t)f * max_blobs + pos) * 2, a00, a10, a01, xy_float);
     }
     __syncthreads();
     if (tid == 0) {

@@ -1,31 +1,11 @@
-// Suzuki-Abe border following on a packed binary image (shared by the per-frame general path, detect_blobs.cu, and the
-// per-cluster path, detect_cluster.cu).  Restates what cv.findContours(RETR_TREE, CHAIN_APPROX_SIMPLE) does per border
-// (lib/ImageOperations.py:41) plus the Green sums / perimeter of cv.moments / cv.arcLength (:44-45, :59).
+// Suzuki-Abe border following on a packed binary image: one walker, trace_border, for every border of the library -- the
+// per-cluster traces and hole-parent walks (detect_cluster.cu), the general path's traces, canonical-start tests and
+// parent walks, and the outline of drawContours (detect_blobs.cu).  Restates what cv.findContours(RETR_TREE,
+// CHAIN_APPROX_SIMPLE) does per border (lib/ImageOperations.py:41) plus the Green sums / perimeter of cv.moments /
+// cv.arcLength (:44-45, :59).  A step is one byte of a step table in shared memory, looked up with the walker's 3x3
+// neighbourhood taken from bit rows held in registers.
 #pragma once
 #include "common.cuh"
-
-// Walker state for Suzuki-Abe border following started from the west (side 4) or east (side 0) edge of a pixel.
-struct Walk {
-    int x0, y0;      // start pixel
-    int x1, y1;      // its predecessor on the border
-    int x, y;        // current pixel
-    int s;           // direction from current pixel to the previous one
-    bool single;
-};
-
-__device__ __forceinline__ void walk_init(const BitImg& im, Walk& w, int x, int y, int side)
-{
-    w.x0 = x; w.y0 = y; w.x = x; w.y = y;
-    // clockwise search (side-1, side-2, ... side-7) for the border's predecessor of the start pixel
-    uint32_t m = im.nbr8(x, y);
-    uint32_t rev = __brev(m) >> 24;                               // bit i = m[7 - i]
-    uint32_t sh = (8 - side) & 7;
-    uint32_t r = (((rev | (rev << 8)) >> sh) & 0x7fu);            // bit j = m[(side - 1 - j) & 7], j = 0..6
-    w.single = r == 0;
-    int s = w.single ? (side + 1) & 7 : (side - 1 - (__ffs(r) - 1)) & 7;
-    w.s = s;
-    w.x1 = x + dir_dx(s); w.y1 = y + dir_dy(s);
-}
 
 // The rule of one step: counter-clockwise search of the 8-neighbour mask m from s + 1 (s = direction to the previous
 // pixel); returns the step direction, `zeros` = bitmask of neighbour directions examined and found empty.
@@ -39,101 +19,9 @@ __device__ __forceinline__ int walk_rule(uint32_t m, int s, unsigned& zeros)
     return (start + k) & 7;
 }
 
-// One step: walk_rule at the walker's pixel.  Advances the walker.  `done` when back at the start.
-__device__ __forceinline__ int walk_step(const BitImg& im, Walk& w, unsigned& zeros, bool& done)
-{
-    int d = walk_rule(im.nbr8(w.x, w.y), w.s, zeros);
-    int nx = w.x + dir_dx(d), ny = w.y + dir_dy(d);
-    done = (nx == w.x0 && ny == w.y0 && w.x == w.x1 && w.y == w.y1);
-    w.x = nx; w.y = ny;
-    w.s = (d + 4) & 7;
-    return d;
-}
-
 #define WALK_BUDGET (1 << 22)
 
-// key of a west/east edge: 2 * pixel index + (east ? 1 : 0)
-__device__ __forceinline__ long long edge_key(int x, int y, int W, int east) { return 2LL * ((long long)y * W + x) + east; }
-
-// Walk the border owning edge (x, y, side).  mode 0: stop as soon as a smaller west/east edge of the same border is
-// seen (returns 1 if the start edge is the border's smallest edge).  mode 1: full loop, *min_key = smallest edge key.
-static __device__ int walk_min_edge(const BitImg& im, int x, int y, int side, int mode, long long* min_key, int* overflow)
-{
-    const int W = im.W;
-    long long key0 = edge_key(x, y, W, side == 0);
-    long long best = key0;
-    Walk w; walk_init(im, w, x, y, side);
-    if (w.single) { if (min_key) *min_key = edge_key(x, y, W, 0); return side == 4; }   // isolated pixel: its west edge is smaller
-    for (int step = 0; step < WALK_BUDGET; ++step) {
-        int cx = w.x, cy = w.y;
-        unsigned zeros; bool done;
-        walk_step(im, w, zeros, done);
-        if (zeros & (1u << 4)) { long long k = edge_key(cx, cy, W, 0); if (k < best) { best = k; if (!mode) return 0; } }
-        if (zeros & (1u << 0)) { long long k = edge_key(cx, cy, W, 1); if (k < best) { best = k; if (!mode) return 0; } }
-        if (done) { if (min_key) *min_key = best; return best == key0; }
-    }
-    *overflow = 1;
-    if (min_key) *min_key = best;
-    return 0;
-}
-
-// Full trace of a border from its start edge: Green sums over the CHAIN_APPROX_SIMPLE vertices, perimeter, length.
-// key0 >= 0: also verify that the start edge is the border's smallest west/east edge (i.e. where cv.findContours starts
-// it); returns 0 as soon as a smaller one is met.  key0 < 0: no check.  Returns 1 for a completed trace.
-// (ox, oy, Wabs): the image `im` may be a window of the frame (cluster path): vertices and edge keys are taken in frame
-// coordinates (x + ox, y + oy) of a frame of width Wabs.
-static __device__ int trace_contour(const BitImg& im, int x, int y, int side, long long key0, long long* a, double* per, int* n_chain, int* overflow,
-                             int ox, int oy, int Wabs, int* bbox = nullptr)
-{
-    const int W = Wabs;
-    Walk w; walk_init(im, w, x, y, side);
-    if (bbox) { bbox[0] = bbox[2] = x + ox; bbox[1] = bbox[3] = y + oy; }
-    if (w.single) { a[0] = a[1] = a[2] = 0; *per = 0.0; *n_chain = 1; return key0 < 0 || side == 4; }
-    long long a00 = 0, a10 = 0, a01 = 0;
-    double perim = 0.0;
-    int n = 0;
-    int prev_dir = w.s ^ 4;             // direction of the closing step (predecessor -> start)
-    bool have_v = false;
-    int vx = 0, vy = 0, fx = 0, fy = 0; // previous vertex, first vertex
-    for (int step = 0; step < WALK_BUDGET; ++step) {
-        int cx = w.x + ox, cy = w.y + oy;
-        unsigned zeros; bool done;
-        int d = walk_step(im, w, zeros, done);
-        ++n;
-        if (key0 >= 0) {
-            if ((zeros & (1u << 4)) && edge_key(cx, cy, W, 0) < key0) return 0;
-            if ((zeros & (1u << 0)) && edge_key(cx, cy, W, 1) < key0) return 0;
-        }
-        if (d != prev_dir) {            // direction change: (cx, cy) is a vertex
-            if (have_v) {
-                long long dxy = (long long)vx * cy - (long long)cx * vy;
-                a00 += dxy; a10 += dxy * (vx + cx); a01 += dxy * (vy + cy);
-                float ddx = (float)(cx - vx), ddy = (float)(cy - vy);
-                perim += (double)__fsqrt_rn(__fadd_rn(__fmul_rn(ddx, ddx), __fmul_rn(ddy, ddy)));
-            } else { fx = cx; fy = cy; have_v = true; }
-            vx = cx; vy = cy;
-            if (bbox) { bbox[0] = min(bbox[0], cx); bbox[1] = min(bbox[1], cy); bbox[2] = max(bbox[2], cx); bbox[3] = max(bbox[3], cy); }
-        }
-        prev_dir = d;
-        if (done) {
-            if (have_v) {               // closing segment last vertex -> first vertex
-                long long dxy = (long long)vx * fy - (long long)fx * vy;
-                a00 += dxy; a10 += dxy * (vx + fx); a01 += dxy * (vy + fy);
-                float ddx = (float)(fx - vx), ddy = (float)(fy - vy);
-                float q = __fadd_rn(__fmul_rn(ddx, ddx), __fmul_rn(ddy, ddy));
-                if (q > 0.f) perim += (double)__fsqrt_rn(q);
-            }
-            a[0] = a00; a[1] = a10; a[2] = a01; *per = perim; *n_chain = n;
-            return 1;
-        }
-    }
-    *overflow = 1;
-    a[0] = a[1] = a[2] = 0; *per = 0.0; *n_chain = n;
-    return 0;
-}
-
-
-// Step table of trace_contour64: walk_rule's outcome for every 3x3 neighbourhood and every s, so that a step is one
+// Step table of trace_border: walk_rule's outcome for every 3x3 neighbourhood and every s, so that a step is one
 // shared-memory byte instead of gathering eight neighbour bits and searching them.  Index (raw9 << 3) + s, where raw9 is
 // the walker's 3x3 neighbourhood as three row triples side by side: bits 0-2 the row above (columns x-1, x, x+1), 3-5 the
 // walker's row, 6-8 the row below.  Entry: bits 0-1 what the abandon test needs from the empty neighbours walk_rule passed
@@ -141,7 +29,7 @@ static __device__ int trace_contour(const BitImg& im, int x, int y, int side, lo
 // the next step, d ^ 4 for the step direction d; bit 5 set when the step goes up (dir_dy(d) < 0); bits 6-7 dir_dx(d) + 1.
 // The step changes row when bits 2-3 are not both zero (d is neither east nor west).
 #define STEP_TAB_BYTES 4096
-// One table per CTA, in the shared memory of every kernel that calls trace_contour64 (4 KB).  Such a kernel must fill it
+// One table per CTA, in the shared memory of every kernel that calls trace_border (4 KB).  Such a kernel must fill it
 // with step_table_build() and synchronise the block before its first trace: the table is not initialised otherwise.
 __shared__ uint32_t step_tab[STEP_TAB_BYTES / 4];                // four entries per word, little-endian
 
@@ -184,7 +72,18 @@ __device__ __forceinline__ uint32_t step_index(unsigned long long up, unsigned l
 template <bool WINDOW> struct GreenAcc { typedef uint32_t T; };
 template <> struct GreenAcc<true> { typedef long long T; };
 
-// trace_contour for boxes at most 64 pixels wide and 1024 high (two 32-bit words per row).  Same results, cheaper steps:
+// trace_border's default per-step visitor: none
+struct NoVisit { __device__ __forceinline__ void operator()(int, int, int, int) const {} };
+
+// Full trace of the border that starts at the west (side 4) or east (side 0) edge of pixel (x, y) of a box of mw x mh pixels
+// (bit rows of wpr words, bits at x >= mw zero).  Writes the Green sums a00/a10/a01 of its CHAIN_APPROX_SIMPLE polygon, the
+// perimeter, the number of steps and, given bbox, the bounding box of the border's pixels.  Vertices and edge keys are
+// taken in frame coordinates (x + ox, y + oy) of a frame of width Wabs; the frame sizes the library accepts (at most 16384 x
+// 16384) keep them in 32 bits.  key0 >= 0: also verify that the start edge, key0 = 2 * (frame pixel index) + east, is the
+// border's smallest west/east edge (where cv.findContours starts it); returns 0 as soon as a smaller one is met.  key0 < 0:
+// no check.  Returns 1 for a completed trace; *overflow = 1 when the border is longer than WALK_BUDGET steps.
+//
+// How a step is taken:
 //  * the five rows y-2 .. y+2 around the walker live in registers as 64-bit words, and a step looks up its direction in the
 //    step table (step_table_build).  When the walker changes row the rows shift and the load of the new outer row is issued
 //    at once; it is first read when the walker changes row again, a step later at the soonest (a walker moves one row per
@@ -194,49 +93,61 @@ template <> struct GreenAcc<true> { typedef long long T; };
 //    of a diagonal segment longer than one pixel (rare);
 //  * Green sums per unit step instead of per CHAIN_APPROX_SIMPLE vertex: the sums are linear along a straight run, so the
 //    terms of a run's unit steps add up exactly to the term of its end points.  Box-local coordinates, translated at the
-//    end: a10 = a10' + 3 ox a00, a01 = a01' + 3 oy a00 (exact integer identity for a closed polygon).  In a box of 64 x 1024
-//    pixels the totals are below 2^29 (|a01'| <= 6 * 2^16 * 2^10), so they are summed modulo 2^32;
+//    end: a10 = a10' + 3 ox a00, a01 = a01' + 3 oy a00 (exact integer identity for a closed polygon);
 //  * bounding box over every pixel of the walk: a pixel of a straight run lies between the run's end vertices;
 //  * perimeter: CHAIN_APPROX_SIMPLE segments are the runs of one step direction, axis-parallel (length = an integer, exact in
 //    float32) or diagonal (length = float32 sqrt(2 k^2)); the double sum of such float32 values is exact in any order, so
 //    axis and diagonal steps are counted, and a longer diagonal is added when its run ends.  The run that closes the border
 //    continues the run the trace started on when the start pixel is no vertex.
 //
-// WINDOW = true: the same trace on a sliding 64-pixel wide window of a wider box (wpr words per row, mw > 64 pixels wide;
-// a blob of a wide cluster box is usually narrow).  The window starts at column wx0 (0 <= wx0 <= mw - 64); (x, ox) and all
-// coordinates are relative to wx0.  When the walker reaches a window column whose outer neighbour is not known, the
-// window is re-centred on it (five row loads).  Coordinates then exceed 64, so a10/a01 are summed in 64 bits.
+// WINDOW = false: a box at most 64 pixels wide and 1024 high with two words per row, 8-byte aligned; a row is one 64-bit
+// load.  In such a box the Green sums stay below 2^29 (|a01'| <= 6 * 2^16 * 2^10), so they are summed modulo 2^32.
+// WINDOW = true: any box, e.g. a whole frame (ox = oy = 0, Wabs = mw); rows are read with 32-bit loads only.  The rows are
+// seen through a 64-pixel window, first centred on the start pixel, that is re-centred on the walker (five row loads) when
+// it reaches a window column whose outer neighbour is not known.  A box at most 64 wide (wpr = 1 or 2) fits the window at
+// origin 0, which never moves.  Coordinates then exceed 64, so a10/a01 are summed in 64 bits.
+//
+// Compile-time extras, off by default:
+//  * MIN_KEY: *min_key = the border's smallest west/east edge key 2 * (frame pixel index) + east, the start edge included;
+//    a single pixel gives its west edge.  Used with key0 < 0.
+//  * visit(x, y, dx, dy) at every step: the walker's pixel in frame coordinates and the step it takes from there.
 //
 // Precondition: the calling block has filled step_tab (step_table_build) and passed a __syncthreads() since.
-template <bool WINDOW>
-static __device__ int trace_contour64(const uint32_t* __restrict__ rows, int mh, int wpr, int wx0, int mw,
-                                      int x, int y, int side, long long key0, long long* a, double* per, int* n_chain, int* overflow,
-                                      int ox, int oy, int Wabs, int* bbox)
+template <bool WINDOW, bool MIN_KEY = false, class Visit = NoVisit>
+static __device__ int trace_border(const uint32_t* __restrict__ rows, int mh, int wpr, int mw,
+                                   int x, int y, int side, long long key0, long long* a, double* per, int* n_chain, int* overflow,
+                                   int ox, int oy, int Wabs, int* bbox, long long* min_key = nullptr, Visit visit = Visit())
 {
+    const int wx0 = WINDOW ? max(min(x - 32, mw - 64), 0) : 0;     // window origin in the box; coordinates below are relative to it
+    x -= wx0; ox += wx0;
     int wofs = 0;                                   // window origin relative to wx0 (WINDOW only)
     int wi0 = wx0 >> 5, wsh = wx0 & 31;
     const unsigned long long* rows64 = (const unsigned long long*)rows;                             // rows of a two-word box are 8-byte aligned
     auto load = [&](int yy) -> unsigned long long {
         if ((unsigned)yy >= (unsigned)mh) return 0ull;
         if (!WINDOW) return rows64[(unsigned)yy];
-        const uint32_t* r = rows + (size_t)yy * wpr + wi0;                                          // origin + 63 < mw: words wi0, wi0 + 1 exist
-        const uint32_t w0 = r[0], w1 = r[1], w2 = (wsh && wi0 + 2 < wpr) ? r[2] : 0u;
+        const uint32_t* r = rows + (size_t)yy * wpr + wi0;         // origin + 63 < mw or origin 0: word wi0 + 1 exists unless wpr = 1
+        const uint32_t w0 = r[0], w1 = wpr > 1 ? r[1] : 0u, w2 = (wsh && wi0 + 2 < wpr) ? r[2] : 0u;
         const unsigned long long lo = (unsigned long long)w0 | ((unsigned long long)w1 << 32);
         return wsh ? (lo >> wsh) | ((unsigned long long)w2 << (64 - wsh)) : lo;
     };
     unsigned long long u2 = load(y - 2), up = load(y - 1), mid = load(y), dn = load(y + 1), d2 = load(y + 2);
     if (bbox) { bbox[0] = bbox[2] = x + ox; bbox[1] = bbox[3] = y + oy; }
-    // start: clockwise search for the predecessor (see walk_init)
+    // start: clockwise search (side-1, side-2, ... side-7) for the border's predecessor of the start pixel
     uint32_t m0 = nbr8_of_raw9(step_index(up, mid, dn, x - 1, 0) >> 3);
     uint32_t rev = __brev(m0) >> 24, sh = (8 - side) & 7;
-    uint32_t r0 = (((rev | (rev << 8)) >> sh) & 0x7fu);
-    if (r0 == 0) { a[0] = a[1] = a[2] = 0; *per = 0.0; *n_chain = 1; return key0 < 0 || side == 4; }
+    uint32_t r0 = (((rev | (rev << 8)) >> sh) & 0x7fu);           // bit j = m0[(side - 1 - j) & 7], j = 0..6
+    if (r0 == 0) {                                              // single pixel
+        if (MIN_KEY) *min_key = 2LL * ((long long)(y + oy) * Wabs + x + ox);
+        a[0] = a[1] = a[2] = 0; *per = 0.0; *n_chain = 1; return key0 < 0 || side == 4;
+    }
     const int s0 = (side - 1 - (__ffs(r0) - 1)) & 7;            // the closing step predecessor -> start goes in direction s0 ^ 4
     const int lin1 = (y + dir_dy(s0)) * Wabs + x + dir_dx(s0);  // the predecessor as cy * Wabs + cx
-    // edge keys in 32 bits: key = 2 * (row * Wabs + col) + east = 2 * (oy * Wabs + ox) + 2 * (cy * Wabs + cx) + east; the frame
-    // sizes the library accepts keep this below 2^31.  An edge smaller than key0 is met when kt - 2 * (cy * Wabs + cx) exceeds
-    // the step table's threshold (0 for the west edge, 1 for the east edge).
+    // edge keys in 32 bits: key = 2 * (row * Wabs + col) + east = 2 * (oy * Wabs + ox) + 2 * (cy * Wabs + cx) + east.  An edge
+    // smaller than key0 is met when kt - 2 * (cy * Wabs + cx) exceeds the step table's threshold (0 for the west edge, 1 for
+    // the east edge).
     const int kt = key0 >= 0 ? (int)key0 - 2 * (oy * Wabs + ox) : -(1 << 30);
+    int kmin = 2 * (y * Wabs + x) + (side == 0);                // MIN_KEY: smallest edge key so far, relative like kt
     uint32_t a00 = 0;
     typename GreenAcc<WINDOW>::T a10 = 0, a01 = 0;
     int n_diag = 0, n_long = 0;                                 // diagonal steps, those of them on runs longer than one
@@ -254,6 +165,8 @@ static __device__ int trace_contour64(const uint32_t* __restrict__ rows, int mh,
         const int dx = (int)(e >> 6) - 1, dy = (e & 0x20u) ? -1 : (e & 0x0cu) ? 1 : 0;
         const int lin = wy * Wabs + wx;
         ++n;
+        visit(wx + ox, wy + oy, dx, dy);
+        if (MIN_KEY && thr < 2) kmin = min(kmin, 2 * lin + thr);
         abandon = thr < 2 && kt - 2 * lin > thr;
         done = lin == lin1 && sn == s0;
         const int dxy = wx * dy - dx * wy;
@@ -291,6 +204,7 @@ static __device__ int trace_contour64(const uint32_t* __restrict__ rows, int mh,
         }
         wx = nx; wy = ny;
     }
+    if (MIN_KEY) *min_key = 2LL * ((long long)oy * Wabs + ox) + kmin;
     if (!abandon && !done) {
         *overflow = 1;
         a[0] = a[1] = a[2] = 0; *per = 0.0; *n_chain = n;

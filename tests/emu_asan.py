@@ -56,6 +56,12 @@ def run():
     img[90:120, 0:130] = 255
     assert eng.detect(torch.from_numpy(img[None].copy()), K, D, min_area=0.0).points(0) == \
         eng.detect(torch.from_numpy(img[None].copy()), K, D, min_area=0.0, outputs=("bits", "labels")).points(0)
+    from test_border_walker import narrow_frame
+    from util import pack_bits
+    bits = torch.from_numpy(pack_bits(narrow_frame())[None].copy())                    # rows of one word, blobs on the last row
+    res = eng.blobs(bits, 28, min_area=0.0, outputs=("contours",))
+    res.extras["bits"] = bits
+    eng.draw_contours(torch.zeros((1, 30, 28), dtype=torch.uint8), res)
     for shape in [(3, 4), (5, 8), (34, 132), (64, 128), (97, 260), (7, 10), (33, 65), (3, 8), (12, 1032), (129, 1040), (75, 16)]:  # Bayer front step, both kernels
         eng.bayer_gr2gray(torch.from_numpy(rng.integers(0, 256, (2,) + shape).astype(np.uint8)))
         eng.bayer_gr2gray_scan(torch.from_numpy(rng.integers(0, 256, (2,) + shape).astype(np.uint8)), thresh=int(rng.integers(0, 256)))
